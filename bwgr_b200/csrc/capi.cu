@@ -169,10 +169,8 @@ struct Fit {
   bool weighted = false;
   DevBuf<SysScalars> sc;
   DevBuf<int> perm;                     // [kPermRing][p]
-  DevBuf<long long> gacc, trace;
-  DevBuf<unsigned int> bar;
+  DevBuf<long long> trace;
   // pipelined sweep (sweep_pipe.cu)
-  bool pipe = false;
   int lookahead = 0, nbuf = 0, sring = 2, nworkers = 0, nc = 1, nband = 1, full_inv = 0, cl = 0, nclusters = 0;
   DevBuf<float> tinv;                   // (I + A L)^-1 of every block of the current sweep (block_inv.cu)
   uint32_t tag = 0;
@@ -264,7 +262,6 @@ struct bwgr_handle {
   DevBuf<int> err;
   // tuning
   int path = BWGR_PATH_AUTO, grid = 0;
-  int gram_simt = 0;
   DevBuf<float> gram_nat;  // Gram band of the natural marker order (Gibbs / KMUP / wgr): depends on the store only
   int gram_nat_band = 0;
   // row-sharded fit over the GPUs of a node (bwgr_dist_*)
@@ -277,8 +274,6 @@ struct bwgr_handle {
   bool hx_connected = false;
   unsigned long long dist_gen = 0;          // global block sequence number (same on every rank)
   DevBuf<double> dscratch;                  // small all-reduce scratch
-  alignas(64) unsigned char tmap[128];  // CUtensorMap of the int8 store (TMA tile::gather4)
-  bool tmap_ok = false;
   // side stream for work that overlaps the clustered sweep, gated by a flag word the sweep kernel stores (stream memory operations)
   cudaStream_t side = nullptr;
   cudaEvent_t side_done[2] = {nullptr, nullptr};
@@ -289,16 +284,6 @@ struct bwgr_handle {
   int fp8_codes = 0;  // all genotypes are codes 0..7 (and n small enough): the Gram kernel may use the exact E4M3 path
   int64_t launches = 0;
   Fit fit;
-  // debug (BWGR_GAPS=1): events at the kernel boundaries of every sweep on the main stream, printed by bwgr_em_end
-  std::vector<cudaEvent_t> gap_ev;
-  void gap_mark() {
-    static const bool on = getenv("BWGR_GAPS") != nullptr;
-    if (!on) return;
-    cudaEvent_t e;
-    cudaEventCreate(&e);
-    cudaEventRecord(e, stream);
-    gap_ev.push_back(e);
-  }
   // optional per-kernel timing (bwgr_profile)
   bool profiling = false;
   std::vector<std::pair<cudaEvent_t, cudaEvent_t>> prof_ev[4];  // gram, sweep, epilogue, block inverses
@@ -395,18 +380,11 @@ int finish_store(bwgr_handle* h, int storage) {
   for (int64_t j = 0; j < h->p; j++) xf[j] = (float)xx[j];
   CU(cudaMemcpyAsync(h->xx_f.p, xf.data(), sizeof(float) * h->p, cudaMemcpyHostToDevice, h->stream));
   CU(cudaStreamSynchronize(h->stream));
-  {
-    // TMA tile::gather4 for the Gram tiles is built and bit-exact, but at 128 B per column per visit it is 2x SLOWER than
-    // the cp.async gather (2.43 vs 1.24 ms at 50k x 50k, band 2): opt-in only (BWGR_TMA=1), see profiles/r1_v5_summary.md
-    const char* te = getenv("BWGR_TMA");
-    h->tmap_ok = te && !strcmp(te, "1") && make_geno_tensor_map(h->x8, h->ld, h->p, h->tmap);
-  }
   {  // codes 0..7 everywhere?  (one more streaming pass at load time)
     h->fp8_codes = 0;
-    const char* ge = getenv("BWGR_GRAM");
     double xxmax = 0;  // every Gram entry and every partial sum of non-negative codes is bounded by max_j xx_j (Cauchy-Schwarz)
     for (double v : h->h_xx) xxmax = std::max(xxmax, v);
-    if (!(ge && !strcmp(ge, "i8")) && xxmax < 16777216.0) {
+    if (xxmax < 16777216.0) {
       launch_check_range_i8(h->x8, h->ld, (int)h->n, (int)h->p, 0, 7, h->err.p, h->stream);
       h->launches++;
       int flag = 0;
@@ -418,8 +396,7 @@ int finish_store(bwgr_handle* h, int storage) {
   }
   h->x2f.release();
   if (h->fp8_codes && storage == BWGR_STORE_I8) {  // FP4 Gram shadow copy (gram_fp4.cu): only when every code is 0, 1 or 2
-    const char* fe = getenv("BWGR_GRAM");
-    if (!(fe && !strcmp(fe, "fp8")) && h->x2f.alloc((size_t)(h->ld / 4) * h->p) == cudaSuccess) {
+    if (h->x2f.alloc((size_t)(h->ld / 4) * h->p) == cudaSuccess) {
       launch_pack_2bit_fp4(h->x8, h->ld, (int)h->p, h->x2f.p, h->err.p, h->stream);
       h->launches++;
       int flag = 0;
@@ -430,8 +407,7 @@ int finish_store(bwgr_handle* h, int storage) {
   }
   h->x2g.release();
   if (h->fp8_codes && storage == BWGR_STORE_I8 && !h->x2f.p) {  // E4M3 Gram shadow copy (codes 0..3)
-    const char* pe = getenv("BWGR_GRAM_PACKED");
-    if (!(pe && !strcmp(pe, "0")) && h->x2g.alloc((size_t)(h->ld / 4) * h->p) == cudaSuccess) {
+    if (h->x2g.alloc((size_t)(h->ld / 4) * h->p) == cudaSuccess) {
       launch_pack_2bit_gram(h->x8, h->ld, (int)h->p, h->x2g.p, h->err.p, h->stream);
       h->launches++;
       int flag = 0;
@@ -452,7 +428,6 @@ int finish_store(bwgr_handle* h, int storage) {
     h->storage = BWGR_STORE_2BIT;
     h->x8_own.release();  // the 2-bit store is the only copy kept in HBM
     h->x8 = nullptr;
-    h->tmap_ok = false;
   }
   return 0;
 }
@@ -532,8 +507,6 @@ int bwgr_create(int device, bwgr_handle** out) {
   }
   if (h->err.alloc(1) != cudaSuccess) { delete h; return fail(BWGR_ERR_CUDA, "cudaMalloc failed"); }
   cudaMemset(h->err.p, 0, sizeof(int));
-  const char* gs = getenv("BWGR_GRAM");
-  h->gram_simt = gs && !strcmp(gs, "simt");
   *out = h;
   return 0;
 }
@@ -664,7 +637,7 @@ static int load_f64_real(bwgr_handle* h, const double* X, int64_t n, int64_t p, 
   CU(cudaStreamSynchronize(h->stream));
   h->n_global = h->n;
   h->storage = BWGR_STORE_F32;
-  h->fp8_codes = 0; h->tmap_ok = false;
+  h->fp8_codes = 0;
   h->x2f.release(); h->x2g.release();
   return 0;
 }
@@ -888,12 +861,9 @@ struct FitSpec {
 // nbuf X tiles per worker.  False if the shape does not fit one SM's shared memory / TMEM.
 struct PipePlan { int R, W, nbuf, D, sring, full_inv, cl, nclusters; };
 bool plan_pipe(const bwgr_handle* h, int model, int ns, PipePlan* pl) {
-  const char* sw = getenv("BWGR_SWEEP");
-  if (sw && !strcmp(sw, "v4")) return false;
   if (h->storage != BWGR_STORE_I8 || ns > 32) return false;
-  int sms = h->grid > 1 ? std::min(h->grid, h->num_sms) : h->num_sms;
-  if (const char* ge = getenv("BWGR_GRID")) { const int v = atoi(ge); if (v > 1) sms = std::min(v, h->num_sms); }  // CTAs of the flat topology
-  else if (h->world > 1 && h->grid <= 1 && h->x2f.p && h->comm_side && h->num_sms > 64) {
+  int sms = h->grid > 1 ? std::min(h->grid, h->num_sms) : h->num_sms;  // CTAs of the flat topology
+  if (h->world > 1 && h->grid <= 1 && h->x2f.p && h->comm_side && h->num_sms > 64) {
     // row-sharded fit, flat topology: the per-block chain is latency-bound, so ~104 CTAs sweep as fast as 148 and the SMs left idle
     // compute the next sweep's Gram band meanwhile (measured at 50k x 50k: 104 CTAs 1.54 ms per sweep, 120: 1.68, 148: 1.84)
     const int want = h->num_sms - 44;
@@ -906,31 +876,25 @@ bool plan_pipe(const bwgr_handle* h, int model, int ns, PipePlan* pl) {
   const int W = (int)((h->ld + R - 1) / R);
   const int NA = (R + 127) / 128, N = ((4 * ns + 15) / 16) * 16;
   if ((NA + 1) * N > 512) return false;
-  const char* la = getenv("BWGR_LOOKAHEAD");
-  int D = la ? atoi(la) : 1;
-  if (D < 0 || h->gram_simt) D = 0;
-  if (D > 1) D = 1;
-  // one linear system: the in-block solve applies the precomputed block inverse (block_inv.cu); BWGR_TINV=0 keeps the
-  // four dependent 32-marker steps.  (MRR3's centred systems keep the stepwise solve.)
-  const char* ti = getenv("BWGR_TINV");
-  const int full_inv = model_is_linear(model) && ns == 1 && model != M_MRR && !(ti && !strcmp(ti, "0"));
+  int D = 1;
+  // one linear system on uncentred columns: the in-block solve applies the precomputed block inverse (block_inv.cu).
+  // (MRR3's centred systems keep the stepwise solve.)
+  const int full_inv = model_is_linear(model) && ns == 1 && model != M_MRR;
   pl->cl = 0; pl->nclusters = 0;
   // Clustered topology (sweep_pipe.cu): thread-block clusters of one solver + seven workers; partial sums and steps travel
   // through distributed shared memory, one L2 hop per block is left (the exchange of the cluster sums between the solvers).
-  // Single GPU, at most four systems; BWGR_CLUSTER=0 keeps the flat topology (one solver CTA, two-hop L2 tree).  Row-sharded fits use
-  // the flat one: a clustered variant with a third (NVLink) hop after the cluster exchange measured 1.79 ms against 1.43 ms per sweep.
-  const char* ce = getenv("BWGR_CLUSTER");
-  if (D >= 1 && h->world <= 1 && h->grid <= 1 && !(ce && !strcmp(ce, "0")) && sweep_pipe_cluster_ok(model, ns, full_inv)) {
+  // Single GPU at the default grid, at most four systems; otherwise the flat topology (one solver CTA, two-hop L2 tree).  Row-sharded
+  // fits use the flat one: a clustered variant with a third (NVLink) hop after the cluster exchange measured 1.79 ms against 1.43 ms per sweep.
+  if (h->world <= 1 && h->grid <= 1 && sweep_pipe_cluster_ok(model, ns, full_inv)) {
     {
       // The sweep is latency-bound: 14 clusters sweep as fast as 15 (measured 1.226 against 1.235 ms at 50k x 50k), and every SM left
       // idle works on the next sweep's Gram band meanwhile (capi.cu fit_sweeps).  First choice: leave at least 36 SMs; if the rows per
-      // worker then exceed the tile (512), take every cluster that fits.  BWGR_MAXCL=k overrides.
+      // worker then exceed the tile (512), take every cluster that fits.
       const int cap_side = std::max(2, (h->num_sms - 36) / 8);
       for (int nbuf = D + 2; nbuf >= D + 1; nbuf--)
       for (int pass = 0; pass < 2; pass++) {
         // rows per worker depend on the number of co-resident clusters, which depends on the shared memory per CTA: iterate
         int C = pass == 0 ? std::min(18, cap_side) : 18;
-        if (const char* mc = getenv("BWGR_MAXCL")) { const int v = atoi(mc); if (v >= 2) C = std::min(v, 18); }
         for (int iter = 0; iter < 4 && C >= 2; iter++) {
           const int Wc = 7 * C;
           const int Rc = (int)(((h->ld + Wc - 1) / Wc + 15) / 16 * 16);
@@ -976,11 +940,8 @@ void grid_geometry(bwgr_handle* h, int* rp, int* grid) {
 int choose_path(bwgr_handle* h, const FitSpec& s, int* family) {
   const GenoView g = h->view();
   const bool small_ok = h->storage != BWGR_STORE_F32 && small_n_fits(g, s.row_mask != nullptr, h->smem_optin, s.row_cnt != nullptr);
-  const int grid = h->grid > 0 ? std::min(h->grid, h->num_sms) : h->num_sms;
-  const int64_t rows = ((h->ld + grid - 1) / grid + 15) / 16 * 16;
   PipePlan pl;
-  const bool blocked_ok = h->storage == BWGR_STORE_I8 && !s.row_mask && s.nsys <= 32 &&
-                          (plan_pipe(h, s.model, s.nsys, &pl) || (rows <= 512 && sweep_blocked_smem((int)rows, s.nsys) <= h->smem_optin));
+  const bool blocked_ok = !s.row_mask && plan_pipe(h, s.model, s.nsys, &pl);
   int grp = 0, ggrid = 0;
   grid_geometry(h, &grp, &ggrid);
   const bool grid_ok = (h->storage == BWGR_STORE_I8 || h->storage == BWGR_STORE_F32) && h->world <= 1 && s.nsys <= 32 && s.model != M_MRR &&
@@ -1284,9 +1245,8 @@ int fit_begin(bwgr_handle* h, const FitSpec& s, const double* y) {
   if (blocked) {
     f.nblocks = (int)((p + kBlk - 1) / kBlk);
     PipePlan pl;
-    f.pipe = plan_pipe(h, s.model, ns, &pl);
+    if (!plan_pipe(h, s.model, ns, &pl)) return fail(BWGR_ERR_UNSUPPORTED, "the shape does not fit the pipelined blocked sweep");
     if (dist) {
-      if (!f.pipe) return fail(BWGR_ERR_UNSUPPORTED, "row-sharded fit: the shape does not fit the pipelined blocked sweep");
       {  // the per-rank Gram bands are summed in float by ncclAllReduce: exact (= independent of the sharding) only below 2^24.
          // |G_jk| <= max_j xx_j (Cauchy-Schwarz) over ALL individuals; h_xx holds the all-reduced column statistics.
         double xxmax = 0;
@@ -1301,55 +1261,42 @@ int fit_begin(bwgr_handle* h, const FitSpec& s, const double* y) {
       rc = dist_allreduce_host(h, &one, 1, false);
       if (rc) return rc;
     }
-    if (f.pipe) {
-      f.rows_per_cta = pl.R; f.nworkers = pl.W; f.grid = pl.cl ? pl.nclusters * 8 : pl.W + 1; f.nbuf = pl.nbuf; f.sring = pl.sring; f.lookahead = pl.D; f.full_inv = pl.full_inv; f.nband = pl.D + 1;
-      f.cl = pl.cl; f.nclusters = pl.nclusters;
-      f.nc = std::max(1, 16 / ns);
-      f.tag = 0;
-      const size_t gram_n = (size_t)f.nblocks * kBlk * kBlk * f.nband;
-      if (!s.shuffled) {  // natural order: one Gram band per genotype store, kept on the handle
-        if (h->gram_nat_band != f.nband || h->gram_nat.n != gram_n) {
-          h->gram_nat_band = 0;
-          if (h->gram_nat.alloc(gram_n) != cudaSuccess) return fail(BWGR_ERR_CUDA, "cudaMalloc(Gram band) failed");
-        } else {
-          f.gram_cached = true;
-        }
-        f.gram_p = h->gram_nat.p;
+    f.rows_per_cta = pl.R; f.nworkers = pl.W; f.grid = pl.cl ? pl.nclusters * 8 : pl.W + 1; f.nbuf = pl.nbuf; f.sring = pl.sring; f.lookahead = pl.D; f.full_inv = pl.full_inv; f.nband = pl.D + 1;
+    f.cl = pl.cl; f.nclusters = pl.nclusters;
+    f.nc = std::max(1, 16 / ns);
+    f.tag = 0;
+    const size_t gram_n = (size_t)f.nblocks * kBlk * kBlk * f.nband;
+    if (!s.shuffled) {  // natural order: one Gram band per genotype store, kept on the handle
+      if (h->gram_nat_band != f.nband || h->gram_nat.n != gram_n) {
+        h->gram_nat_band = 0;
+        if (h->gram_nat.alloc(gram_n) != cudaSuccess) return fail(BWGR_ERR_CUDA, "cudaMalloc(Gram band) failed");
       } else {
-        if (f.gram.alloc(gram_n) != cudaSuccess) return fail(BWGR_ERR_CUDA, "cudaMalloc(Gram band) failed");
-        f.gram_p = f.gram.p;
-        // the clustered sweep occupies 8 x nclusters of the SMs: the next sweep's Gram band (a function of the marker order only)
-        // is computed on the others meanwhile.  BWGR_OVERLAP=0 keeps everything on one stream.
-        const char* ov = getenv("BWGR_OVERLAP");
-        f.overlap = (h->world <= 1 || h->comm_side) && h->wait32 && h->x2f.p && f.nband == 2 && !h->gram_simt && !(ov && !strcmp(ov, "0")) &&
-                    f.grid + 8 <= h->num_sms;  // at least a few SMs are left idle by the sweep
-        if (f.overlap && f.gram2.alloc(gram_n) != cudaSuccess) { cudaGetLastError(); f.overlap = false; }
+        f.gram_cached = true;
       }
-      if (!f.overlap) f.gram2.release();
-      f.gram_ahead = -1;
-      if (f.full_inv && f.tinv.alloc((size_t)f.nblocks * kBlk * kBlk) != cudaSuccess) return fail(BWGR_ERR_CUDA, "cudaMalloc(block inverses) failed");
-      if (!f.full_inv) f.tinv.release();
-      if (
-          f.part.alloc((size_t)8 * ns * 128 * 161) != cudaSuccess || f.dew.alloc((size_t)f.nblocks * ns * 136) != cudaSuccess)
-        return fail(BWGR_ERR_CUDA, "cudaMalloc(blocked workspace) failed");
-      if (f.cl && f.cx.alloc((size_t)8 * f.nclusters * ns * 128) != cudaSuccess) return fail(BWGR_ERR_CUDA, "cudaMalloc(cluster ring) failed");
-      if (!f.cl) f.cx.release();
-      CU(cudaMemsetAsync(f.dew.p, 0, sizeof(unsigned long long) * f.dew.n, h->stream));
+      f.gram_p = h->gram_nat.p;
     } else {
-      const int grid0 = h->grid > 0 ? std::min(h->grid, h->num_sms) : h->num_sms;
-      f.rows_per_cta = (int)(((ld + grid0 - 1) / grid0 + 15) / 16 * 16);
-      f.grid = (int)((ld + f.rows_per_cta - 1) / f.rows_per_cta);
-      f.nband = 1;
-      if (f.gram.alloc((size_t)f.nblocks * kBlk * kBlk) != cudaSuccess || f.gacc.alloc((size_t)f.nblocks * kNC * ns * kBlk) != cudaSuccess || f.bar.alloc(1) != cudaSuccess)
-        return fail(BWGR_ERR_CUDA, "cudaMalloc(blocked workspace) failed");
+      if (f.gram.alloc(gram_n) != cudaSuccess) return fail(BWGR_ERR_CUDA, "cudaMalloc(Gram band) failed");
       f.gram_p = f.gram.p;
+      // the clustered sweep occupies 8 x nclusters of the SMs: the next sweep's Gram band (a function of the marker order only)
+      // is computed on the others meanwhile
+      f.overlap = (h->world <= 1 || h->comm_side) && h->wait32 && h->x2f.p && f.nband == 2 &&
+                  f.grid + 8 <= h->num_sms;  // at least a few SMs are left idle by the sweep
+      if (f.overlap && f.gram2.alloc(gram_n) != cudaSuccess) { cudaGetLastError(); f.overlap = false; }
     }
+    if (!f.overlap) f.gram2.release();
+    f.gram_ahead = -1;
+    if (f.full_inv && f.tinv.alloc((size_t)f.nblocks * kBlk * kBlk) != cudaSuccess) return fail(BWGR_ERR_CUDA, "cudaMalloc(block inverses) failed");
+    if (!f.full_inv) f.tinv.release();
+    if (f.part.alloc((size_t)8 * ns * 128 * 161) != cudaSuccess || f.dew.alloc((size_t)f.nblocks * ns * 136) != cudaSuccess)
+      return fail(BWGR_ERR_CUDA, "cudaMalloc(blocked workspace) failed");
+    if (f.cl && f.cx.alloc((size_t)8 * f.nclusters * ns * 128) != cudaSuccess) return fail(BWGR_ERR_CUDA, "cudaMalloc(cluster ring) failed");
+    if (!f.cl) f.cx.release();
+    CU(cudaMemsetAsync(f.dew.p, 0, sizeof(unsigned long long) * f.dew.n, h->stream));
   }
   if (f.gridfam) {
     grid_geometry(h, &f.rows_per_cta, &f.grid);
-    // unmasked systems: blocks of markers per grid sum, if the block ring fits next to the residual slabs (BWGR_GRID_BLOCK=0: one marker per sum)
-    const char* gb = getenv("BWGR_GRID_BLOCK");
-    f.grid_blocked = !f.masked && s.model != M_KMUP2 && !(gb && !strcmp(gb, "0")) &&
+    // unmasked systems: blocks of markers per grid sum, if the block ring fits next to the residual slabs (else one marker per sum)
+    f.grid_blocked = !f.masked && s.model != M_KMUP2 &&
                      grid_block_smem(ns, f.rows_per_cta, h->storage == BWGR_STORE_F32, model_is_gibbs(s.model)) <= h->smem_optin;
     const size_t words = f.grid_blocked ? grid_block_acc_words(ns, (int)p) : (size_t)p * kGridCopies * 32;
     if (f.gridacc.alloc(words) != cudaSuccess) return fail(BWGR_ERR_CUDA, "cudaMalloc(grid accumulators) failed");
@@ -1378,7 +1325,7 @@ int fit_sweeps(bwgr_handle* h, int nsweeps) {
   const int64_t p = h->p, ld = h->ld;
   const GenoView g = h->view();
   float quantum = 1, limit = 1;
-  if (f.blocked || f.gridfam) g_fixed_point(h, f, &quantum, &limit);
+  if (f.gridfam) g_fixed_point(h, f, &quantum, &limit);
   for (int k = 0; k < nsweeps; k++) {
     const int sweep = f.sweeps_issued;
     const int slot = sweep % kPermRing;
@@ -1404,11 +1351,10 @@ int fit_sweeps(bwgr_handle* h, int nsweeps) {
         CU(cudaStreamWaitEvent(h->stream, h->side_done[sweep & 1], 0));
       } else if (f.shuffled || !f.gram_cached) {
         cudaEvent_t pe = h->prof_begin(0);
-        if (h->gram_simt) launch_gram_simt(g, d_perm, f.nblocks, f.gram_p, 1, h->stream);
-        else if (h->x2f.p && f.nband == 2) {
+        if (h->x2f.p && f.nband == 2) {
           const cudaError_t ge = launch_gram_fp4(h->x2f.p, h->ld, (int)h->p, (int)h->n_global, d_perm, f.nblocks, f.gram_p, h->err.p, h->num_sms, f.sx_dev.p, h->stream);
           if (ge != cudaSuccess) return fail(BWGR_ERR_CUDA, "FP4 Gram launch failed: %s", cudaGetErrorString(ge));
-        } else launch_gram_tc(gram_view(h), d_perm, f.nblocks, f.gram_p, 1, f.nband, h->fp8_codes, h->err.p, h->num_sms, f.sx_dev.p, h->tmap_ok ? h->tmap : nullptr, h->stream);
+        } else launch_gram_tc(gram_view(h), d_perm, f.nblocks, f.gram_p, 1, f.nband, h->fp8_codes, h->err.p, h->num_sms, f.sx_dev.p, h->stream);
         h->prof_end(pe);
         h->launches++;
         f.gram_cached = true;
@@ -1416,79 +1362,57 @@ int fit_sweeps(bwgr_handle* h, int nsweeps) {
         if (h->world > 1)  // row shards: the Gram band is a sum over individuals (exact: integers below 2^24 in fp32)
           NC(nccl().AllReduce(f.gram_p, f.gram_p, (size_t)f.nblocks * kBlk * kBlk * f.nband, ncclFloat, ncclSum, h->comm, h->stream));
       }
-      h->gap_mark();  // 0: band of this sweep available
-      if (f.pipe && f.full_inv) {  // the step coefficients change every sweep (lambda), the inverses with them
+      if (f.full_inv) {  // the step coefficients change every sweep (lambda), the inverses with them
         cudaEvent_t pi = h->prof_begin(3);
         launch_block_inverse(f.model, d_perm, (int)p, f.nblocks, f.gram_p, f.nband, f.xx_over.p ? f.xx_over.p : h->xx_f.p, f.vbv.p, f.sc.p,
                              f.tinv.p, h->stream);
         h->prof_end(pi);
         h->launches++;
       }
-      if (f.pipe) {
-        if (f.cl) CU(cudaMemsetAsync(f.cx.p, 0, sizeof(unsigned long long) * f.cx.n, h->stream));
-        else CU(cudaMemsetAsync(f.part.p, 0, sizeof(unsigned long long) * f.part.n, h->stream));
-        PipeArgs a;
-        memset(&a, 0, sizeof a);
-        a.g = g; a.model = rule_model(f.model); a.nsys = f.nsys; a.perm = d_perm; a.nblocks = f.nblocks; a.gram = f.gram_p; a.nband = f.nband; a.tinv = f.full_inv ? f.tinv.p : nullptr;
-        a.e = f.e.p; a.b = f.b.p; a.d = f.d.p; a.vbv = f.vbv.p; a.xx = f.xx_over.p ? f.xx_over.p : h->xx_f.p; a.sx = f.sx_dev.p; a.cshift = f.cshift.p; a.sc = f.sc.p;
-        a.part = f.part.p; a.hred = f.part.p + (size_t)8 * f.nsys * 128 * 160; a.dew = f.dew.p; a.tag = ++f.tag;
-        a.seed_lo = (uint32_t)f.seed; a.seed_hi = (uint32_t)(f.seed >> 32); a.chain0 = 0;
-        a.rows_per_cta = f.rows_per_cta; a.nworkers = f.nworkers; a.D = f.lookahead; a.nbuf = f.nbuf; a.sring = f.sring; a.err = h->err.p;
-        a.world = h->world; a.rank = h->rank; a.gen0 = h->dist_gen;
-        a.cl = f.cl; a.nclusters = f.nclusters; a.cx = f.cx.p;
-        for (int r = 0; r < 8; r++) a.hx[r] = h->hx[r];
-        if (h->world > 1) h->dist_gen += (unsigned long long)f.nblocks;
-        if (getenv("BWGR_TRACE")) {
-          if (!f.trace.p) { f.trace.alloc((size_t)f.grid * f.nblocks * 32); cudaMemsetAsync(f.trace.p, 0, sizeof(long long) * f.trace.n, h->stream); }
-          a.trace = f.trace.p;
-        }
-        if (f.overlap) { a.started = h->started.p; a.started_val = ++h->started_seq; }
-        h->gap_mark();  // 1: inverses done, rings zeroed
-        cudaEvent_t pe = h->prof_begin(1);
-        const cudaError_t le = launch_sweep_pipe(a, h->stream);
-        h->prof_end(pe);
-        h->gap_mark();  // 2: sweep done
-        if (le != cudaSuccess) return fail(BWGR_ERR_CUDA, "pipelined sweep launch failed: %s", cudaGetErrorString(le));
-        h->launches++;
-        if (f.overlap) {
-          // the flag is also set when the sweep has drained, whatever happened inside it: the side stream never waits forever
-          const CUdeviceptr flag = reinterpret_cast<CUdeviceptr>(h->started.p);
-          if (h->write32(h->stream, flag, a.started_val, 0) != CUDA_SUCCESS) return fail(BWGR_ERR_CUDA, "cuStreamWriteValue32 failed");
-          const bool more = k + 1 < nsweeps || sweep + 1 < f.it_target;
-          if (more && !h->profiling) {  // sweep + 1: order + Gram band on the SMs this sweep leaves idle, as soon as it is resident
-            if (h->wait32(h->side, flag, a.started_val, CU_STREAM_WAIT_VALUE_GEQ) != CUDA_SUCCESS) return fail(BWGR_ERR_CUDA, "cuStreamWaitValue32 failed");
-            CU(upload_order(sweep + 1, h->side));
-            const int* np_ = f.perm.p + (size_t)((sweep + 1) % kPermRing) * p;
-            const cudaError_t ge = launch_gram_fp4(h->x2f.p, h->ld, (int)h->p, (int)h->n_global, np_, f.nblocks, ((sweep + 1) & 1) ? f.gram2.p : f.gram.p,
-                                                   h->err.p, h->num_sms, f.sx_dev.p, h->side, true);
-            if (ge != cudaSuccess) return fail(BWGR_ERR_CUDA, "FP4 Gram launch failed: %s", cudaGetErrorString(ge));
-            if (h->world > 1) {  // row shards: the band is a sum over individuals; its own communicator, so it never queues behind (or ahead of) the main stream's
-              float* gn = ((sweep + 1) & 1) ? f.gram2.p : f.gram.p;
-              NC(nccl().AllReduce(gn, gn, (size_t)f.nblocks * kBlk * kBlk * f.nband, ncclFloat, ncclSum, h->comm_side, h->side));
-            }
-            CU(cudaEventRecord(h->side_done[(sweep + 1) & 1], h->side));
-            f.gram_ahead = sweep + 1;
-            h->launches++;
+      if (f.cl) CU(cudaMemsetAsync(f.cx.p, 0, sizeof(unsigned long long) * f.cx.n, h->stream));
+      else CU(cudaMemsetAsync(f.part.p, 0, sizeof(unsigned long long) * f.part.n, h->stream));
+      PipeArgs a;
+      memset(&a, 0, sizeof a);
+      a.g = g; a.model = rule_model(f.model); a.nsys = f.nsys; a.perm = d_perm; a.nblocks = f.nblocks; a.gram = f.gram_p; a.nband = f.nband; a.tinv = f.full_inv ? f.tinv.p : nullptr;
+      a.e = f.e.p; a.b = f.b.p; a.d = f.d.p; a.vbv = f.vbv.p; a.xx = f.xx_over.p ? f.xx_over.p : h->xx_f.p; a.sx = f.sx_dev.p; a.cshift = f.cshift.p; a.sc = f.sc.p;
+      a.part = f.part.p; a.hred = f.part.p + (size_t)8 * f.nsys * 128 * 160; a.dew = f.dew.p; a.tag = ++f.tag;
+      a.seed_lo = (uint32_t)f.seed; a.seed_hi = (uint32_t)(f.seed >> 32); a.chain0 = 0;
+      a.rows_per_cta = f.rows_per_cta; a.nworkers = f.nworkers; a.D = f.lookahead; a.nbuf = f.nbuf; a.sring = f.sring; a.err = h->err.p;
+      a.world = h->world; a.rank = h->rank; a.gen0 = h->dist_gen;
+      a.cl = f.cl; a.nclusters = f.nclusters; a.cx = f.cx.p;
+      for (int r = 0; r < 8; r++) a.hx[r] = h->hx[r];
+      if (h->world > 1) h->dist_gen += (unsigned long long)f.nblocks;
+      if (getenv("BWGR_TRACE")) {
+        const size_t tn = (size_t)f.grid * f.nblocks * 32;  // a previous fit on this handle may have had another geometry
+        if (f.trace.n != tn) { f.trace.alloc(tn); cudaMemsetAsync(f.trace.p, 0, sizeof(long long) * f.trace.n, h->stream); }
+        a.trace = f.trace.p;
+      }
+      if (f.overlap) { a.started = h->started.p; a.started_val = ++h->started_seq; }
+      cudaEvent_t pe = h->prof_begin(1);
+      const cudaError_t le = launch_sweep_pipe(a, h->stream);
+      h->prof_end(pe);
+      if (le != cudaSuccess) return fail(BWGR_ERR_CUDA, "pipelined sweep launch failed: %s", cudaGetErrorString(le));
+      h->launches++;
+      if (f.overlap) {
+        // the flag is also set when the sweep has drained, whatever happened inside it: the side stream never waits forever
+        const CUdeviceptr flag = reinterpret_cast<CUdeviceptr>(h->started.p);
+        if (h->write32(h->stream, flag, a.started_val, 0) != CUDA_SUCCESS) return fail(BWGR_ERR_CUDA, "cuStreamWriteValue32 failed");
+        const bool more = k + 1 < nsweeps || sweep + 1 < f.it_target;
+        if (more && !h->profiling) {  // sweep + 1: order + Gram band on the SMs this sweep leaves idle, as soon as it is resident
+          if (h->wait32(h->side, flag, a.started_val, CU_STREAM_WAIT_VALUE_GEQ) != CUDA_SUCCESS) return fail(BWGR_ERR_CUDA, "cuStreamWaitValue32 failed");
+          CU(upload_order(sweep + 1, h->side));
+          const int* np_ = f.perm.p + (size_t)((sweep + 1) % kPermRing) * p;
+          const cudaError_t ge = launch_gram_fp4(h->x2f.p, h->ld, (int)h->p, (int)h->n_global, np_, f.nblocks, ((sweep + 1) & 1) ? f.gram2.p : f.gram.p,
+                                                 h->err.p, h->num_sms, f.sx_dev.p, h->side, true);
+          if (ge != cudaSuccess) return fail(BWGR_ERR_CUDA, "FP4 Gram launch failed: %s", cudaGetErrorString(ge));
+          if (h->world > 1) {  // row shards: the band is a sum over individuals; its own communicator, so it never queues behind (or ahead of) the main stream's
+            float* gn = ((sweep + 1) & 1) ? f.gram2.p : f.gram.p;
+            NC(nccl().AllReduce(gn, gn, (size_t)f.nblocks * kBlk * kBlk * f.nband, ncclFloat, ncclSum, h->comm_side, h->side));
           }
+          CU(cudaEventRecord(h->side_done[(sweep + 1) & 1], h->side));
+          f.gram_ahead = sweep + 1;
+          h->launches++;
         }
-      } else {
-        CU(cudaMemsetAsync(f.gacc.p, 0, sizeof(long long) * (size_t)f.nblocks * kNC * f.nsys * kBlk, h->stream));
-        CU(cudaMemsetAsync(f.bar.p, 0, sizeof(unsigned int), h->stream));
-        SweepArgs a;
-        memset(&a, 0, sizeof a);
-        a.g = g; a.model = rule_model(f.model); a.nsys = f.nsys; a.perm = d_perm; a.nblocks = f.nblocks; a.gram = f.gram_p;
-        a.e = f.e.p; a.b = f.b.p; a.d = f.d.p; a.vbv = f.vbv.p; a.xx = f.xx_over.p ? f.xx_over.p : h->xx_f.p; a.sc = f.sc.p;
-        a.gacc = f.gacc.p; a.bar = f.bar.p; a.g_quantum = quantum; a.g_limit = limit;
-        a.seed_lo = (uint32_t)f.seed; a.seed_hi = (uint32_t)(f.seed >> 32); a.chain0 = 0;
-        a.rows_per_cta = f.rows_per_cta; a.err = h->err.p;
-        if (getenv("BWGR_TRACE")) {
-          if (!f.trace.p) f.trace.alloc((size_t)f.nblocks * 16);
-          a.trace = f.trace.p;
-        }
-        cudaEvent_t pe = h->prof_begin(1);
-        launch_sweep_blocked(a, f.grid, h->stream);
-        h->prof_end(pe);
-        h->launches++;
       }
     } else if (f.gridfam) {
       GridArgs a;
@@ -1554,7 +1478,6 @@ int fit_sweeps(bwgr_handle* h, int nsweeps) {
       launch_epilogue(ea, h->stream);
       h->prof_end(pe2);
       h->launches++;
-      h->gap_mark();  // 3: epilogue done
     }
     f.sweeps_issued++;
     cudaError_t le = cudaGetLastError();
@@ -1619,34 +1542,15 @@ int bwgr_em_sweeps(bwgr_handle* h, int nsweeps) {
   return fit_sweeps(h, nsweeps);
 }
 
-// debug (BWGR_TRACE=file): raw int64 stamps of the last sweep, [cta][block][32]
+// debug (BWGR_TRACE=file): header {CTAs, blocks, 32, look-ahead D}, then the raw int64 stamps of the last sweep, [cta][block][32]
 static void dump_trace(bwgr_handle* h) {
   Fit& f = h->fit;
-  if (!h->gap_ev.empty()) {  // BWGR_GAPS: median time between consecutive marks of the main stream (4 marks per sweep)
-    cudaStreamSynchronize(h->stream);
-    const size_t ns = h->gap_ev.size() / 4;
-    if (ns > 12) {
-      const char* names[4] = {"band ready -> inverses + ring memset done", "-> sweep done", "-> epilogue done", "-> next band ready (wait for the side stream)"};
-      for (int k = 0; k < 4; k++) {
-        std::vector<float> v;
-        for (size_t s = 8; s + 1 < ns; s++) {
-          float ms = 0;
-          cudaEventElapsedTime(&ms, h->gap_ev[4 * s + k], h->gap_ev[4 * s + k + 1]);
-          v.push_back(ms);
-        }
-        std::sort(v.begin(), v.end());
-        fprintf(stderr, "[bwgr gaps] %-52s median %.1f us  (min %.1f, max %.1f)\n", names[k], 1e3 * v[v.size() / 2], 1e3 * v.front(), 1e3 * v.back());
-      }
-    }
-    for (cudaEvent_t e : h->gap_ev) cudaEventDestroy(e);
-    h->gap_ev.clear();
-  }
   if (!f.trace.p || !getenv("BWGR_TRACE")) return;
   cudaStreamSynchronize(h->stream);
   std::vector<long long> tr(f.trace.n);
   cudaMemcpy(tr.data(), f.trace.p, tr.size() * sizeof(long long), cudaMemcpyDeviceToHost);
   if (FILE* fp = fopen(getenv("BWGR_TRACE"), "wb")) {
-    const long long hdr[4] = {f.pipe ? f.grid : 1, f.nblocks, 32, f.lookahead};
+    const long long hdr[4] = {f.grid, f.nblocks, 32, f.lookahead};
     fwrite(hdr, sizeof(long long), 4, fp);
     fwrite(tr.data(), sizeof(long long), tr.size(), fp);
     fclose(fp);
@@ -2763,7 +2667,7 @@ int bwgr_mrr3_fit(bwgr_handle* h, int f32_variant, const double* Y, int k, const
   int rc = fit_begin(h, s, Y);
   h->path = saved_path;
   Fit& f = h->fit;
-  if (rc == BWGR_ERR_UNSUPPORTED || (!rc && !f.pipe)) {  // the shape does not fit the pipelined blocked sweep (row slabs above 512 rows): general path
+  if (rc == BWGR_ERR_UNSUPPORTED) {  // the shape does not fit the pipelined blocked sweep (row slabs above 512 rows): general path
     f.reset();
     return mrr3_general(h, f32_variant, Y, k, F, mu_out, b_out, hat_out, h2_out, GC_out, vb_out, ve_out, MSx_out, cnv_out, W_out, its_out);
   }
@@ -2983,7 +2887,7 @@ int bwgr_debug_gram_band(bwgr_handle* h, const int32_t* perm, float* gram_out, i
     const cudaError_t ge = launch_gram_fp4(h->x2f.p, h->ld, (int)p, (int)h->n, dperm.p, nblocks, dg.p, h->err.p, h->num_sms, nullptr, h->stream);
     if (ge != cudaSuccess) return fail(BWGR_ERR_CUDA, "FP4 Gram launch failed: %s", cudaGetErrorString(ge));
   } else {
-    launch_gram_tc(gram_view(h), dperm.p, nblocks, dg.p, 1, 2, h->fp8_codes, h->err.p, h->num_sms, nullptr, h->tmap_ok ? h->tmap : nullptr, h->stream);
+    launch_gram_tc(gram_view(h), dperm.p, nblocks, dg.p, 1, 2, h->fp8_codes, h->err.p, h->num_sms, nullptr, h->stream);
   }
   if (kind_out) *kind_out = h->x2f.p ? 4 : 8;
   h->launches++;
@@ -3004,8 +2908,7 @@ int bwgr_debug_gram(bwgr_handle* h, const int32_t* perm, int block, int32_t* gra
   DevBuf<int32_t> dg;
   if (dperm.alloc(p) != cudaSuccess || dg.alloc((size_t)nblocks * kBlk * kBlk) != cudaSuccess) return fail(BWGR_ERR_CUDA, "cudaMalloc failed");
   CU(cudaMemcpyAsync(dperm.p, perm, sizeof(int) * p, cudaMemcpyHostToDevice, h->stream));
-  if (h->gram_simt) launch_gram_simt(h->view(), dperm.p, nblocks, dg.p, 0, h->stream);
-  else launch_gram_tc(gram_view(h), dperm.p, nblocks, dg.p, 0, 1, h->fp8_codes, h->err.p, h->num_sms, nullptr, h->tmap_ok ? h->tmap : nullptr, h->stream);
+  launch_gram_tc(gram_view(h), dperm.p, nblocks, dg.p, 0, 1, h->fp8_codes, h->err.p, h->num_sms, nullptr, h->stream);
   h->launches++;
   CU(cudaMemcpyAsync(gram_out, dg.p, sizeof(int32_t) * dg.n, cudaMemcpyDeviceToHost, h->stream));
   CU(cudaStreamSynchronize(h->stream));

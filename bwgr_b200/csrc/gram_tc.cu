@@ -13,10 +13,6 @@
 // issues the MMAs (one elected lane) and owns the TMEM allocation, warps 5-8 drain the accumulator (tcgen05.ld -> st.global).
 // Two accumulator stages (2 x 128 TMEM columns) overlap the drain of block i with the MMAs of block i+1.
 // One CTA per SM, persistent over blocks.  HBM traffic: every genotype byte is read exactly once.
-#include <cuda.h>
-#include <stdlib.h>
-#include <string.h>
-
 #include "kernels.h"
 
 namespace bwgr {
@@ -69,19 +65,6 @@ __device__ __forceinline__ bool mbar_wait(uint64_t* bar, uint32_t parity, int* e
   return false;
 }
 
-__device__ __forceinline__ void mbar_arrive_expect_tx(uint64_t* bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-// TMA tile::gather4: four rows (= four marker columns, by index) of the 2-D genotype tensor [p][ld], 128 bytes each from
-// row offset crd0, land as four consecutive 128-byte rows at dst in the SWIZZLE_128B pattern the UMMA descriptor expects.
-// An index outside [0, p) is filled with zeros (and still counts its bytes on the mbarrier).
-__device__ __forceinline__ void tma_gather4(uint32_t dst, const CUtensorMap* tmap, int crd0, int i0, int i1, int i2, int i3,
-                                            uint64_t* bar) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.shared::cta.global.tile::gather4.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3, %4, %5, %6}], [%7];"
-      ::"r"(dst), "l"(reinterpret_cast<uint64_t>(tmap)), "r"(crd0), "r"(i0), "r"(i1), "r"(i2), "r"(i3), "r"(smem_u32(bar))
-      : "memory");
-}
 __device__ __forceinline__ void cp_async16_zfill(uint32_t dst, const void* src, uint32_t src_bytes) {
   asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(dst), "l"(src), "r"(src_bytes) : "memory");
 }
@@ -130,11 +113,11 @@ struct GramSmem {
   float sxc[128];  // column sums of this block's markers (centred Gram)
 };
 
-template <int NBAND, bool FP8, int PROD>
+// PACKED: the tiles are expanded from the 2-bit shadow copy g.x2 (codes 0..3) instead of gathered from the int8 store
+template <int NBAND, bool FP8, bool PACKED>
 __global__ void __launch_bounds__(416, 1) gram_tc_kernel(GenoView g, const int* __restrict__ perm, int nblocks,
                                                          int32_t* __restrict__ gram, int out_f32, int* err,
-                                                         const float* __restrict__ sx, float inv_n, int dbg,
-                                                         const __grid_constant__ CUtensorMap tmap) {
+                                                         const float* __restrict__ sx, float inv_n) {
   constexpr int kStages = GramCfg<NBAND>::kStages;
   constexpr int kLag = GramCfg<NBAND>::kLag;  // cp.async groups kept in flight per producer thread
   constexpr int kSub = GramCfg<NBAND>::kSub;
@@ -150,7 +133,7 @@ __global__ void __launch_bounds__(416, 1) gram_tc_kernel(GenoView g, const int* 
   const int nkg = (nkt + GramCfg<NBAND>::kSub - 1) / GramCfg<NBAND>::kSub;  // stages per block
 
   if (threadIdx.x == 0) {
-    for (int s = 0; s < kStages; s++) { mbar_init(&S->full[s], PROD == 1 ? 1 : PROD == 2 ? 256 : 128); mbar_init(&S->empty[s], 1); }
+    for (int s = 0; s < kStages; s++) { mbar_init(&S->full[s], PACKED ? 256 : 128); mbar_init(&S->empty[s], 1); }
     for (int s = 0; s < 2; s++) { mbar_init(&S->tmem_full[s], 1); mbar_init(&S->tmem_empty[s], 4); }
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
   }
@@ -163,41 +146,7 @@ __global__ void __launch_bounds__(416, 1) gram_tc_kernel(GenoView g, const int* 
   asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
   const uint32_t tmem_base = S->tmem_base;
 
-  if (PROD == 1 && warp < 4) {
-    // ===================== producer: TMA gather4 (one warp; lane l brings markers 4l..4l+3 of every tile) =====================
-    if (warp == 0) {
-      uint32_t it = 0;
-      bool ok = true;
-      for (int blk = blockIdx.x; blk < nblocks && ok; blk += gridDim.x) {
-        int ids[NBAND][4];
-#pragma unroll
-        for (int d = 0; d < NBAND; d++)
-#pragma unroll
-          for (int q = 0; q < 4; q++) {
-            const int pos = (blk - d) * 128 + 4 * lane + q;
-            ids[d][q] = (pos >= 0 && pos < g.p) ? perm[pos] : g.p;  // g.p = out of bounds -> zeros
-          }
-        for (int kg = 0; kg < nkg && ok; kg++, it++) {
-          const uint32_t stage = it % kStages, phase = (it / kStages) & 1u;
-          ok = mbar_wait(&S->empty[stage], phase ^ 1u, err);
-          const uint32_t tbase = smem_u32(tiles + stage * kStageBytes);
-          const int nsub = min(kSub, nkt - kg * kSub);
-          if (lane == 0) mbar_arrive_expect_tx(&S->full[stage], (uint32_t)(nsub * NBAND * kTileBytes));
-          __syncwarp();
-#pragma unroll
-          for (int sub = 0; sub < kSub; sub++) {
-            if (sub < nsub) {
-              const int kt = kg * kSub + sub;
-#pragma unroll
-              for (int d = 0; d < NBAND; d++)
-                tma_gather4(tbase + (sub * NBAND + d) * kTileBytes + lane * 512, &tmap, kt * 128, ids[d][0], ids[d][1], ids[d][2], ids[d][3],
-                            &S->full[stage]);
-            }
-          }
-        }
-      }
-    }
-  } else if (PROD == 2 && (warp < 4 || warp >= 9)) {
+  if (PACKED && (warp < 4 || warp >= 9)) {
     // ===================== producer: 2-bit packed source (codes 0..3), expanded to bytes in flight =====================
     // The gather is what bounds this kernel (~4.3 TB/s of cp.async at 50k x 50k whatever the MMA kind); reading the packed
     // shadow copy moves 4x fewer bytes.  A 16-byte packed chunk = 64 rows of one marker = half a 128-row atom: it is
@@ -267,7 +216,7 @@ __global__ void __launch_bounds__(416, 1) gram_tc_kernel(GenoView g, const int* 
       }
     }
   } else if (warp < 4) {
-    // ===================== producer: gather tiles with cp.async (fallback when no tensor map could be built) =====================
+    // ===================== producer: gather tiles from the int8 store with cp.async =====================
     const int t = threadIdx.x;  // 0..127
     uint32_t it = 0;            // tile counter (runs over blocks and K tiles)
     bool ok = true;
@@ -332,7 +281,7 @@ __global__ void __launch_bounds__(416, 1) gram_tc_kernel(GenoView g, const int* 
 #pragma unroll
           for (int sub = 0; sub < kSub; sub++) {
             const int kt = kg * kSub + sub;
-            if (kt < nkt && !(dbg & 1)) {  // dbg bit 0 (BWGR_GRAM_DBG=1): gather only, no MMAs -- isolates the gather rate
+            if (kt < nkt) {
               const uint64_t desc = make_desc_sw128(smem_u32(tiles + stage * kStageBytes + sub * NBAND * kTileBytes));
 #pragma unroll
               for (int d = 0; d < NBAND; d++) {
@@ -431,83 +380,33 @@ __global__ void __launch_bounds__(416, 1) gram_tc_kernel(GenoView g, const int* 
   }
 }
 
-// Debug / test cross-check: the same Gram blocks with dp4a on the CUDA cores.
-__global__ void __launch_bounds__(256) gram_simt_kernel(GenoView g, const int* __restrict__ perm, int32_t* __restrict__ gram, int out_f32) {
-  const int blk = blockIdx.x;
-  const int nw = (int)(g.ld >> 2);
-  for (int idx = threadIdx.x; idx < 128 * 128; idx += blockDim.x) {
-    const int i = idx >> 7, j = idx & 127;
-    const int pi = blk * 128 + i, pj = blk * 128 + j;
-    int acc = 0;
-    if (pi < g.p && pj < g.p) {
-      const int* ci = reinterpret_cast<const int*>(g.x8 + (int64_t)perm[pi] * g.ld);
-      const int* cj = reinterpret_cast<const int*>(g.x8 + (int64_t)perm[pj] * g.ld);
-      for (int w = 0; w < nw; w++) acc = __dp4a(ci[w], cj[w], acc);
-    }
-    gram[(size_t)blk * 128 * 128 + idx] = out_f32 ? __float_as_int(__int2float_rn(acc)) : acc;
-  }
-}
-
 }  // namespace
 
 template <int NBAND, bool FP8>
 static void launch_gram_band(const GenoView& g, const int* perm, int nblocks, void* gram, int out_f32, int* err, int num_sms,
-                             const float* sx, const void* tmap, cudaStream_t st) {
+                             const float* sx, cudaStream_t st) {
   const size_t smem = (size_t)GramCfg<NBAND>::kStages * GramCfg<NBAND>::kSub * NBAND * kTileBytes + sizeof(GramSmem<NBAND>) + 1024;
   const int grid = nblocks < num_sms ? nblocks : num_sms;
-  const char* de = getenv("BWGR_GRAM_DBG");
-  const int dbg = de ? atoi(de) : 0;
-  CUtensorMap tm;
-  memset(&tm, 0, sizeof tm);
-  if (tmap) memcpy(&tm, tmap, sizeof tm);
   const float inv_n = 1.0f / (float)g.n;
   int32_t* out = static_cast<int32_t*>(gram);
-#define BWGR_GRAM_LAUNCH(PROD)                                                                                              \
+#define BWGR_GRAM_LAUNCH(PACKED)                                                                                            \
   do {                                                                                                                      \
-    cudaFuncSetAttribute(gram_tc_kernel<NBAND, FP8, PROD>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);         \
-    gram_tc_kernel<NBAND, FP8, PROD><<<grid, 416, smem, st>>>(g, perm, nblocks, out, out_f32, err, sx, inv_n, dbg, tm);     \
+    cudaFuncSetAttribute(gram_tc_kernel<NBAND, FP8, PACKED>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);       \
+    gram_tc_kernel<NBAND, FP8, PACKED><<<grid, 416, smem, st>>>(g, perm, nblocks, out, out_f32, err, sx, inv_n);            \
   } while (0)
-  if (FP8 && g.x2 && !tmap) BWGR_GRAM_LAUNCH(2);   // packed 2-bit shadow copy: codes 0..2, exact E4M3 products
-  else if (tmap) BWGR_GRAM_LAUNCH(1);
-  else BWGR_GRAM_LAUNCH(0);
+  if (FP8 && g.x2) BWGR_GRAM_LAUNCH(true);   // packed 2-bit shadow copy: codes 0..3, exact E4M3 products
+  else BWGR_GRAM_LAUNCH(false);
 #undef BWGR_GRAM_LAUNCH
 }
 void launch_gram_tc(const GenoView& g, const int* perm, int nblocks, void* gram, int out_f32, int nband, int fp8_codes,
-                    int* err, int num_sms, const float* sx, const void* tmap, cudaStream_t st) {
+                    int* err, int num_sms, const float* sx, cudaStream_t st) {
   if (fp8_codes) {
-    if (nband == 2) launch_gram_band<2, true>(g, perm, nblocks, gram, out_f32, err, num_sms, sx, tmap, st);
-    else launch_gram_band<1, true>(g, perm, nblocks, gram, out_f32, err, num_sms, sx, tmap, st);
+    if (nband == 2) launch_gram_band<2, true>(g, perm, nblocks, gram, out_f32, err, num_sms, sx, st);
+    else launch_gram_band<1, true>(g, perm, nblocks, gram, out_f32, err, num_sms, sx, st);
   } else {
-    if (nband == 2) launch_gram_band<2, false>(g, perm, nblocks, gram, out_f32, err, num_sms, sx, tmap, st);
-    else launch_gram_band<1, false>(g, perm, nblocks, gram, out_f32, err, num_sms, sx, tmap, st);
+    if (nband == 2) launch_gram_band<2, false>(g, perm, nblocks, gram, out_f32, err, num_sms, sx, st);
+    else launch_gram_band<1, false>(g, perm, nblocks, gram, out_f32, err, num_sms, sx, st);
   }
-}
-
-// Tensor map of the int8 genotype store as a 2-D tensor [p columns][ld rows], box = 128 rows x 1 column, SWIZZLE_128B:
-// the descriptor tile::gather4 needs.  Built through the driver entry point (no link-time dependency on libcuda).
-// tmap_out: 128 bytes, 64-byte aligned.  Returns false if the driver cannot provide it (the kernels then gather with cp.async).
-bool make_geno_tensor_map(const int8_t* x8, int64_t ld, int64_t p, void* tmap_out) {
-  typedef CUresult (*EncodeFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                               const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                               CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-  void* fn = nullptr;
-  cudaDriverEntryPointQueryResult qres;
-  if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &qres) != cudaSuccess || !fn ||
-      qres != cudaDriverEntryPointSuccess)
-    return false;
-  const cuuint64_t dims[2] = {(cuuint64_t)ld, (cuuint64_t)p};
-  const cuuint64_t strides[1] = {(cuuint64_t)ld};
-  const cuuint32_t box[2] = {128, 1}, estr[2] = {1, 1};
-  CUtensorMap tm;
-  const CUresult r = reinterpret_cast<EncodeFn>(fn)(&tm, CU_TENSOR_MAP_DATA_TYPE_UINT8, 2, const_cast<int8_t*>(x8), dims, strides, box,
-                                                    estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
-                                                    CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) return false;
-  memcpy(tmap_out, &tm, sizeof tm);
-  return true;
-}
-void launch_gram_simt(const GenoView& g, const int* perm, int nblocks, void* gram, int out_f32, cudaStream_t st) {
-  gram_simt_kernel<<<nblocks, 256, 0, st>>>(g, perm, static_cast<int32_t*>(gram), out_f32);
 }
 
 }  // namespace bwgr

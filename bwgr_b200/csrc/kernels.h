@@ -76,17 +76,16 @@ bool small_n_fits(const GenoView& g, bool masked, size_t smem_limit, bool weight
 
 // ---- blocked path ---------------------------------------------------------------------------------
 constexpr int kBlk = 128;  // markers per block
-constexpr int kNC = 8;     // copies of every block accumulator: spreads the L2 atomic traffic of the grid over 8x more addresses
 
 // Gram blocks G[blk][i][j] = x_{perm[blk*128+i]}' x_{perm[blk*128+j]} (int32), tcgen05 kind::i8.
 // out_f32: write the (exact) int32 accumulators converted to float, the form the sweep consumes.
 // nband = 2: row r of block b holds [x_{b,r}'X_b | x_{b-1,r}'X_b] (256 entries): the cross block (stored transposed) feeds
 // the one-block look-ahead of the pipelined sweep.
-// fp8_codes != 0: all genotypes are codes 0..7 and n*49 < 2^24 -> kind::f8f6f4 on the same bytes (exact, see gram_tc.cu).
+// fp8_codes != 0: all genotypes are codes 0..7 and n*49 < 2^24 -> kind::f8f6f4 on the same bytes (exact, see gram_tc.cu);
+// with g.x2 set as well (the packed shadow of a store whose codes are 0..3) the tiles are expanded from the 2-bit copy.
 // sx != nullptr (float output): the Gram of the CENTRED columns, x_i'x_k - sx_i sx_k / n (MRR3).
-// tmap != nullptr: the 128-byte CUtensorMap of make_geno_tensor_map -> the tiles are gathered with TMA tile::gather4.
 void launch_gram_tc(const GenoView& g, const int* perm, int nblocks, void* gram, int out_f32, int nband, int fp8_codes,
-                    int* err, int num_sms, const float* sx, const void* tmap, cudaStream_t st);
+                    int* err, int num_sms, const float* sx, cudaStream_t st);
 // FP4 path (gram_fp4.cu): band-2 Gram of a store whose codes are all 0..2, from the packed shadow of launch_pack_2bit_fp4
 // (ld / 4 bytes per column); exact, twice the E4M3 rate.  gram: [nblocks][128][256] floats.
 void launch_pack_2bit_fp4(const int8_t* src, int64_t ld, int p, uint8_t* dst, int* bad, cudaStream_t st);
@@ -96,35 +95,6 @@ cudaError_t launch_gram_fp4(const uint8_t* x2f, int64_t ld, int p, int n, const 
 int narrow_column(const double* src, int64_t n, int8_t* out, int lo, int hi);
 int narrow_column_shifted(const double* src, int64_t n, int8_t* out, double shift, int lo, int hi);
 double column_min(const double* src, int64_t n);
-bool make_geno_tensor_map(const int8_t* x8, int64_t ld, int64_t p, void* tmap_out);
-// SIMT cross-check of the same quantity (debug / tests only; selected with BWGR_GRAM=simt).
-void launch_gram_simt(const GenoView& g, const int* perm, int nblocks, void* gram, int out_f32, cudaStream_t st);
-
-struct SweepArgs {
-  GenoView g;
-  int model;
-  int nsys;
-  const int* perm;       // this sweep's marker order [p] (device)
-  int nblocks;
-  const float* gram;     // [nblocks][128][128] Gram blocks as float (exact below 2^24)
-  float* e;              // [nsys][ld]
-  float* b; float* d; float* vbv;  // [nsys][p]
-  const float* xx;       // [p]
-  SysScalars* sc;        // [nsys]
-  float* B; float* D; float* VBv;  // Gibbs posterior sums or nullptr
-  long long* gacc;       // [nblocks][kNC][nsys][128] block accumulators: (sum of integer partials << 8) + arrival count; zeroed before launch
-  unsigned int* bar;     // grid barrier counter (zeroed before launch)
-  float g_quantum;       // value of one fixed-point unit of g
-  float g_limit;         // |partial g| above this -> err
-  uint32_t seed_lo, seed_hi;
-  int chain0;
-  int rows_per_cta;      // multiple of 16
-  int* err;
-  long long* trace;      // optional [nblocks][16] clock64 stamps of CTA 0 (BWGR_TRACE), else nullptr
-};
-void launch_sweep_blocked(const SweepArgs& a, int grid, cudaStream_t st);
-int sweep_blocked_max_grid(int rows_per_cta, int nsys);
-size_t sweep_blocked_smem(int rows_per_cta, int nsys);
 
 // Pipelined blocked sweep (sweep_pipe.cu): nworkers streaming CTAs + one solver CTA, look-ahead D (0 or 1).
 struct PipeArgs {
@@ -135,7 +105,8 @@ struct PipeArgs {
   int nblocks;
   const float* gram;     // [nblocks][128][nband*128] Gram band as float (exact below 2^24)
   int nband;
-  const float* tinv;     // [nblocks][128][128] (I + A L)^-1 of every block (block_inv.cu; one linear system), or nullptr
+  const float* tinv;     // [nblocks][128][128] (I + A L)^-1 of every block (block_inv.cu), given exactly when the sweep
+                         // has one linear system on uncentred columns; else nullptr
   float* e;              // [nsys][ld]
   float* b; float* d; float* vbv;  // [nsys][p]
   const float* xx;       // [p]

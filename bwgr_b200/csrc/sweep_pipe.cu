@@ -137,7 +137,6 @@ __device__ __forceinline__ unsigned long long gtimer() {
   asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
   return t;
 }
-__device__ __forceinline__ void named_bar_arrive(int id, int nthreads) { asm volatile("bar.arrive %0, %1;" ::"r"(id), "r"(nthreads) : "memory"); }
 __device__ __forceinline__ void named_bar(int id, int nthreads) { asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(nthreads) : "memory"); }
 __device__ __forceinline__ unsigned long long ld_relaxed_u64(const unsigned long long* p) {
   unsigned long long v;
@@ -248,8 +247,6 @@ __host__ __device__ inline SLayout solver_layout(int ns, bool gibbs, bool use_in
   return L;
 }
 __host__ __device__ inline bool pipe_use_inv(int model, int ns) { return model_is_linear(model) && ns <= 2; }
-// one system, linear rule, uncentred columns: the four 32-marker steps of the in-block solve are spread over four warps
-__host__ __device__ inline bool pipe_wps4(int model, int ns, bool centred) { return model_is_linear(model) && ns == 1 && !centred; }
 
 template <int MODEL, bool CL>
 __global__ void __launch_bounds__(kT, 1) sweep_pipe_kernel(PipeArgs a) {
@@ -274,7 +271,7 @@ __global__ void __launch_bounds__(kT, 1) sweep_pipe_kernel(PipeArgs a) {
     mbar_init(&S.dl_full[0], 128); mbar_init(&S.dl_full[1], 128);
     mbar_init(&S.u_done, 1); mbar_init(&S.el_full, 128); mbar_init(&S.g_done, 1); mbar_init(&S.g_empty, 128);
     const int nsw = ns < kSolveWarps ? ns : kSolveWarps;
-    for (int i = 0; i < 3; i++) { mbar_init(&S.raw_ready[i], 128); mbar_init(&S.in_ready[i], 128); mbar_init(&S.solve_done[i], pipe_wps4(MODEL, ns, a.sx != nullptr) ? 4 : nsw); }
+    for (int i = 0; i < 3; i++) { mbar_init(&S.raw_ready[i], 128); mbar_init(&S.in_ready[i], 128); mbar_init(&S.solve_done[i], a.tinv ? 4 : nsw); }
     for (int s = 0; s < 32; s++) {
       mbar_init(&S.corr_ready[s], 128);
       for (int d = 0; d < 4; d++) mbar_init(&S.de_ready[s][d], 1);
@@ -520,15 +517,17 @@ __global__ void __launch_bounds__(kT, 1) sweep_pipe_kernel(PipeArgs a) {
     } else if ((warp >= 5 && warp <= 8) || (warp >= 10 && warp <= 13)) {
       // ------------------------------------------------------------------ X tile gather
       // two groups of four warps take alternate tiles; a group waits for its own tile to land before it signals it,
-      // so a tile is announced the moment it is complete and the other group's tile stays in flight meanwhile
-      const int grp = warp >= 10 ? 1 : 0;
+      // so a tile is announced the moment it is complete and the other group's tile stays in flight meanwhile.
+      // A ring of one tile (the plans without look-ahead) has one group: with two, the group of tile t + 2 could wait on the
+      // parity of a tile_empty phase two uses ahead, which reads as complete, and overwrite the tile still in use.
+      const int grp = warp >= 10 ? 1 : 0, ngrp = nbuf >= 2 ? 2 : 1;
       const int lw = warp - (grp ? 10 : 5);
       const int nchunk = R >> 4;
       const bool act = lane < nchunk && row0 + 16 * lane < a.g.ld;
       const uint32_t choff = (uint32_t)((lane >> 3) * kAtomBytes + ((lane & 7) << 4));
       const int8_t* xrow = a.g.x8 + row0 + 16 * lane;
       const uint64_t pol = policy_evict_first();
-      for (int t = grp; t < nblocks; t += 2) {
+      for (int t = grp; t < nblocks && grp < ngrp; t += ngrp) {
         const int buf = t % nbuf;
         const int pos = t * 128 + lw + 4 * lane;
         const int myid = pos < p ? a.perm[pos] : -1;
@@ -621,7 +620,9 @@ __global__ void __launch_bounds__(kT, 1) sweep_pipe_kernel(PipeArgs a) {
   // Thresholding rules (emEN :431-436, lasso :1478-1486, emBL :378-386): the reciprocals of their denominators are folded one
   // block ahead, the chain keeps an FMA, a compare / clip and a multiply (no division).
   constexpr bool kFoldEM = MODEL == M_EMEN || MODEL == M_LASSO || MODEL == M_EMBL;
-  const bool full_inv = a.tinv != nullptr;  // T = (I + A L)^-1 of every block precomputed (block_inv.cu)
+  // T = (I + A L)^-1 of every block precomputed (block_inv.cu): one system, linear rule, uncentred columns.  The in-block solve
+  // is then one lower-triangular mat-vec, spread over four warps
+  const bool full_inv = a.tinv != nullptr;
   const bool use_inv = !full_inv && pipe_use_inv(MODEL, ns);
   const int sring = a.sring;
   const SLayout L = solver_layout(ns, kGibbs, use_inv, sring, CL);
@@ -735,7 +736,7 @@ __global__ void __launch_bounds__(kT, 1) sweep_pipe_kernel(PipeArgs a) {
         // until the partials of the next block arrive these warps are idle: three of them take one tile each of the lower-
         // triangular product dE = T r of the block they just delivered ((2,2), (3,2), (3,3)); the solve warps add the tile sums in
         // the same order as when they compute all tiles themselves, so the result is bit-identical to the flat topology
-        if (full_inv && pipe_wps4(MODEL, ns, centred) && !sc[0].done) {
+        if (full_inv && !sc[0].done) {
           named_bar(4, 256);  // r of all 128 markers is in shared memory
           const int hw = warp - kCommWarp0;  // 0: tile (2,2); 1: (3,2); 2: (3,3)
           if (hw < 3) {
@@ -757,15 +758,11 @@ __global__ void __launch_bounds__(kT, 1) sweep_pipe_kernel(PipeArgs a) {
         }
       }
     }
-    const bool wps4 = pipe_wps4(MODEL, ns, centred);
-    if (wps4 && warp < 4) {
+    if (full_inv && warp < 4) {
       // ------------------------------------------------------------------ one system on four solve warps
-      // warp w owns markers 32w .. 32w+31 of the block (lane = marker).  Step d: warp d applies the inverse of its diagonal
-      // block (one 32x32 mat-vec through shared memory), the later warps subtract its contribution from their right-hand
-      // sides -- the dependent chain is 4 mat-vecs + 3 (hand-over + update) instead of 4 + 6 serial products on one warp.
+      // warp w owns markers 32w .. 32w+31 of the block (lane = marker)
       const int w = warp;
       float* mxs = cs + 64;  // [2][4] block maxima of |dE| per warp, double buffered by block parity
-      float* rbs = rb + w * 32;
       for (int b = 0; b < nblocks; b++) {
         const int nvalid = min(128, p - b * 128);
         const int slot = b % sring;
@@ -825,12 +822,13 @@ __global__ void __launch_bounds__(kT, 1) sweep_pipe_kernel(PipeArgs a) {
         }
         if (w == 0) SSTAMPW(b, 9);
         const float av = mk[jj].a;
-        float r = fmaf(av, g, mk[jj].c), de = 0.0f;
+        const float r = fmaf(av, g, mk[jj].c);
+        float de = 0.0f;
         if (Sy.done) {
           dehist[jj] = 0.0f;
           __syncwarp();
           if (lane == 0) mbar_arrive(&S.de_ready[0][w]);
-        } else if (full_inv) {
+        } else {
           // dE = T r: all right-hand sides through shared memory, then every warp takes its 32 rows of the lower-triangular
           // product at once -- no dependent 32-marker steps left in the chain
           rb[jj] = r;
@@ -859,44 +857,6 @@ __global__ void __launch_bounds__(kT, 1) sweep_pipe_kernel(PipeArgs a) {
           dehist[jj] = de;
           __syncwarp();
           if (lane == 0) mbar_arrive(&S.de_ready[0][w]);
-        } else {
-#pragma unroll
-          for (int d = 0; d < 4; d++) {
-            if (w == d) {
-              __syncwarp();
-              rbs[lane] = r;
-              __syncwarp();
-              const float* mt = Mt + ((size_t)slot * 4 + d) * 8 * kMS + 4 * lane;
-              float ac[4] = {0.f, 0.f, 0.f, 0.f};
-#pragma unroll
-              for (int k4 = 0; k4 < 8; k4++) {
-                const float4 mv = *reinterpret_cast<const float4*>(mt + k4 * kMS);
-                const float4 rv = *reinterpret_cast<const float4*>(rbs + 4 * k4);
-                ac[0] = fmaf(mv.x, rv.x, ac[0]); ac[1] = fmaf(mv.y, rv.y, ac[1]);
-                ac[2] = fmaf(mv.z, rv.z, ac[2]); ac[3] = fmaf(mv.w, rv.w, ac[3]);
-              }
-              de = (ac[0] + ac[1]) + (ac[2] + ac[3]);
-              dehist[jj] = de;
-              __syncwarp();
-              if (lane == 0) mbar_arrive(&S.de_ready[0][d]);  // for the cross-Gram correction warps
-              named_bar_arrive(4 + d, 128);                    // hand-over to the later solve warps (hardware barrier: ~30 cycles)
-            } else if (w < d) {
-              named_bar_arrive(4 + d, 128);
-            } else {
-              named_bar(4 + d, 128);
-              const float* grow = Gb + (size_t)tri(w, d) * kTileF + lane * kTS;
-              const float* dv4 = dehist + 32 * d;
-              float fa[4] = {0.f, 0.f, 0.f, 0.f};
-#pragma unroll
-              for (int k4 = 0; k4 < 8; k4++) {
-                const float4 gv = *reinterpret_cast<const float4*>(grow + 4 * k4);
-                const float4 dv = *reinterpret_cast<const float4*>(dv4 + 4 * k4);
-                fa[0] = fmaf(gv.x, dv.x, fa[0]); fa[1] = fmaf(gv.y, dv.y, fa[1]);
-                fa[2] = fmaf(gv.z, dv.z, fa[2]); fa[3] = fmaf(gv.w, dv.w, fa[3]);
-              }
-              r = fmaf(-av, (fa[0] + fa[1]) + (fa[2] + fa[3]), r);
-            }
-          }
         }
         if (w == 3) SSTAMPW(b, 10);
         // block maximum of |dE| over the four warps -> the fixed-point scale of the published step
@@ -945,7 +905,7 @@ __global__ void __launch_bounds__(kT, 1) sweep_pipe_kernel(PipeArgs a) {
       }
     }
     // -------------------------------------------------------------------- solve warps (one system at a time)
-    if (!wps4 && warp < nsw) {
+    if (!full_inv && warp < nsw) {
       for (int b = 0; b < nblocks; b++) {
         const int nvalid = min(128, p - b * 128);
         const int slot = b % sring;

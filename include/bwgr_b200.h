@@ -92,7 +92,9 @@ BWGR_API void bwgr_trim(void);
  * handle's own stream. Lets a host framework time the library with its own events. */
 BWGR_API int bwgr_set_stream(bwgr_handle* h, void* cuda_stream);
 /* Tuning knobs: block = markers per block of the blocked sweep (128); path = bwgr_path;
- * grid = persistent CTAs (0 = one per SM). Negative values leave a knob unchanged. */
+ * grid = persistent CTAs (0 = one per SM; grid > 1 runs the blocked sweep in its flat topology on that many CTAs).
+ * Negative values leave a knob unchanged. A shape the blocked sweep cannot take on `grid` CTAs (more than 512 rows per CTA, or
+ * a solver that does not fit one SM) returns BWGR_ERR_UNSUPPORTED under path = BLOCKED; under AUTO another family takes it. */
 BWGR_API int bwgr_set_tuning(bwgr_handle* h, int block, int path, int grid);
 
 /* ---- genotype store (replaces the per-call double->float copy of RcppExports.cpp:115-116) -- */

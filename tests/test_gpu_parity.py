@@ -278,17 +278,18 @@ def test_grid_family_large_n_masks_and_chains(tpod):
         assert np.abs(out["e"] - ref["e"]).max() <= RTOL * np.abs(ref["e"]).max()
 
 
-@pytest.mark.parametrize("blocked", ["1", "0"])
-def test_grid_family_block_variants_multi_system(monkeypatch, blocked):
+@pytest.mark.parametrize("blocked", [True, False])
+def test_grid_family_block_variants_multi_system(blocked):
     """Unmasked systems on the grid family run blocks of 16 markers per grid sum (stale dots corrected by the block's exact integer
-    cross products); BWGR_GRID_BLOCK=0 keeps one marker per sum.  Five traits at once on a ragged shape (p not a multiple of 16,
-    n not a multiple of the row slab) against per-trait oracle fits, both variants; each is bit-reproducible."""
-    monkeypatch.setenv("BWGR_GRID_BLOCK", blocked)
+    cross products); systems with a row mask -- here one that keeps every row -- run one marker per sum.  Five traits at once on a
+    ragged shape (p not a multiple of 16, n not a multiple of the row slab) against per-trait oracle fits, both variants; each is
+    bit-reproducible."""
     X, Y = synth(3001, 333, k=5, seed=31)
+    kw = {} if blocked else {"row_mask": np.ones((X.shape[0], 5), bool)}
     with bw.Genotypes(X, path=bw.PATH_GRID) as g:
         for model in ("emBA", "emBC"):
-            out = bw.em_fit(model, Y, g, it=10)
-            again = bw.em_fit(model, Y, g, it=10)
+            out = bw.em_fit(model, Y, g, it=10, **kw)
+            again = bw.em_fit(model, Y, g, it=10, **kw)
             assert np.array_equal(out["b"], again["b"])
             for t in range(5):
                 ref = O.em(model, Y[:, t], X.astype(np.float32), it=10)
@@ -361,9 +362,10 @@ def test_blocked_sweep_is_deterministic(tpod):
     assert np.array_equal(a["b"], b["b"]) and a["Ve"] == b["Ve"]
 
 
-def test_gram_band_computed_ahead_changes_nothing(monkeypatch):
+def test_gram_band_computed_ahead_changes_nothing():
     """The next sweep's Gram band is computed on a side stream while the clustered sweep runs (capi.cu fit_sweeps): the fit is
-    bit-identical to the one-stream schedule, for straight fits, stepped fits and back-to-back fits on one store."""
+    bit-identical to the one-stream schedule (what a profiled handle runs), for straight fits, stepped fits and back-to-back fits
+    on one store."""
     X, y = synth(20000, 4000, seed=33)
     with bw.Genotypes(X, path=2) as g:
         a = bw.emRR(y, g, it=14)
@@ -372,7 +374,7 @@ def test_gram_band_computed_ahead_changes_nothing(monkeypatch):
             st.sweeps(k)
         s = st.end()
         c = bw.em_fit("emBA", y, g, it=9)
-        monkeypatch.setenv("BWGR_OVERLAP", "0")
+        g.profile(True)
         b = bw.emRR(y, g, it=14)
         d = bw.em_fit("emBA", y, g, it=9)
     assert np.array_equal(a["b"], b["b"]) and a["Ve"] == b["Ve"] and np.array_equal(a["hat"], b["hat"])
@@ -1228,21 +1230,56 @@ def test_emml_marker_weights(tpod, path):
     assert np.abs(out["b"] - bw.emML(y, gen, it=40)["b"]).max() > 1e-2 * np.abs(ref["b"]).max()  # the weights matter
 
 
-@pytest.mark.parametrize("env", [{"BWGR_CLUSTER": "0"}, {"BWGR_CLUSTER": "0", "BWGR_LOOKAHEAD": "0"}, {"BWGR_TINV": "0"}, {"BWGR_SWEEP": "v4"},
-                                 {"BWGR_GRAM": "fp8"}, {"BWGR_GRAM": "i8"}, {"BWGR_GRAM": "simt"}, {"BWGR_TMA": "1", "BWGR_GRAM": "fp8"},
-                                 {"BWGR_GRAM_PACKED": "0", "BWGR_GRAM": "fp8"}, {"BWGR_OVERLAP": "0"}, {"BWGR_MAXCL": "18"},
-                                 {"BWGR_CLUSTER": "0", "BWGR_GRID": "100"}, {"BWGR_LOAD_THREADS": "3", "BWGR_CACHE_GB": "0"}])
-def test_every_kernel_variant_behind_a_switch(monkeypatch, env):
-    """Every alternative kernel the library can select (flat topology, no look-ahead, stepwise in-block solve, the v4 sweep, the
-    E4M3 / int8 / SIMT Gram kernels, the TMA gather4 and unpacked producers) fits the same data to the same parity bar as the default."""
+def _coded(lo, hi, n=3000, p=2000, seed=3):
+    """Genotype codes drawn uniformly from lo..hi and a phenotype with 20 causal markers (h2 = 0.5)."""
+    rng = np.random.default_rng(seed)
+    X = np.asfortranarray(rng.integers(lo, hi + 1, size=(n, p)).astype(np.int8))
+    beta = np.zeros(p)
+    beta[rng.choice(p, 20, replace=False)] = rng.normal(size=20)
+    g = X @ beta
+    g = (g - g.mean()) / g.std() * np.sqrt(0.5)
+    return X, g + rng.normal(size=n) * np.sqrt(0.5)
+
+
+# Each case reaches one kernel variant through what selects it in a fit: the shape, the stored codes or bwgr_set_tuning.
+#   (data, Genotypes keywords, environment, expected trace header {CTAs, blocks, 32, look-ahead D} as (predicate, D), or None)
+_VARIANTS = {
+    # flat topology (one solver CTA, two-hop L2 tree) with the one-block look-ahead: any grid > 1; the clustered plan would take 112 CTAs
+    "flat": (lambda: synth(3000, 2000, seed=3), {"grid": 100}, {}, (lambda ctas: ctas <= 100, 1)),
+    # no look-ahead: 17 systems leave no room in shared memory for a second X tile on two CTAs
+    "lookahead0": (lambda: synth(500, 300, k=17, seed=3), {"grid": 2}, {}, (lambda ctas: ctas == 2, 0)),
+    # Gram kernels: codes 0..2 take FP4 (every other case), 0..3 E4M3 from the packed shadow, 0..7 E4M3 from the int8 gather,
+    # anything else kind::i8
+    "gram_e4m3_packed": (lambda: _coded(0, 3), {}, {}, None),
+    "gram_e4m3_int8": (lambda: _coded(0, 7), {}, {}, None),
+    "gram_i8": (lambda: _coded(-3, 8), {}, {}, None),
+    # n = 52,000 needs more than 14 clusters of 8 CTAs for rows per worker <= 512: the planner's second pass (15 clusters on a B200)
+    "clusters_over_14": (lambda: synth(52000, 300, seed=3), {}, {}, (lambda ctas: ctas > 112 and ctas % 8 == 0, 1)),
+    "load_threads_no_cache": (lambda: synth(3000, 2000, seed=3), {}, {"BWGR_LOAD_THREADS": "3", "BWGR_CACHE_GB": "0"}, None),
+}
+
+
+@pytest.mark.parametrize("model", ["emRR", "emBC"])
+@pytest.mark.parametrize("variant", list(_VARIANTS))
+def test_every_kernel_variant(monkeypatch, tmp_path, variant, model):
+    """Every alternative kernel the blocked family selects (flat topology, no look-ahead, more than 14 clusters, the E4M3 and
+    kind::i8 Gram kernels) fits the same data to the same parity bar as the default; where the variant is a plan, the sweep's trace
+    header shows that plan ran."""
+    make, kw, env, plan = _VARIANTS[variant]
     for k, v in env.items():
         monkeypatch.setenv(k, v)
-    X, y = synth(3000, 2000, seed=3)
-    ref = O.em("emRR", y, X.astype(np.float32), it=6)
-    ref64 = O.em("emRR", y, X.astype(np.float32), it=6, use_double=True)
-    with bw.Genotypes(X, path=2) as g:
-        out = bw.emRR(y, g, it=6)
-        outc = bw.em_fit("emBC", y, g, it=6)
-    _close_em(out, ref, "emRR", ref64)
-    refc = O.em("emBC", y, X.astype(np.float32), it=6)
-    _close_em(outc, refc, "emBC", O.em("emBC", y, X.astype(np.float32), it=6, use_double=True))
+    trace = tmp_path / "trace.bin"
+    if plan:
+        monkeypatch.setenv("BWGR_TRACE", str(trace))
+    X, Y = make()
+    Y2 = Y.reshape(len(Y), -1)
+    with bw.Genotypes(X, path=2, **kw) as g:
+        out = bw.em_fit(model, Y, g, it=6)
+    if plan:
+        hdr = np.fromfile(trace, dtype=np.int64, count=4)
+        assert plan[0](int(hdr[0])) and hdr[1] == (X.shape[1] + 127) // 128 and hdr[2] == 32 and hdr[3] == plan[1], hdr
+    for t in range(Y2.shape[1]):
+        ref = O.em(model, Y2[:, t], X.astype(np.float32), it=6)
+        ref64 = O.em(model, Y2[:, t], X.astype(np.float32), it=6, use_double=True)
+        o = out if Y2.shape[1] == 1 else {k: (v[..., t] if np.ndim(v) else v) for k, v in out.items()}
+        _close_em(o, ref, model, ref64)

@@ -1,5 +1,5 @@
 """Grid family (csrc/grid_sweep.cu) at a chosen shape: emRR sweeps on synthetic genotypes, ms per sweep-kernel launch from the library's CUDA events
-(bwgr_profile; EmStepper keeps everything resident).  usage: python tools/grid_probe.py n p [EM model] [nsweeps]; BWGR_GRID_BLOCK=0 selects the one-marker-per-sum kernel"""
+(bwgr_profile; EmStepper keeps everything resident).  usage: python tools/grid_probe.py n p [EM model] [nsweeps]"""
 import os
 import sys
 import time
