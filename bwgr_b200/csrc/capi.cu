@@ -95,6 +95,10 @@ struct DevBuf {
   size_t n = 0;
   int dev = 0;
   bool cacheable = true;  // false: memory other processes have mapped (cudaIpc)
+  DevBuf() = default;
+  DevBuf(const DevBuf&) = delete;  // a copy would hand the same block back to the cache twice
+  DevBuf& operator=(const DevBuf&) = delete;
+  void swap(DevBuf& o) { std::swap(p, o.p); std::swap(n, o.n); std::swap(dev, o.dev); std::swap(cacheable, o.cacheable); }
   cudaError_t alloc(size_t count) {
     release();
     n = count;
@@ -328,17 +332,22 @@ GenoView gram_view(const bwgr_handle* h) {
   return g;
 }
 
+// Reads the device error word into *flag (0: no kernel raised one) and clears it.
+int take_err_flag(bwgr_handle* h, int* flag) {
+  *flag = 0;
+  CU(cudaMemcpyAsync(flag, h->err.p, sizeof(int), cudaMemcpyDeviceToHost, h->stream));
+  CU(cudaStreamSynchronize(h->stream));
+  if (*flag) CU(cudaMemsetAsync(h->err.p, 0, sizeof(int), h->stream));
+  return 0;
+}
+
 int check_err_flag(bwgr_handle* h, const char* where) {
   int flag = 0;
-  CU(cudaMemcpyAsync(&flag, h->err.p, sizeof(int), cudaMemcpyDeviceToHost, h->stream));
-  CU(cudaStreamSynchronize(h->stream));
-  if (flag) {
-    cudaMemsetAsync(h->err.p, 0, sizeof(int), h->stream);
-    const char* what = flag == 1 ? "non-integer or out-of-range genotype" : flag == 2 ? "tensor-core pipeline watchdog"
-                       : flag == 3 ? "grid barrier watchdog" : flag == 4 ? "fixed-point range of g exceeded" : "device error";
-    return fail(flag == 1 ? BWGR_ERR_ARG : BWGR_ERR_NUMERIC, "%s: %s", where, what);
-  }
-  return 0;
+  const int rc = take_err_flag(h, &flag);
+  if (rc || !flag) return rc;
+  const char* what = flag == 1 ? "non-integer or out-of-range genotype" : flag == 2 ? "tensor-core pipeline watchdog"
+                     : flag == 3 ? "grid barrier watchdog" : flag == 4 ? "fixed-point range of g exceeded" : "device error";
+  return fail(flag == 1 ? BWGR_ERR_ARG : BWGR_ERR_NUMERIC, "%s: %s", where, what);
 }
 
 // Row-sharded fit: all-reduce `cnt` host doubles over the ranks (sum or max) through a device scratch buffer.
@@ -380,6 +389,7 @@ int finish_store(bwgr_handle* h, int storage) {
   for (int64_t j = 0; j < h->p; j++) xf[j] = (float)xx[j];
   CU(cudaMemcpyAsync(h->xx_f.p, xf.data(), sizeof(float) * h->p, cudaMemcpyHostToDevice, h->stream));
   CU(cudaStreamSynchronize(h->stream));
+  int flag = 0, rc = 0;
   {  // codes 0..7 everywhere?  (one more streaming pass at load time)
     h->fp8_codes = 0;
     double xxmax = 0;  // every Gram entry and every partial sum of non-negative codes is bounded by max_j xx_j (Cauchy-Schwarz)
@@ -387,10 +397,7 @@ int finish_store(bwgr_handle* h, int storage) {
     if (xxmax < 16777216.0) {
       launch_check_range_i8(h->x8, h->ld, (int)h->n, (int)h->p, 0, 7, h->err.p, h->stream);
       h->launches++;
-      int flag = 0;
-      CU(cudaMemcpyAsync(&flag, h->err.p, sizeof(int), cudaMemcpyDeviceToHost, h->stream));
-      CU(cudaStreamSynchronize(h->stream));
-      if (flag) CU(cudaMemsetAsync(h->err.p, 0, sizeof(int), h->stream));
+      if ((rc = take_err_flag(h, &flag))) return rc;
       h->fp8_codes = flag ? 0 : 1;
     }
   }
@@ -399,10 +406,8 @@ int finish_store(bwgr_handle* h, int storage) {
     if (h->x2f.alloc((size_t)(h->ld / 4) * h->p) == cudaSuccess) {
       launch_pack_2bit_fp4(h->x8, h->ld, (int)h->p, h->x2f.p, h->err.p, h->stream);
       h->launches++;
-      int flag = 0;
-      CU(cudaMemcpyAsync(&flag, h->err.p, sizeof(int), cudaMemcpyDeviceToHost, h->stream));
-      CU(cudaStreamSynchronize(h->stream));
-      if (flag) { CU(cudaMemsetAsync(h->err.p, 0, sizeof(int), h->stream)); h->x2f.release(); }  // a code 3..7: the E4M3 path
+      if ((rc = take_err_flag(h, &flag))) return rc;
+      if (flag) h->x2f.release();  // a code 3..7: the E4M3 path
     }
   }
   h->x2g.release();
@@ -410,10 +415,8 @@ int finish_store(bwgr_handle* h, int storage) {
     if (h->x2g.alloc((size_t)(h->ld / 4) * h->p) == cudaSuccess) {
       launch_pack_2bit_gram(h->x8, h->ld, (int)h->p, h->x2g.p, h->err.p, h->stream);
       h->launches++;
-      int flag = 0;
-      CU(cudaMemcpyAsync(&flag, h->err.p, sizeof(int), cudaMemcpyDeviceToHost, h->stream));
-      CU(cudaStreamSynchronize(h->stream));
-      if (flag) { CU(cudaMemsetAsync(h->err.p, 0, sizeof(int), h->stream)); h->x2g.release(); }  // a code 3..7: keep the int8 gather
+      if ((rc = take_err_flag(h, &flag))) return rc;
+      if (flag) h->x2g.release();  // a code 3..7: keep the int8 gather
     }
   }
   CU(cudaGetLastError());  // a store kernel that failed to launch must not go unnoticed
@@ -423,7 +426,7 @@ int finish_store(bwgr_handle* h, int storage) {
     if (h->x2.alloc((size_t)h->ldb * h->p) != cudaSuccess) return fail(BWGR_ERR_CUDA, "cudaMalloc(2-bit store) failed");
     launch_pack_2bit(h->x8, h->ld, (int)h->n, (int)h->p, h->x2.p, h->ldb, h->err.p, h->stream);
     h->launches++;
-    int rc = check_err_flag(h, "bwgr_geno_load (2-bit needs codes {0,1,2})");
+    rc = check_err_flag(h, "bwgr_geno_load (2-bit needs codes {0,1,2})");
     if (rc) { h->x2.release(); return rc; }
     h->storage = BWGR_STORE_2BIT;
     h->x8_own.release();  // the 2-bit store is the only copy kept in HBM
@@ -465,6 +468,22 @@ float fvar_f(const std::vector<float>& x) {  // fvar, Rcpp20260726ai.cpp:7-9 (su
   for (float v : x) { const float t = v - mean; s += (double)t * t; }
   return (float)s / (float)(x.size() - 1);
 }
+
+// Fixed-point scale of the residuals in the tensor-core passes: 8x headroom over emax = max|e|.
+void set_e_scale(SysScalars& c, float emax) {
+  int ex = 0;
+  if (emax > 0) std::frexp(emax, &ex);
+  if (ex < -60) ex = -60;
+  c.e_q = std::ldexp(1.0f, ex + 3 - 30);
+  c.e_qinv = std::ldexp(1.0f, 30 - 3 - ex);
+}
+
+// Held by a one-shot entry point from the start of its fit to its return: the fit is released whatever the exit, so a failed call
+// leaves no fit that bwgr_em_sweeps / bwgr_em_end could continue.
+struct FitGuard {
+  bwgr_handle* h;
+  ~FitGuard() { if (h) h->fit.reset(); }
+};
 
 }  // namespace
 
@@ -936,8 +955,8 @@ void grid_geometry(bwgr_handle* h, int* rp, int* grid) {
   *grid = (int)((h->ld + r - 1) / r);
 }
 
-// family: 0 = small-n, 1 = blocked, 2 = grid
-int choose_path(bwgr_handle* h, const FitSpec& s, int* family) {
+// family: 0 = small-n, 1 = blocked, 2 = grid; path: the BWGR_PATH_* to honour
+int choose_path(bwgr_handle* h, const FitSpec& s, int path, int* family) {
   const GenoView g = h->view();
   const bool small_ok = h->storage != BWGR_STORE_F32 && small_n_fits(g, s.row_mask != nullptr, h->smem_optin, s.row_cnt != nullptr);
   PipePlan pl;
@@ -946,13 +965,13 @@ int choose_path(bwgr_handle* h, const FitSpec& s, int* family) {
   grid_geometry(h, &grp, &ggrid);
   const bool grid_ok = (h->storage == BWGR_STORE_I8 || h->storage == BWGR_STORE_F32) && h->world <= 1 && s.nsys <= 32 && s.model != M_MRR &&
                        ggrid <= 255 && grid_sweep_smem(s.nsys, grp, s.row_mask != nullptr, h->storage == BWGR_STORE_F32) <= h->smem_optin;
-  if (h->path == BWGR_PATH_SMALL_N) {
+  if (path == BWGR_PATH_SMALL_N) {
     if (!small_ok) return fail(BWGR_ERR_UNSUPPORTED, "small-n path: residual of n=%lld does not fit one SM", (long long)h->n);
     *family = 0;
-  } else if (h->path == BWGR_PATH_BLOCKED) {
+  } else if (path == BWGR_PATH_BLOCKED) {
     if (!blocked_ok) return fail(BWGR_ERR_UNSUPPORTED, "blocked path needs the int8 store, no row mask, nsys<=32 and n <= 512 rows x grid");
     *family = 1;
-  } else if (h->path == BWGR_PATH_GRID) {
+  } else if (path == BWGR_PATH_GRID) {
     if (!grid_ok) return fail(BWGR_ERR_UNSUPPORTED, "grid path needs the int8 or float32 store, one GPU, nsys<=32 and the row slabs of all systems in shared memory");
     *family = 2;
   } else {
@@ -963,6 +982,53 @@ int choose_path(bwgr_handle* h, const FitSpec& s, int* family) {
     else if (grid_ok) *family = 2;
     else return fail(BWGR_ERR_UNSUPPORTED, "no kernel family fits n=%lld nsys=%d storage=%d", (long long)h->n, s.nsys, h->storage);
   }
+  return 0;
+}
+
+// Device scratch of rows_col_stats: exact int64 sums (int8 store, 0/1 mask) or double sums, allocated on first use
+struct ColStatBufs {
+  DevBuf<long long> xx_i, sx_i;
+  DevBuf<double> xx_d, sx_d;
+};
+
+// Column statistics over the rows a system uses -- a 0/1 row mask, or (cnt) the multiplicity of every row -- with
+// xx_j = sum_i w_i x_ij^2 as floats into slot t of f.xx_sys.  With xx / sx, both sums also come back as host doubles, and the float
+// conversion runs on the host.
+int rows_col_stats(bwgr_handle* h, ColStatBufs& s, const uint8_t* rows, bool cnt, int t, std::vector<double>* xx, std::vector<double>* sx) {
+  const int64_t p = h->p;
+  float* xx_sys = h->fit.xx_sys.p + (size_t)t * p;
+  const bool exact = !cnt && h->storage != BWGR_STORE_F32;
+  if (exact) {
+    if (s.xx_i.n < (size_t)p && (s.xx_i.alloc(p) != cudaSuccess || s.sx_i.alloc(p) != cudaSuccess)) return fail(BWGR_ERR_CUDA, "cudaMalloc failed");
+    launch_col_stats_masked(h->view(), rows, s.xx_i.p, s.sx_i.p, h->stream);
+  } else {
+    if (s.xx_d.n < (size_t)p && (s.xx_d.alloc(p) != cudaSuccess || s.sx_d.alloc(p) != cudaSuccess)) return fail(BWGR_ERR_CUDA, "cudaMalloc failed");
+    if (cnt) launch_col_stats_cnt(h->view(), rows, s.xx_d.p, s.sx_d.p, h->stream);
+    else launch_col_stats_f32(h->view(), rows, s.xx_d.p, s.sx_d.p, h->stream);
+  }
+  h->launches++;
+  if (!xx) {
+    if (exact) launch_ll_to_float(s.xx_i.p, xx_sys, (int)p, h->stream);
+    else launch_d_to_float(s.xx_d.p, xx_sys, (int)p, h->stream);
+    h->launches++;
+    return 0;
+  }
+  xx->resize(p); sx->resize(p);
+  if (exact) {
+    std::vector<long long> hx(p), hs(p);
+    CU(cudaMemcpyAsync(hx.data(), s.xx_i.p, sizeof(long long) * p, cudaMemcpyDeviceToHost, h->stream));
+    CU(cudaMemcpyAsync(hs.data(), s.sx_i.p, sizeof(long long) * p, cudaMemcpyDeviceToHost, h->stream));
+    CU(cudaStreamSynchronize(h->stream));
+    xx->assign(hx.begin(), hx.end()); sx->assign(hs.begin(), hs.end());  // exact: |sums| < 2^45
+  } else {
+    CU(cudaMemcpyAsync(xx->data(), s.xx_d.p, sizeof(double) * p, cudaMemcpyDeviceToHost, h->stream));
+    CU(cudaMemcpyAsync(sx->data(), s.sx_d.p, sizeof(double) * p, cudaMemcpyDeviceToHost, h->stream));
+    CU(cudaStreamSynchronize(h->stream));
+  }
+  std::vector<float> xf(p);
+  for (int64_t j = 0; j < p; j++) xf[j] = (float)(*xx)[j];
+  CU(cudaMemcpyAsync(xx_sys, xf.data(), sizeof(float) * p, cudaMemcpyHostToDevice, h->stream));
+  CU(cudaStreamSynchronize(h->stream));
   return 0;
 }
 
@@ -983,10 +1049,8 @@ int fit_begin(bwgr_handle* h, const FitSpec& s, const double* y) {
     if (s.row_mask) return fail(BWGR_ERR_UNSUPPORTED, "row-sharded fits take unmasked systems");
     if (s.model == M_MRR || s.model == M_KMUP || s.model == M_KMUP2) return fail(BWGR_ERR_UNSUPPORTED, "row sharding covers the univariate EM and Gibbs solvers");
   }
-  const int saved_path_ = h->path;
-  if (dist) h->path = BWGR_PATH_BLOCKED;
-  int rc = choose_path(h, s, &family);
-  h->path = saved_path_;
+  // row-sharded fits and MRR3's rotated systems run on the pipelined blocked sweep only
+  int rc = choose_path(h, s, dist || s.model == M_MRR ? BWGR_PATH_BLOCKED : h->path, &family);
   if (rc) return rc;
   const bool blocked = family == 1;
   const int64_t n = h->n, p = h->p, ld = h->ld;
@@ -1011,35 +1075,10 @@ int fit_begin(bwgr_handle* h, const FitSpec& s, const double* y) {
     }
     if (f.mask.alloc(m.size()) != cudaSuccess || f.xx_sys.alloc((size_t)ns * p) != cudaSuccess) return fail(BWGR_ERR_CUDA, "cudaMalloc failed");
     CU(cudaMemcpyAsync(f.mask.p, m.data(), m.size(), cudaMemcpyHostToDevice, h->stream));
-    DevBuf<long long> txx, tsx;
-    if (txx.alloc(p) != cudaSuccess || tsx.alloc(p) != cudaSuccess) return fail(BWGR_ERR_CUDA, "cudaMalloc failed");
     xx_s.resize(ns); sx_s.resize(ns);
-    std::vector<long long> hx(p), hs(p);
-    std::vector<float> xf(p);
-    for (int t = 0; t < ns; t++) {
-      if (h->storage == BWGR_STORE_F32) {  // real-valued store: the same sums in double (two long long = two double buffers)
-        double* dxx = reinterpret_cast<double*>(txx.p); double* dsx = reinterpret_cast<double*>(tsx.p);
-        launch_col_stats_f32(h->view(), f.mask.p + (size_t)t * ld, dxx, dsx, h->stream);
-        h->launches++;
-        xx_s[t].resize(p); sx_s[t].resize(p);
-        CU(cudaMemcpyAsync(xx_s[t].data(), dxx, sizeof(double) * p, cudaMemcpyDeviceToHost, h->stream));
-        CU(cudaMemcpyAsync(sx_s[t].data(), dsx, sizeof(double) * p, cudaMemcpyDeviceToHost, h->stream));
-        CU(cudaStreamSynchronize(h->stream));
-        for (int64_t j = 0; j < p; j++) xf[j] = (float)xx_s[t][j];
-        CU(cudaMemcpyAsync(f.xx_sys.p + (size_t)t * p, xf.data(), sizeof(float) * p, cudaMemcpyHostToDevice, h->stream));
-        CU(cudaStreamSynchronize(h->stream));
-        continue;
-      }
-      launch_col_stats_masked(h->view(), f.mask.p + (size_t)t * ld, txx.p, tsx.p, h->stream);
-      h->launches++;
-      CU(cudaMemcpyAsync(hx.data(), txx.p, sizeof(long long) * p, cudaMemcpyDeviceToHost, h->stream));
-      CU(cudaMemcpyAsync(hs.data(), tsx.p, sizeof(long long) * p, cudaMemcpyDeviceToHost, h->stream));
-      CU(cudaStreamSynchronize(h->stream));
-      xx_s[t].assign(hx.begin(), hx.end()); sx_s[t].assign(hs.begin(), hs.end());
-      for (int64_t j = 0; j < p; j++) xf[j] = (float)hx[j];
-      CU(cudaMemcpyAsync(f.xx_sys.p + (size_t)t * p, xf.data(), sizeof(float) * p, cudaMemcpyHostToDevice, h->stream));
-      CU(cudaStreamSynchronize(h->stream));
-    }
+    ColStatBufs cs;
+    for (int t = 0; t < ns; t++)
+      if ((rc = rows_col_stats(h, cs, f.mask.p + (size_t)t * ld, false, t, &xx_s[t], &sx_s[t]))) return rc;
   }
 
   // ---- initial state per system (SURVEY A.1), float arithmetic
@@ -1187,7 +1226,7 @@ int fit_begin(bwgr_handle* h, const FitSpec& s, const double* y) {
       default: return fail(BWGR_ERR_ARG, "bad model %d", s.model);
     }
     c.C = -0.5f / std::sqrt(c.ve);
-    {  // fixed-point scale of the residuals (tensor-core passes): 8x headroom over max|y - mu|
+    {  // fixed-point scale of the residuals, from max|y - mu|
       float emax = 0;
       for (float v : yt) emax = std::max(emax, std::fabs(v - mu));
       if (dist) {  // the fixed-point scale must be the same on every rank
@@ -1196,11 +1235,7 @@ int fit_begin(bwgr_handle* h, const FitSpec& s, const double* y) {
         if (rc) return rc;
         emax = (float)em;
       }
-      int ex = 0;
-      if (emax > 0) std::frexp(emax, &ex);
-      if (ex < -60) ex = -60;
-      c.e_q = std::ldexp(1.0f, ex + 3 - 30);
-      c.e_qinv = std::ldexp(1.0f, 30 - 3 - ex);
+      set_e_scale(c, emax);
     }
     f.sc0[t] = c;
     f.vy[t] = vy; f.MSx[t] = c.MSx; f.cxx[t] = c.cxx;
@@ -1496,6 +1531,26 @@ int fit_hat(bwgr_handle* h, const float* b_dev, const float* mu_dev, float* hat_
   return 0;
 }
 
+// Fitted values of nsys systems read back to the host: hat[t * n + i] = mu[t] + x_i'b_t.  b: nsys x p floats, on the device or, with
+// b_on_host, on the host.
+int fitted_values(bwgr_handle* h, int nsys, const float* b, bool b_on_host, const float* mu, std::vector<float>& hat) {
+  const int64_t n = h->n, p = h->p;
+  DevBuf<float> bdev, mudev, hatd;
+  if ((b_on_host && bdev.alloc((size_t)nsys * p) != cudaSuccess) || mudev.alloc(nsys) != cudaSuccess || hatd.alloc(h->ld) != cudaSuccess)
+    return fail(BWGR_ERR_CUDA, "cudaMalloc failed");
+  if (b_on_host) CU(cudaMemcpyAsync(bdev.p, b, sizeof(float) * nsys * p, cudaMemcpyHostToDevice, h->stream));
+  CU(cudaMemcpyAsync(mudev.p, mu, sizeof(float) * nsys, cudaMemcpyHostToDevice, h->stream));
+  const float* bd = b_on_host ? bdev.p : b;
+  hat.resize((size_t)nsys * n);
+  for (int t = 0; t < nsys; t++) {
+    const int rc = fit_hat(h, bd + (size_t)t * p, mudev.p + t, hatd.p);
+    if (rc) return rc;
+    CU(cudaMemcpyAsync(hat.data() + (size_t)t * n, hatd.p, sizeof(float) * n, cudaMemcpyDeviceToHost, h->stream));
+  }
+  CU(cudaStreamSynchronize(h->stream));
+  return 0;
+}
+
 }  // namespace
 
 extern "C" {
@@ -1560,29 +1615,25 @@ static void dump_trace(bwgr_handle* h) {
 int bwgr_em_end(bwgr_handle* h, bwgr_em_out* out) {
   if (!h || !h->fit.active) return fail(BWGR_ERR_STATE, "no fit in progress");
   if (!out) return fail(BWGR_ERR_ARG, "out NULL");
+  FitGuard guard{h};
   Fit& f = h->fit;
   const int64_t n = h->n, p = h->p, ld = h->ld;
   const int ns = f.nsys;
   int rc = check_err_flag(h, "sweep");
-  if (rc) { f.reset(); return rc; }
+  if (rc) return rc;
   dump_trace(h);
   std::vector<SysScalars> sc(ns);
   CU(cudaMemcpyAsync(sc.data(), f.sc.p, sizeof(SysScalars) * ns, cudaMemcpyDeviceToHost, h->stream));
-  std::vector<float> hb((size_t)ns * p), hd, hv, hh((size_t)ns * n), he;
+  std::vector<float> hb((size_t)ns * p), hd, hv, hh, he;
   std::vector<uint8_t> hmask;  // row masks of masked systems (emBL's var(e))
   CU(cudaMemcpyAsync(hb.data(), f.b.p, sizeof(float) * hb.size(), cudaMemcpyDeviceToHost, h->stream));
   if (f.d.p && out->d) { hd.resize((size_t)ns * p); CU(cudaMemcpyAsync(hd.data(), f.d.p, sizeof(float) * hd.size(), cudaMemcpyDeviceToHost, h->stream)); }
   if (f.vbv.p && (out->vb || f.model == M_EMDE)) { hv.resize((size_t)ns * p); CU(cudaMemcpyAsync(hv.data(), f.vbv.p, sizeof(float) * hv.size(), cudaMemcpyDeviceToHost, h->stream)); }
   if (f.model == M_EMBL) { he.resize((size_t)ns * ld); CU(cudaMemcpyAsync(he.data(), f.e.p, sizeof(float) * he.size(), cudaMemcpyDeviceToHost, h->stream)); }
-  DevBuf<float> hat;
-  if (hat.alloc((size_t)ld) != cudaSuccess) return fail(BWGR_ERR_CUDA, "cudaMalloc failed");
-  for (int t = 0; t < ns; t++) {
-    rc = fit_hat(h, f.b.p + (size_t)t * p, &f.sc.p[t].mu, hat.p);
-    if (rc) return rc;
-    CU(cudaMemcpyAsync(hh.data() + (size_t)t * n, hat.p, sizeof(float) * n, cudaMemcpyDeviceToHost, h->stream));
-    CU(cudaStreamSynchronize(h->stream));
-  }
   CU(cudaStreamSynchronize(h->stream));
+  std::vector<float> mu(ns);
+  for (int t = 0; t < ns; t++) mu[t] = sc[t].mu;
+  if ((rc = fitted_values(h, ns, f.b.p, false, mu.data(), hh))) return rc;
   for (int t = 0; t < ns; t++) {
     const SysScalars& c = sc[t];
     if (out->mu) out->mu[t] = c.mu;
@@ -1645,11 +1696,11 @@ int bwgr_em_end(bwgr_handle* h, bwgr_em_out* out) {
   if (out->d && !hd.empty()) for (size_t i = 0; i < hd.size(); i++) out->d[i] = hd[i];
   if (out->vb && !hv.empty()) for (size_t i = 0; i < hv.size(); i++) out->vb[i] = hv[i];
   if (out->hat) for (size_t i = 0; i < hh.size(); i++) out->hat[i] = hh[i];
-  f.reset();
   return 0;
 }
 
 int bwgr_em_fit(bwgr_handle* h, const bwgr_em_params* par, const double* y, bwgr_em_out* out) {
+  FitGuard guard{h};
   int rc = bwgr_em_begin(h, par, y);
   if (rc) return rc;
   Fit& f = h->fit;
@@ -1684,6 +1735,7 @@ int bwgr_gs_fit(bwgr_handle* h, int which, const double* y, double* e, double* b
   s.model = which == 0 ? M_GSRR : M_GSFLM; s.nsys = 1; s.shuffled = false; s.row_mask = nullptr;  // natural marker order (:1581)
   s.df = 10; s.R2 = 0.5f; s.Pi = 0; s.alpha = 0; s.pi = 0; s.it = maxit; s.bi = 0; s.seed = 0;
   // fit_begin on the residual as passed in: mu = mean(e), e <- e - mu (:1574), and the y slot keeps e0 for vna = e.e0/n (:1587)
+  FitGuard guard{h};
   int rc = fit_begin(h, s, e);
   if (rc) return rc;
   Fit& f = h->fit;
@@ -1710,7 +1762,7 @@ int bwgr_gs_fit(bwgr_handle* h, int which, const double* y, double* e, double* b
     done = sc.done;
   }
   rc = check_err_flag(h, "sweep");
-  if (rc) { f.reset(); return rc; }
+  if (rc) return rc;
   std::vector<float> he(ld);
   CU(cudaMemcpyAsync(he.data(), f.e.p, sizeof(float) * ld, cudaMemcpyDeviceToHost, h->stream));
   CU(cudaMemcpyAsync(hb.data(), f.b.p, sizeof(float) * p, cudaMemcpyDeviceToHost, h->stream));
@@ -1724,7 +1776,6 @@ int bwgr_gs_fit(bwgr_handle* h, int which, const double* y, double* e, double* b
     if (vb) vb[j] = which == 0 ? sc.vb : sc.cxx * sc.ve / (L * L);  // GSFLM: Lmb_j = sqrt(phi vna / Vb_j) (:1589)
   }
   if (scal) { scal[0] = sc.mu; scal[1] = 1.0f - sc.ve / c.vy; scal[2] = sc.ve; scal[3] = sc.its; }
-  f.reset();
   return 0;
 }
 
@@ -1744,13 +1795,14 @@ int bwgr_gibbs_fit(bwgr_handle* h, const bwgr_gibbs_params* par, const double* y
   s.model = kGibbsModel[par->model]; s.nsys = nc; s.shuffled = false; s.row_mask = nullptr;
   s.df = (float)par->df; s.R2 = (float)par->R2; s.Pi = 0; s.alpha = 0; s.pi = has_pi ? 0.5f : (float)par->pi;
   s.it = par->it; s.bi = par->bi; s.seed = par->seed;
+  FitGuard guard{h};
   int rc = fit_begin(h, s, yy.data());
   if (rc) return rc;
   Fit& f = h->fit;
   rc = fit_sweeps(h, par->it);
   if (rc) return rc;
   rc = check_err_flag(h, "gibbs sweep");
-  if (rc) { f.reset(); return rc; }
+  if (rc) return rc;
   std::vector<SysScalars> sc(nc);
   CU(cudaMemcpyAsync(sc.data(), f.sc.p, sizeof(SysScalars) * nc, cudaMemcpyDeviceToHost, h->stream));
   std::vector<float> B((size_t)nc * p), D, V;
@@ -1759,25 +1811,18 @@ int bwgr_gibbs_fit(bwgr_handle* h, const bwgr_gibbs_params* par, const double* y
   if (f.VBv.p) { V.resize((size_t)nc * p); CU(cudaMemcpyAsync(V.data(), f.VBv.p, sizeof(float) * V.size(), cudaMemcpyDeviceToHost, h->stream)); }
   CU(cudaStreamSynchronize(h->stream));
   const float MCMC = (float)par->it - (float)par->bi;  // sic (:626): divisor it-bi although i>bi keeps it-bi-1 draws
-  std::vector<float> Bm(B.size()), hh((size_t)nc * n);
+  std::vector<float> Bm(B.size()), MU(nc), hh;
   for (size_t i = 0; i < B.size(); i++) Bm[i] = B[i] / MCMC;
-  DevBuf<float> bdev, mudev, hat;
-  if (bdev.alloc(p) != cudaSuccess || mudev.alloc(1) != cudaSuccess || hat.alloc(h->ld) != cudaSuccess) return fail(BWGR_ERR_CUDA, "cudaMalloc failed");
+  for (int c = 0; c < nc; c++) MU[c] = (float)(sc[c].MU / MCMC);
+  if ((rc = fitted_values(h, nc, Bm.data(), true, MU.data(), hh))) return rc;
   for (int c = 0; c < nc; c++) {
-    const float MU = (float)(sc[c].MU / MCMC);
-    CU(cudaMemcpyAsync(bdev.p, Bm.data() + (size_t)c * p, sizeof(float) * p, cudaMemcpyHostToDevice, h->stream));
-    CU(cudaMemcpyAsync(mudev.p, &MU, sizeof(float), cudaMemcpyHostToDevice, h->stream));
-    rc = fit_hat(h, bdev.p, mudev.p, hat.p);
-    if (rc) return rc;
-    CU(cudaMemcpyAsync(hh.data() + (size_t)c * n, hat.p, sizeof(float) * n, cudaMemcpyDeviceToHost, h->stream));
-    CU(cudaStreamSynchronize(h->stream));
     const float VE = (float)(sc[c].VE / MCMC), VBs = (float)(sc[c].VB / MCMC);
     float vg;
     if (f.VBv.p) { double sv = 0; for (int64_t j = 0; j < p; j++) sv += V[(size_t)c * p + j] / MCMC; vg = (float)sv; }
     else vg = VBs * f.MSx[c];
     const float pi_out = has_pi ? 1.0f - (float)(sc[c].PI / MCMC) : 0.0f;  // :911, :975
     if (f.model == M_BCPI) vg = VBs * f.MSx[c] / pi_out;                   // :913
-    if (out->mu) out->mu[c] = MU;
+    if (out->mu) out->mu[c] = MU[c];
     if (out->scal) {
       double* sc_out = out->scal + (size_t)BWGR_NSCAL * c;
       sc_out[0] = VBs; sc_out[1] = VE; sc_out[2] = vg / (vg + VE); sc_out[3] = f.MSx[c]; sc_out[4] = pi_out; sc_out[5] = 0;
@@ -1790,7 +1835,6 @@ int bwgr_gibbs_fit(bwgr_handle* h, const bwgr_gibbs_params* par, const double* y
   if (out->b) for (size_t i = 0; i < Bm.size(); i++) out->b[i] = Bm[i];
   if (out->d && !D.empty()) for (size_t i = 0; i < D.size(); i++) out->d[i] = D[i] / MCMC;
   if (out->hat) for (size_t i = 0; i < hh.size(); i++) out->hat[i] = hh[i];
-  f.reset();
   return 0;
 }
 
@@ -1800,19 +1844,17 @@ int bwgr_gibbs_fit(bwgr_handle* h, const bwgr_gibbs_params* par, const double* y
 // likelihood ratio).  The 0/1 mask (cnt != 0) is the caller's.
 static int set_row_multiplicities(bwgr_handle* h, const uint8_t* cnt) {
   Fit& f = h->fit;
-  const int64_t n = h->n, p = h->p, ld = h->ld;
+  const int64_t n = h->n, ld = h->ld;
   std::vector<uint8_t> c8((size_t)ld, 0);
   std::vector<float> cf((size_t)ld, 0.0f);
   for (int64_t i = 0; i < n; i++) { c8[i] = cnt[i]; cf[i] = (float)cnt[i]; }
-  DevBuf<double> txx, tsx;
-  if (f.cnt.alloc(ld) != cudaSuccess || f.row_w.alloc(ld) != cudaSuccess || txx.alloc(p) != cudaSuccess || tsx.alloc(p) != cudaSuccess)
-    return fail(BWGR_ERR_CUDA, "cudaMalloc failed");
+  if (f.cnt.alloc(ld) != cudaSuccess || f.row_w.alloc(ld) != cudaSuccess) return fail(BWGR_ERR_CUDA, "cudaMalloc failed");
   CU(cudaMemcpyAsync(f.cnt.p, c8.data(), (size_t)ld, cudaMemcpyHostToDevice, h->stream));
   CU(cudaMemcpyAsync(f.row_w.p, cf.data(), sizeof(float) * ld, cudaMemcpyHostToDevice, h->stream));
-  launch_col_stats_cnt(h->view(), f.cnt.p, txx.p, tsx.p, h->stream);
-  launch_d_to_float(txx.p, f.xx_sys.p, (int)p, h->stream);
-  h->launches += 2;
-  CU(cudaStreamSynchronize(h->stream));  // c8 / cf / txx go out of scope
+  ColStatBufs cs;
+  const int rc = rows_col_stats(h, cs, f.cnt.p, true, 0, nullptr, nullptr);
+  if (rc) return rc;
+  CU(cudaStreamSynchronize(h->stream));  // c8 / cf / the scratch go out of scope
   f.weighted = true;
   return 0;
 }
@@ -1839,14 +1881,9 @@ static int kmup_begin(bwgr_handle* h, const double* b, const double* d, const do
   SysScalars c = f.sc0[0];
   c.mu = 0; c.ve = (float)Ve; c.pi_mix = (float)pi; c.C = -0.5f / std::sqrt((float)Ve);  // C = -0.5/sqrt(Ve) (:17, sic)
   c.sweep = 0; c.burn = 0;
-  {
-    int ex = 0;
-    if (emax > 0) std::frexp(emax, &ex);
-    if (ex < -60) ex = -60;
-    c.e_q = std::ldexp(1.0f, ex + 3 - 30);
-    c.e_qinv = std::ldexp(1.0f, 30 - 3 - ex);
-  }
+  set_e_scale(c, emax);
   f.sc0[0] = c;
+  f.skip_epilogue = true;  // the state is advanced by the caller's sweeps alone (KMUP) or by the wgr driver's steps
   CU(cudaMemcpyAsync(f.e.p, he.data(), sizeof(float) * ld, cudaMemcpyHostToDevice, h->stream));
   CU(cudaMemcpyAsync(f.b.p, hb.data(), sizeof(float) * p, cudaMemcpyHostToDevice, h->stream));
   CU(cudaMemcpyAsync(f.d.p, hd.data(), sizeof(float) * p, cudaMemcpyHostToDevice, h->stream));
@@ -1866,27 +1903,33 @@ static int kmup_begin(bwgr_handle* h, const double* b, const double* d, const do
   return 0;
 }
 
-// KMUP(X,b,d,xx,e,L,Ve,pi) (:12-38): one sweep, state updated in place.  X = the handle's store.
-int bwgr_kmup_sweep(bwgr_handle* h, double* b, double* d, const double* xx, double* e, const double* L, double Ve, double pi,
-                    uint64_t seed) {
-  int rc = kmup_begin(h, b, d, xx, e, L, Ve, pi, seed);
-  if (rc) return rc;
+// One sweep of the KMUP / KMUP2 fit kmup_begin set up, and its read-out: b, d and the residuals, e_out[q] = e[rows[q]] (KMUP2: the
+// rows of Use, in that order) or, with rows null, all n rows.
+static int kmup_sweep_out(bwgr_handle* h, const char* where, double* b, double* d, double* e_out, const double* rows, int64_t nrows) {
   Fit& f = h->fit;
-  f.skip_epilogue = true;
-  rc = fit_sweeps(h, 1);
+  int rc = fit_sweeps(h, 1);
   if (rc) return rc;
-  rc = check_err_flag(h, "kmup sweep");
-  if (rc) { f.reset(); return rc; }
+  rc = check_err_flag(h, where);
+  if (rc) return rc;
   const int64_t n = h->n, p = h->p;
   std::vector<float> he(n), hb(p), hd(p);
   CU(cudaMemcpyAsync(he.data(), f.e.p, sizeof(float) * n, cudaMemcpyDeviceToHost, h->stream));
   CU(cudaMemcpyAsync(hb.data(), f.b.p, sizeof(float) * p, cudaMemcpyDeviceToHost, h->stream));
   CU(cudaMemcpyAsync(hd.data(), f.d.p, sizeof(float) * p, cudaMemcpyDeviceToHost, h->stream));
   CU(cudaStreamSynchronize(h->stream));
-  for (int64_t i = 0; i < n; i++) e[i] = he[i];
+  if (rows) for (int64_t q = 0; q < nrows; q++) e_out[q] = he[(int64_t)rows[q]];
+  else for (int64_t i = 0; i < n; i++) e_out[i] = he[i];
   for (int64_t j = 0; j < p; j++) { b[j] = hb[j]; if (d) d[j] = hd[j]; }
-  f.reset();
   return 0;
+}
+
+// KMUP(X,b,d,xx,e,L,Ve,pi) (:12-38): one sweep, state updated in place.  X = the handle's store.
+int bwgr_kmup_sweep(bwgr_handle* h, double* b, double* d, const double* xx, double* e, const double* L, double Ve, double pi,
+                    uint64_t seed) {
+  FitGuard guard{h};
+  const int rc = kmup_begin(h, b, d, xx, e, L, Ve, pi, seed);
+  if (rc) return rc;
+  return kmup_sweep_out(h, "kmup sweep", b, d, e, nullptr, 0);
 }
 
 // Fitted values of the handle's store: hat = mu + X b.  What the reference's drivers form as X * b (emML2's u1 = X1 * b1,
@@ -1898,157 +1941,32 @@ int bwgr_fitted(bwgr_handle* h, const double* b, double mu, double* hat) {
   if (h->col_offset.size()) return fail(BWGR_ERR_UNSUPPORTED, "this store holds integer codes + a constant per column: use the solvers that centre the columns themselves");
   CU(cudaSetDevice(h->device));
   const int64_t n = h->n, p = h->p;
-  std::vector<float> bf(p), hh(n);
+  std::vector<float> bf(p), hh;
   for (int64_t j = 0; j < p; j++) bf[j] = (float)b[j];
   const float m0 = (float)mu;
-  DevBuf<float> bdev, mudev, hatd;
-  if (bdev.alloc(p) != cudaSuccess || mudev.alloc(1) != cudaSuccess || hatd.alloc(h->ld) != cudaSuccess) return fail(BWGR_ERR_CUDA, "cudaMalloc failed");
-  CU(cudaMemcpyAsync(bdev.p, bf.data(), sizeof(float) * p, cudaMemcpyHostToDevice, h->stream));
-  CU(cudaMemcpyAsync(mudev.p, &m0, sizeof(float), cudaMemcpyHostToDevice, h->stream));
-  int rc = fit_hat(h, bdev.p, mudev.p, hatd.p);
+  const int rc = fitted_values(h, 1, bf.data(), true, &m0, hh);
   if (rc) return rc;
-  CU(cudaMemcpyAsync(hh.data(), hatd.p, sizeof(float) * n, cudaMemcpyDeviceToHost, h->stream));
-  CU(cudaStreamSynchronize(h->stream));
   for (int64_t i = 0; i < n; i++) hat[i] = hh[i];
   return 0;
 }
 
-// wgr(y, X, it, bi, th, bag = 1, rp = FALSE, iv, de, pi, df, R2, eigK = NULL) (R/wgr.R:2-169) with the MCMC loop on the device.
-int bwgr_wgr_fit(bwgr_handle* h, const double* y, int it, int bi, int th, int iv, int de, double pi, double df, double R2,
-                 uint64_t seed, double* b, double* d, double* Vb, double* hat, double* scal) {
+// wgr(y, X, it, bi, th, bag, rp, iv, de, pi, df, R2, eigK = NULL) (R/wgr.R:2-169) with the MCMC loop on the device.
+// bag = 1: `it` KMUP sweeps, each followed by the driver's step on the device (wgr_mode).
+// bag != 1 (:21, :49, :68, :87, :121): every iteration sweeps a fresh sorted sample of floor(n * bag) rows with KMUP2, estimates Ve
+// from their residuals, and rebuilds e = y - mu - X b over all rows.  The row samples come from std::mt19937_64(seed), not from R's
+// sample().
+static int wgr_fit(bwgr_handle* h, const double* y, int it, int bi, int th, double bag, int rp, int iv, int de, double pi, double df,
+                   double R2, uint64_t seed, double* b, double* d, double* Vb, double* hat, double* scal) {
   if (!h || !h->p) return fail(BWGR_ERR_STATE, "no genotypes loaded");
   if (!y) return fail(BWGR_ERR_ARG, "y is NULL");
   if (it < 1 || bi < 1 || bi > it || th < 1) return fail(BWGR_ERR_ARG, "need 1 <= bi <= it and th >= 1");
-  if (de) iv = 1;  // R/wgr.R:10
-  const int64_t n = h->n, p = h->p;
-  // initial state (R/wgr.R:46-59): b = 0, d = 1, mu = mean(y), e = y - mu, Va = MSx, Vb = Va, Ve = 1, L = Vb/Ve (sic)
-  double mu = 0;
-  for (int64_t i = 0; i < n; i++) { if (!(y[i] == y[i])) return fail(BWGR_ERR_ARG, "y contains NaN"); mu += y[i]; }
-  mu /= (double)n;
-  double vy = 0;
-  for (int64_t i = 0; i < n; i++) vy += (y[i] - mu) * (y[i] - mu);
-  vy /= (double)(n - 1);
-  double MSx = 0, sxx = 0;
-  for (int64_t j = 0; j < p; j++) { MSx += (h->h_xx[j] - h->h_sx[j] * h->h_sx[j] / (double)n) / ((double)n - 1.0); sxx += h->h_xx[j]; }
-  if (!(MSx > 0)) return fail(BWGR_ERR_ARG, "genotypes have no variance");
-  std::vector<double> e0(n), b0(p, 0.0), d0(p, 1.0), L0(p, MSx / 1.0);
-  for (int64_t i = 0; i < n; i++) e0[i] = y[i] - mu;
-  int rc = kmup_begin(h, b0.data(), d0.data(), nullptr, e0.data(), L0.data(), 1.0, pi, seed);
-  if (rc) return rc;
-  Fit& f = h->fit;
-  {
-    SysScalars c = f.sc0[0];
-    c.mu = (float)mu;
-    CU(cudaMemcpyAsync(f.sc.p, &c, sizeof(SysScalars), cudaMemcpyHostToDevice, h->stream));
-    CU(cudaStreamSynchronize(h->stream));
-  }
-  if (f.wst.alloc(1) != cudaSuccess) return fail(BWGR_ERR_CUDA, "cudaMalloc failed");
-  CU(cudaMemsetAsync(f.wst.p, 0, sizeof(WgrState), h->stream));
-  WgrArgs& w = f.wgr_args;
-  memset(&w, 0, sizeof w);
-  w.n = (int)n; w.p = (int)p; w.ld = h->ld; w.e = f.e.p; w.b = f.b.p; w.d = f.d.p; w.L = f.vbv.p;
-  w.B = f.B.p; w.D = f.D.p; w.VB = f.VBv.p; w.sc = f.sc.p; w.st = f.wst.p; w.iv = iv; w.de = de;
-  w.Sb = (float)(R2 * df * vy / MSx); w.Se = (float)((1 - R2) * df * vy); w.df = (float)df; w.MSx = (float)MSx;  // :58-59
-  w.it = it; w.bi = bi; w.th = th; w.seed_lo = (uint32_t)seed; w.seed_hi = (uint32_t)(seed >> 32);
-  f.wgr_mode = true;
-  rc = fit_sweeps(h, it);
-  if (rc) return rc;
-  rc = check_err_flag(h, "wgr sweep");
-  if (rc) { f.reset(); return rc; }
-  dump_trace(h);
-  WgrState st;
-  CU(cudaMemcpyAsync(&st, f.wst.p, sizeof st, cudaMemcpyDeviceToHost, h->stream));
-  std::vector<float> B(p), D(p), V(p);
-  CU(cudaMemcpyAsync(B.data(), f.B.p, sizeof(float) * p, cudaMemcpyDeviceToHost, h->stream));
-  CU(cudaMemcpyAsync(D.data(), f.D.p, sizeof(float) * p, cudaMemcpyDeviceToHost, h->stream));
-  CU(cudaMemcpyAsync(V.data(), f.VBv.p, sizeof(float) * p, cudaMemcpyDeviceToHost, h->stream));
-  CU(cudaStreamSynchronize(h->stream));
-  const double mc = (double)((it - bi) / th + 1);  // length(seq(bi, it, th)) (:41-42)
-  double mD = 0;
-  for (int64_t j = 0; j < p; j++) mD += D[j] / mc;
-  mD /= (double)p;
-  std::vector<float> Bm(p);
-  for (int64_t j = 0; j < p; j++) Bm[j] = (float)(B[j] / mc / mD);  // B = B/mc/mean(D) (:143)
-  const float B0 = (float)(st.B0 / mc);
-  DevBuf<float> bdev, mudev, hatd;
-  if (bdev.alloc(p) != cudaSuccess || mudev.alloc(1) != cudaSuccess || hatd.alloc(h->ld) != cudaSuccess) return fail(BWGR_ERR_CUDA, "cudaMalloc failed");
-  CU(cudaMemcpyAsync(bdev.p, Bm.data(), sizeof(float) * p, cudaMemcpyHostToDevice, h->stream));
-  CU(cudaMemcpyAsync(mudev.p, &B0, sizeof(float), cudaMemcpyHostToDevice, h->stream));
-  rc = fit_hat(h, bdev.p, mudev.p, hatd.p);  // HAT = B0 + gen0 %*% B (:152)
-  if (rc) return rc;
-  std::vector<float> hh(n);
-  CU(cudaMemcpyAsync(hh.data(), hatd.p, sizeof(float) * n, cudaMemcpyDeviceToHost, h->stream));
-  CU(cudaStreamSynchronize(h->stream));
-  if (b) for (int64_t j = 0; j < p; j++) b[j] = Bm[j];
-  if (d) for (int64_t j = 0; j < p; j++) d[j] = D[j] / mc;
-  if (Vb && iv) for (int64_t j = 0; j < p; j++) Vb[j] = V[j] / mc;
-  if (hat) for (int64_t i = 0; i < n; i++) hat[i] = hh[i];
-  if (scal) { scal[0] = B0; scal[1] = st.VE / mc; scal[2] = iv ? 0.0 : st.VA / mc; scal[3] = sxx / (double)p; }
-  f.reset();
-  return 0;
-}
-
-// Rows of one bagged iteration as a 0/1 mask plus the multiplicity of every row.  use: 0-based row indices as R passes them
-// (doubles).  *repeats = some row occurs more than once (sampling with replacement, rp = TRUE).
-static int use_to_mask(const double* use, int64_t nuse, int64_t n, std::vector<uint8_t>& mask, std::vector<uint8_t>& cnt, bool* repeats) {
-  mask.assign((size_t)n, 0);
-  cnt.assign((size_t)n, 0);
-  *repeats = false;
-  for (int64_t q = 0; q < nuse; q++) {
-    const int64_t r = (int64_t)use[q];
-    if (r < 0 || r >= n) return fail(BWGR_ERR_ARG, "Use[%lld] = %lld is not a row of X", (long long)q, (long long)r);
-    if (cnt[r] == 255) return fail(BWGR_ERR_UNSUPPORTED, "KMUP2: row %lld occurs more than 255 times in Use", (long long)r);
-    if (mask[r]) *repeats = true;
-    mask[r] = 1;
-    cnt[r]++;
-  }
-  return 0;
-}
-
-// KMUP2(X,Use,b,d,xx,E,L,Ve,pi) (:41-77): one Kuo-Mallick sweep over the rows Use.  b, d updated in place; e_out [nuse] = the
-// residuals of the rows in use, in the order of Use (the reference's third list element).  Runs on the small-n family (row mask).
-int bwgr_kmup2_sweep(bwgr_handle* h, const double* use, int64_t nuse, double* b, double* d, const double* xx, const double* E,
-                     double* e_out, const double* L, double Ve, double pi, uint64_t seed) {
-  if (!h || !h->p) return fail(BWGR_ERR_STATE, "no genotypes loaded");
-  if (!use || !E || !e_out || nuse < 2) return fail(BWGR_ERR_ARG, "KMUP2: bad Use / E / e_out");
-  const int64_t n = h->n, p = h->p;
-  std::vector<uint8_t> mask, cnt;
-  bool repeats = false;
-  int rc = use_to_mask(use, nuse, n, mask, cnt, &repeats);
-  if (rc) return rc;
-  rc = kmup_begin(h, b, d, xx, E, L, Ve, pi, seed, mask.data(), (double)((float)n / (float)nuse), repeats ? cnt.data() : nullptr);
-  if (rc) return rc;
-  Fit& f = h->fit;
-  f.skip_epilogue = true;
-  rc = fit_sweeps(h, 1);
-  if (rc) return rc;
-  rc = check_err_flag(h, "kmup2 sweep");
-  if (rc) { f.reset(); return rc; }
-  std::vector<float> he(n), hb(p), hd(p);
-  CU(cudaMemcpyAsync(he.data(), f.e.p, sizeof(float) * n, cudaMemcpyDeviceToHost, h->stream));
-  CU(cudaMemcpyAsync(hb.data(), f.b.p, sizeof(float) * p, cudaMemcpyDeviceToHost, h->stream));
-  CU(cudaMemcpyAsync(hd.data(), f.d.p, sizeof(float) * p, cudaMemcpyDeviceToHost, h->stream));
-  CU(cudaStreamSynchronize(h->stream));
-  for (int64_t q = 0; q < nuse; q++) e_out[q] = he[(int64_t)use[q]];
-  for (int64_t j = 0; j < p; j++) { b[j] = hb[j]; if (d) d[j] = hd[j]; }
-  f.reset();
-  return 0;
-}
-
-// wgr(y,X,it,bi,th,bag,rp=FALSE,iv,de,pi,df,R2) for bag != 1 (R/wgr.R:21, :49, :68, :87, :121): every iteration sweeps a fresh sorted sample
-// of floor(n * bag) rows with KMUP2, estimates Ve from their residuals, and rebuilds e = y - mu - X b over all rows.  The row samples
-// come from std::mt19937_64(seed), not from R's sample().  Same outputs as bwgr_wgr_fit.
-int bwgr_wgr_fit_bag(bwgr_handle* h, const double* y, int it, int bi, int th, double bag, int rp, int iv, int de, double pi, double df,
-                     double R2, uint64_t seed, double* b, double* d, double* Vb, double* hat, double* scal) {
-  if (bag == 1.0) return bwgr_wgr_fit(h, y, it, bi, th, iv, de, pi, df, R2, seed, b, d, Vb, hat, scal);
-  if (!h || !h->p) return fail(BWGR_ERR_STATE, "no genotypes loaded");
-  if (!y) return fail(BWGR_ERR_ARG, "y is NULL");
-  if (it < 1 || bi < 1 || bi > it || th < 1) return fail(BWGR_ERR_ARG, "need 1 <= bi <= it and th >= 1");
+  const bool bagged = bag != 1.0;
   const int64_t n = h->n, p = h->p, ld = h->ld;
   const int64_t nuse = (int64_t)((double)n * bag);
-  if (!(bag > 0) || nuse < 2 || (!rp && nuse > n)) return fail(BWGR_ERR_ARG, "bag must give 2 <= n * bag (<= n rows without replacement)");
-  if (de) iv = 1;
-  df = df / (bag * bag);  // :21
+  if (bagged && (!(bag > 0) || nuse < 2 || (!rp && nuse > n))) return fail(BWGR_ERR_ARG, "bag must give 2 <= n * bag (<= n rows without replacement)");
+  if (de) iv = 1;  // R/wgr.R:10
+  if (bagged) df = df / (bag * bag);  // :21
+  // initial state (R/wgr.R:46-59): b = 0, d = 1, mu = mean(y), e = y - mu, Va = MSx, Vb = Va, Ve = 1, L = Vb/Ve (sic)
   double mu = 0;
   for (int64_t i = 0; i < n; i++) { if (!(y[i] == y[i])) return fail(BWGR_ERR_ARG, "y contains NaN"); mu += y[i]; }
   mu /= (double)n;
@@ -2078,66 +1996,64 @@ int bwgr_wgr_fit_bag(bwgr_handle* h, const double* y, int it, int bi, int th, do
     for (int64_t r = 0; r < n; r++) rows[r] = r;
     for (int64_t r = 0; r < nuse; r++) { std::uniform_int_distribution<int64_t> pick(r, n - 1); std::swap(rows[r], rows[pick(gen)]); mask[rows[r]] = 1; }
   };
-  draw();
-  int rc = kmup_begin(h, b0.data(), d0.data(), xxb.data(), e0.data(), L0.data(), 1.0, pi, seed, mask.data(), (double)((float)n / (float)nuse),
-                      rp ? cnt.data() : nullptr);
+  FitGuard guard{h};
+  int rc;
+  if (bagged) {
+    draw();
+    rc = kmup_begin(h, b0.data(), d0.data(), xxb.data(), e0.data(), L0.data(), 1.0, pi, seed, mask.data(), (double)((float)n / (float)nuse),
+                    rp ? cnt.data() : nullptr);
+  } else {
+    rc = kmup_begin(h, b0.data(), d0.data(), nullptr, e0.data(), L0.data(), 1.0, pi, seed);
+  }
   if (rc) return rc;
   Fit& f = h->fit;
-  f.skip_epilogue = true;
   {
     SysScalars c = f.sc0[0];
     c.mu = (float)mu;
     CU(cudaMemcpyAsync(f.sc.p, &c, sizeof(SysScalars), cudaMemcpyHostToDevice, h->stream));
     CU(cudaStreamSynchronize(h->stream));
   }
-  DevBuf<float> yd, hatd;
-  DevBuf<long long> txx, tsx;
-  if (f.wst.alloc(1) != cudaSuccess || yd.alloc(ld) != cudaSuccess || hatd.alloc(ld) != cudaSuccess || txx.alloc(p) != cudaSuccess ||
-      tsx.alloc(p) != cudaSuccess)
-    return fail(BWGR_ERR_CUDA, "cudaMalloc failed");
-  {
-    std::vector<float> yf(ld, 0.0f);
-    for (int64_t i = 0; i < n; i++) yf[i] = (float)y[i];
-    CU(cudaMemcpyAsync(yd.p, yf.data(), sizeof(float) * ld, cudaMemcpyHostToDevice, h->stream));
-    CU(cudaStreamSynchronize(h->stream));
-  }
+  if (f.wst.alloc(1) != cudaSuccess) return fail(BWGR_ERR_CUDA, "cudaMalloc failed");
   CU(cudaMemsetAsync(f.wst.p, 0, sizeof(WgrState), h->stream));
   WgrArgs& w = f.wgr_args;
   memset(&w, 0, sizeof w);
   w.n = (int)n; w.p = (int)p; w.ld = ld; w.e = f.e.p; w.b = f.b.p; w.d = f.d.p; w.L = f.vbv.p;
   w.B = f.B.p; w.D = f.D.p; w.VB = f.VBv.p; w.sc = f.sc.p; w.st = f.wst.p; w.iv = iv; w.de = de;
-  w.Sb = (float)(R2 * df * vy / MSx); w.Se = (float)((1 - R2) * df * vy); w.df = (float)df; w.MSx = (float)MSx;
+  w.Sb = (float)(R2 * df * vy / MSx); w.Se = (float)((1 - R2) * df * vy); w.df = (float)df; w.MSx = (float)MSx;  // :58-59
   w.it = it; w.bi = bi; w.th = th; w.seed_lo = (uint32_t)seed; w.seed_hi = (uint32_t)(seed >> 32);
-  w.mask = rp ? f.cnt.p : f.mask.p; w.nsub = (float)nuse; w.y = yd.p; w.hat = hatd.p;  // phase 1 weighs e^2 by the byte (0/1 or the multiplicity)
-  for (int i = 0; i < it; i++) {
-    if (i > 0) {  // this iteration's rows: mask, and H'H of every marker over them (the rule's likelihood-ratio scale)
-      draw();
-      CU(cudaMemcpyAsync(f.mask.p, mask.data(), (size_t)ld, cudaMemcpyHostToDevice, h->stream));
-      if (rp) {
-        if (overflow) { f.reset(); return fail(BWGR_ERR_UNSUPPORTED, "wgr(rp = TRUE): a row was drawn more than 255 times in one iteration"); }
-        CU(cudaMemcpyAsync(f.cnt.p, cnt.data(), (size_t)ld, cudaMemcpyHostToDevice, h->stream));
-        CU(cudaMemcpyAsync(f.row_w.p, cntf.data(), sizeof(float) * ld, cudaMemcpyHostToDevice, h->stream));
-        launch_col_stats_cnt(h->view(), f.cnt.p, reinterpret_cast<double*>(txx.p), reinterpret_cast<double*>(tsx.p), h->stream);
-        launch_d_to_float(reinterpret_cast<double*>(txx.p), f.xx_sys.p, (int)p, h->stream);
-      } else if (h->storage == BWGR_STORE_F32) {
-        launch_col_stats_f32(h->view(), f.mask.p, reinterpret_cast<double*>(txx.p), reinterpret_cast<double*>(tsx.p), h->stream);
-        launch_d_to_float(reinterpret_cast<double*>(txx.p), f.xx_sys.p, (int)p, h->stream);
-      } else {
-        launch_col_stats_masked(h->view(), f.mask.p, txx.p, tsx.p, h->stream);
-        launch_ll_to_float(txx.p, f.xx_sys.p, (int)p, h->stream);
+  if (!bagged) {
+    f.wgr_mode = true;
+    if ((rc = fit_sweeps(h, it))) return rc;
+  } else {
+    DevBuf<float> yd, hatd;
+    if (yd.alloc(ld) != cudaSuccess || hatd.alloc(ld) != cudaSuccess) return fail(BWGR_ERR_CUDA, "cudaMalloc failed");
+    std::vector<float> yf(ld, 0.0f);
+    for (int64_t i = 0; i < n; i++) yf[i] = (float)y[i];
+    CU(cudaMemcpyAsync(yd.p, yf.data(), sizeof(float) * ld, cudaMemcpyHostToDevice, h->stream));
+    CU(cudaStreamSynchronize(h->stream));
+    w.mask = rp ? f.cnt.p : f.mask.p; w.nsub = (float)nuse; w.y = yd.p; w.hat = hatd.p;  // phase 1 weighs e^2 by the byte (0/1 or the multiplicity)
+    ColStatBufs cs;
+    for (int i = 0; i < it; i++) {
+      if (i > 0) {  // this iteration's rows: mask, and H'H of every marker over them (the rule's likelihood-ratio scale)
+        draw();
+        CU(cudaMemcpyAsync(f.mask.p, mask.data(), (size_t)ld, cudaMemcpyHostToDevice, h->stream));
+        if (rp) {
+          if (overflow) return fail(BWGR_ERR_UNSUPPORTED, "wgr(rp = TRUE): a row was drawn more than 255 times in one iteration");
+          CU(cudaMemcpyAsync(f.cnt.p, cnt.data(), (size_t)ld, cudaMemcpyHostToDevice, h->stream));
+          CU(cudaMemcpyAsync(f.row_w.p, cntf.data(), sizeof(float) * ld, cudaMemcpyHostToDevice, h->stream));
+        }
+        if ((rc = rows_col_stats(h, cs, rp ? f.cnt.p : f.mask.p, rp, 0, nullptr, nullptr))) return rc;
       }
-      h->launches += 2;
+      if ((rc = fit_sweeps(h, 1))) return rc;                                    // KMUP2 over the rows in use
+      launch_wgr_bag_phase(w, 1, h->num_sms, h->stream);                          // Vb (with the old Ve), Va, Ve from the rows in use
+      if ((rc = fit_hat(h, f.b.p, reinterpret_cast<const float*>(f.sc.p), hatd.p))) return rc;  // mu + X b  (SysScalars starts with mu)
+      launch_wgr_bag_phase(w, 2, h->num_sms, h->stream);                          // e = y - hat, intercept draw, L, posterior sums
+      h->launches += 3;
     }
-    rc = fit_sweeps(h, 1);  // KMUP2 over the rows in use
-    if (rc) return rc;
-    launch_wgr_bag_phase(w, 1, h->num_sms, h->stream);                       // Vb (with the old Ve), Va, Ve from the rows in use
-    rc = fit_hat(h, f.b.p, reinterpret_cast<const float*>(f.sc.p), hatd.p);  // mu + X b  (SysScalars starts with mu)
-    if (rc) return rc;
-    launch_wgr_bag_phase(w, 2, h->num_sms, h->stream);                       // e = y - hat, intercept draw, L, posterior sums
-    h->launches += 3;
   }
-  rc = check_err_flag(h, "wgr (bagged) sweep");
-  if (rc) { f.reset(); return rc; }
+  rc = check_err_flag(h, bagged ? "wgr (bagged) sweep" : "wgr sweep");
+  if (rc) return rc;
+  if (!bagged) dump_trace(h);
   WgrState st;
   CU(cudaMemcpyAsync(&st, f.wst.p, sizeof st, cudaMemcpyDeviceToHost, h->stream));
   std::vector<float> B(p), D(p), V(p);
@@ -2145,29 +2061,66 @@ int bwgr_wgr_fit_bag(bwgr_handle* h, const double* y, int it, int bi, int th, do
   CU(cudaMemcpyAsync(D.data(), f.D.p, sizeof(float) * p, cudaMemcpyDeviceToHost, h->stream));
   CU(cudaMemcpyAsync(V.data(), f.VBv.p, sizeof(float) * p, cudaMemcpyDeviceToHost, h->stream));
   CU(cudaStreamSynchronize(h->stream));
-  const double mc = (double)((it - bi) / th + 1);
+  const double mc = (double)((it - bi) / th + 1);  // length(seq(bi, it, th)) (:41-42)
   double mD = 0;
   for (int64_t j = 0; j < p; j++) mD += D[j] / mc;
   mD /= (double)p;
-  std::vector<float> Bm(p);
-  for (int64_t j = 0; j < p; j++) Bm[j] = (float)(B[j] / mc / mD);
+  std::vector<float> Bm(p), hh;
+  for (int64_t j = 0; j < p; j++) Bm[j] = (float)(B[j] / mc / mD);  // B = B/mc/mean(D) (:143)
   const float B0 = (float)(st.B0 / mc);
-  DevBuf<float> bdev, mudev;
-  if (bdev.alloc(p) != cudaSuccess || mudev.alloc(1) != cudaSuccess) return fail(BWGR_ERR_CUDA, "cudaMalloc failed");
-  CU(cudaMemcpyAsync(bdev.p, Bm.data(), sizeof(float) * p, cudaMemcpyHostToDevice, h->stream));
-  CU(cudaMemcpyAsync(mudev.p, &B0, sizeof(float), cudaMemcpyHostToDevice, h->stream));
-  rc = fit_hat(h, bdev.p, mudev.p, hatd.p);
+  rc = fitted_values(h, 1, Bm.data(), true, &B0, hh);  // HAT = B0 + gen0 %*% B (:152)
   if (rc) return rc;
-  std::vector<float> hh(n);
-  CU(cudaMemcpyAsync(hh.data(), hatd.p, sizeof(float) * n, cudaMemcpyDeviceToHost, h->stream));
-  CU(cudaStreamSynchronize(h->stream));
   if (b) for (int64_t j = 0; j < p; j++) b[j] = Bm[j];
   if (d) for (int64_t j = 0; j < p; j++) d[j] = D[j] / mc;
   if (Vb && iv) for (int64_t j = 0; j < p; j++) Vb[j] = V[j] / mc;
   if (hat) for (int64_t i = 0; i < n; i++) hat[i] = hh[i];
   if (scal) { scal[0] = B0; scal[1] = st.VE / mc; scal[2] = iv ? 0.0 : st.VA / mc; scal[3] = sxx / (double)p; }
-  f.reset();
   return 0;
+}
+
+int bwgr_wgr_fit(bwgr_handle* h, const double* y, int it, int bi, int th, int iv, int de, double pi, double df, double R2,
+                 uint64_t seed, double* b, double* d, double* Vb, double* hat, double* scal) {
+  return wgr_fit(h, y, it, bi, th, 1.0, 0, iv, de, pi, df, R2, seed, b, d, Vb, hat, scal);
+}
+
+// Rows of one bagged iteration as a 0/1 mask plus the multiplicity of every row.  use: 0-based row indices as R passes them
+// (doubles).  *repeats = some row occurs more than once (sampling with replacement, rp = TRUE).
+static int use_to_mask(const double* use, int64_t nuse, int64_t n, std::vector<uint8_t>& mask, std::vector<uint8_t>& cnt, bool* repeats) {
+  mask.assign((size_t)n, 0);
+  cnt.assign((size_t)n, 0);
+  *repeats = false;
+  for (int64_t q = 0; q < nuse; q++) {
+    const int64_t r = (int64_t)use[q];
+    if (r < 0 || r >= n) return fail(BWGR_ERR_ARG, "Use[%lld] = %lld is not a row of X", (long long)q, (long long)r);
+    if (cnt[r] == 255) return fail(BWGR_ERR_UNSUPPORTED, "KMUP2: row %lld occurs more than 255 times in Use", (long long)r);
+    if (mask[r]) *repeats = true;
+    mask[r] = 1;
+    cnt[r]++;
+  }
+  return 0;
+}
+
+// KMUP2(X,Use,b,d,xx,E,L,Ve,pi) (:41-77): one Kuo-Mallick sweep over the rows Use.  b, d updated in place; e_out [nuse] = the
+// residuals of the rows in use, in the order of Use (the reference's third list element).  Runs on the small-n family (row mask).
+int bwgr_kmup2_sweep(bwgr_handle* h, const double* use, int64_t nuse, double* b, double* d, const double* xx, const double* E,
+                     double* e_out, const double* L, double Ve, double pi, uint64_t seed) {
+  if (!h || !h->p) return fail(BWGR_ERR_STATE, "no genotypes loaded");
+  if (!use || !E || !e_out || nuse < 2) return fail(BWGR_ERR_ARG, "KMUP2: bad Use / E / e_out");
+  const int64_t n = h->n;
+  std::vector<uint8_t> mask, cnt;
+  bool repeats = false;
+  int rc = use_to_mask(use, nuse, n, mask, cnt, &repeats);
+  if (rc) return rc;
+  FitGuard guard{h};
+  rc = kmup_begin(h, b, d, xx, E, L, Ve, pi, seed, mask.data(), (double)((float)n / (float)nuse), repeats ? cnt.data() : nullptr);
+  if (rc) return rc;
+  return kmup_sweep_out(h, "kmup2 sweep", b, d, e_out, use, nuse);
+}
+
+// wgr(y,X,it,bi,th,bag,rp,iv,de,pi,df,R2): bwgr_wgr_fit with row bagging (see wgr_fit); bag = 1 is bwgr_wgr_fit.  Same outputs.
+int bwgr_wgr_fit_bag(bwgr_handle* h, const double* y, int it, int bi, int th, double bag, int rp, int iv, int de, double pi, double df,
+                     double R2, uint64_t seed, double* b, double* d, double* Vb, double* hat, double* scal) {
+  return wgr_fit(h, y, it, bi, th, bag, rp, iv, de, pi, df, R2, seed, b, d, Vb, hat, scal);
 }
 
 }  // extern "C"
@@ -2258,12 +2211,74 @@ struct MrrFlags {
     DeflateMax = par[q++]; DeflateBy = par[q++]; OneVarB = par[q++] != 0; OneVarE = par[q++] != 0;
   }
 };
-// The k x k state of the variance components that survives from sweep to sweep.
+// The state of MRR3's outer loop that survives from sweep to sweep, the same on the rotated fast path and the general path.
 struct MrrVar {
   Mat vb, iG, GC, Sb;
   std::vector<double> vbInit;
   double Deflate = 1, inflate = 0;
+  std::vector<double> mu, vy, MSx, nn;  // per trait: mean and variance of y, sum of the marker variances, observations (the path's)
+  std::vector<double> ve, iVe, veInit, h2, Se, iNp;
+  std::vector<double> cnvB, cnvH2, cnvV;  // convergence records (:662-666)
+  int numit = 0;
 };
+// Output arrays of bwgr_mrr3_fit (any may be null)
+struct MrrOut {
+  double *mu, *b, *hat, *h2, *GC, *vb, *ve, *MSx, *cnv, *W;
+  int* its;
+};
+
+// Starting values (:394-432) from V.vy, V.MSx and V.nn.
+void mrr_start(const MrrFlags& F, int k, MrrVar& V) {
+  auto M = [k](int r, int c) { return (size_t)r + (size_t)c * k; };
+  Mat& vb = V.vb;
+  vb.assign((size_t)k * k, 0.0); V.iG.assign((size_t)k * k, 0.0); V.GC.assign((size_t)k * k, 0.0);
+  for (auto* v : {&V.vbInit, &V.ve, &V.iVe, &V.veInit, &V.h2, &V.Se, &V.iNp}) v->resize(k);
+  for (int t = 0; t < k; t++) {
+    V.ve[t] = V.vy[t] * (1 - F.R2); V.iVe[t] = 1.0 / V.ve[t]; V.veInit[t] = V.ve[t];
+    V.vbInit[t] = V.vy[t] * F.R2 / V.MSx[t]; vb[M(t, t)] = V.vbInit[t]; V.iG[M(t, t)] = 1.0 / V.vbInit[t]; V.h2[t] = 1 - V.ve[t] / V.vy[t];
+    V.Se[t] = V.ve[t] * F.df0; V.iNp[t] = 1.0 / (V.nn[t] + F.df0 - 1.0);
+  }
+  for (int i = 0; i < k; i++) for (int j = 0; j < i; j++) { const double v = F.gc0 * std::sqrt(vb[M(i, i)] * vb[M(j, j)]); vb[M(i, j)] = v; vb[M(j, i)] = v; }
+  V.Sb = vb;
+  for (auto& v : V.Sb) v *= F.df0;
+}
+
+// Residual variances of one sweep (:536-543) from e'y of trait t at ey[t * stride].
+void mrr_residual_var(const MrrFlags& F, int k, const double* ey, int stride, MrrVar& V) {
+  for (int t = 0; t < k; t++) { V.ve[t] = (ey[(size_t)t * stride] + V.Se[t]) * V.iNp[t]; V.h2[t] = 1 - V.ve[t] / V.vy[t]; }
+  if (F.wph2 > 0) for (int t = 0; t < k; t++) V.ve[t] = V.ve[t] * (1 - F.wph2) + F.wph2 * V.veInit[t];
+  if (F.OneVarE) { double m = 0; for (int t = 0; t < k; t++) m += V.ve[t]; m /= k; for (int t = 0; t < k; t++) V.ve[t] = m; }
+  for (int t = 0; t < k; t++) V.iVe[t] = 1.0 / V.ve[t];
+}
+
+// Convergence records of one sweep (:662-666) from |beta0 - b|^2 of every trait; vb0 and h20 are vb and h2 before the sweep.
+// False: the outer loop ends here.
+bool mrr_record(const MrrFlags& F, int k, const double* db, const Mat& vb0, const std::vector<double>& h20, MrrVar& V) {
+  double mx = -1e300;
+  for (int t = 0; t < k; t++) mx = std::max(mx, db[t]);
+  const double cnv = std::log10(mx);
+  V.cnvB.push_back(cnv);
+  if (cnv != cnv) return false;  // :663
+  { double sH = 0; for (int t = 0; t < k; t++) sH += (h20[t] - V.h2[t]) * (h20[t] - V.h2[t]); V.cnvH2.push_back(std::log10(sH)); }
+  { double sV = 0; for (size_t i = 0; i < V.vb.size(); i++) sV += (vb0[i] - V.vb[i]) * (vb0[i] - V.vb[i]); V.cnvV.push_back(std::log10(sV)); }
+  ++V.numit;
+  return !(cnv < std::log10(F.tol));
+}
+
+// The outputs (:676-700) both paths share; b, hat and W are the path's own.
+void mrr_copy_out(const MrrFlags& F, int k, const MrrVar& V, const MrrOut& o) {
+  for (int t = 0; t < k; t++) {
+    if (o.mu) o.mu[t] = V.mu[t];
+    if (o.h2) o.h2[t] = V.h2[t];
+    if (o.ve) o.ve[t] = V.ve[t];
+    if (o.MSx) o.MSx[t] = V.MSx[t];
+  }
+  if (o.GC) for (int i = 0; i < k * k; i++) o.GC[i] = V.GC[i];
+  if (o.vb) for (int i = 0; i < k * k; i++) o.vb[i] = V.vb[i];
+  if (o.cnv)
+    for (int i = 0; i < V.numit; i++) { o.cnv[i] = V.cnvB[i]; o.cnv[F.maxit + i] = V.cnvH2[i]; o.cnv[2 * F.maxit + i] = V.cnvV[i]; }
+  if (o.its) *o.its = V.numit;
+}
 // Genetic (co)variances of one sweep (:559-648): TildeHat and the traces Tr (TrXSX, or TrDinvXSX under TH) in, vb / GC / iG out.
 // Shared by the rotated fast path and the general path; double, on the host (k <= 32).
 void mrr_varcomp(const MrrFlags& F, int k, const Mat& TildeHat, const std::vector<double>& Tr, const std::vector<double>& h2, MrrVar& V) {
@@ -2358,9 +2373,7 @@ void mrr_varcomp(const MrrFlags& F, int k, const Mat& TildeHat, const std::vecto
 
 // MRR3 / MRR3F on the general device path (mrr_gen.cu): per-trait observation masks, InnerGS, NLfactor, TH, MRR3F's NoInv system.
 // Host side = the reference's set-up (:359-432) and the k x k variance block; everything O(n), O(p) or O(n p) is a kernel.
-int mrr3_general(bwgr_handle* h, int f32_variant, const double* Y, int k, const MrrFlags& F, double* mu_out, double* b_out,
-                 double* hat_out, double* h2_out, double* GC_out, double* vb_out, double* ve_out, double* MSx_out, double* cnv_out,
-                 double* W_out, int* its_out) {
+int mrr3_general(bwgr_handle* h, int f32_variant, const double* Y, int k, const MrrFlags& F, const MrrOut& out) {
   if (h->storage != BWGR_STORE_I8 || !h->x8) return fail(BWGR_ERR_UNSUPPORTED, "MRR3 (general path) reads the int8 store");
   if (h->world > 1) return fail(BWGR_ERR_UNSUPPORTED, "MRR3 does not run on a row-sharded store");
   const int64_t n = h->n, p = h->p, ld = h->ld;
@@ -2370,8 +2383,11 @@ int mrr3_general(bwgr_handle* h, int f32_variant, const double* Y, int k, const 
   auto M = [k](int r, int c) { return (size_t)r + (size_t)c * k; };
   CU(cudaSetDevice(h->device));
   // ---- incidence, counts, centred phenotypes (:359-376)
+  MrrVar V;
+  std::vector<double> &nn = V.nn, &mu = V.mu, &vy = V.vy, &MSx = V.MSx;
+  nn.resize(k); mu.resize(k); vy.resize(k); MSx.assign(k, 0.0);
   std::vector<uint32_t> zb((size_t)ld, 0u);
-  std::vector<double> nn(k), mu(k), ysum(k), vy(k), yh((size_t)k * ld, 0.0);
+  std::vector<double> ysum(k), yh((size_t)k * ld, 0.0);
   for (int t = 0; t < k; t++) {
     double sum = 0; int64_t cnt = 0;
     for (int64_t i = 0; i < n; i++) { const double v = Y[(size_t)t * n + i]; if (v == v) { zb[i] |= 1u << t; sum += v; cnt++; } }
@@ -2421,7 +2437,7 @@ int mrr3_general(bwgr_handle* h, int f32_variant, const double* Y, int k, const 
     CU(cudaMemcpyAsync(tilde.data(), tilded.p, sizeof(double) * p * k, cudaMemcpyDeviceToHost, st));
     CU(cudaStreamSynchronize(st));
   }
-  std::vector<double> MSx(k, 0.0), TrXSX(k), see(k);
+  std::vector<double> TrXSX(k), see(k);
   double xxmax = 0;
   for (int64_t j = 0; j < p; j++) xxmax = std::max(xxmax, h->h_xx[j]);
   for (int t = 0; t < k; t++) see[t] = vy[t] * (nn[t] - 1.0);  // e = y at the start
@@ -2448,40 +2464,28 @@ int mrr3_general(bwgr_handle* h, int f32_variant, const double* Y, int k, const 
   CU(cudaMemcpyAsync(meand.p, meanv.data(), sizeof(double) * p, cudaMemcpyHostToDevice, st));
   CU(cudaMemcpyAsync(tilded.p, tilde.data(), sizeof(double) * p * k, cudaMemcpyHostToDevice, st));
   if (F.TH) CU(cudaMemcpyAsync(xsxd.p, xsx.data(), sizeof(double) * p * k, cudaMemcpyHostToDevice, st));
-  // ---- starting values (:394-432)
-  std::vector<double> ve(k), iVe(k), veInit(k), h2(k), Se(k), iNp(k);
-  MrrVar V;
-  Mat &vb = V.vb, &iG = V.iG, &GC = V.GC, TildeHat((size_t)kk);
-  vb.assign((size_t)kk, 0.0); iG.assign((size_t)kk, 0.0); GC.assign((size_t)kk, 0.0);
-  V.vbInit.resize(k);
-  for (int t = 0; t < k; t++) {
-    ve[t] = vy[t] * (1 - F.R2); iVe[t] = 1.0 / ve[t]; veInit[t] = ve[t];
-    V.vbInit[t] = vy[t] * F.R2 / MSx[t]; vb[M(t, t)] = V.vbInit[t]; iG[M(t, t)] = 1.0 / V.vbInit[t]; h2[t] = 1 - ve[t] / vy[t];
-    Se[t] = ve[t] * F.df0; iNp[t] = 1.0 / (nn[t] + F.df0 - 1.0);
-  }
-  for (int i = 0; i < k; i++) for (int j = 0; j < i; j++) { const double v = F.gc0 * std::sqrt(vb[M(i, i)] * vb[M(j, j)]); vb[M(i, j)] = v; vb[M(j, i)] = v; }
-  V.Sb = vb;
-  for (auto& v : V.Sb) v *= F.df0;
+  mrr_start(F, k, V);
+  Mat TildeHat((size_t)kk);
   std::vector<int> order(p), irgs(32);
   for (int64_t j = 0; j < p; j++) order[j] = (int)j;
   for (int j = 0; j < 32; j++) irgs[j] = j;
-  std::vector<double> W, bh, cnvB, cnvH2, cnvV, hsmall(32 * 4 + kk), trd(k);
+  std::vector<double> W, bh, hsmall(32 * 4 + kk), trd(k);
   if (NonLinear) { W.assign((size_t)p * k, 1.0); CU(cudaMemcpyAsync(Wd.p, W.data(), sizeof(double) * p * k, cudaMemcpyHostToDevice, st)); }
-  const double logtol = std::log10(F.tol);
-  int numit = 0, rc = 0;
+  int rc = 0;
   MrrGenArgs a;
   a.g = h->view(); a.k = k; a.rows_per_cta = rp; a.innergs = innergs ? 1 : 0; a.perm = permd.p; a.irgs = permd.p + p; a.zbits = zbits.p;
   a.e = ed.p; a.b = bd.p; a.fixed = fixd.p; a.mean = meand.p; a.sol = sold.p; a.se0 = d_se; a.acc = accd.p; a.scale = d_scale; a.err = h->err.p;
-  while (numit < maxit) {
-    const Mat vb0(vb); const std::vector<double> h20(h2);
+  while (V.numit < maxit) {
+    const Mat vb0(V.vb); const std::vector<double> h20(V.h2);
+    const int numit = V.numit;
     CU(cudaMemcpyAsync(bold.p, bd.p, sizeof(double) * p * k, cudaMemcpyDeviceToDevice, st));  // beta0 (:475)
     std::shuffle(order.begin(), order.end(), std::mt19937(numit));                           // :483-484, cumulative
     std::shuffle(irgs.begin(), irgs.begin() + k, std::mt19937(numit));
     CU(cudaMemcpyAsync(permd.p, order.data(), sizeof(int) * p, cudaMemcpyHostToDevice, st));
     CU(cudaMemcpyAsync(permd.p + p, irgs.data(), sizeof(int) * 32, cudaMemcpyHostToDevice, st));
-    CU(cudaMemcpyAsync(d_iG, iG.data(), sizeof(double) * kk, cudaMemcpyHostToDevice, st));
-    CU(cudaMemcpyAsync(d_vb, vb.data(), sizeof(double) * kk, cudaMemcpyHostToDevice, st));
-    CU(cudaMemcpyAsync(d_iVe, iVe.data(), sizeof(double) * k, cudaMemcpyHostToDevice, st));
+    CU(cudaMemcpyAsync(d_iG, V.iG.data(), sizeof(double) * kk, cudaMemcpyHostToDevice, st));
+    CU(cudaMemcpyAsync(d_vb, V.vb.data(), sizeof(double) * kk, cudaMemcpyHostToDevice, st));
+    CU(cudaMemcpyAsync(d_iVe, V.iVe.data(), sizeof(double) * k, cudaMemcpyHostToDevice, st));
     // MRR3 applies the marker weights in the solve (:504); MRR3F never does (its weights are an output only)
     launch_mrr_gen_systems((int)p, k, fixd.p, (NonLinear && !f32_variant) ? Wd.p : nullptr, d_iG, d_vb, d_iVe, noinv_system ? 1 : 0,
                            innergs ? 1 : 0, sold.p, st);
@@ -2520,15 +2524,11 @@ int mrr3_general(bwgr_handle* h, int f32_variant, const double* Y, int k, const 
       }
       CU(cudaMemcpyAsync(Wd.p, W.data(), sizeof(double) * p * k, cudaMemcpyHostToDevice, st));
     }
-    // ---- residual variances (:536-543)
-    for (int t = 0; t < k; t++) { ve[t] = (hsmall[t] + Se[t]) * iNp[t]; h2[t] = 1 - ve[t] / vy[t]; }
-    if (F.wph2 > 0) for (int t = 0; t < k; t++) ve[t] = ve[t] * (1 - F.wph2) + F.wph2 * veInit[t];
-    if (F.OneVarE) { double m = 0; for (int t = 0; t < k; t++) m += ve[t]; m /= k; for (int t = 0; t < k; t++) ve[t] = m; }
-    for (int t = 0; t < k; t++) iVe[t] = 1.0 / ve[t];
+    mrr_residual_var(F, k, hsmall.data(), 1, V);
     // ---- tilde-hat (:546-556) and the convergence sums (:662)
     if (F.TH) {
       std::vector<double> par(64, 0.0);
-      for (int t = 0; t < k; t++) { par[t] = ve[t]; par[k + t] = iG[M(t, t)]; }
+      for (int t = 0; t < k; t++) { par[t] = V.ve[t]; par[k + t] = V.iG[M(t, t)]; }
       CU(cudaMemcpyAsync(d_par, par.data(), sizeof(double) * 2 * k, cudaMemcpyHostToDevice, st));
       launch_mrr_gen_pk(2, xsxd.p, nullptr, dinvd.p, d_par, (int)p, k, d_trd, st);
       launch_mrr_gen_pk(0, bd.p, tilded.p, dinvd.p, nullptr, (int)p, k, d_th, st);
@@ -2543,7 +2543,7 @@ int mrr3_general(bwgr_handle* h, int f32_variant, const double* Y, int k, const 
     CU(cudaStreamSynchronize(st));
     for (int i = 0; i < k; i++) for (int j = 0; j < k; j++) TildeHat[M(i, j)] = hsmall[128 + (size_t)i * k + j];
     for (int t = 0; t < k; t++) trd[t] = hsmall[32 + t];
-    mrr_varcomp(F, k, TildeHat, F.TH ? trd : TrXSX, h2, V);
+    mrr_varcomp(F, k, TildeHat, F.TH ? trd : TrXSX, V.h2, V);
     if (F.updateMu) {  // :651-655; iN is 1 / (n_t - 1) by now (:395)
       launch_mrr_gen_colred(ed.p, nullptr, ld, (int)n, k, d_se, st);
       std::vector<double> sh(k);
@@ -2555,50 +2555,25 @@ int mrr3_general(bwgr_handle* h, int f32_variant, const double* Y, int k, const 
       CU(cudaStreamSynchronize(st));
       h->launches += 2;
     }
-    double mx = -1e300;
-    for (int t = 0; t < k; t++) mx = std::max(mx, hsmall[t]);
-    const double cnv = std::log10(mx);
-    cnvB.push_back(cnv);
-    if (cnv != cnv) break;  // :663
-    { double sH = 0; for (int t = 0; t < k; t++) sH += (h20[t] - h2[t]) * (h20[t] - h2[t]); cnvH2.push_back(std::log10(sH)); }
-    { double sV = 0; for (size_t i = 0; i < vb.size(); i++) sV += (vb0[i] - vb[i]) * (vb0[i] - vb[i]); cnvV.push_back(std::log10(sV)); }
-    ++numit;
-    if (cnv < logtol) break;
+    if (!mrr_record(F, k, hsmall.data(), vb0, h20, V)) break;
   }
   // ---- outputs (:676-700): hat = X_c b + mu = X b + (mu - sum_j mean_j b_j)
   bh.resize((size_t)p * k);
   CU(cudaMemcpyAsync(bh.data(), bd.p, sizeof(double) * p * k, cudaMemcpyDeviceToHost, st));
   CU(cudaStreamSynchronize(st));
-  {
-    DevBuf<float> bf, mud, hatd;
-    std::vector<float> bt(p), hh(n);
-    if (bf.alloc(p) != cudaSuccess || mud.alloc(1) != cudaSuccess || hatd.alloc(ld) != cudaSuccess) return fail(BWGR_ERR_CUDA, "cudaMalloc failed");
-    for (int t = 0; t < k && hat_out; t++) {
+  if (out.hat) {
+    std::vector<float> bt((size_t)k * p), m0(k), hh;
+    for (int t = 0; t < k; t++) {
       double shift = 0;
-      for (int64_t j = 0; j < p; j++) { const double v = bh[(size_t)j * k + t]; shift += meanv[j] * v; bt[j] = (float)v; }
-      const float m0 = (float)(mu[t] - shift);
-      CU(cudaMemcpyAsync(bf.p, bt.data(), sizeof(float) * p, cudaMemcpyHostToDevice, st));
-      CU(cudaMemcpyAsync(mud.p, &m0, sizeof(float), cudaMemcpyHostToDevice, st));
-      rc = fit_hat(h, bf.p, mud.p, hatd.p);
-      if (rc) return rc;
-      CU(cudaMemcpyAsync(hh.data(), hatd.p, sizeof(float) * n, cudaMemcpyDeviceToHost, st));
-      CU(cudaStreamSynchronize(st));
-      for (int64_t i = 0; i < n; i++) hat_out[(size_t)t * n + i] = hh[i];
+      for (int64_t j = 0; j < p; j++) { const double v = bh[(size_t)j * k + t]; shift += meanv[j] * v; bt[(size_t)t * p + j] = (float)v; }
+      m0[t] = (float)(mu[t] - shift);
     }
+    if ((rc = fitted_values(h, k, bt.data(), true, m0.data(), hh))) return rc;
+    for (size_t i = 0; i < hh.size(); i++) out.hat[i] = hh[i];
   }
-  for (int t = 0; t < k; t++) {
-    if (mu_out) mu_out[t] = mu[t];
-    if (h2_out) h2_out[t] = h2[t];
-    if (ve_out) ve_out[t] = ve[t];
-    if (MSx_out) MSx_out[t] = MSx[t];
-  }
-  if (b_out) for (int t = 0; t < k; t++) for (int64_t j = 0; j < p; j++) b_out[(size_t)t * p + j] = bh[(size_t)j * k + t];
-  if (W_out) for (int t = 0; t < k; t++) for (int64_t j = 0; j < p; j++) W_out[(size_t)t * p + j] = NonLinear ? W[(size_t)j * k + t] : 1.0;
-  if (GC_out) for (int i = 0; i < kk; i++) GC_out[i] = GC[i];
-  if (vb_out) for (int i = 0; i < kk; i++) vb_out[i] = vb[i];
-  if (cnv_out)
-    for (int i = 0; i < numit; i++) { cnv_out[i] = cnvB[i]; cnv_out[maxit + i] = cnvH2[i]; cnv_out[2 * maxit + i] = cnvV[i]; }
-  if (its_out) *its_out = numit;
+  if (out.b) for (int t = 0; t < k; t++) for (int64_t j = 0; j < p; j++) out.b[(size_t)t * p + j] = bh[(size_t)j * k + t];
+  if (out.W) for (int t = 0; t < k; t++) for (int64_t j = 0; j < p; j++) out.W[(size_t)t * p + j] = NonLinear ? W[(size_t)j * k + t] : 1.0;
+  mrr_copy_out(F, k, V, out);
   return 0;
 }
 }  // namespace
@@ -2614,8 +2589,8 @@ int bwgr_mrr3_fit(bwgr_handle* h, int f32_variant, const double* Y, int k, const
   if (!Y || !par) return fail(BWGR_ERR_ARG, "null argument");
   if (k < 1 || k > 32) return fail(BWGR_ERR_UNSUPPORTED, "MRR3 on the B200 path takes 1..32 traits (k=%d)", k);
   const MrrFlags F(par);
-  const int maxit = F.maxit; const double tol = F.tol, R2 = F.R2, gc0 = F.gc0, df0 = F.df0, wph2 = F.wph2;
-  const bool updateMu = F.updateMu, OneVarE = F.OneVarE;
+  const MrrOut out{mu_out, b_out, hat_out, h2_out, GC_out, vb_out, ve_out, MSx_out, cnv_out, W_out, its_out};
+  const int maxit = F.maxit;
   if (maxit < 1) return fail(BWGR_ERR_ARG, "maxit < 1");
   const int64_t n = h->n, p = h->p, ld = h->ld;
   bool missing = false;
@@ -2624,18 +2599,18 @@ int bwgr_mrr3_fit(bwgr_handle* h, int f32_variant, const double* Y, int k, const
   // MRR3F's NoInv system, the tilde-hat estimator -- runs on the general device path (mrr_gen.cu); BWGR_MRR=general forces it.
   const char* force = getenv("BWGR_MRR");
   if (missing || F.TH || F.NLfactor != 0 || F.InnerGS || (f32_variant && F.NoInv) || (force && !strcmp(force, "general")))
-    return mrr3_general(h, f32_variant, Y, k, F, mu_out, b_out, hat_out, h2_out, GC_out, vb_out, ve_out, MSx_out, cnv_out, W_out, its_out);
+    return mrr3_general(h, f32_variant, Y, k, F, out);
   auto M = [k](int r, int c) { return (size_t)r + (size_t)c * k; };
   // ---- setup (:359-432), double on the host
-  std::vector<double> mu(k), vy(k), ve(k), iVe(k), vbInit(k), veInit(k), h2(k), MSx(k), Se(k);
-  std::vector<double> yc((size_t)n * k);
+  MrrVar V;
+  V.mu.resize(k); V.vy.resize(k); V.nn.assign(k, (double)n);
   for (int t = 0; t < k; t++) {
     double s = 0;
     for (int64_t i = 0; i < n; i++) s += Y[(size_t)t * n + i];
-    mu[t] = s / (double)n;
+    V.mu[t] = s / (double)n;
     double ss = 0;
-    for (int64_t i = 0; i < n; i++) { const double v = Y[(size_t)t * n + i] - mu[t]; yc[(size_t)t * n + i] = v; ss += v * v; }
-    vy[t] = ss / ((double)n - 1.0);
+    for (int64_t i = 0; i < n; i++) { const double v = Y[(size_t)t * n + i] - V.mu[t]; ss += v * v; }
+    V.vy[t] = ss / ((double)n - 1.0);
   }
   std::vector<float> xxc(p), sxf(p);
   double msx = 0;
@@ -2645,33 +2620,19 @@ int bwgr_mrr3_fit(bwgr_handle* h, int f32_variant, const double* Y, int k, const
     msx += c / (double)n;                                              // XSX (:386-388): the centred column sums to zero
   }
   if (!(msx > 0)) return fail(BWGR_ERR_ARG, "genotypes have no variance");
-  const double TrXSX = (double)n * msx, iNp = 1.0 / ((double)n + df0 - 1.0);
-  MrrVar V;
-  Mat &vb = V.vb, &iG = V.iG, &GC = V.GC, &Sb = V.Sb, TildeHat((size_t)k * k);
-  vb.assign((size_t)k * k, 0.0); iG.assign((size_t)k * k, 0.0); GC.assign((size_t)k * k, 0.0);
-  for (int t = 0; t < k; t++) {
-    MSx[t] = msx; ve[t] = vy[t] * (1 - R2); iVe[t] = 1.0 / ve[t]; veInit[t] = ve[t];
-    vbInit[t] = vy[t] * R2 / msx; vb[M(t, t)] = vbInit[t]; iG[M(t, t)] = 1.0 / vbInit[t]; h2[t] = 1 - ve[t] / vy[t];
-  }
-  for (int i = 0; i < k; i++) for (int j = 0; j < i; j++) { const double v = gc0 * std::sqrt(vb[M(i, i)] * vb[M(j, j)]); vb[M(i, j)] = v; vb[M(j, i)] = v; }
-  Sb = vb;
-  for (auto& v : Sb) v *= df0;
-  V.vbInit = vbInit;
-  for (int t = 0; t < k; t++) Se[t] = ve[t] * df0;
+  const double TrXSX = (double)n * msx;
+  V.MSx.assign(k, msx);
+  mrr_start(F, k, V);
   // ---- device state through the common fit machinery: k systems of the rotated ridge rule
   FitSpec s;
   s.model = M_MRR; s.nsys = k; s.shuffled = true; s.row_mask = nullptr;
-  s.df = 0; s.R2 = (float)R2; s.Pi = 0; s.alpha = 0; s.pi = 0; s.it = maxit; s.bi = 0; s.seed = 0;
-  const int saved_path = h->path;
-  h->path = BWGR_PATH_BLOCKED;
+  s.df = 0; s.R2 = (float)F.R2; s.Pi = 0; s.alpha = 0; s.pi = 0; s.it = maxit; s.bi = 0; s.seed = 0;
+  FitGuard guard{h};
   int rc = fit_begin(h, s, Y);
-  h->path = saved_path;
-  Fit& f = h->fit;
-  if (rc == BWGR_ERR_UNSUPPORTED) {  // the shape does not fit the pipelined blocked sweep (row slabs above 512 rows): general path
-    f.reset();
-    return mrr3_general(h, f32_variant, Y, k, F, mu_out, b_out, hat_out, h2_out, GC_out, vb_out, ve_out, MSx_out, cnv_out, W_out, its_out);
-  }
+  if (rc == BWGR_ERR_UNSUPPORTED)  // the shape does not fit the pipelined blocked sweep (row slabs above 512 rows): general path
+    return mrr3_general(h, f32_variant, Y, k, F, out);
   if (rc) return rc;
+  Fit& f = h->fit;
   f.skip_epilogue = true;
   DevBuf<float> tilde, e_alt, b_alt, b_old, Tdev, amax;
   DevBuf<double> red, red2;
@@ -2687,16 +2648,16 @@ int bwgr_mrr3_fit(bwgr_handle* h, int f32_variant, const double* Y, int k, const
   CU(cudaMemcpyAsync(f.y.p, f.e.p, sizeof(float) * k * ld, cudaMemcpyDeviceToDevice, h->stream));
   launch_xty(h->view(), f.y.p, k, tilde.p, h->stream);  // tilde = X'y (:420)
   h->launches++;
-  std::vector<double> cnvB, cnvH2, cnvV, hred((size_t)k * k + 3 * k);
+  std::vector<double> hred((size_t)k * k + 3 * k);
   std::vector<float> Tf(32 * 32), Tif(32 * 32), hmax(32);
   std::vector<SysScalars> sc(f.sc0);
-  const double logtol = std::log10(tol);
-  int numit = 0;
-  while (numit < maxit) {
-    const Mat vb0(vb); const std::vector<double> h20(h2);
+  Mat TildeHat((size_t)k * k);
+  while (V.numit < maxit) {
+    const Mat vb0(V.vb); const std::vector<double> h20(V.h2);
+    const std::vector<double>& iVe = V.iVe;
     // ---- rotation of this sweep: S^-1 iG S^-1 = U Lambda U', T = S U, T^-1 = U' S^-1
     Mat Ms((size_t)k * k), U; std::vector<double> lam;
-    for (int i = 0; i < k; i++) for (int j = 0; j < k; j++) Ms[M(i, j)] = iG[M(i, j)] / std::sqrt(iVe[i] * iVe[j]);
+    for (int i = 0; i < k; i++) for (int j = 0; j < k; j++) Ms[M(i, j)] = V.iG[M(i, j)] / std::sqrt(iVe[i] * iVe[j]);
     sym_eig(Ms, k, lam, U);
     for (int sI = 0; sI < k; sI++) for (int t = 0; t < k; t++) {
       Tf[sI * k + t] = (float)(std::sqrt(iVe[sI]) * U[M(sI, t)]);       // T[s][t]
@@ -2709,26 +2670,23 @@ int bwgr_mrr3_fit(bwgr_handle* h, int f32_variant, const double* Y, int k, const
     launch_rotate(f.e.p, e_alt.p, ld, (int)n, k, Tdev.p, nullptr, amax.p, h->num_sms, h->stream);
     launch_rotate(f.b.p, b_alt.p, p, (int)p, k, Tdev.p, nullptr, nullptr, h->num_sms, h->stream);
     h->launches += 2;
-    std::swap(f.e.p, e_alt.p); std::swap(f.b.p, b_alt.p);
+    f.e.swap(e_alt); f.b.swap(b_alt);
     CU(cudaMemcpyAsync(hmax.data(), amax.p, sizeof(float) * 32, cudaMemcpyDeviceToHost, h->stream));
     CU(cudaStreamSynchronize(h->stream));
     for (int t = 0; t < k; t++) {
       SysScalars& c = sc[t];
       c.lmb = (float)std::max(lam[t], 0.0);
-      int ex = 0;
-      if (hmax[t] > 0) std::frexp(hmax[t], &ex);
-      if (ex < -60) ex = -60;
-      c.e_q = std::ldexp(1.0f, ex + 3 - 30); c.e_qinv = std::ldexp(1.0f, 30 - 3 - ex);
-      c.done = 0; c.sweep = numit;
+      set_e_scale(c, hmax[t]);
+      c.done = 0; c.sweep = V.numit;
     }
     CU(cudaMemcpyAsync(f.sc.p, sc.data(), sizeof(SysScalars) * k, cudaMemcpyHostToDevice, h->stream));
     CU(cudaMemsetAsync(f.cshift.p, 0, sizeof(float) * 32, h->stream));
     rc = fit_sweeps(h, 1);  // marker order shuffle(mt19937(numit)) (:483), centred Gram band, k-system sweep
-    if (rc) { std::swap(f.e.p, e_alt.p); std::swap(f.b.p, b_alt.p); return rc; }
+    if (rc) return rc;
     // ---- back to trait space: E = (E~ + c) T^-1, b = b~ T^-1
     launch_rotate(f.e.p, e_alt.p, ld, (int)n, k, Tdev.p + 1024, f.cshift.p, nullptr, h->num_sms, h->stream);
     launch_rotate(f.b.p, b_alt.p, p, (int)p, k, Tdev.p + 1024, nullptr, nullptr, h->num_sms, h->stream);
-    std::swap(f.e.p, e_alt.p); std::swap(f.b.p, b_alt.p);
+    f.e.swap(e_alt); f.b.swap(b_alt);
     // ---- reductions of the sweep epilogue: b'tilde (:549), e.y (:536), |beta0 - b|^2 (:662), column sums of e (:652)
     launch_pair_reduce(f.b.p, tilde.p, p, p, (int)p, k, 0, red.p, h->stream);
     launch_pair_reduce(f.e.p, f.y.p, ld, ld, (int)n, k, 0, red2.p, h->stream);
@@ -2742,68 +2700,40 @@ int bwgr_mrr3_fit(bwgr_handle* h, int f32_variant, const double* Y, int k, const
     for (int i = 0; i < k; i++) for (int j = 0; j < k; j++) TildeHat[M(i, j)] = hred[(size_t)i * k + j];
     for (int t = 0; t < 2 * k; t++) small[t] = hred[(size_t)k * k + t];
     rc = check_err_flag(h, "MRR3 sweep");
-    if (rc) { f.reset(); return rc; }
+    if (rc) return rc;
     // ---- variance components (:536-648), double
-    for (int t = 0; t < k; t++) { ve[t] = (ey[(size_t)t * k + t] + Se[t]) * iNp; h2[t] = 1 - ve[t] / vy[t]; }
-    if (wph2 > 0) for (int t = 0; t < k; t++) ve[t] = ve[t] * (1 - wph2) + wph2 * veInit[t];
-    if (OneVarE) { double m = 0; for (int t = 0; t < k; t++) m += ve[t]; m /= k; for (int t = 0; t < k; t++) ve[t] = m; }
-    for (int t = 0; t < k; t++) iVe[t] = 1.0 / ve[t];
-    { const std::vector<double> Tr((size_t)k, TrXSX); mrr_varcomp(F, k, TildeHat, Tr, h2, V); }
-    if (updateMu) {  // :651-655 (complete Y: Z = 1)
+    mrr_residual_var(F, k, ey.data(), k + 1, V);  // e.y of trait t: the diagonal of the k x k products
+    { const std::vector<double> Tr((size_t)k, TrXSX); mrr_varcomp(F, k, TildeHat, Tr, V.h2, V); }
+    if (F.updateMu) {  // :651-655 (complete Y: Z = 1)
       std::vector<float> sh(k);
-      for (int t = 0; t < k; t++) { const double m = small[k + t] / ((double)n - 1.0); mu[t] += m; sh[t] = (float)(-m); }
+      for (int t = 0; t < k; t++) { const double m = small[k + t] / ((double)n - 1.0); V.mu[t] += m; sh[t] = (float)(-m); }
       // e -= m: a rotation by the identity with a shift
       std::vector<float> I((size_t)k * k, 0.0f);
       for (int t = 0; t < k; t++) I[(size_t)t * k + t] = 1.0f;
       CU(cudaMemcpyAsync(Tdev.p, I.data(), sizeof(float) * k * k, cudaMemcpyHostToDevice, h->stream));
       CU(cudaMemcpyAsync(f.cshift.p, sh.data(), sizeof(float) * k, cudaMemcpyHostToDevice, h->stream));
       launch_rotate(f.e.p, e_alt.p, ld, (int)n, k, Tdev.p, f.cshift.p, nullptr, h->num_sms, h->stream);
-      std::swap(f.e.p, e_alt.p);
+      f.e.swap(e_alt);
       CU(cudaStreamSynchronize(h->stream));
     }
-    double mx = -1e300;
-    for (int t = 0; t < k; t++) mx = std::max(mx, small[t]);
-    const double cnv = std::log10(mx);
-    cnvB.push_back(cnv);
-    if (cnv != cnv) break;  // :663
-    { double sH = 0; for (int t = 0; t < k; t++) sH += (h20[t] - h2[t]) * (h20[t] - h2[t]); cnvH2.push_back(std::log10(sH)); }
-    { double sV = 0; for (size_t i = 0; i < vb.size(); i++) sV += (vb0[i] - vb[i]) * (vb0[i] - vb[i]); cnvV.push_back(std::log10(sV)); }
-    ++numit;
-    if (cnv < logtol) break;
+    if (!mrr_record(F, k, small.data(), vb0, h20, V)) break;
   }
   // ---- outputs (:676-700): hat = X_c b + mu = X b + (mu - sum_j mean_j b_j)
-  std::vector<float> hb((size_t)k * p), hh(n);
+  std::vector<float> hb((size_t)k * p), m0(k), hh;
   CU(cudaMemcpyAsync(hb.data(), f.b.p, sizeof(float) * k * p, cudaMemcpyDeviceToHost, h->stream));
   CU(cudaStreamSynchronize(h->stream));
-  DevBuf<float> mud, hatd;
-  if (mud.alloc(1) != cudaSuccess || hatd.alloc(ld) != cudaSuccess) return fail(BWGR_ERR_CUDA, "cudaMalloc failed");
   for (int t = 0; t < k; t++) {
     double shift = 0;
     for (int64_t j = 0; j < p; j++) shift += (h->h_sx[j] / (double)n) * (double)hb[(size_t)t * p + j];
-    const float m0 = (float)(mu[t] - shift);
-    CU(cudaMemcpyAsync(mud.p, &m0, sizeof(float), cudaMemcpyHostToDevice, h->stream));
-    rc = fit_hat(h, f.b.p + (size_t)t * p, mud.p, hatd.p);
-    if (rc) return rc;
-    CU(cudaMemcpyAsync(hh.data(), hatd.p, sizeof(float) * n, cudaMemcpyDeviceToHost, h->stream));
-    CU(cudaStreamSynchronize(h->stream));
-    if (hat_out) for (int64_t i = 0; i < n; i++) hat_out[(size_t)t * n + i] = hh[i];
+    m0[t] = (float)(V.mu[t] - shift);
   }
-  for (int t = 0; t < k; t++) {
-    if (mu_out) mu_out[t] = mu[t];
-    if (h2_out) h2_out[t] = h2[t];
-    if (ve_out) ve_out[t] = ve[t];
-    if (MSx_out) MSx_out[t] = MSx[t];
-  }
+  rc = fitted_values(h, k, f.b.p, false, m0.data(), hh);
+  if (rc) return rc;
+  if (hat_out) for (size_t i = 0; i < hh.size(); i++) hat_out[i] = hh[i];
   if (b_out) for (size_t i = 0; i < hb.size(); i++) b_out[i] = hb[i];
   if (W_out) for (size_t i = 0; i < (size_t)k * p; i++) W_out[i] = 1.0;
-  if (GC_out) for (int i = 0; i < k * k; i++) GC_out[i] = GC[i];
-  if (vb_out) for (int i = 0; i < k * k; i++) vb_out[i] = vb[i];
-  if (cnv_out)
-    for (int i = 0; i < numit; i++) { cnv_out[i] = cnvB[i]; cnv_out[maxit + i] = cnvH2[i]; cnv_out[2 * maxit + i] = cnvV[i]; }
-  if (its_out) *its_out = numit;
-  // the swapped buffers go back to their owners before the fit is released
+  mrr_copy_out(F, k, V, out);
   dump_trace(h);
-  f.reset();
   return 0;
 }
 

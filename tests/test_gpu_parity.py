@@ -605,6 +605,20 @@ def test_error_paths_and_edges(tpod):
         assert np.abs(o["b"] - ref["b"]).max() <= RTOL * np.abs(ref["b"]).max(), (n, p)
 
 
+def test_failed_one_shot_call_releases_its_fit(tpod):
+    """A one-shot entry point that fails after its fit has started leaves no fit behind: the stepper calls that follow report
+    BWGR_ERR_STATE instead of sweeping the failed fit."""
+    y, gen = tpod
+    with bw.Genotypes(gen) as g:
+        yn = y.copy(); yn[7] = np.nan                        # GSRR checks y after fit_begin has taken e
+        p = g.p
+        with pytest.raises(bw.BwgrError):
+            bw.GSRR(yn, y - y.mean(), g, np.zeros(p), np.ones(p), np.ones(p), 1.0)
+        assert g.lib.bwgr_em_sweeps(g.h, 1) == -3
+        buf = bw.api._EmBuffers(g.n, g.p, 1)
+        assert g.lib.bwgr_em_end(g.h, ctypes.byref(buf.c)) == -3
+
+
 def test_signed_genotypes_blocked_path():
     """General int8 genotypes (centred / negative codes): the kind::i8 Gram path and the limb products stay exact."""
     rng = np.random.default_rng(4)
