@@ -2031,7 +2031,9 @@ static int wgr_fit(bwgr_handle* h, const double* y, int it, int bi, int th, doub
     for (int64_t i = 0; i < n; i++) yf[i] = (float)y[i];
     CU(cudaMemcpyAsync(yd.p, yf.data(), sizeof(float) * ld, cudaMemcpyHostToDevice, h->stream));
     CU(cudaStreamSynchronize(h->stream));
-    w.mask = rp ? f.cnt.p : f.mask.p; w.nsub = (float)nuse; w.y = yd.p; w.hat = hatd.p;  // phase 1 weighs e^2 by the byte (0/1 or the multiplicity)
+    // phase 1 weighs e^2 by the byte (0/1 or the multiplicity); Ve's chi-square has n * bag + df degrees of freedom (:121), n * bag
+    // unrounded although the sample holds floor(n * bag) rows
+    w.mask = rp ? f.cnt.p : f.mask.p; w.nsub = (float)((double)n * bag); w.y = yd.p; w.hat = hatd.p;
     ColStatBufs cs;
     for (int i = 0; i < it; i++) {
       if (i > 0) {  // this iteration's rows: mask, and H'H of every marker over them (the rule's likelihood-ratio scale)

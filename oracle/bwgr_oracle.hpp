@@ -25,7 +25,8 @@
 //     accumulators, then horizontal add), LLT, self-adjoint EVD (Jacobi here) and the
 //     pseudo-inverse (EVD based here; vb is symmetric).
 //   Rmath (R >= 4.0): rnorm / rchisq / rbinom -> std::mt19937_64 + <random> distributions.
-//     R's RNG stream is irreproducible outside R; Gibbs parity is statistical (posterior means).
+//     R's RNG stream is irreproducible outside R; Gibbs parity with it is statistical (posterior means).  PhiloxDraws replays the
+//     device's own draws instead, which makes each chain a deterministic function of the seed.
 #pragma once
 #include <algorithm>
 #include <cmath>
@@ -597,8 +598,14 @@ static void em_fit(int model, const R* y, const R* X, int n, int p, const EmPar<
 }
 
 // ------------------------------------------------------------------------------------------------
-// RNG stand-in for Rmath (R::rnorm / R::rchisq / R::rbinom).
+// Draw sources.  The samplers below ask for every random number at a named site:
+//   effect(m, s)    marker effect  ~ N(m, s)          excluded(s)    excluded effect ~ N(0, s)
+//   include(q)      inclusion test, true with prob. q  chi_marker(nu) per-marker chi-square
+//   intercept(m, s) intercept of a Gibbs sweep         chi_e(nu), chi_b(nu)  residual / marker variance of a Gibbs sweep
+//   wgr_Ve, wgr_Va, wgr_mu0, wgr_Vb(j, .), wgr_Vp  the draws of wgr's driver      rows(...)  wgr's row sample of one iteration
+// and tell the source where they are (set_sweep, set_marker, set_chain).
 // ------------------------------------------------------------------------------------------------
+// Rng: the stand-in for Rmath (R::rnorm / R::rchisq / R::rbinom), one std::mt19937_64 stream consumed in the reference's order.
 struct Rng {
   std::mt19937_64 g;
   explicit Rng(uint64_t seed) : g(seed) {}
@@ -609,6 +616,135 @@ struct Rng {
     if (!(p == p)) return std::numeric_limits<double>::quiet_NaN();
     std::uniform_real_distribution<double> u(0.0, 1.0);
     return u(g) < p ? 1.0 : 0.0;
+  }
+  void set_sweep(int) {}
+  void set_marker(int) {}
+  double effect(double m, double s) { return rnorm(m, s); }
+  double excluded(double s) { return rnorm(0, s); }
+  bool include(double q) { return rbinom1(q) == 1; }
+  double chi_marker(double nu) { return rchisq(nu); }
+  double intercept(double m, double s) { return rnorm(m, s); }
+  double chi_e(double nu) { return rchisq(nu); }
+  double chi_b(double nu) { return rchisq(nu); }
+  double wgr_Ve(double nu) { return rchisq(nu); }
+  double wgr_Va(double nu) { return rchisq(nu); }
+  double wgr_mu0(double m, double s) { return rnorm(m, s); }
+  double wgr_Vb(int, double nu) { return rchisq(nu); }
+  double wgr_Vp(double nu) { return rchisq(nu); }
+  // sample(n, nuse, rp) of R/wgr.R:68, unsorted, in rows[0, nuse)
+  void rows(int n, int nuse, bool rp, std::vector<int>& rows) {
+    if (rp) {
+      rows.resize(std::max(n, nuse));
+      std::uniform_int_distribution<int> pick(0, n - 1);
+      for (int r = 0; r < nuse; r++) rows[r] = pick(g);
+    } else {
+      for (int r = 0; r < n; r++) rows[r] = r;
+      for (int r = 0; r < nuse; r++) { std::uniform_int_distribution<int> pick(r, n - 1); std::swap(rows[r], rows[pick(g)]); }
+    }
+  }
+};
+
+// PhiloxDraws: the device's counter-addressed draws (Philox4x32-10, key = the seed), restated on the host so that a chain is a
+// deterministic function of the seed and can be compared with the device draw for draw.  Counters:
+//   marker draws z1, z2, u    (marker, sweep, chain, 0)        per-marker chi-square   (marker, sweep, chain, 1 + (attempt << 8))
+//   Gibbs sweep epilogue      (0xFFFFFFFF, sweep, chain, p): intercept p = 0, chi_e p = 1, chi_b p = 2
+//   wgr driver                (0xFFFFFFFE, sweep, 0, p): mu0 p = 0, Ve p = 1, Va p = 2       wgr per-marker Vb  (marker, sweep, 0, 3)
+// Every draw is made in float, as on the device; the sampler may then run in float or double on the same draws.  wgr's row samples
+// come from std::mt19937_64(seed ^ 0x9E3779B97F4A7C15) with int64 uniform_int_distribution, as in the C ABI's bagged driver.
+// The source records how close every accept / reject decision came to the other outcome: q[] (the inclusion probability of each
+// include() call) and u[] (the uniform it was tested with), and mt_margin, the smallest |log u - (0.5 x^2 + d - d v + d log v)| / (1 + d)
+// of every Marsaglia-Tsang acceptance test.
+namespace philox {
+inline void philox4x32_10(uint32_t c[4], uint32_t k0, uint32_t k1) {
+  const uint32_t M0 = 0xD2511F53u, M1 = 0xCD9E8D57u, W0 = 0x9E3779B9u, W1 = 0xBB67AE85u;
+  for (int r = 0; r < 10; r++) {
+    const uint64_t p0 = (uint64_t)M0 * c[0], p1 = (uint64_t)M1 * c[2];
+    const uint32_t n0 = (uint32_t)(p1 >> 32) ^ c[1] ^ k0, n1 = (uint32_t)p1;
+    const uint32_t n2 = (uint32_t)(p0 >> 32) ^ c[3] ^ k1, n3 = (uint32_t)p0;
+    c[0] = n0; c[1] = n1; c[2] = n2; c[3] = n3;
+    k0 += W0; k1 += W1;
+  }
+}
+inline float u01(uint32_t x) { return (float)((x >> 8) + 1) * (1.0f / 16777216.0f); }  // (0, 1], 24 bits
+// sincospi(t) as sin / cos of pi t in double, rounded to float
+inline void box_muller(uint32_t a, uint32_t b, float& z0, float& z1) {
+  const float r = std::sqrt(-2.0f * std::log(u01(a)));
+  const double t = 3.14159265358979323846 * (double)(2.0f * u01(b));
+  z0 = r * (float)std::cos(t);
+  z1 = r * (float)std::sin(t);
+}
+// chi-square(nu) = 2 Gamma(nu / 2) by Marsaglia-Tsang, each attempt its own counter; a < 1 is boosted by u^(1/a)
+inline float rchisq(float nu, uint32_t c0, uint32_t c1, uint32_t c2, uint32_t purpose, uint32_t k0, uint32_t k1, double& margin) {
+  float a = 0.5f * nu;
+  const bool boost = a < 1.0f;
+  if (boost) a += 1.0f;
+  const float d = a - (1.0f / 3.0f), cc = 1.0f / std::sqrt(9.0f * d);
+  float out = d, ub = 1.0f;
+  for (uint32_t att = 0; att < 64; att++) {
+    uint32_t c[4] = {c0, c1, c2, purpose + (att << 8)};
+    philox4x32_10(c, k0, k1);
+    float x, unused;
+    box_muller(c[0], c[1], x, unused);
+    const float u = u01(c[2]);
+    ub = u01(c[3]);
+    float v = 1.0f + cc * x;
+    if (v <= 0.0f) continue;
+    v = v * v * v;
+    const float lhs = std::log(u), rhs = 0.5f * x * x + d - d * v + d * std::log(v);
+    margin = std::min(margin, (double)std::fabs(lhs - rhs) / (1.0 + d));
+    if (lhs < rhs) { out = d * v; break; }
+  }
+  if (boost) out *= std::pow(ub, 1.0f / (0.5f * nu));
+  return 2.0f * out;
+}
+}  // namespace philox
+
+struct PhiloxDraws {
+  uint32_t k0, k1, chain = 0, sweep = 0, marker = 0;
+  float z1 = 0, z2 = 0, u = 0;
+  std::vector<float> q, uq;
+  double mt_margin = std::numeric_limits<double>::infinity();
+  uint64_t seed;
+  std::mt19937_64 row_gen;
+  explicit PhiloxDraws(uint64_t s) : k0((uint32_t)s), k1((uint32_t)(s >> 32)), seed(s), row_gen(s ^ 0x9E3779B97F4A7C15ull) {}
+  void set_chain(int c) { chain = (uint32_t)c; }
+  void set_sweep(int i) { sweep = (uint32_t)i; }
+  void set_marker(int j) {
+    marker = (uint32_t)j;
+    uint32_t c[4] = {marker, sweep, chain, 0u};
+    philox::philox4x32_10(c, k0, k1);
+    philox::box_muller(c[0], c[1], z1, z2);
+    u = philox::u01(c[2]);
+  }
+  double effect(double m, double s) { return m + s * (double)z1; }
+  double excluded(double s) { return s * (double)z2; }
+  bool include(double qj) { q.push_back((float)qj); uq.push_back(u); return (double)u < qj; }
+  double chi_marker(double nu) { return philox::rchisq((float)nu, marker, sweep, chain, 1u, k0, k1, mt_margin); }
+  double scalar_normal(uint32_t c0, uint32_t ch) {
+    uint32_t c[4] = {c0, sweep, ch, 0u};
+    philox::philox4x32_10(c, k0, k1);
+    float z, unused;
+    philox::box_muller(c[0], c[1], z, unused);
+    return z;
+  }
+  double intercept(double m, double s) { return m + s * scalar_normal(0xFFFFFFFFu, chain); }
+  double chi_e(double nu) { return philox::rchisq((float)nu, 0xFFFFFFFFu, sweep, chain, 1u, k0, k1, mt_margin); }
+  double chi_b(double nu) { return philox::rchisq((float)nu, 0xFFFFFFFFu, sweep, chain, 2u, k0, k1, mt_margin); }
+  double wgr_mu0(double m, double s) { return m + s * scalar_normal(0xFFFFFFFEu, 0u); }
+  double wgr_Ve(double nu) { return philox::rchisq((float)nu, 0xFFFFFFFEu, sweep, 0u, 1u, k0, k1, mt_margin); }
+  double wgr_Va(double nu) { return philox::rchisq((float)nu, 0xFFFFFFFEu, sweep, 0u, 2u, k0, k1, mt_margin); }
+  double wgr_Vb(int j, double nu) { return philox::rchisq((float)nu, (uint32_t)j, sweep, 0u, 3u, k0, k1, mt_margin); }
+  // wgr with eigK has no device counters (its driver draws with numpy): a replay of it is not defined
+  double wgr_Vp(double) { return std::numeric_limits<double>::quiet_NaN(); }
+  void rows(int n, int nuse, bool rp, std::vector<int>& rows) {
+    if (rp) {
+      rows.resize(std::max(n, nuse));
+      std::uniform_int_distribution<int64_t> pick(0, n - 1);
+      for (int r = 0; r < nuse; r++) rows[r] = (int)pick(row_gen);
+    } else {
+      for (int r = 0; r < n; r++) rows[r] = r;
+      for (int r = 0; r < nuse; r++) { std::uniform_int_distribution<int64_t> pick(r, n - 1); std::swap(rows[r], rows[pick(row_gen)]); }
+    }
   }
 };
 
@@ -627,10 +763,9 @@ struct GibbsOut {
 // BayesDpi :922-987 of Rcpp20260726ai.cpp.  BayesL = BayesA with Lmb_j = sqrt(Phi ve / vb_j) after the first sweep;
 // BayesCpi = BayesC started at pi = 0.5 whose prior scale Sb follows the mean inclusion (the mixing odds Pi0 stay fixed);
 // BayesDpi = per-marker variances with the Kuo-Mallick style acceptance min(1, (1 - pi) exp(C(|e1|^2 - |e2|^2))), pi = mean(d).
-template <class R>
+template <class R, class Draws>
 static void gibbs_fit(int model, const R* y, const R* X, int n, int p, R it_f, R bi_f, R pi, R df, R R2,
-                      uint64_t seed, GibbsOut<R>& o) {
-  Rng rng(seed);
+                      Draws& rng, GibbsOut<R>& o) {
   const int iit = (int)it_f, ibi = (int)bi_f;
   const R MCMC = it_f - bi_f;
   std::vector<R> xx, vx;
@@ -656,48 +791,50 @@ static void gibbs_fit(int model, const R* y, const R* X, int n, int p, R it_f, R
   const R Pi0 = pi / (R(1.0) - pi);
   for (int i = 0; i < iit; i++) {
     const R C = R(-0.5) / std::sqrt(ve);
+    rng.set_sweep(i);
     for (int j = 0; j < p; j++) {
+      rng.set_marker(j);
       const R* x = X + (size_t)j * n;
       const R L = per_marker ? Lmbv[j] : Lmb;
       const R b0 = b[j];
       const R sd = std::sqrt(ve / (xx[j] + L));
-      const R b1 = (R)rng.rnorm((vdot(x, e.data(), n) + xx[j] * b0) / (xx[j] + L), sd);
+      const R b1 = (R)rng.effect((vdot(x, e.data(), n) + xx[j] * b0) / (xx[j] + L), sd);
       if (model == GB_CPI || model == GB_DPI) {  // both draw b2 before the test (:886, :951)
-        const R b2 = (R)rng.rnorm(0, sd);
+        const R b2 = (R)rng.excluded(sd);
         const R n1 = sq_after(e.data(), x, b1 - b0, t1.data(), n);
         const R n2 = sq_after(e.data(), x, (model == GB_DPI ? b2 : R(0)) - b0, t2.data(), n);
         R pj;
         if (model == GB_CPI) pj = R(1.0) / (R(1.0) + Pi0 * std::exp(C * (n2 - n1)));
         else { pj = (1 - pi) * std::exp(C * (n1 - n2)); if (pj > 1) pj = 1; }
-        if (rng.rbinom1(pj) == 1) { b[j] = b1; d[j] = 1; }
+        if (rng.include(pj)) { b[j] = b1; d[j] = 1; }
         else { b[j] = b2; d[j] = 0; }
       } else if (spike) {
         const R n1 = sq_after(e.data(), x, b1 - b0, t1.data(), n);
         const R n2 = sq_after(e.data(), x, R(0) - b0, t2.data(), n);
         const R LR = Pi0 * std::exp(C * (n2 - n1));
         const R pj = R(1.0) / (R(1.0) + LR);
-        if (rng.rbinom1(pj) == 1) { b[j] = b1; d[j] = 1; }
-        else { b[j] = (R)rng.rnorm(0, sd); d[j] = 0; }
+        if (rng.include(pj)) { b[j] = b1; d[j] = 1; }
+        else { b[j] = (R)rng.excluded(sd); d[j] = 0; }
       } else {
         b[j] = b1;
       }
-      if (per_marker) vbv[j] = (Sb + b[j] * b[j]) / (R)rng.rchisq(df + 1);
+      if (per_marker) vbv[j] = (Sb + b[j] * b[j]) / (R)rng.chi_marker(df + 1);
       axpy_sub(e.data(), x, b[j] - b0, n);
     }
-    const R eM = (R)rng.rnorm(vmean(e.data(), n), std::sqrt(ve / n));
+    const R eM = (R)rng.intercept(vmean(e.data(), n), std::sqrt(ve / n));
     mu += eM;
     for (int r = 0; r < n; r++) e[r] -= eM;
     if (model == GB_RR) {  // :841-843 (ve first, then vb)
-      ve = (vsq(e.data(), n) + Se) / (R)rng.rchisq(n + df);
-      vb = (vsq(b.data(), p) + Sb) / (R)rng.rchisq(p + df);
+      ve = (vsq(e.data(), n) + Se) / (R)rng.chi_e(n + df);
+      vb = (vsq(b.data(), p) + Sb) / (R)rng.chi_b(p + df);
       Lmb = ve / vb;
     } else if (c_like) {  // :745-747, :903-907 (vb first, then ve)
-      vb = (vsq(b.data(), p) + Sb) / (R)rng.rchisq(df + p);
-      ve = (vsq(e.data(), n) + Se) / (R)rng.rchisq(n + df);
+      vb = (vsq(b.data(), p) + Sb) / (R)rng.chi_b(df + p);
+      ve = (vsq(e.data(), n) + Se) / (R)rng.chi_e(n + df);
       Lmb = ve / vb;
       if (model == GB_CPI) { pi = vmean(d.data(), p); Sb = df * R2 * vy / MSx / (1 - pi); }  // Pi0 is NOT refreshed (:906-907)
     } else {
-      ve = (vsq(e.data(), n) + Se) / (R)rng.rchisq(n + df);
+      ve = (vsq(e.data(), n) + Se) / (R)rng.chi_e(n + df);
       if (model == GB_L) for (int j = 0; j < p; j++) Lmbv[j] = std::sqrt(Phi * ve / vbv[j]);  // :799
       else for (int j = 0; j < p; j++) Lmbv[j] = ve * (R(1) / vbv[j]);
       if (model == GB_DPI) pi = vmean(d.data(), p);  // :969
@@ -725,31 +862,32 @@ static void gibbs_fit(int model, const R* y, const R* X, int n, int p, R it_f, R
 // ratio_form=false restates the reference literally (exp(C*||e1||^2) etc., which underflows to
 // NaN -> "else" branch for large n*Ve); ratio_form=true is the algebraically identical
 // 1/(1+pi/(1-pi)*exp(C*(||e2||^2-||e1||^2))) that the CUDA path implements.
-static inline void kmup(const float* X, int n, int p, float* b, float* d, const float* xx, float* e,
-                        const float* L, float Ve, float pi, Rng& rng, bool ratio_form) {
-  std::vector<float> e1(n), e2(n);
-  const float C = -0.5f / std::sqrt(Ve);
+template <class R, class Draws>
+static void kmup(const R* X, int n, int p, R* b, R* d, const R* xx, R* e, const R* L, R Ve, R pi, Draws& rng, bool ratio_form) {
+  std::vector<R> e1(n), e2(n);
+  const R C = R(-0.5f) / std::sqrt(Ve);
   for (int j = 0; j < p; j++) {
-    const float* x = X + (size_t)j * n;
-    const float b0 = b[j];
-    const float sd = std::sqrt(Ve / (xx[j] + L[j]));
-    const float b1 = (float)rng.rnorm((vdot(x, e, n) + xx[j] * b0) / (xx[j] + L[j]), sd);
-    const float b2 = (float)rng.rnorm(0, sd);
+    rng.set_marker(j);
+    const R* x = X + (size_t)j * n;
+    const R b0 = b[j];
+    const R sd = std::sqrt(Ve / (xx[j] + L[j]));
+    const R b1 = (R)rng.effect((vdot(x, e, n) + xx[j] * b0) / (xx[j] + L[j]), sd);
+    const R b2 = (R)rng.excluded(sd);
     for (int i = 0; i < n; i++) e1[i] = e[i] - x[i] * (b1 - b0);
     if (pi > 0) {
       for (int i = 0; i < n; i++) e2[i] = e[i] - x[i] * (b2 - b0);
-      float pj;
+      R pj;
       if (ratio_form) {
-        pj = 1.0f / (1.0f + (pi / (1 - pi)) * std::exp(C * (vsq(e2.data(), n) - vsq(e1.data(), n))));
+        pj = R(1.0f) / (R(1.0f) + (pi / (1 - pi)) * std::exp(C * (vsq(e2.data(), n) - vsq(e1.data(), n))));
       } else {
-        const float cj = (1 - pi) * std::exp(C * vsq(e1.data(), n));
-        const float dj = (pi)*std::exp(C * vsq(e2.data(), n));
+        const R cj = (1 - pi) * std::exp(C * vsq(e1.data(), n));
+        const R dj = (pi)*std::exp(C * vsq(e2.data(), n));
         pj = cj / (cj + dj);
       }
-      if (rng.rbinom1(pj) == 1) { b[j] = b1; d[j] = 1; std::memcpy(e, e1.data(), sizeof(float) * n); }
-      else { b[j] = b2; d[j] = 0; std::memcpy(e, e2.data(), sizeof(float) * n); }
+      if (rng.include(pj)) { b[j] = b1; d[j] = 1; std::memcpy(e, e1.data(), sizeof(R) * n); }
+      else { b[j] = b2; d[j] = 0; std::memcpy(e, e2.data(), sizeof(R) * n); }
     } else {
-      d[j] = 1; b[j] = b1; std::memcpy(e, e1.data(), sizeof(float) * n);
+      d[j] = 1; b[j] = b1; std::memcpy(e, e1.data(), sizeof(R) * n);
     }
   }
 }
@@ -909,36 +1047,38 @@ static inline void emml2_fit(const float* y, const float* X1, const float* X2, i
 
 // KMUP2: Rcpp20260726ai.cpp:41-77.  The bagged sweep of wgr(bag != 1): only the rows `use` enter; note (H.e0 + b0) without the xx
 // factor (:59, sic) and xx scaled by bg = n0 / n.  e_out has length nuse.
-static inline void kmup2(const float* X, int n0, int p, const float* use, int nuse, float* b, float* d, const float* xx, const float* E,
-                         float* e_out, const float* L, float Ve, float pi, Rng& rng, bool ratio_form) {
+template <class R, class Draws>
+static void kmup2(const R* X, int n0, int p, const float* use, int nuse, R* b, R* d, const R* xx, const R* E, R* e_out, const R* L, R Ve,
+                  R pi, Draws& rng, bool ratio_form) {
   const int n = nuse;
-  const float C = -0.5f / std::sqrt(Ve);
-  const float bg = (float)n0 / (float)n;
-  std::vector<float> e0(n), H(n), e1(n), e2(n);
+  const R C = R(-0.5f) / std::sqrt(Ve);
+  const R bg = (R)((float)n0 / (float)n);
+  std::vector<R> e0(n), H(n), e1(n), e2(n);
   for (int k = 0; k < n; k++) e0[k] = E[(int)use[k]];
   for (int j = 0; j < p; j++) {
+    rng.set_marker(j);
     for (int x = 0; x < n; x++) H[x] = X[(size_t)j * n0 + (int)use[x]];
-    const float b0 = b[j];
-    const float sd = std::sqrt(Ve / (xx[j] * bg + L[j]));
-    const float b1 = (float)rng.rnorm((vdot(H.data(), e0.data(), n) + b0) / (xx[j] * bg + L[j]), sd);
-    const float b2 = (float)rng.rnorm(0, sd);
+    const R b0 = b[j];
+    const R sd = std::sqrt(Ve / (xx[j] * bg + L[j]));
+    const R b1 = (R)rng.effect((vdot(H.data(), e0.data(), n) + b0) / (xx[j] * bg + L[j]), sd);
+    const R b2 = (R)rng.excluded(sd);
     for (int i = 0; i < n; i++) e1[i] = e0[i] - H[i] * (b1 - b0);
     if (pi > 0) {
       for (int i = 0; i < n; i++) e2[i] = e0[i] - H[i] * (b2 - b0);
-      float pj;
-      if (ratio_form) pj = 1.0f / (1.0f + (pi / (1 - pi)) * std::exp(C * (vsq(e2.data(), n) - vsq(e1.data(), n))));
+      R pj;
+      if (ratio_form) pj = R(1.0f) / (R(1.0f) + (pi / (1 - pi)) * std::exp(C * (vsq(e2.data(), n) - vsq(e1.data(), n))));
       else {
-        const float cj = (1 - pi) * std::exp(C * vsq(e1.data(), n));
-        const float dj = (pi)*std::exp(C * vsq(e2.data(), n));
+        const R cj = (1 - pi) * std::exp(C * vsq(e1.data(), n));
+        const R dj = (pi)*std::exp(C * vsq(e2.data(), n));
         pj = cj / (cj + dj);
       }
-      if (rng.rbinom1(pj) == 1) { b[j] = b1; d[j] = 1; e0 = e1; }
+      if (rng.include(pj)) { b[j] = b1; d[j] = 1; e0 = e1; }
       else { b[j] = b2; d[j] = 0; e0 = e2; }
     } else {
       d[j] = 1; b[j] = b1; e0 = e1;
     }
   }
-  std::memcpy(e_out, e0.data(), sizeof(float) * n);
+  std::memcpy(e_out, e0.data(), sizeof(R) * n);
 }
 
 // GSRR :1597-1628 / GSFLM :1564-1594: the warm-start Gauss-Seidel solvers of mm() (R/mix.R:890-892); natural marker order, the
@@ -1010,18 +1150,20 @@ struct WgrOut {
   double mu = 0, Ve = 0, Va = 0, cxx = 0, Vk = 0;
   std::vector<double> b, d, Vb, hat, u;
 };
-static inline void wgr(const double* y, const double* Xd, int n, int p, int it, int bi, int th, bool iv, bool de,
-                       double pi, double df, double R2, uint64_t seed, bool ratio_form, WgrOut& o, double bag = 1.0,
-                       const double* Ud = nullptr, const double* Vd = nullptr, int pk = 0, bool rp = false) {
-  Rng rng(seed);
+// K: the arithmetic of the KMUP sweeps (float, as across the Rcpp boundary; double for a float64 replay of the same draws).
+template <class K, class Draws>
+static void wgr(const double* y, const double* Xd, int n, int p, int it, int bi, int th, bool iv, bool de,
+                double pi, double df, double R2, Draws& rng, bool ratio_form, WgrOut& o, double bag = 1.0,
+                const double* Ud = nullptr, const double* Vd = nullptr, int pk = 0, bool rp = false) {
   if (de) iv = true;
   const bool bagged = bag != 1.0;
   if (bagged) df = df / (bag * bag);  // :21
   const int nuse = bagged ? (int)(n * bag) : n;
   std::vector<int> rows(n);
-  std::vector<float> usef(nuse), esub(nuse);
-  std::vector<float> Xf((size_t)n * p);
-  for (size_t i = 0; i < Xf.size(); i++) Xf[i] = (float)Xd[i];
+  std::vector<float> usef(nuse);
+  std::vector<K> esub(nuse);
+  std::vector<K> Xf((size_t)n * p);
+  for (size_t i = 0; i < Xf.size(); i++) Xf[i] = (K)(float)Xd[i];
   std::vector<int> post;
   for (int v = bi; v <= it; v += th) post.push_back(v);  // seq(bi,it,th)
   const int mc = (int)post.size();
@@ -1048,61 +1190,56 @@ static inline void wgr(const double* y, const double* Xd, int n, int p, int it, 
   const double Sb = R2 * df * vy / MSx, Se = (1 - R2) * df * vy;
   double B0 = 0, VA = 0, VE = 0;
   std::vector<double> VB(p, 0.0), D(p, 0.0), B(p, 0.0);
-  std::vector<float> bf(p), dfl(p), xxf(p), ef(n), Lf(p);
+  std::vector<K> bf(p), dfl(p), xxf(p), ef(n), Lf(p);
   // polygenic term (:23-33, :60): h = effects of the eigenvectors, xxK = bag, Vk = 1, Sk = R2 var(y) (df + 2)
   const bool poly = Ud != nullptr && pk > 0;
   std::vector<double> h(pk, 0.0), H(pk, 0.0), Vk(pk, 1.0);
-  std::vector<float> Uf((size_t)n * pk), hf(pk), dhf(pk), xxKf(pk, (float)bag), Lkf(pk);
-  for (size_t i = 0; i < Uf.size(); i++) Uf[i] = (float)Ud[i];
+  std::vector<K> Uf((size_t)n * pk), hf(pk), dhf(pk), xxKf(pk, (K)(float)bag), Lkf(pk);
+  for (size_t i = 0; i < Uf.size(); i++) Uf[i] = (K)(float)Ud[i];
   const double Sk = R2 * vy * (df + 2);
   double Vp = 0, VP = 0;
   size_t next_post = 0;
   for (int i = 1; i <= it; i++) {
-    for (int j = 0; j < p; j++) { bf[j] = (float)b[j]; dfl[j] = (float)d[j]; xxf[j] = (float)xx[j]; Lf[j] = (float)L[j]; }
-    for (int r = 0; r < n; r++) ef[r] = (float)e[r];
+    rng.set_sweep(i - 1);
+    for (int j = 0; j < p; j++) { bf[j] = (K)(float)b[j]; dfl[j] = (K)(float)d[j]; xxf[j] = (K)(float)xx[j]; Lf[j] = (K)(float)L[j]; }
+    for (int r = 0; r < n; r++) ef[r] = (K)(float)e[r];
     if (poly) {  // :77-84: Lk = Ve / (V Vk); KMUP(U, h, dh, xxK, e, Lk, Ve, 0)
-      for (int q = 0; q < pk; q++) { Lkf[q] = (float)(Ve / (Vd[q] * Vk[q])); hf[q] = (float)h[q]; dhf[q] = 0.0f; }
-      kmup(Uf.data(), n, pk, hf.data(), dhf.data(), xxKf.data(), ef.data(), Lkf.data(), (float)Ve, 0.0f, rng, ratio_form);
+      for (int q = 0; q < pk; q++) { Lkf[q] = (K)(float)(Ve / (Vd[q] * Vk[q])); hf[q] = (K)(float)h[q]; dhf[q] = 0; }
+      kmup(Uf.data(), n, pk, hf.data(), dhf.data(), xxKf.data(), ef.data(), Lkf.data(), (K)(float)Ve, K(0), rng, ratio_form);
       for (int q = 0; q < pk; q++) h[q] = hf[q];
     }
     if (bagged) {  // :68, :87: a fresh sorted row sample, swept by KMUP2; e becomes the residual of the rows in use
-      if (rp) {  // sample(n, n*bag, TRUE): rows may repeat; KMUP2 then counts a repeated row once per draw (:51-60)
-        rows.resize(std::max(n, nuse));
-        std::uniform_int_distribution<int> pick(0, n - 1);
-        for (int r = 0; r < nuse; r++) rows[r] = pick(rng.g);
-      } else {
-        for (int r = 0; r < n; r++) rows[r] = r;
-        for (int r = 0; r < nuse; r++) { std::uniform_int_distribution<int> pick(r, n - 1); std::swap(rows[r], rows[pick(rng.g)]); }
-      }
+      // sample(n, n*bag, rp): with rp = TRUE rows may repeat; KMUP2 then counts a repeated row once per draw (:51-60)
+      rng.rows(n, nuse, rp, rows);
       std::sort(rows.begin(), rows.begin() + nuse);
       for (int r = 0; r < nuse; r++) usef[r] = (float)rows[r];
-      kmup2(Xf.data(), n, p, usef.data(), nuse, bf.data(), dfl.data(), xxf.data(), ef.data(), esub.data(), Lf.data(), (float)Ve, (float)pi, rng,
-            ratio_form);
+      kmup2(Xf.data(), n, p, usef.data(), nuse, bf.data(), dfl.data(), xxf.data(), ef.data(), esub.data(), Lf.data(), (K)(float)Ve,
+            (K)(float)pi, rng, ratio_form);
     } else {
-      kmup(Xf.data(), n, p, bf.data(), dfl.data(), xxf.data(), ef.data(), Lf.data(), (float)Ve, (float)pi, rng, ratio_form);
+      kmup(Xf.data(), n, p, bf.data(), dfl.data(), xxf.data(), ef.data(), Lf.data(), (K)(float)Ve, (K)(float)pi, rng, ratio_form);
     }
     if (pi > 0) for (int j = 0; j < p; j++) d[j] = dfl[j];
     for (int j = 0; j < p; j++) b[j] = bf[j];
     for (int r = 0; r < n; r++) e[r] = ef[r];
     if (iv) {
       if (de) for (int j = 0; j < p; j++) Vb[j] = std::sqrt(b[j] * b[j] * Ve / MSx);
-      else for (int j = 0; j < p; j++) Vb[j] = (Sb + b[j] * b[j]) / rng.rchisq(df + 1);
+      else for (int j = 0; j < p; j++) Vb[j] = (Sb + b[j] * b[j]) / rng.wgr_Vb(j, df + 1);
     } else {
       double bb = 0;
       for (int j = 0; j < p; j++) bb += b[j] * b[j];
-      Va = (bb + Sb) / rng.rchisq(df + p);
+      Va = (bb + Sb) / rng.wgr_Va(df + p);
       for (int j = 0; j < p; j++) Vb[j] = Va;
     }
     if (poly) {  // :116-119
       double hh = 0;
       for (int q = 0; q < pk; q++) hh += h[q] * h[q] / Vd[q];
-      Vp = (hh + Sk) / rng.rchisq(df + pk);
+      Vp = (hh + Sk) / rng.wgr_Vp(df + pk);
       for (int q = 0; q < pk; q++) Vk[q] = Vp;
     }
     double ee = 0;
     if (bagged) for (int r = 0; r < nuse; r++) ee += (double)esub[r] * (double)esub[r];
     else for (int r = 0; r < n; r++) ee += e[r] * e[r];
-    Ve = (ee + Se) / rng.rchisq(n * bag + df);  // :121
+    Ve = (ee + Se) / rng.wgr_Ve(n * bag + df);  // :121
     for (int j = 0; j < p; j++) L[j] = Ve / Vb[j];
     for (int r = 0; r < n; r++) e[r] = y[r] - mu;  // e = y-mu-X%*%b
     for (int j = 0; j < p; j++) {
@@ -1119,7 +1256,7 @@ static inline void wgr(const double* y, const double* Xd, int n, int p, int it, 
     double em = 0;
     for (int r = 0; r < n; r++) em += e[r];
     em /= n;
-    const double mu0 = rng.rnorm(em, Ve / n);  // sic: sd argument is Ve/n (wgr.R:125)
+    const double mu0 = rng.wgr_mu0(em, Ve / n);  // sic: sd argument is Ve/n (wgr.R:125)
     mu += mu0;
     for (int r = 0; r < n; r++) e[r] -= mu0;
     if (next_post < post.size() && post[next_post] == i) {

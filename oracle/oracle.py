@@ -109,7 +109,27 @@ def emML_weighted(y, gen, D, it=-1, use_double=False):
     return {"mu": mu.value, "b": b, "hat": hat, "h2": scal[2], "Vb": scal[3], "Va": scal[0], "Ve": scal[1], "its": its.value}
 
 
-def gibbs(model, y, X, it=1500, bi=500, pi=0.95, df=5.0, R2=0.5, seed=1):
+class _Margins:
+    """Decision record of a replay on the device's Philox draws (see orc::PhiloxDraws)."""
+
+    def __init__(self, cap):
+        self.q, self.u = np.zeros(cap), np.zeros(cap)
+        self.nq, self.mt = C.c_int(), np.zeros(1)
+        self.args = (_p(self.q, C.c_double), _p(self.u, C.c_double), C.c_int(cap), C.byref(self.nq), _p(self.mt, C.c_double))
+
+    def add_to(self, out):
+        k = self.nq.value
+        assert k <= self.q.size
+        # q / u: the inclusion probability and the uniform of every accept / reject decision, in the order they were made;
+        # margin: the smallest |u - q|; mt_margin: the smallest normalised Marsaglia-Tsang acceptance margin
+        out.update(q=self.q[:k].copy(), u=self.u[:k].copy(), margin=float(np.abs(self.u[:k] - self.q[:k]).min()) if k else np.inf,
+                   mt_margin=float(self.mt[0]))
+        return out
+
+
+def gibbs(model, y, X, it=1500, bi=500, pi=0.95, df=5.0, R2=0.5, seed=1, draws="mt", chain=0, use_double=False):
+    """draws = "mt": the reference's draw order on one std::mt19937_64 stream; "philox": the device's counter-addressed draws of chain
+    `chain`, with the decision record of _Margins.  use_double (philox only): the same recipe in float64 on the same float draws."""
     y = _f32(y)
     X = _f32(X)
     n, p = X.shape
@@ -117,13 +137,24 @@ def gibbs(model, y, X, it=1500, bi=500, pi=0.95, df=5.0, R2=0.5, seed=1):
     b, d, vbv = (np.zeros(p) for _ in range(3))
     hat = np.zeros(n)
     scal = np.zeros(5)
-    rc = lib().orc_gibbs(C.c_int(GIBBS_MODELS[model]), _p(y, C.c_float), _p(X, C.c_float), C.c_int(n), C.c_int(p),
-                         C.c_float(it), C.c_float(bi), C.c_float(pi), C.c_float(df), C.c_float(R2),
-                         C.c_uint64(seed), C.byref(mu), _p(b, C.c_double), _p(d, C.c_double), _p(hat, C.c_double),
-                         _p(vbv, C.c_double), _p(scal, C.c_double))
+    if draws == "philox":
+        m = _Margins(int(it) * p)
+        rc = lib().orc_gibbs_philox(C.c_int(GIBBS_MODELS[model]), C.c_int(int(use_double)), C.c_int(chain), _p(y, C.c_float), _p(X, C.c_float),
+                                    C.c_int(n), C.c_int(p), C.c_float(it), C.c_float(bi), C.c_float(pi), C.c_float(df), C.c_float(R2),
+                                    C.c_uint64(seed), C.byref(mu), _p(b, C.c_double), _p(d, C.c_double), _p(hat, C.c_double),
+                                    _p(vbv, C.c_double), _p(scal, C.c_double), *m.args)
+    else:
+        assert draws == "mt" and chain == 0 and not use_double
+        m = None
+        rc = lib().orc_gibbs(C.c_int(GIBBS_MODELS[model]), _p(y, C.c_float), _p(X, C.c_float), C.c_int(n), C.c_int(p),
+                             C.c_float(it), C.c_float(bi), C.c_float(pi), C.c_float(df), C.c_float(R2),
+                             C.c_uint64(seed), C.byref(mu), _p(b, C.c_double), _p(d, C.c_double), _p(hat, C.c_double),
+                             _p(vbv, C.c_double), _p(scal, C.c_double))
     assert rc == 0
     vb, ve, h2, MSx, pi_out = scal
     out = {"mu": mu.value, "b": b, "hat": hat, "ve": ve, "h2": h2, "MSx": MSx}
+    if m is not None:
+        m.add_to(out)
     out["vb"] = vbv if model in ("BayesA", "BayesB", "BayesL", "BayesDpi") else vb
     if model in ("BayesB", "BayesC", "BayesCpi", "BayesDpi"):
         out["d"] = d
@@ -135,7 +166,28 @@ def gibbs(model, y, X, it=1500, bi=500, pi=0.95, df=5.0, R2=0.5, seed=1):
     return out
 
 
-def kmup(X, b, d, xx, e, L, Ve, pi, seed=1, ratio_form=False):
+def _kmup_philox(X, use, b, d, xx, e, L, Ve, pi, seed, use_double):
+    """One KMUP (use None) or KMUP2 sweep on the device's Philox draws, in the ratio form the device evaluates."""
+    X = _f32(X)
+    n, p = X.shape
+    b, d, xx, e, L = (np.array(v, dtype=np.float64).ravel() for v in (b, d, xx, e, L))
+    if use is not None:
+        use = np.array(use, dtype=np.float32).ravel()
+    e_out = np.zeros(n if use is None else use.size)
+    m = _Margins(p)
+    rc = lib().orc_kmup_philox(C.c_int(int(use_double)), _p(X, C.c_float), C.c_int(n), C.c_int(p), None if use is None else _p(use, C.c_float),
+                               C.c_int(0 if use is None else use.size), _p(b, C.c_double), _p(d, C.c_double), _p(xx, C.c_double),
+                               _p(e, C.c_double), _p(e_out, C.c_double), _p(L, C.c_double), C.c_double(Ve), C.c_double(pi),
+                               C.c_uint64(seed), *m.args)
+    assert rc == 0
+    return m.add_to({"b": b, "d": d, "e": e_out})
+
+
+def kmup(X, b, d, xx, e, L, Ve, pi, seed=1, ratio_form=False, draws="mt", use_double=False):
+    """draws = "philox": the device's draws of a standalone sweep (sweep 0, chain 0), ratio form, use_double as for gibbs()."""
+    if draws == "philox":
+        return _kmup_philox(X, None, b, d, xx, e, L, Ve, pi, seed, use_double)
+    assert draws == "mt" and not use_double
     X = _f32(X)
     n, p = X.shape
     b, d, xx, e, L = (np.array(v, dtype=np.float32) for v in (b, d, xx, e, L))
@@ -145,7 +197,11 @@ def kmup(X, b, d, xx, e, L, Ve, pi, seed=1, ratio_form=False):
     return {"b": b, "d": d, "e": e}
 
 
-def kmup2(X, use, b, d, xx, E, L, Ve, pi, seed=1, ratio_form=False):
+def kmup2(X, use, b, d, xx, E, L, Ve, pi, seed=1, ratio_form=False, draws="mt", use_double=False):
+    """draws = "philox": as kmup()."""
+    if draws == "philox":
+        return _kmup_philox(X, use, b, d, xx, E, L, Ve, pi, seed, use_double)
+    assert draws == "mt" and not use_double
     X = _f32(X)
     n, p = X.shape
     use = np.array(use, dtype=np.float32)
@@ -187,13 +243,27 @@ def eigk_rank(values, VarK=0.95):
     return int(np.argmax(np.cumsum(V) / V.size > VarK)) + 1
 
 
-def wgr(y, X, it=1500, bi=500, th=1, iv=False, de=False, pi=0.0, df=5.0, R2=0.5, seed=1, ratio_form=False, bag=1.0, eigK=None, VarK=0.95, rp=False):
+def wgr(y, X, it=1500, bi=500, th=1, iv=False, de=False, pi=0.0, df=5.0, R2=0.5, seed=1, ratio_form=False, bag=1.0, eigK=None, VarK=0.95, rp=False,
+        draws="mt", use_double=False):
+    """draws = "philox": the device's draws (native or bagged; not eigK), KMUP sweeps in the ratio form; use_double: the KMUP sweeps
+    in float64 on the same float draws."""
     y = np.ascontiguousarray(y, dtype=np.float64)
     X = np.asfortranarray(X, dtype=np.float64)
     n, p = X.shape
     b, d, Vb = (np.zeros(p) for _ in range(3))
     hat = np.zeros(n)
     scal = np.zeros(4)
+    if draws == "philox":
+        assert eigK is None
+        m = _Margins(int(it) * p)
+        rc = lib().orc_wgr_philox(C.c_int(int(use_double)), _p(y, C.c_double), _p(X, C.c_double), C.c_int(n), C.c_int(p), C.c_int(it), C.c_int(bi),
+                                  C.c_int(th), C.c_double(bag), C.c_int(int(rp)), C.c_int(int(iv)), C.c_int(int(de)), C.c_double(pi),
+                                  C.c_double(df), C.c_double(R2), C.c_uint64(seed), _p(b, C.c_double), _p(d, C.c_double), _p(Vb, C.c_double),
+                                  _p(hat, C.c_double), _p(scal, C.c_double), *m.args)
+        assert rc == 0
+        mu, Ve, Va, cxx = scal
+        return m.add_to({"mu": mu, "b": b, "Vb": Vb if (iv or de) else Va, "d": d, "Ve": Ve, "hat": hat, "cxx": cxx})
+    assert draws == "mt" and not use_double
     if eigK is not None:  # R/wgr.R:23-33 (bag == 1)
         assert bag == 1.0
         pk = eigk_rank(eigK["values"], VarK)

@@ -67,7 +67,8 @@ int orc_gibbs(int model, const float* y, const float* X, int n, int p, float it,
               uint64_t seed, double* mu, double* b, double* d, double* hat, double* vbv, double* scal) {
   if (model < 0 || model > 6) return -1;
   orc::GibbsOut<float> o;
-  orc::gibbs_fit<float>(model, y, X, n, p, it, bi, pi, df, R2, seed, o);
+  orc::Rng rng(seed);
+  orc::gibbs_fit<float>(model, y, X, n, p, it, bi, pi, df, R2, rng, o);
   *mu = o.mu;
   for (int j = 0; j < p; j++) { b[j] = o.b[j]; d[j] = o.d[j]; vbv[j] = o.vbv[j]; }
   for (int i = 0; i < n; i++) hat[i] = o.hat[i];
@@ -119,7 +120,8 @@ int orc_two_design(int model, const float* y, const float* X1, const float* X2, 
 int orc_wgr(const double* y, const double* X, int n, int p, int it, int bi, int th, int iv, int de, double pi, double df,
             double R2, uint64_t seed, int ratio_form, double* b, double* d, double* Vb, double* hat, double* scal) {
   orc::WgrOut o;
-  orc::wgr(y, X, n, p, it, bi, th, iv != 0, de != 0, pi, df, R2, seed, ratio_form != 0, o);
+  orc::Rng rng(seed);
+  orc::wgr<float>(y, X, n, p, it, bi, th, iv != 0, de != 0, pi, df, R2, rng, ratio_form != 0, o);
   for (int j = 0; j < p; j++) { b[j] = o.b[j]; d[j] = o.d[j]; Vb[j] = o.Vb[j]; }
   for (int i = 0; i < n; i++) hat[i] = o.hat[i];
   scal[0] = o.mu; scal[1] = o.Ve; scal[2] = o.Va; scal[3] = o.cxx;
@@ -131,7 +133,8 @@ int orc_wgr_eigk(const double* y, const double* X, int n, int p, const double* U
                  int de, double pi, double df, double R2, uint64_t seed, int ratio_form, double* b, double* d, double* Vb, double* hat,
                  double* u, double* scal) {
   orc::WgrOut o;
-  orc::wgr(y, X, n, p, it, bi, th, iv != 0, de != 0, pi, df, R2, seed, ratio_form != 0, o, 1.0, U, V, pk);
+  orc::Rng rng(seed);
+  orc::wgr<float>(y, X, n, p, it, bi, th, iv != 0, de != 0, pi, df, R2, rng, ratio_form != 0, o, 1.0, U, V, pk);
   for (int j = 0; j < p; j++) { b[j] = o.b[j]; d[j] = o.d[j]; Vb[j] = o.Vb[j]; }
   for (int i = 0; i < n; i++) { hat[i] = o.hat[i]; u[i] = o.u[i]; }
   scal[0] = o.mu; scal[1] = o.Ve; scal[2] = o.Va; scal[3] = o.cxx; scal[4] = o.Vk;
@@ -141,7 +144,8 @@ int orc_wgr_eigk(const double* y, const double* X, int n, int p, const double* U
 int orc_wgr_bag(const double* y, const double* X, int n, int p, int it, int bi, int th, double bag, int iv, int de, double pi, double df,
                 double R2, uint64_t seed, int ratio_form, double* b, double* d, double* Vb, double* hat, double* scal) {
   orc::WgrOut o;
-  orc::wgr(y, X, n, p, it, bi, th, iv != 0, de != 0, pi, df, R2, seed, ratio_form != 0, o, bag);
+  orc::Rng rng(seed);
+  orc::wgr<float>(y, X, n, p, it, bi, th, iv != 0, de != 0, pi, df, R2, rng, ratio_form != 0, o, bag);
   for (int j = 0; j < p; j++) { b[j] = o.b[j]; d[j] = o.d[j]; Vb[j] = o.Vb[j]; }
   for (int i = 0; i < n; i++) hat[i] = o.hat[i];
   scal[0] = o.mu; scal[1] = o.Ve; scal[2] = o.Va; scal[3] = o.cxx;
@@ -152,7 +156,8 @@ int orc_wgr_bag(const double* y, const double* X, int n, int p, int it, int bi, 
 int orc_wgr_bag_rp(const double* y, const double* X, int n, int p, int it, int bi, int th, double bag, int rp, int iv, int de, double pi,
                    double df, double R2, uint64_t seed, int ratio_form, double* b, double* d, double* Vb, double* hat, double* scal) {
   orc::WgrOut o;
-  orc::wgr(y, X, n, p, it, bi, th, iv != 0, de != 0, pi, df, R2, seed, ratio_form != 0, o, bag, nullptr, nullptr, 0, rp != 0);
+  orc::Rng rng(seed);
+  orc::wgr<float>(y, X, n, p, it, bi, th, iv != 0, de != 0, pi, df, R2, rng, ratio_form != 0, o, bag, nullptr, nullptr, 0, rp != 0);
   for (int j = 0; j < p; j++) { b[j] = o.b[j]; d[j] = o.d[j]; Vb[j] = o.Vb[j]; }
   for (int i = 0; i < n; i++) hat[i] = o.hat[i];
   scal[0] = o.mu; scal[1] = o.Ve; scal[2] = o.Va; scal[3] = o.cxx;
@@ -190,6 +195,104 @@ int orc_mrr3(int f32_variant, const double* Y, const double* X, int n, int k, in
     *its = o.its;
   };
   if (f32_variant) run(float{}); else run(double{});
+  return 0;
+}
+
+}  // extern "C"
+
+// ---- replays on the device's Philox draws (orc::PhiloxDraws) --------------------------------------------------------------------
+// use_double = 1 runs the same recipe in float64 on the same float draws.  Every replay reports how close its accept / reject
+// decisions came to the other outcome: q / u (the inclusion probability and the uniform of each decision, at most qcap of them,
+// *nq = how many there were) and mt[0] = the smallest normalised Marsaglia-Tsang acceptance margin.
+namespace {
+void margins_out(const orc::PhiloxDraws& rng, double* q, double* u, int qcap, int* nq, double* mt) {
+  *nq = (int)rng.q.size();
+  for (int i = 0; i < *nq && i < qcap; i++) { q[i] = rng.q[i]; u[i] = rng.uq[i]; }
+  mt[0] = rng.mt_margin;
+}
+template <class R>
+void gibbs_philox_run(int model, const float* y, const float* X, int n, int p, float it, float bi, float pi, float df, float R2,
+                      orc::PhiloxDraws& rng, double* mu, double* b, double* d, double* hat, double* vbv, double* scal) {
+  std::vector<R> yy(y, y + n), XX(X, X + (size_t)n * p);
+  orc::GibbsOut<R> o;
+  orc::gibbs_fit<R>(model, yy.data(), XX.data(), n, p, it, bi, pi, df, R2, rng, o);
+  *mu = o.mu;
+  for (int j = 0; j < p; j++) { b[j] = o.b[j]; d[j] = o.d[j]; vbv[j] = o.vbv[j]; }
+  for (int i = 0; i < n; i++) hat[i] = o.hat[i];
+  scal[0] = o.vb; scal[1] = o.ve; scal[2] = o.h2; scal[3] = o.MSx; scal[4] = o.pi;
+}
+template <class R>
+void kmup_philox_run(const float* X, int n, int p, const float* use, int nuse, double* b, double* d, const double* xx, const double* e,
+                     double* e_out, const double* L, double Ve, double pi, orc::PhiloxDraws& rng) {
+  std::vector<R> XX(X, X + (size_t)n * p), bb(b, b + p), dd(d, d + p), x2(xx, xx + p), LL(L, L + p), ee(e, e + n), eo(use ? nuse : n);
+  for (int j = 0; j < p; j++) { bb[j] = (R)(float)b[j]; dd[j] = (R)(float)d[j]; x2[j] = (R)(float)xx[j]; LL[j] = (R)(float)L[j]; }
+  for (int i = 0; i < n; i++) ee[i] = (R)(float)e[i];
+  if (use) orc::kmup2<R>(XX.data(), n, p, use, nuse, bb.data(), dd.data(), x2.data(), ee.data(), eo.data(), LL.data(), (R)(float)Ve,
+                         (R)(float)pi, rng, true);
+  else { orc::kmup<R>(XX.data(), n, p, bb.data(), dd.data(), x2.data(), ee.data(), LL.data(), (R)(float)Ve, (R)(float)pi, rng, true); eo = ee; }
+  for (int j = 0; j < p; j++) { b[j] = bb[j]; d[j] = dd[j]; }
+  for (size_t i = 0; i < eo.size(); i++) e_out[i] = eo[i];
+}
+}  // namespace
+
+extern "C" {
+
+// Gibbs fit of chain `chain`; scal as orc_gibbs.
+int orc_gibbs_philox(int model, int use_double, int chain, const float* y, const float* X, int n, int p, float it, float bi, float pi,
+                     float df, float R2, uint64_t seed, double* mu, double* b, double* d, double* hat, double* vbv, double* scal, double* q,
+                     double* u, int qcap, int* nq, double* mt) {
+  if (model < 0 || model > 6) return -1;
+  orc::PhiloxDraws rng(seed);
+  rng.set_chain(chain);
+  if (use_double) gibbs_philox_run<double>(model, y, X, n, p, it, bi, pi, df, R2, rng, mu, b, d, hat, vbv, scal);
+  else gibbs_philox_run<float>(model, y, X, n, p, it, bi, pi, df, R2, rng, mu, b, d, hat, vbv, scal);
+  margins_out(rng, q, u, qcap, nq, mt);
+  return 0;
+}
+
+// One KMUP sweep (use = NULL; e_out has n values) or KMUP2 sweep over the rows `use` (e_out has nuse values), at sweep 0, chain 0,
+// in the ratio form the device evaluates.  b and d are updated in place.
+int orc_kmup_philox(int use_double, const float* X, int n, int p, const float* use, int nuse, double* b, double* d, const double* xx,
+                    const double* e, double* e_out, const double* L, double Ve, double pi, uint64_t seed, double* q, double* u, int qcap,
+                    int* nq, double* mt) {
+  orc::PhiloxDraws rng(seed);
+  if (use_double) kmup_philox_run<double>(X, n, p, use, nuse, b, d, xx, e, e_out, L, Ve, pi, rng);
+  else kmup_philox_run<float>(X, n, p, use, nuse, b, d, xx, e, e_out, L, Ve, pi, rng);
+  margins_out(rng, q, u, qcap, nq, mt);
+  return 0;
+}
+
+// wgr (bag = 1: native; bag != 1: bagged, rp as orc_wgr_bag_rp), KMUP sweeps in the ratio form; scal as orc_wgr.
+int orc_wgr_philox(int use_double, const double* y, const double* X, int n, int p, int it, int bi, int th, double bag, int rp, int iv, int de,
+                   double pi, double df, double R2, uint64_t seed, double* b, double* d, double* Vb, double* hat, double* scal, double* q,
+                   double* u, int qcap, int* nq, double* mt) {
+  orc::WgrOut o;
+  orc::PhiloxDraws rng(seed);
+  if (use_double) orc::wgr<double>(y, X, n, p, it, bi, th, iv != 0, de != 0, pi, df, R2, rng, true, o, bag, nullptr, nullptr, 0, rp != 0);
+  else orc::wgr<float>(y, X, n, p, it, bi, th, iv != 0, de != 0, pi, df, R2, rng, true, o, bag, nullptr, nullptr, 0, rp != 0);
+  for (int j = 0; j < p; j++) { b[j] = o.b[j]; d[j] = o.d[j]; Vb[j] = o.Vb[j]; }
+  for (int i = 0; i < n; i++) hat[i] = o.hat[i];
+  scal[0] = o.mu; scal[1] = o.Ve; scal[2] = o.Va; scal[3] = o.cxx;
+  margins_out(rng, q, u, qcap, nq, mt);
+  return 0;
+}
+
+// Known-answer check of the restated generator: out[4] = Philox4x32-10(counter, key)
+int orc_philox4x32_10(const uint32_t* counter, uint32_t k0, uint32_t k1, uint32_t* out) {
+  uint32_t c[4] = {counter[0], counter[1], counter[2], counter[3]};
+  orc::philox::philox4x32_10(c, k0, k1);
+  for (int i = 0; i < 4; i++) out[i] = c[i];
+  return 0;
+}
+
+// The draws of one marker update at (marker, sweep, chain): {z1, z2, u, chi(nu)} (chi with nu <= 0: not drawn, 1)
+int orc_marker_draws(uint32_t marker, uint32_t sweep, uint32_t chain, float nu, uint64_t seed, float* out) {
+  orc::PhiloxDraws rng(seed);
+  rng.set_chain((int)chain);
+  rng.set_sweep((int)sweep);
+  rng.set_marker((int)marker);
+  out[0] = rng.z1; out[1] = rng.z2; out[2] = rng.u;
+  out[3] = nu > 0 ? (float)rng.chi_marker(nu) : 1.0f;
   return 0;
 }
 
