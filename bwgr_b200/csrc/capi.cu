@@ -469,15 +469,6 @@ float fvar_f(const std::vector<float>& x) {  // fvar, Rcpp20260726ai.cpp:7-9 (su
   return (float)s / (float)(x.size() - 1);
 }
 
-// Fixed-point scale of the residuals in the tensor-core passes: 8x headroom over emax = max|e|.
-void set_e_scale(SysScalars& c, float emax) {
-  int ex = 0;
-  if (emax > 0) std::frexp(emax, &ex);
-  if (ex < -60) ex = -60;
-  c.e_q = std::ldexp(1.0f, ex + 3 - 30);
-  c.e_qinv = std::ldexp(1.0f, 30 - 3 - ex);
-}
-
 // Held by a one-shot entry point from the start of its fit to its return: the fit is released whatever the exit, so a failed call
 // leaves no fit that bwgr_em_sweeps / bwgr_em_end could continue.
 struct FitGuard {
@@ -2404,9 +2395,8 @@ int mrr3_general(bwgr_handle* h, int f32_variant, const double* Y, int k, const 
     if (!(vy[t] > 0)) return fail(BWGR_ERR_ARG, "MRR3: trait %d has no variance", t + 1);
   }
   // ---- launch geometry: one CTA per row slab, all co-resident
-  int rp = (int)((ld + h->num_sms - 1) / h->num_sms);
-  rp = std::max(64, (rp + 15) / 16 * 16);
-  const int grid = (int)((ld + rp - 1) / rp);
+  int rp = 0, grid = 0;
+  grid_geometry(h, &rp, &grid);
   const size_t smem = mrr_gen_smem(k, rp, innergs);
   if (smem > h->smem_optin || grid > h->num_sms)
     return fail(BWGR_ERR_UNSUPPORTED, "MRR3 (general path): %lld rows x %d traits do not fit the shared memory of %d SMs", (long long)n, k, h->num_sms);
@@ -2417,7 +2407,7 @@ int mrr3_general(bwgr_handle* h, int f32_variant, const double* Y, int k, const 
       bd.alloc((size_t)p * k) != cudaSuccess || bold.alloc((size_t)p * k) != cudaSuccess || fixd.alloc((size_t)p * 2 * k) != cudaSuccess ||
       meand.alloc(p) != cudaSuccess || tilded.alloc((size_t)p * k) != cudaSuccess || sold.alloc((size_t)p * nmat * kk) != cudaSuccess ||
       (NonLinear && Wd.alloc((size_t)p * k) != cudaSuccess) || (F.TH && (xsxd.alloc((size_t)p * k) != cudaSuccess || dinvd.alloc((size_t)p * k) != cudaSuccess)) ||
-      small.alloc(nsmall + kk) != cudaSuccess || accd.alloc((size_t)p * 32 * kMrrGenCopies) != cudaSuccess || grid > 255 ||
+      small.alloc(nsmall + kk) != cudaSuccess || accd.alloc((size_t)p * 32 * kGridCopies) != cudaSuccess || grid > 255 ||
       permd.alloc(p + 32) != cudaSuccess)
     return fail(BWGR_ERR_CUDA, "cudaMalloc(MRR3 general workspace) failed");
   double *d_iG = small.p, *d_vb = small.p + kk, *d_iVe = d_vb + kk, *d_se = d_iVe + 32, *d_ey = d_se + 32, *d_cnv = d_ey + 32,
@@ -2501,7 +2491,7 @@ int mrr3_general(bwgr_handle* h, int f32_variant, const double* Y, int k, const 
         scl[t] = std::ldexp(1.0, 52 - ex); scl[32 + t] = std::ldexp(1.0, ex - 52);
       }
       CU(cudaMemcpyAsync(d_scale, scl.data(), sizeof(double) * 64, cudaMemcpyHostToDevice, st));
-      CU(cudaMemsetAsync(accd.p, 0, sizeof(unsigned long long) * p * 32 * kMrrGenCopies, st));
+      CU(cudaMemsetAsync(accd.p, 0, sizeof(unsigned long long) * p * 32 * kGridCopies, st));
       const cudaError_t le = launch_mrr_gen_sweep(a, grid, st);
       if (le != cudaSuccess) return fail(BWGR_ERR_CUDA, "MRR3 general sweep launch failed: %s", cudaGetErrorString(le));
     }

@@ -42,6 +42,15 @@ struct SysScalars {
   double MU, VE, VB, PI;
 };
 
+// Fixed-point scale of the residuals for the next sweep, from bound >= max|e|: |e| may grow 8x before it saturates 2^30.
+__host__ __device__ inline void set_e_scale(SysScalars& s, float bound) {
+  int ex = 0;
+  if (bound > 0.0f && bound < 3.0e38f) frexpf(bound, &ex);
+  if (ex < -60) ex = -60;
+  s.e_q = ldexpf(1.0f, ex + 3 - 30);
+  s.e_qinv = ldexpf(1.0f, 30 - 3 - ex);
+}
+
 struct MarkerDraws {  // pre-generated per marker per sweep (Gibbs only)
   float z1, z2, u, chi;
 };

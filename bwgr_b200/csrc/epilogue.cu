@@ -234,14 +234,7 @@ __global__ void __cluster_dims__(kEpiCl, 1, 1) __launch_bounds__(1024) epilogue_
     }
     s.mu += eM;
     s.sweep += 1;
-    {  // fixed-point scale of the residuals for the next sweep: |e| may grow 8x before it saturates 2^30
-      int ex = 0;
-      const float bound = emax + fabsf(eM);
-      if (bound > 0.0f && bound < 3.0e38f) frexpf(bound, &ex);
-      if (ex < -60) ex = -60;
-      s.e_q = ldexpf(1.0f, ex + 3 - 30);
-      s.e_qinv = ldexpf(1.0f, 30 - 3 - ex);
-    }
+    set_e_scale(s, emax + fabsf(eM));
     *scp = s;
     s_eM = eM;
     s_acc = accumulate;
@@ -349,14 +342,7 @@ __global__ void __launch_bounds__(1024) wgr_scalars_kernel(WgrArgs a) {
       s.C = -0.5f / sqrtf(s.ve);
       s.sweep += 1;
       s.its += 1;
-      {
-        int ex = 0;
-        const float bound = emax + fabsf(w.mu0);
-        if (bound > 0.0f && bound < 3.0e38f) frexpf(bound, &ex);
-        if (ex < -60) ex = -60;
-        s.e_q = ldexpf(1.0f, ex + 3 - 30);
-        s.e_qinv = ldexpf(1.0f, 30 - 3 - ex);
-      }
+      set_e_scale(s, emax + fabsf(w.mu0));
       *a.sc = s;
     }
     *a.st = w;

@@ -23,7 +23,7 @@
 #include <stdint.h>
 #include <string.h>
 
-#include "kernels.h"
+#include "device.cuh"
 
 namespace bwgr {
 
@@ -33,35 +33,8 @@ constexpr int kStages = 6;
 constexpr int kProducers = 512;             // warps 0-3 and 9-20: one packed 16-byte chunk of one marker of each tile per thread and stage
 constexpr int kThreads = kProducers + 160;  // + MMA warp (4) + four epilogue warps (5-8)
 constexpr int kStageBytes = 2 * 128 * 128;  // two tiles (block b, block b + 1) x 128 markers x 128 bytes (256 rows as FP4)
-constexpr uint32_t kSpinLimit = 1u << 22;
 constexpr uint32_t kAccCols = 256, kSfCol = 256, kSfCols = 64, kTmemCols = 512;
 
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ bool elect_one() {
-  uint32_t pred;
-  asm volatile("{\n\t.reg .pred P;\n\telect.sync _|P, 0xffffffff;\n\tselp.u32 %0, 1, 0, P;\n\t}" : "=r"(pred));
-  return pred != 0;
-}
-__device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count));
-}
-__device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ bool mbar_wait(uint64_t* bar, uint32_t parity, int* err) {
-  const uint32_t addr = smem_u32(bar);
-  for (uint32_t spin = 0; spin < kSpinLimit; spin++) {
-    uint32_t done;
-    asm volatile("{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}"
-                 : "=r"(done) : "r"(addr), "r"(parity) : "memory");
-    if (done) return true;
-  }
-  atomicExch(err, 2);
-  return false;
-}
-__device__ __forceinline__ uint64_t make_desc_sw128(uint32_t saddr) {
-  return (uint64_t)((saddr & 0x3FFFFu) >> 4) | ((uint64_t)1 << 16) | ((uint64_t)(1024 >> 4) << 32) | ((uint64_t)1 << 46) | ((uint64_t)2 << 61);
-}
 // block-scaled instruction descriptor (cute/arch/mma_sm100_desc.hpp, InstrDescriptorBlockScaled): A, B = E2M1 (kind::mxf4 format 1),
 // both K-major, N = 256, scale format UE8M0, M = 128, K = 64, scale-factor ids 0
 constexpr uint32_t kIdescMxf4 = (1u << 7) | (1u << 10) | ((256u >> 3) << 17) | (1u << 23) | ((128u >> 4) << 24);
@@ -71,9 +44,6 @@ __device__ __forceinline__ void umma_mxf4(uint32_t tmem_d, uint64_t adesc, uint6
       "setp.ne.b32 p, %6, 0;\n\t"
       "tcgen05.mma.cta_group::1.kind::mxf4.block_scale.scale_vec::2X [%0], %1, %2, %3, [%4], [%5], p;\n\t}"
       ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(kIdescMxf4), "r"(sfa), "r"(sfb), "r"(accumulate) : "memory");
-}
-__device__ __forceinline__ void umma_commit(uint64_t* bar) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");
 }
 
 struct Fp4Smem {
@@ -94,15 +64,12 @@ __global__ void __launch_bounds__(kThreads, 1) gram_fp4_kernel(const uint8_t* __
   if (threadIdx.x == 0) {
     for (int s = 0; s < kStages; s++) { mbar_init(&S->full[s], kProducers); mbar_init(&S->empty[s], 1); }
     mbar_init(&S->tmem_full, 1); mbar_init(&S->tmem_empty, 4);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    fence_mbar_init();
   }
-  if (warp == 4) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&S->tmem_base)), "r"(kTmemCols) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+  if (warp == 4) tmem_alloc(&S->tmem_base, kTmemCols);
+  tc_fence_before();
   __syncthreads();
-  asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+  tc_fence_after();
   const uint32_t tmem_base = S->tmem_base;
   if (warp >= 5 && warp <= 8) {
     // every block scale = 0x7F (UE8M0 2^0): the whole scale region is filled with that byte, so whichever rows / columns / byte
@@ -114,9 +81,9 @@ __global__ void __launch_bounds__(kThreads, 1) gram_fp4_kernel(const uint8_t* __
       asm volatile("tcgen05.st.sync.aligned.32x32b.x4.b32 [%0], {%1, %1, %1, %1};" ::"r"(taddr + (uint32_t)c), "r"(one) : "memory");
     asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
   }
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+  tc_fence_before();
   __syncthreads();
-  asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+  tc_fence_after();
 
   if (warp < 4 || warp >= 9) {
     // ===================== producer: packed 2-bit chunks -> E2M1 nibbles, SWIZZLE_128B K-major tiles =====================
@@ -169,7 +136,7 @@ __global__ void __launch_bounds__(kThreads, 1) gram_fp4_kernel(const uint8_t* __
             asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(rowb + ((((uint32_t)(2 * c + 1)) ^ sw) << 4)),
                          "r"((pk.z & 0x33333333u) << 1), "r"((pk.z >> 1) & 0x66666666u), "r"((pk.w & 0x33333333u) << 1), "r"((pk.w >> 1) & 0x66666666u) : "memory");
           }
-          asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+          fence_proxy_async();
           mbar_arrive(&S->full[stage]);
           it++;
         }
@@ -182,13 +149,13 @@ __global__ void __launch_bounds__(kThreads, 1) gram_fp4_kernel(const uint8_t* __
     const uint32_t sfa = tmem_base + kSfCol, sfb = tmem_base + kSfCol + 16;
     for (int blk = blockIdx.x; blk < nblocks && ok; blk += gridDim.x, bi++) {
       ok = mbar_wait(&S->tmem_empty, (bi & 1u) ^ 1u, err);
-      asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+      tc_fence_after();
       for (int kg = 0; kg < nkg && ok; kg++, it++) {
         const uint32_t stage = it % kStages, phase = (it / kStages) & 1u;
         ok = mbar_wait(&S->full[stage], phase, err);
-        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+        tc_fence_after();
         if (elect_one()) {
-          const uint64_t desc = make_desc_sw128(smem_u32(tiles + stage * kStageBytes));  // A = tile of block b; B = both tiles (256 rows)
+          const uint64_t desc = desc_k_sw128(smem_u32(tiles + stage * kStageBytes));  // A = tile of block b; B = both tiles (256 rows)
 #pragma unroll
           for (int k4 = 0; k4 < 4; k4++)
             umma_mxf4(tmem_base, desc + (uint64_t)(k4 * 2), desc + (uint64_t)(k4 * 2), sfa, sfb, (kg | k4) != 0 ? 1u : 0u);
@@ -207,32 +174,23 @@ __global__ void __launch_bounds__(kThreads, 1) gram_fp4_kernel(const uint8_t* __
     bool ok = true;
     for (int blk = blockIdx.x; blk < nblocks && ok; blk += gridDim.x, bi++) {
       ok = mbar_wait(&S->tmem_full, bi & 1u, err);
-      asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+      tc_fence_after();
       float* out_d = gram + ((size_t)blk * 128 + row) * 256;              // diagonal block of b
       float* out_c = gram + ((size_t)(blk + 1) * 128 + row) * 256 + 128;  // cross block of b + 1 (its row r = marker r of block b)
       float sxr = 0.0f;
       if (sx) {  // centred Gram (MRR3 centres every column): x_ci'x_ck = x_i'x_k - sx_i sx_k / n
         const int pos = blk * 128 + row;
         sxr = pos < p ? sx[perm[pos]] * inv_n : 0.0f;
-        asm volatile("bar.sync 1, 128;" ::: "memory");
+        named_bar(1, 128);
         for (int q = row; q < 256; q += 128) { const int pq = blk * 128 + q; S->sxc[q] = pq < p ? sx[perm[pq]] : 0.0f; }
-        asm volatile("bar.sync 1, 128;" ::: "memory");
+        named_bar(1, 128);
       }
 #pragma unroll
       for (int c = 0; c < 8; c++) {
         uint32_t v[32];
         const uint32_t taddr = tmem_base + ((uint32_t)(quarter * 32) << 16) + (uint32_t)c * 32u;
-        asm volatile(
-            "tcgen05.ld.sync.aligned.32x32b.x32.b32 "
-            "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, "
-            "%16, %17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31}, [%32];"
-            : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]),
-              "=r"(v[8]), "=r"(v[9]), "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15]),
-              "=r"(v[16]), "=r"(v[17]), "=r"(v[18]), "=r"(v[19]), "=r"(v[20]), "=r"(v[21]), "=r"(v[22]), "=r"(v[23]),
-              "=r"(v[24]), "=r"(v[25]), "=r"(v[26]), "=r"(v[27]), "=r"(v[28]), "=r"(v[29]), "=r"(v[30]), "=r"(v[31])
-            : "r"(taddr)
-            : "memory");
-        asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+        tmem_ld_x32(taddr, v);
+        tmem_ld_wait();
         if (sx) {
 #pragma unroll
           for (int q = 0; q < 32; q++) v[q] = __float_as_uint(fmaf(-sxr, S->sxc[c * 32 + q], __uint_as_float(v[q])));
@@ -249,18 +207,15 @@ __global__ void __launch_bounds__(kThreads, 1) gram_fp4_kernel(const uint8_t* __
 #pragma unroll
         for (int q = 0; q < 128; q += 4) *reinterpret_cast<uint4*>(gram + (size_t)row * 256 + 128 + q) = make_uint4(0, 0, 0, 0);
       }
-      asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+      tc_fence_before();
       __syncwarp();
       if (lane == 0) mbar_arrive(&S->tmem_empty);
     }
   }
 
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+  tc_fence_before();
   __syncthreads();
-  if (warp == 4) {
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(kTmemCols) : "memory");
-  }
+  if (warp == 4) tmem_dealloc(tmem_base, kTmemCols);
 }
 
 // int8 store -> the packed shadow this kernel reads: word k of a column = rows 16k .. 16k+15, nibble i = {row 16k+i, row 16k+8+i}

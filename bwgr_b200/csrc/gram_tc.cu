@@ -13,7 +13,7 @@
 // issues the MMAs (one elected lane) and owns the TMEM allocation, warps 5-8 drain the accumulator (tcgen05.ld -> st.global).
 // Two accumulator stages (2 x 128 TMEM columns) overlap the drain of block i with the MMAs of block i+1.
 // One CTA per SM, persistent over blocks.  HBM traffic: every genotype byte is read exactly once.
-#include "kernels.h"
+#include "device.cuh"
 
 namespace bwgr {
 
@@ -30,58 +30,6 @@ template <int NBAND> struct GramCfg {
   static constexpr int kStages = 3;
   static constexpr int kLag = 2;
 };
-constexpr uint32_t kSpinLimit = 1u << 22;
-
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-
-// one elected lane of a converged warp: the form ptxas turns into back-to-back UTC*MMA issue (a plain `lane == 0`
-// branch makes it wrap every tcgen05.mma in a per-lane loop, ~250 cycles per instruction)
-__device__ __forceinline__ bool elect_one() {
-  uint32_t pred;
-  asm volatile("{\n\t.reg .pred P;\n\telect.sync _|P, 0xffffffff;\n\tselp.u32 %0, 1, 0, P;\n\t}" : "=r"(pred));
-  return pred != 0;
-}
-__device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count));
-}
-__device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-// Bounded wait: a protocol bug must not hang the GPU (it sets *err and lets the kernel drain).
-__device__ __forceinline__ bool mbar_wait(uint64_t* bar, uint32_t parity, int* err) {
-  const uint32_t addr = smem_u32(bar);
-  for (uint32_t spin = 0; spin < kSpinLimit; spin++) {
-    uint32_t done;
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-        "selp.u32 %0, 1, 0, p;\n\t}"
-        : "=r"(done)
-        : "r"(addr), "r"(parity)
-        : "memory");
-    if (done) return true;
-  }
-  atomicExch(err, 2);
-  return false;
-}
-
-__device__ __forceinline__ void cp_async16_zfill(uint32_t dst, const void* src, uint32_t src_bytes) {
-  asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(dst), "l"(src), "r"(src_bytes) : "memory");
-}
-
-__device__ __forceinline__ uint64_t make_desc_sw128(uint32_t saddr) {
-  uint64_t d = 0;
-  d |= (uint64_t)((saddr & 0x3FFFFu) >> 4);  // start address, 16 B units
-  d |= (uint64_t)1 << 16;                    // leading byte offset (unused for swizzled K-major) = 16 B
-  d |= (uint64_t)(1024 >> 4) << 32;          // stride byte offset: 8 rows x 128 B
-  d |= (uint64_t)1 << 46;                    // descriptor version (Blackwell)
-  d |= (uint64_t)2 << 61;                    // SWIZZLE_128B
-  return d;
-}
-
-// kind::i8, D = S32, A = B = signed int8, both K-major, M = 128, N = 128.
-constexpr uint32_t kIdescI8 = (2u << 4) | (1u << 7) | (1u << 10) | ((128u >> 3) << 17) | ((128u >> 4) << 24);
-
 // kind::f8f6f4 with both operands E4M3 and an F32 accumulator.  Genotype codes 0..7 stored as int8 are, read as E4M3,
 // the subnormals code * 2^-9: the SAME bytes feed this (4x faster) instruction, every product code_i*code_j*2^-18 is
 // exact, and so is the fp32 sum while max_j xx_j < 2^24 -- the epilogue rescales by 2^18 and lands on the exact integer.
@@ -93,17 +41,6 @@ __device__ __forceinline__ void umma_f8(uint32_t tmem_d, uint64_t adesc, uint64_
       "tcgen05.mma.cta_group::1.kind::f8f6f4 [%0], %1, %2, %3, p;\n\t}"
       ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
       : "memory");
-}
-__device__ __forceinline__ void umma_i8(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::i8 [%0], %1, %2, %3, p;\n\t}"
-      ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-__device__ __forceinline__ void umma_commit(uint64_t* bar) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");
 }
 
 template <int NBAND>
@@ -135,15 +72,12 @@ __global__ void __launch_bounds__(416, 1) gram_tc_kernel(GenoView g, const int* 
   if (threadIdx.x == 0) {
     for (int s = 0; s < kStages; s++) { mbar_init(&S->full[s], PACKED ? 256 : 128); mbar_init(&S->empty[s], 1); }
     for (int s = 0; s < 2; s++) { mbar_init(&S->tmem_full[s], 1); mbar_init(&S->tmem_empty[s], 4); }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    fence_mbar_init();
   }
-  if (warp == 4) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&S->tmem_base)), "r"(2u * kAccCols) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+  if (warp == 4) tmem_alloc(&S->tmem_base, 2u * kAccCols);
+  tc_fence_before();
   __syncthreads();
-  asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+  tc_fence_after();
   const uint32_t tmem_base = S->tmem_base;
 
   if (PACKED && (warp < 4 || warp >= 9)) {
@@ -207,7 +141,7 @@ __global__ void __launch_bounds__(416, 1) gram_tc_kernel(GenoView g, const int* 
                            "r"((w4[q] >> 6) & 0x03030303u) : "memory");
             }
           }
-        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+        fence_proxy_async();
         mbar_arrive(&S->full[stage]);
         if (kg + 1 < nkg) {
 #pragma unroll
@@ -252,17 +186,17 @@ __global__ void __launch_bounds__(416, 1) gram_tc_kernel(GenoView g, const int* 
               }
           }
         }
-        asm volatile("cp.async.commit_group;" ::: "memory");
+        cp_async_commit();
         if (it >= kLag) {
-          asm volatile("cp.async.wait_group %0;" ::"n"(kLag) : "memory");
-          asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+          cp_async_wait<kLag>();
+          fence_proxy_async();
           mbar_arrive(&S->full[(it - kLag) % kStages]);
         }
       }
     }
     // drain: signal the last (up to kLag) tiles
-    asm volatile("cp.async.wait_group 0;" ::: "memory");
-    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+    cp_async_wait<0>();
+    fence_proxy_async();
     for (uint32_t q = (it > kLag ? it - kLag : 0); q < it; q++) mbar_arrive(&S->full[q % kStages]);
   } else if (warp == 4) {
     // ===================== MMA issuer =====================
@@ -271,21 +205,21 @@ __global__ void __launch_bounds__(416, 1) gram_tc_kernel(GenoView g, const int* 
     for (int blk = blockIdx.x; blk < nblocks && ok; blk += gridDim.x, bi++) {
       const uint32_t as = bi & 1u, aphase = (bi >> 1) & 1u;
       ok = mbar_wait(&S->tmem_empty[as], aphase ^ 1u, err);
-      asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+      tc_fence_after();
       const uint32_t tmem_d = tmem_base + as * kAccCols;
       for (int kg = 0; kg < nkg && ok; kg++, it++) {
         const uint32_t stage = it % kStages, phase = (it / kStages) & 1u;
         ok = mbar_wait(&S->full[stage], phase, err);
-        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+        tc_fence_after();
         if (elect_one()) {
 #pragma unroll
           for (int sub = 0; sub < kSub; sub++) {
             const int kt = kg * kSub + sub;
             if (kt < nkt) {
-              const uint64_t desc = make_desc_sw128(smem_u32(tiles + stage * kStageBytes + sub * NBAND * kTileBytes));
+              const uint64_t desc = desc_k_sw128(smem_u32(tiles + stage * kStageBytes + sub * NBAND * kTileBytes));
 #pragma unroll
               for (int d = 0; d < NBAND; d++) {
-                const uint64_t bdesc = make_desc_sw128(smem_u32(tiles + stage * kStageBytes + (sub * NBAND + d) * kTileBytes));
+                const uint64_t bdesc = desc_k_sw128(smem_u32(tiles + stage * kStageBytes + (sub * NBAND + d) * kTileBytes));
 #pragma unroll
                 for (int k4 = 0; k4 < 4; k4++) {
                   // band d >= 1 is stored transposed: row r = marker r of block b-d, columns = markers of block b, so that
@@ -295,8 +229,8 @@ __global__ void __launch_bounds__(416, 1) gram_tc_kernel(GenoView g, const int* 
                     if (d == 0) umma_f8(tmem_d, desc + (uint64_t)(k4 * 2), desc + (uint64_t)(k4 * 2), kIdescF8, acc);
                     else umma_f8(tmem_d + (uint32_t)d * 128u, bdesc + (uint64_t)(k4 * 2), desc + (uint64_t)(k4 * 2), kIdescF8, acc);
                   } else {
-                    if (d == 0) umma_i8(tmem_d, desc + (uint64_t)(k4 * 2), desc + (uint64_t)(k4 * 2), kIdescI8, acc);
-                    else umma_i8(tmem_d + (uint32_t)d * 128u, bdesc + (uint64_t)(k4 * 2), desc + (uint64_t)(k4 * 2), kIdescI8, acc);
+                    if (d == 0) umma_i8(tmem_d, desc + (uint64_t)(k4 * 2), desc + (uint64_t)(k4 * 2), idesc_i8(128, 0), acc);
+                    else umma_i8(tmem_d + (uint32_t)d * 128u, bdesc + (uint64_t)(k4 * 2), desc + (uint64_t)(k4 * 2), idesc_i8(128, 0), acc);
                   }
                 }
               }
@@ -318,7 +252,7 @@ __global__ void __launch_bounds__(416, 1) gram_tc_kernel(GenoView g, const int* 
     for (int blk = blockIdx.x; blk < nblocks && ok; blk += gridDim.x, bi++) {
       const uint32_t as = bi & 1u, aphase = (bi >> 1) & 1u;
       ok = mbar_wait(&S->tmem_full[as], aphase, err);
-      asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+      tc_fence_after();
       int32_t* out = gram + ((size_t)blk * 128 + row) * (NBAND * 128);
       // centred Gram (MRR3 centres every column, RcppEigen20230423.cpp:378-379): x_ci'x_ck = x_i'x_k - sx_i sx_k / n
       float sxr0 = 0.0f, sxr1 = 0.0f;
@@ -326,25 +260,16 @@ __global__ void __launch_bounds__(416, 1) gram_tc_kernel(GenoView g, const int* 
         const int pos0 = blk * 128 + row, pos1 = (blk - 1) * 128 + row;
         sxr0 = pos0 < g.p ? sx[perm[pos0]] : 0.0f;
         sxr1 = (pos1 >= 0 && pos1 < g.p) ? sx[perm[pos1]] : 0.0f;
-        asm volatile("bar.sync 1, 128;" ::: "memory");  // previous block's reads of sxc are done
+        named_bar(1, 128);  // previous block's reads of sxc are done
         S->sxc[row] = sxr0;
-        asm volatile("bar.sync 1, 128;" ::: "memory");
+        named_bar(1, 128);
       }
 #pragma unroll
       for (int c = 0; c < 4 * NBAND; c++) {
         uint32_t v[32];
         const uint32_t taddr = tmem_base + ((uint32_t)(quarter * 32) << 16) + as * kAccCols + (uint32_t)c * 32u;
-        asm volatile(
-            "tcgen05.ld.sync.aligned.32x32b.x32.b32 "
-            "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, "
-            "%16, %17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31}, [%32];"
-            : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]),
-              "=r"(v[8]), "=r"(v[9]), "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15]),
-              "=r"(v[16]), "=r"(v[17]), "=r"(v[18]), "=r"(v[19]), "=r"(v[20]), "=r"(v[21]), "=r"(v[22]), "=r"(v[23]),
-              "=r"(v[24]), "=r"(v[25]), "=r"(v[26]), "=r"(v[27]), "=r"(v[28]), "=r"(v[29]), "=r"(v[30]), "=r"(v[31])
-            : "r"(taddr)
-            : "memory");
-        asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+        tmem_ld_x32(taddr, v);
+        tmem_ld_wait();
         if (FP8) {  // accumulator = exact integer * 2^-18 in fp32
 #pragma unroll
           for (int q = 0; q < 32; q++) {
@@ -366,18 +291,15 @@ __global__ void __launch_bounds__(416, 1) gram_tc_kernel(GenoView g, const int* 
             *reinterpret_cast<uint4*>(out + c * 32 + q) = make_uint4(v[q], v[q + 1], v[q + 2], v[q + 3]);
         }
       }
-      asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+      tc_fence_before();
       __syncwarp();
       if (lane == 0) mbar_arrive(&S->tmem_empty[as]);
     }
   }
 
-  asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+  tc_fence_before();
   __syncthreads();
-  if (warp == 4) {
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(2u * kAccCols) : "memory");
-  }
+  if (warp == 4) tmem_dealloc(tmem_base, 2u * kAccCols);
 }
 
 }  // namespace

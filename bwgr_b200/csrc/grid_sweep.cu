@@ -5,13 +5,12 @@
 //
 // One persistent cooperative grid; CTA c keeps its row slab of the residuals (and masks) of all systems in shared memory for the whole
 // sweep and streams its slab of the genotype columns in marker order through a cp.async ring.  Per marker: slab dot products -> ONE
-// grid-wide sum through L2 -> the rule, evaluated by every CTA alike -> rank-one update of the slab.  The grid sum: each CTA adds its
-// fixed-point partial to the marker's own 64-bit accumulator word with one atomic per system; the low byte of a word counts the
-// arrivals, so the data is its own flag (one L2 hop, no fence, no barrier).  Integer sums are order-free: every CTA reads bit-identical
-// totals, takes bit-identical decisions, and a fit is bit-reproducible.  Same-address atomics serialise in L2, so CTA c adds to copy
-// c % 8 of the word.  The per-marker chain is latency-bound (~2-3 us per marker): this family is the fallback, not the fast path.
+// grid-wide sum through L2 (the accumulator word of device.cuh, one atomic per system and CTA) -> the rule, evaluated by every CTA
+// alike -> rank-one update of the slab.  The integer sums are order-free: every CTA reads bit-identical totals, takes bit-identical
+// decisions, and a fit is bit-reproducible.  The per-marker chain is latency-bound (~2-3 us per marker): this family is the fallback,
+// not the fast path.
 // HBM traffic per sweep: n p bytes.
-#include "kernels.h"
+#include "device.cuh"
 
 namespace bwgr {
 
@@ -19,29 +18,6 @@ namespace {
 
 constexpr int kT = 256;  // threads per CTA
 constexpr int kD = 4;    // markers in flight
-constexpr int kC = kGridCopies;
-
-__device__ __forceinline__ void gcp16(void* smem, const void* gmem) {
-  const uint32_t s = (uint32_t)__cvta_generic_to_shared(smem);
-  asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(s), "l"(gmem) : "memory");
-}
-__device__ __forceinline__ void gcp4(void* smem, const void* gmem) {
-  const uint32_t s = (uint32_t)__cvta_generic_to_shared(smem);
-  asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(s), "l"(gmem) : "memory");
-}
-__device__ __forceinline__ void gcp_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
-template <int N>
-__device__ __forceinline__ void gcp_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
-__device__ __forceinline__ unsigned long long gld_relaxed(const unsigned long long* p) {
-  unsigned long long v;
-  asm volatile("ld.relaxed.gpu.global.u64 %0, [%1];" : "=l"(v) : "l"(p) : "memory");
-  return v;
-}
-__device__ __forceinline__ unsigned long long gtimer() {
-  unsigned long long t;
-  asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t));
-  return t;
-}
 
 struct GridSmem {
   float* E;          // [ns][rp]
@@ -105,26 +81,26 @@ __global__ void __launch_bounds__(kT, 1) grid_sweep_kernel(GridArgs a) {
       const unsigned char* col = sizeof(XT) == 1 ? reinterpret_cast<const unsigned char*>(a.g.x8 + (int64_t)J * ld + r0)
                                                  : reinterpret_cast<const unsigned char*>(a.g.xf + (int64_t)J * ld + r0);
       for (int c = tid; c < nch; c += kT)
-        if (r0 + (int64_t)kRowsPerChunk * c < ld) gcp16(s.xs[slot] + 16 * c, col + 16 * c);
+        if (r0 + (int64_t)kRowsPerChunk * c < ld) cp_async16(s.xs[slot] + 16 * c, col + 16 * c);
       float* v = s.vin[slot];
-      if (tid < 32) { if (tid < ns) gcp4(v + tid, a.b + (size_t)tid * p + J); }
-      else if (tid < 64) { const int t = tid - 32; if (t < ns && a.vbv) gcp4(v + 32 + t, a.vbv + (size_t)t * p + J); }
-      else if (tid < 96) { const int t = tid - 64; if (t < ns) gcp4(v + 64 + t, xxbase + (a.xx_per_sys ? (size_t)t * p : 0) + J); }
-      else if (tid == 96 && a.xx2) gcp4(v + 96, a.xx2 + J);
+      if (tid < 32) { if (tid < ns) cp_async4(v + tid, a.b + (size_t)tid * p + J); }
+      else if (tid < 64) { const int t = tid - 32; if (t < ns && a.vbv) cp_async4(v + 32 + t, a.vbv + (size_t)t * p + J); }
+      else if (tid < 96) { const int t = tid - 64; if (t < ns) cp_async4(v + 64 + t, xxbase + (a.xx_per_sys ? (size_t)t * p : 0) + J); }
+      else if (tid == 96 && a.xx2) cp_async4(v + 96, a.xx2 + J);
       if (tid == 0) s.Js[slot] = J;
     }
-    gcp_commit();
+    cp_async_commit();
   };
   __syncthreads();  // the zeroed ring slots are in place before any cp.async lands in them
   for (int m = 0; m < kD - 1; m++) prefetch(m);
   __syncthreads();
   if (model_is_gibbs(MODEL) && warp == 1 && lane < ns)  // draws of marker 0
     s.dr[lane] = marker_draws(MODEL, (uint32_t)s.Js[0], (uint32_t)s.sc[lane].sweep, (uint32_t)(a.chain0 + lane), s.sc[lane].df, a.seed_lo, a.seed_hi);
-  const unsigned long long t_start = gtimer();
+  const unsigned long long t_start = globaltimer_ns();
   const double inv_q = (double)a.g_quantum;  // value of one fixed-point unit
   const double qinv = 1.0 / (double)a.g_quantum;
   for (int m = 0; m < p; m++) {
-    gcp_wait<kD - 2>();
+    cp_async_wait<kD - 2>();
     __syncthreads();  // marker m's slot has landed; step m - 1 is finished by every thread
     prefetch(m + kD - 1);
     const int slot = m % kD;
@@ -164,35 +140,10 @@ __global__ void __launch_bounds__(kT, 1) grid_sweep_kernel(GridArgs a) {
         double v = 0.0;
 #pragma unroll
         for (int w = 0; w < 8; w++) v += (double)s_wred[w][lane];
-        v *= qinv;
-        if (!(fabs(v) < 4503599627370496.0)) atomicExch(a.err, 4);  // 2^52: the fixed-point range of g is exceeded
-        atomicAdd(a.acc + ((size_t)m * kC + (cta & (kC - 1))) * 32 + lane, ((unsigned long long)__double2ll_rn(v) << 8) + 1ull);
+        grid_add(a.acc + ((size_t)m * kGridCopies + (cta & (kGridCopies - 1))) * 32 + lane, v * qinv, a.err);
       }
-      // the marker's totals: a word is complete when its low byte counts all the CTAs that add to that copy
-      const unsigned long long* accw = a.acc + (size_t)m * kC * 32 + (on ? lane : 0);
-      unsigned long long w[kC];
-      unsigned int spins = 0;
-      for (;;) {
-        bool pending = false;
-#pragma unroll
-        for (int c = 0; c < kC; c++) w[c] = gld_relaxed(accw + c * 32);
-#pragma unroll
-        for (int c = 0; c < kC; c++) pending |= (int)(w[c] & 0xffull) != (G + kC - 1 - c) / kC;
-        if (!__any_sync(0xffffffffu, on && pending)) break;
-        if ((++spins & 0xfffu) == 0) {
-          int ab = 0;
-          if (lane == 0) {
-            if (*reinterpret_cast<volatile int*>(a.err) != 0) ab = 1;
-            else if (gtimer() - t_start > 120000000000ull) { atomicExch(a.err, 3); ab = 1; }  // two minutes without the grid
-            if (ab) s_abort = 1;
-          }
-          if (__shfl_sync(0xffffffffu, ab, 0)) break;
-        }
-      }
+      const long long tot = grid_wait_total(a.acc + (size_t)m * kGridCopies * 32 + (on ? lane : 0), on, G, a.err, t_start, &s_abort);
       if (on) {
-        long long tot = 0;
-#pragma unroll
-        for (int c = 0; c < kC; c++) tot += (long long)w[c] >> 8;
         const float g = (float)((double)tot * inv_q);
         const SysScalars& sc = s.sc[lane];
         float de = 0.0f;
@@ -231,7 +182,7 @@ __global__ void __launch_bounds__(kT, 1) grid_sweep_kernel(GridArgs a) {
       }
     }
   }
-  gcp_wait<0>();
+  cp_async_wait<0>();
   __syncthreads();
   for (int q = tid; q < ns * rp; q += kT) {
     const int t = q / rp, i = q - t * rp;
@@ -252,7 +203,6 @@ constexpr int kGP = kGB * (kGB - 1) / 2;      // cross products per block
 constexpr int kGR = 3;                        // blocks in flight
 constexpr int kJR = kGR + 1;                  // marker indices are staged one block further ahead
 constexpr int kTB = 1024;                     // threads per CTA of the blocked variant: its phases are short dependent chains, 32 warps hide them
-constexpr int kCB = kGridCopies;              // accumulator copies (power of two; 4, 8, 16 measured alike)
 static_assert(kGB <= 32 && kGB * 32 + kGP <= kTB, "one dot warp per marker, one polling thread per word");
 
 struct GridBlockSmem {
@@ -334,7 +284,7 @@ __global__ void __launch_bounds__(kTB, 1) grid_block_kernel(GridArgs a) {
         if (r0 + (int64_t)kRowsPerChunk * c < ld) {
           const int64_t off = (int64_t)Jv[j] * ld + r0;
           const unsigned char* col = sizeof(XT) == 1 ? reinterpret_cast<const unsigned char*>(a.g.x8 + off) : reinterpret_cast<const unsigned char*>(a.g.xf + off);
-          gcp16(s.xs[slot] + (size_t)j * rp * sizeof(XT) + 16 * c, col + 16 * c);
+          cp_async16(s.xs[slot] + (size_t)j * rp * sizeof(XT) + 16 * c, col + 16 * c);
         }
       }
       // the markers' inputs (b0 | vb_j | xx per system), dealt from the other end of the CTA
@@ -343,13 +293,13 @@ __global__ void __launch_bounds__(kTB, 1) grid_block_kernel(GridArgs a) {
         if (t < ns) {
           const int J = Jv[j];
           float* v = s.vin[slot] + j * 100 + 32 * w + t;
-          if (w == 0) gcp4(v, a.b + (size_t)t * p + J);
-          else if (w == 1) { if (a.vbv) gcp4(v, a.vbv + (size_t)t * p + J); }
-          else gcp4(v, a.xx + (a.xx_per_sys ? (size_t)t * p : 0) + J);
+          if (w == 0) cp_async4(v, a.b + (size_t)t * p + J);
+          else if (w == 1) { if (a.vbv) cp_async4(v, a.vbv + (size_t)t * p + J); }
+          else cp_async4(v, a.xx + (a.xx_per_sys ? (size_t)t * p : 0) + J);
         }
       }
     }
-    gcp_commit();
+    cp_async_commit();
   };
   auto draws_for = [&](int blk) {  // Gibbs draws of a block's markers, one (marker, system) per thread of warps 1..7
     if (!model_is_gibbs(MODEL) || blk >= nblk) return;
@@ -361,7 +311,7 @@ __global__ void __launch_bounds__(kTB, 1) grid_block_kernel(GridArgs a) {
                                                           s.sc[t].df, a.seed_lo, a.seed_hi);
     }
   };
-  const unsigned long long t_start = gtimer();
+  const unsigned long long t_start = globaltimer_ns();
   const double inv_q = (double)a.g_quantum, qinv = 1.0 / (double)a.g_quantum;
   const double inv_qG = (double)a.gram_quantum, qinvG = 1.0 / (double)a.gram_quantum;
   // cross products x_j'x_i (i < j) of a block: E-independent, so they are summed over the grid one block AHEAD of their use -- while the
@@ -369,7 +319,7 @@ __global__ void __launch_bounds__(kTB, 1) grid_block_kernel(GridArgs a) {
   auto cross_tasks = [&](int blk, int w0) {
     if (blk >= nblk) return;
     const XT* xs = reinterpret_cast<const XT*>(s.xs[blk % kGR]);
-    unsigned long long* accw = a.acc + ((size_t)blk * kCB + (cta & (kCB - 1))) * W + ndot;
+    unsigned long long* accw = a.acc + ((size_t)blk * kGridCopies + (cta & (kGridCopies - 1))) * W + ndot;
     for (int pr = warp - w0; pr < kGP; pr += kTB / 32 - w0) {
       const int j = s.pj[pr], i2 = pr - j * (j - 1) / 2;
       double v;
@@ -388,7 +338,7 @@ __global__ void __launch_bounds__(kTB, 1) grid_block_kernel(GridArgs a) {
         for (int q = lane; q < rp; q += 32) acc = fmaf(fj[q], fi[q], acc);
         v = (double)warp_sum(acc) * qinvG;
       }
-      if (lane == 0) atomicAdd(accw + pr, ((unsigned long long)__double2ll_rn(v) << 8) + 1ull);
+      if (lane == 0) atomicAdd(accw + pr, grid_word(v));
     }
   };
   const int nw = ndot + kGP;            // words of a block: one polling thread each (nw <= 16 * 32 + 120 < kTB)
@@ -397,17 +347,17 @@ __global__ void __launch_bounds__(kTB, 1) grid_block_kernel(GridArgs a) {
   __syncthreads();
   for (int b = 0; b < kGR - 1; b++) prefetch(b);
   draws_for(0);
-  gcp_wait<0>();
+  cp_async_wait<0>();
   __syncthreads();
   cross_tasks(0, 0);
   for (int blk = 0; blk < nblk; blk++) {
-    gcp_wait<0>();    // block blk + 1's slab (issued one whole block ago) has landed, block blk's long since
+    cp_async_wait<0>();    // block blk + 1's slab (issued one whole block ago) has landed, block blk's long since
     __syncthreads();  // ... for every thread; block blk - 1 is finished by every thread
     prefetch(blk + kGR - 1);
     const int slot = blk % kGR, nb = min(kGB, p - blk * kGB);
     const int* Jcur = s.Js[blk % kJR];
     const XT* xs = reinterpret_cast<const XT*>(s.xs[slot]);
-    unsigned long long* accw = a.acc + ((size_t)blk * kCB + (cta & (kCB - 1))) * W;
+    unsigned long long* accw = a.acc + ((size_t)blk * kGridCopies + (cta & (kGridCopies - 1))) * W;
     // ---- the block's dot tasks (marker j with the residuals as they stand), one warp each
     if (warp < nb) {
       const int j = warp;
@@ -416,10 +366,7 @@ __global__ void __launch_bounds__(kTB, 1) grid_block_kernel(GridArgs a) {
         float acc = 0.0f;
         for (int i = lane; i < rp; i += 32) acc = fmaf((float)xj[i], s.E[i], acc);
         const double v = (double)warp_sum(acc) * qinv;
-        if (lane == 0) {
-          if (!(fabs(v) < 4503599627370496.0)) atomicExch(a.err, 4);
-          atomicAdd(accw + j, ((unsigned long long)__double2ll_rn(v) << 8) + 1ull);
-        }
+        if (lane == 0) grid_add(accw + j, v, a.err);
       } else {
         for (int t0 = 0; t0 < ns; t0 += 4) {
           const int nt = min(4, ns - t0);
@@ -434,10 +381,7 @@ __global__ void __launch_bounds__(kTB, 1) grid_block_kernel(GridArgs a) {
           for (int q = 0; q < 4; q++) {
             if (q < nt) {
               const double v = (double)warp_sum(acc[q]) * qinv;
-              if (lane == 0) {
-                if (!(fabs(v) < 4503599627370496.0)) atomicExch(a.err, 4);
-                atomicAdd(accw + j * ns + t0 + q, ((unsigned long long)__double2ll_rn(v) << 8) + 1ull);
-              }
+              if (lane == 0) grid_add(accw + j * ns + t0 + q, v, a.err);
             }
           }
         }
@@ -448,21 +392,21 @@ __global__ void __launch_bounds__(kTB, 1) grid_block_kernel(GridArgs a) {
       cross_tasks(blk + 1, npollw);  // next block's cross products, under this block's wait
     } else if (tid < nw && !(tid < ndot && tid / ns >= nb)) {  // markers past the end of the last block are never added
       // ---- the block's totals, one word per polling thread: a word is complete when its low byte counts all the CTAs of its copy
-      const unsigned long long* src = a.acc + (size_t)blk * kCB * W + tid;
+      const unsigned long long* src = a.acc + (size_t)blk * kGridCopies * W + tid;
       unsigned int spins = 0;
       for (;;) {
         long long tot = 0;
         bool done = true;
 #pragma unroll
-        for (int c = 0; c < kCB; c++) {
-          const unsigned long long w = gld_relaxed(src + (size_t)c * W);
-          done &= (int)(w & 0xffull) == (G + kCB - 1 - c) / kCB;
-          tot += (long long)w >> 8;
+        for (int c = 0; c < kGridCopies; c++) {
+          const unsigned long long w = ld_relaxed_u64(src + (size_t)c * W);
+          done &= grid_word_count(w) == grid_copy_count(G, c);
+          tot += grid_word_value(w);
         }
         if (done) { s.tot[tid] = (float)((double)tot * (tid < ndot ? inv_q : inv_qG)); break; }
         if ((++spins & 0x3ffu) == 0) {
           if (*reinterpret_cast<volatile int*>(a.err) != 0) { s_abort = 1; break; }
-          if (gtimer() - t_start > 120000000000ull) { atomicExch(a.err, 3); s_abort = 1; break; }  // two minutes without the grid
+          if (globaltimer_ns() - t_start > kGridTimeoutNs) { atomicExch(a.err, 3); s_abort = 1; break; }
         }
       }
     }
@@ -514,7 +458,7 @@ __global__ void __launch_bounds__(kTB, 1) grid_block_kernel(GridArgs a) {
       }
     }
   }
-  gcp_wait<0>();
+  cp_async_wait<0>();
   __syncthreads();
   for (int q = tid; q < ns * rp; q += kTB) {
     const int t = q / rp, i = q - t * rp;
@@ -547,7 +491,7 @@ cudaError_t launch_grid_model(const GridArgs& a, int grid, cudaStream_t st) {
 size_t grid_block_smem(int nsys, int rows_per_cta, bool real_store, bool gibbs) {
   return grid_block_carve(nullptr, nsys, rows_per_cta, real_store ? 4 : 1, gibbs, nullptr) + 16;
 }
-size_t grid_block_acc_words(int nsys, int p) { return (size_t)((p + kGB - 1) / kGB) * kCB * grid_block_words(nsys); }
+size_t grid_block_acc_words(int nsys, int p) { return (size_t)((p + kGB - 1) / kGB) * kGridCopies * grid_block_words(nsys); }
 
 size_t grid_sweep_smem(int nsys, int rows_per_cta, bool masked, bool real_store) {
   return grid_carve(nullptr, nsys, rows_per_cta, masked, real_store ? 4 : 1, nullptr) + 16;

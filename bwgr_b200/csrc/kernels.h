@@ -201,7 +201,9 @@ void launch_pair_reduce(const float* A, const float* B, int64_t lda, int64_t ldb
                         cudaStream_t st);
 
 // ---- grid family (grid_sweep.cu): the per-marker step with the individuals spread over the whole GPU; any n, row masks, every rule ----
-constexpr int kGridCopies = 8;  // accumulator copies per marker (power of two)
+// copies of each L2 grid-sum word of the grid family and the general MRR3 sweep (the word format is in device.cuh); a power of two
+// (4, 8 and 16 measured alike with grid_block_kernel)
+constexpr int kGridCopies = 8;
 struct GridArgs {
   GenoView g;
   int model;
@@ -229,7 +231,6 @@ size_t grid_sweep_smem(int nsys, int rows_per_cta, bool masked, bool real_store)
 cudaError_t launch_grid_sweep(const GridArgs& a, int grid, cudaStream_t st);
 
 // ---- general multivariate ridge sweep (mrr_gen.cu): missing phenotypes, InnerGS, marker weights, NoInv, TH --------------
-constexpr int kMrrGenCopies = 8;  // accumulator copies per marker (power of two)
 struct MrrGenArgs {
   GenoView g;
   int k;
@@ -244,7 +245,7 @@ struct MrrGenArgs {
   const double* mean;     // [p] column means
   const double* sol;      // [p][nmat * k * k] from launch_mrr_gen_systems
   const double* se0;      // [k] column sums of e at launch
-  unsigned long long* acc;  // [p][kMrrGenCopies][32] the grid sums of marker position m: (fixed-point sum << 8) + arrivals; zeroed before launch
+  unsigned long long* acc;  // [p][kGridCopies][32] the grid sums of marker position m: (fixed-point sum << 8) + arrivals; zeroed before launch
   const double* scale;    // [64]: fixed-point scale of trait t (a power of two) | its inverse
   int* err;
 };

@@ -10,13 +10,12 @@
 //   * mrr_gen_sweep_kernel: one persistent cooperative grid; CTA c keeps its row slab of the k residual columns and of the
 //     observation mask in shared memory for the whole sweep (float64: this path is the reference's MRR3 arithmetic), streams
 //     its slab of the genotype columns in marker order through a cp.async ring together with the marker's matrix and
-//     vectors, and per marker: slab dot products -> one grid-wide sum through L2 (each warp adds its fixed-point partials to the
-//     marker's own 64-bit accumulator words with one atomic each; the low byte of a word counts the arrivals, so the data is its
-//     own flag: one L2 hop, no fence, no barrier; integer sums are order-free, so all CTAs read bit-identical totals and no
+//     vectors, and per marker: slab dot products -> one grid-wide sum through L2 (the accumulator words of device.cuh: each warp
+//     adds its fixed-point partials with one atomic each; integer sums are order-free, so all CTAs read bit-identical totals and no
 //     broadcast is needed) -> mat-vec (or the inner Gauss-Seidel walk) -> masked rank-one update of the slab.  Column centring (:378-379) is analytic: x_c'e = x'e - mean_J * sum(e), with the
 //     running column sums of e carried in registers.
 // HBM traffic per sweep: n p bytes of genotypes + 8 k^2 p bytes of matrices; the bound is the grid sum's latency per marker.
-#include "kernels.h"
+#include "device.cuh"
 
 namespace bwgr {
 
@@ -24,28 +23,10 @@ namespace {
 
 constexpr int kGT = 256;  // threads of a sweep CTA
 constexpr int kGD = 4;    // ring depth (markers in flight)
-constexpr int kGC = kMrrGenCopies;  // copies of a marker's accumulator words: CTA c adds to copy c % kGC (same-address atomics serialise in L2)
 
-__device__ __forceinline__ void cpa16(void* smem, const void* gmem) {
-  const uint32_t s = (uint32_t)__cvta_generic_to_shared(smem);
-  asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(s), "l"(gmem) : "memory");
-}
-__device__ __forceinline__ void cpa8(void* smem, const void* gmem) {
-  const uint32_t s = (uint32_t)__cvta_generic_to_shared(smem);
-  asm volatile("cp.async.ca.shared.global [%0], [%1], 8;" ::"r"(s), "l"(gmem) : "memory");
-}
-__device__ __forceinline__ void cpa_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
-template <int N>
-__device__ __forceinline__ void cpa_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
-__device__ __forceinline__ unsigned long long ld_relaxed_u64(const unsigned long long* p) {
-  unsigned long long v;
-  asm volatile("ld.relaxed.gpu.global.u64 %0, [%1];" : "=l"(v) : "l"(p) : "memory");
-  return v;
-}
-__device__ __forceinline__ unsigned long long globaltimer_ns() {
-  unsigned long long t;
-  asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t));
-  return t;
+// 8 B, through L1
+__device__ __forceinline__ void cp_async8(void* smem, const void* gmem) {
+  asm volatile("cp.async.ca.shared.global [%0], [%1], 8;" ::"r"(smem_u32(smem)), "l"(gmem) : "memory");
 }
 __device__ __forceinline__ double shfl_d(double v, int src) { return __shfl_sync(0xffffffffu, v, src); }
 
@@ -240,22 +221,22 @@ __global__ void __launch_bounds__(kGT, 1) mrr_gen_sweep_kernel(MrrGenArgs a) {
       if (m + 1 < p) Jnext = a.perm[m + 1];
       const int8_t* col = a.g.x8 + (int64_t)J * a.g.ld + r0;
       for (int c = tid; c < nch; c += kGT)
-        if (r0 + 16 * c < a.g.ld) cpa16(s.xs[slot] + 16 * c, col + 16 * c);  // rows past the padded column stay as they are: e = z = 0 there
+        if (r0 + 16 * c < a.g.ld) cp_async16(s.xs[slot] + 16 * c, col + 16 * c);  // rows past the padded column stay as they are: e = z = 0 there
       const double* src = a.sol + (size_t)J * nmat * kk;
-      for (int c = tid; c < nmat * kk; c += kGT) cpa8(s.mats[slot] + c, src + c);
-      if (tid < 2 * k) cpa8(s.vec[slot] + tid, a.fixed + (size_t)J * 2 * k + tid);
-      else if (tid < 3 * k) cpa8(s.vec[slot] + tid, a.b + (size_t)J * k + (tid - 2 * k));
-      else if (tid == 3 * k) cpa8(s.vec[slot] + 3 * k, a.mean + J);
+      for (int c = tid; c < nmat * kk; c += kGT) cp_async8(s.mats[slot] + c, src + c);
+      if (tid < 2 * k) cp_async8(s.vec[slot] + tid, a.fixed + (size_t)J * 2 * k + tid);
+      else if (tid < 3 * k) cp_async8(s.vec[slot] + tid, a.b + (size_t)J * k + (tid - 2 * k));
+      else if (tid == 3 * k) cp_async8(s.vec[slot] + 3 * k, a.mean + J);
       if (tid == 0) s.Js[slot] = J;
     }
-    cpa_commit();
+    cp_async_commit();
   };
   Jnext = a.perm[0];
   __syncthreads();  // the zeroed ring slots are in place before any cp.async lands in them
   for (int m = 0; m < kGD - 1; m++) prefetch(m);
   const unsigned long long t_start = globaltimer_ns();
   for (int m = 0; m < p; m++) {
-    cpa_wait<kGD - 2>();
+    cp_async_wait<kGD - 2>();
     __syncthreads();  // marker m's slot has landed for every thread; step m - 1 is finished by every thread
     prefetch(m + kGD - 1);
     const int slot = m % kGD;
@@ -284,48 +265,20 @@ __global__ void __launch_bounds__(kGT, 1) mrr_gen_sweep_kernel(MrrGenArgs a) {
           }
         }
       }
-      unsigned long long* accw = a.acc + ((size_t)m * kGC + (cta & (kGC - 1))) * 32;
+      unsigned long long* accw = a.acc + ((size_t)m * kGridCopies + (cta & (kGridCopies - 1))) * 32;
 #pragma unroll
       for (int q = 0; q < 4; q++) {
         const int t = warp + 8 * q;
         if (t < k) {
           const double v = warp_sum(acc[q]) * sc4[q];
-          if (lane == 0) {
-            if (!(fabs(v) < 4503599627370496.0)) atomicExch(a.err, 4);  // 2^52: the fixed-point range of this sweep is exceeded
-            atomicAdd(accw + t, ((unsigned long long)__double2ll_rn(v) << 8) + 1ull);
-          }
+          if (lane == 0) grid_add(accw + t, v, a.err);
         }
       }
     }
     if (warp == 0) {
       const bool on = lane < k;
-      double dot = 0.0;
-      {  // the marker's totals: word t is complete when its low byte counts all G CTAs
-        const unsigned long long* accw = a.acc + (size_t)m * kGC * 32 + (on ? lane : 0);
-        unsigned long long w[kGC];
-        unsigned int spins = 0;
-        for (;;) {
-          bool pending = false;
-#pragma unroll
-          for (int c = 0; c < kGC; c++) w[c] = ld_relaxed_u64(accw + c * 32);
-#pragma unroll
-          for (int c = 0; c < kGC; c++) pending |= (int)(w[c] & 0xffull) != (G + kGC - 1 - c) / kGC;  // CTAs with cta % kGC == c
-          if (!__any_sync(0xffffffffu, on && pending)) break;
-          if ((++spins & 0xfffu) == 0) {
-            int ab = 0;
-            if (lane == 0) {
-              if (*reinterpret_cast<volatile int*>(a.err) != 0) ab = 1;
-              else if (globaltimer_ns() - t_start > 120000000000ull) { atomicExch(a.err, 3); ab = 1; }  // two minutes without the grid
-              if (ab) s_abort = 1;
-            }
-            if (__shfl_sync(0xffffffffu, ab, 0)) break;
-          }
-        }
-        long long tot = 0;
-#pragma unroll
-        for (int c = 0; c < kGC; c++) tot += (long long)w[c] >> 8;
-        dot = (double)tot * inv_scale;
-      }
+      const long long tot = grid_wait_total(a.acc + (size_t)m * kGridCopies * 32 + (on ? lane : 0), on, G, a.err, t_start, &s_abort);
+      const double dot = (double)tot * inv_scale;
       const double XXt = on ? vec[lane] : 0.0, sxzc = on ? vec[k + lane] : 0.0, b0 = on ? vec[2 * k + lane] : 0.0;
       const double mean = vec[3 * k];
       const double r = on ? dot - mean * se + XXt * b0 : 0.0;  // x_c'e_t + XX(J,t) b0_t  (:506)
@@ -388,7 +341,7 @@ __global__ void __launch_bounds__(kGT, 1) mrr_gen_sweep_kernel(MrrGenArgs a) {
       }
     }
   }
-  cpa_wait<0>();
+  cp_async_wait<0>();
   __syncthreads();
   if constexpr (NJ > 0) {
 #pragma unroll

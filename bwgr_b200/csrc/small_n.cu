@@ -7,24 +7,12 @@
 // streamed from HBM/L2 through a cp.async ring in marker order (the order is known up front), and
 // the only block-wide synchronisation per marker is the one barrier of the dot-product reduction.
 // Independent systems = independent CTAs: no communication (SURVEY 8e, "replicas").
-#include "kernels.h"
+#include "device.cuh"
 
 namespace bwgr {
 
 namespace {
 
-
-__device__ __forceinline__ void cp_async16(void* smem, const void* gmem) {
-  const uint32_t s = (uint32_t)__cvta_generic_to_shared(smem);
-  asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(s), "l"(gmem) : "memory");
-}
-__device__ __forceinline__ void cp_async4(void* smem, const void* gmem) {
-  const uint32_t s = (uint32_t)__cvta_generic_to_shared(smem);
-  asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(s), "l"(gmem) : "memory");
-}
-__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
-template <int N>
-__device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
 
 // Expand 4 packed 2-bit bytes (16 rows) into 16 int8 bytes.
 __device__ __forceinline__ uint4 expand_2bit(uint32_t pk) {

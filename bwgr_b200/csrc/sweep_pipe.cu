@@ -28,7 +28,7 @@
 // both tensor-core passes, quantisation, L2 round trips) runs beside it.
 #include <string.h>
 
-#include "kernels.h"
+#include "device.cuh"
 
 namespace bwgr {
 
@@ -46,10 +46,6 @@ constexpr int kRing = 8;               // blocks of partial / reduced h kept in 
 constexpr int kWPad = 160;             // worker slots per (block, system, marker) row of the partials
 constexpr int kRedWarp = 9;            // worker warp that reduces its share of the partials
 
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void cp_async16(uint32_t dst, const void* src, uint32_t nbytes) {
-  asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(dst), "l"(src), "r"(nbytes) : "memory");
-}
 // genotype bytes are streamed once per sweep: L2 evict-first keeps the small hot arrays (Gram band, b, xx, order) resident
 __device__ __forceinline__ uint64_t policy_evict_first() {
   uint64_t pol;
@@ -60,21 +56,6 @@ __device__ __forceinline__ void cp_async16_stream(uint32_t dst, const void* src,
   asm volatile("cp.async.cg.shared.global.L2::cache_hint [%0], [%1], 16, %2, %3;" ::"r"(dst), "l"(src), "r"(nbytes), "l"(pol) : "memory");
 }
 __device__ __forceinline__ void prefetch_l2(const void* p) { asm volatile("prefetch.global.L2 [%0];" ::"l"(p)); }
-__device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count));
-}
-__device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ bool mbar_try(uint64_t* bar, uint32_t parity) {
-  uint32_t done;
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-      "selp.u32 %0, 1, 0, p;\n\t}"
-      : "=r"(done) : "r"(smem_u32(bar)), "r"(parity) : "memory");
-  return done != 0;
-}
 // Bounded wait.  A protocol bug or a dead peer must not hang the GPU: on time-out (or when another CTA
 // already raised the error flag) the thread turns `dead` and every later wait returns at once.
 __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity, bool& dead, int* err) {
@@ -86,32 +67,14 @@ __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity, bool& 
   dead = true;
   atomicCAS(err, 0, 2);
 }
-__device__ __forceinline__ uint64_t desc_k_sw128(uint32_t saddr) {
-  return (uint64_t)((saddr & 0x3FFFFu) >> 4) | ((uint64_t)1 << 16) | ((uint64_t)(1024 >> 4) << 32) | ((uint64_t)1 << 46) |
-         ((uint64_t)2 << 61);
-}
 __device__ __forceinline__ uint64_t desc_mn_sw128(uint32_t saddr) {
   return (uint64_t)((saddr & 0x3FFFFu) >> 4) | ((uint64_t)(kAtomBytes >> 4) << 16) | ((uint64_t)(1024 >> 4) << 32) |
          ((uint64_t)1 << 46) | ((uint64_t)2 << 61);
-}
-__host__ __device__ constexpr uint32_t idesc_i8(int N, int a_mn) {
-  return (2u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)a_mn << 15) | ((uint32_t)(N >> 3) << 17) | ((128u >> 4) << 24);
-}
-__device__ __forceinline__ void umma_i8(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t acc) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::i8 [%0], %1, %2, %3, p;\n\t}"
-      ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(acc) : "memory");
-}
-__device__ __forceinline__ void umma_commit(uint64_t* bar) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");
 }
 __device__ __forceinline__ void tmem_ld4(uint32_t taddr, int& v0, int& v1, int& v2, int& v3) {
   asm volatile("tcgen05.ld.sync.aligned.32x32b.x4.b32 {%0, %1, %2, %3}, [%4];"
                : "=r"(v0), "=r"(v1), "=r"(v2), "=r"(v3) : "r"(taddr) : "memory");
 }
-__device__ __forceinline__ void tmem_ld_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
 __device__ __forceinline__ long long combine_limbs(int s0, int s1, int s2, int s3) {
   return (long long)s0 + ((long long)s1 << 8) + ((long long)s2 << 16) + ((long long)s3 << 24);
 }
@@ -125,23 +88,6 @@ __device__ __forceinline__ void split_limbs(int q, int& l0, int& l1, int& l2, in
 // byte offset of element (row n, K byte kb) inside one K-major SWIZZLE_128B atom stack
 __device__ __forceinline__ uint32_t sw128_off(int n, int kb) {
   return (uint32_t)((n >> 3) * 1024 + (n & 7) * 128 + ((((kb >> 4) ^ (n & 7)) & 7) << 4) + (kb & 15));
-}
-// one elected lane of a converged warp (the form ptxas recognises: tcgen05.mma is then issued without a per-lane loop)
-__device__ __forceinline__ bool elect_one() {
-  uint32_t pred;
-  asm volatile("{\n\t.reg .pred P;\n\telect.sync _|P, 0xffffffff;\n\tselp.u32 %0, 1, 0, P;\n\t}" : "=r"(pred));
-  return pred != 0;
-}
-__device__ __forceinline__ unsigned long long gtimer() {
-  unsigned long long t;
-  asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-  return t;
-}
-__device__ __forceinline__ void named_bar(int id, int nthreads) { asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(nthreads) : "memory"); }
-__device__ __forceinline__ unsigned long long ld_relaxed_u64(const unsigned long long* p) {
-  unsigned long long v;
-  asm volatile("ld.relaxed.gpu.global.u64 %0, [%1];" : "=l"(v) : "l"(p) : "memory");
-  return v;
 }
 __device__ __forceinline__ void st_relaxed_u64(unsigned long long* p, unsigned long long v) {
   asm volatile("st.relaxed.gpu.global.u64 [%0], %1;" ::"l"(p), "l"(v) : "memory");
@@ -277,7 +223,7 @@ __global__ void __launch_bounds__(kT, 1) sweep_pipe_kernel(PipeArgs a) {
       for (int d = 0; d < 4; d++) mbar_init(&S.de_ready[s][d], 1);
     }
     for (int i = 0; i < 2; i++) { mbar_init(&S.de_in[i], 1); mbar_init(&S.h_in[i], 1); mbar_init(&S.h_ready[i], 128); }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    fence_mbar_init();
     if (CL) {  // expected bytes of the first two blocks (every later phase is armed by the consumer of the phase before)
       for (int i = 0; i < 2 && i < nblocks; i++) {
         if (is_solver) mbar_expect_tx(&S.h_in[i], (uint32_t)(kClWorkers * ns * 128 * 8));
@@ -327,18 +273,15 @@ __global__ void __launch_bounds__(kT, 1) sweep_pipe_kernel(PipeArgs a) {
       }
     uint32_t tmem_cols = 32;
     while ((int)tmem_cols < (NA + 1) * N) tmem_cols <<= 1;
-    if (warp == 0) {
-      asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&S.tmem_base)), "r"(tmem_cols) : "memory");
-      asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
-    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");  // initial limbs (generic stores) -> tensor core
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+    if (warp == 0) tmem_alloc(&S.tmem_base, tmem_cols);
+    fence_proxy_async();  // initial limbs (generic stores) -> tensor core
+    tc_fence_before();
     __syncthreads();
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+    tc_fence_after();
     const uint32_t tmem_base = S.tmem_base;
     const uint32_t tmem_g = tmem_base + (uint32_t)(NA * N);
     const bool tracing = a.trace != nullptr;
-#define WSTAMP(blk, k) do { if (tracing) { long long* tp_ = a.trace + ((size_t)blockIdx.x * nblocks + (blk)) * 32 + (k); tp_[0] = (long long)gtimer(); tp_[16] = clock64(); } } while (0)
+#define WSTAMP(blk, k) do { if (tracing) { long long* tp_ = a.trace + ((size_t)blockIdx.x * nblocks + (blk)) * 32 + (k); tp_[0] = (long long)globaltimer_ns(); tp_[16] = clock64(); } } while (0)
 
     if (warp == 0) {
       // ------------------------------------------------------------------ tcgen05 issuer
@@ -353,7 +296,7 @@ __global__ void __launch_bounds__(kT, 1) sweep_pipe_kernel(PipeArgs a) {
         if (c > 0) mbar_wait(&S.g_empty, (uint32_t)(c - 1) & 1u, dead, a.err);
         for (int g = 0; g * kAtomsPerGroup < NA; g++) {
           if (use >= 0) mbar_wait(&S.el_full_at[g], (uint32_t)use & 1u, dead, a.err);
-          asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+          tc_fence_after();
           if (elect_one()) {
             for (int at = g * kAtomsPerGroup; at < NA && at < (g + 1) * kAtomsPerGroup; at++) {
               const uint64_t ad = desc_k_sw128(smem_u32(Xt + (size_t)at * kAtomBytes));
@@ -371,7 +314,7 @@ __global__ void __launch_bounds__(kT, 1) sweep_pipe_kernel(PipeArgs a) {
       for (int b = 0; b < nblocks; b++) {
         const unsigned char* Xt = Xs + (size_t)(b % nbuf) * NA * kAtomBytes;
         mbar_wait(&S.dl_full[b & 1], (uint32_t)(b >> 1) & 1u, dead, a.err);
-        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+        tc_fence_after();
         if (tracing && lane == 0) WSTAMP(b, 8);
         if (elect_one()) {
           const uint64_t bd = desc_k_sw128(smem_u32(DL + (size_t)(b & 1) * (N / 8) * 1024));
@@ -401,7 +344,7 @@ __global__ void __launch_bounds__(kT, 1) sweep_pipe_kernel(PipeArgs a) {
       auto g_epilogue = [&](int c) {
         mbar_wait(&S.g_done, (uint32_t)c & 1u, dead, a.err);
         if (t0) WSTAMP(c, 6);
-        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+        tc_fence_after();
         // partial of marker q, system s -> part[c % ring][s][this worker][q] (full 32-byte sectors): (value << 12) | block tag
         unsigned long long* hb = a.part + (((size_t)(c % kRing) * ns) * kWPad + (CL ? 0 : blockIdx.x)) * 128 + q;
         const unsigned long long tagc = tag_of((unsigned long long)(c / kRing));
@@ -416,7 +359,7 @@ __global__ void __launch_bounds__(kT, 1) sweep_pipe_kernel(PipeArgs a) {
           if (CL) st_async_u64(rdst + (uint32_t)s * 1024u, (unsigned long long)gq, rbar);
           else st_relaxed_u64(hb + (size_t)s * kWPad * 128, pack_word(gq, tagc));
         }
-        asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+        tc_fence_before();
         mbar_arrive(&S.g_empty);
         if (t0) WSTAMP(c, 7);
       };
@@ -461,7 +404,7 @@ __global__ void __launch_bounds__(kT, 1) sweep_pipe_kernel(PipeArgs a) {
           if (t0) WSTAMP(b, 0);
           // this inbox slot is next used by block b + 2, whose step cannot be sent before this worker's partial of b + 2
           if (CL && q == 0 && b + 2 < nblocks) mbar_expect_tx(&S.de_in[b & 1], (uint32_t)(ns * 129 * 4));
-          asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+          fence_proxy_async();
           mbar_arrive(&S.dl_full[b & 1]);
           named_bar(1, 128);  // the scales (dqs) of all systems visible to the four epilogue warps
           if (t0) WSTAMP(b, 1);
@@ -471,7 +414,7 @@ __global__ void __launch_bounds__(kT, 1) sweep_pipe_kernel(PipeArgs a) {
         for (int g = 0; g * kAtomsPerGroup < NA; g++) {
           mbar_wait(&S.u_done_at[g], (uint32_t)b & 1u, dead, a.err);
           if (t0 && g == 0) WSTAMP(b, 3);
-          asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+          tc_fence_after();
           const int at0 = g * kAtomsPerGroup;
           for (int s = 0; s < ns; s++) {
             int acc[kAtomsPerGroup][4];
@@ -499,8 +442,8 @@ __global__ void __launch_bounds__(kT, 1) sweep_pipe_kernel(PipeArgs a) {
               }
             }
           }
-          asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-          asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+          tc_fence_before();
+          fence_proxy_async();
           mbar_arrive(&S.el_full_at[g]);
         }
         if (t0) WSTAMP(b, 4);
@@ -543,10 +486,10 @@ __global__ void __launch_bounds__(kT, 1) sweep_pipe_kernel(PipeArgs a) {
             cp_async16_stream(dm, ok ? xrow + (int64_t)j * a.g.ld : a.g.x8, ok ? 16u : 0u, pol);
           }
         }
-        asm volatile("cp.async.commit_group;" ::: "memory");
+        cp_async_commit();
         if (tracing && lw == 0 && lane == 0) WSTAMP(t, 12);
-        asm volatile("cp.async.wait_group 0;" ::: "memory");
-        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+        cp_async_wait<0>();
+        fence_proxy_async();
         mbar_arrive(&S.tile_full[buf]);
         if (tracing && lw == 0 && lane == 0) WSTAMP(t, 13);
       }
@@ -594,12 +537,9 @@ __global__ void __launch_bounds__(kT, 1) sweep_pipe_kernel(PipeArgs a) {
       }
     }
     if (bad) atomicExch(a.err, 4);
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+    tc_fence_before();
     __syncthreads();
-    if (warp == 0) {
-      asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-      asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(tmem_cols) : "memory");
-    }
+    if (warp == 0) tmem_dealloc(tmem_base, tmem_cols);
 #undef WSTAMP
     if (CL) cluster_sync_all();  // nobody leaves while a peer may still store into its shared memory
     return;
@@ -646,8 +586,8 @@ __global__ void __launch_bounds__(kT, 1) sweep_pipe_kernel(PipeArgs a) {
   const int nsw = ns < kSolveWarps ? ns : kSolveWarps;
   __syncthreads();
   const bool tracing = a.trace != nullptr;
-#define SSTAMPW(blk, k) do { if (tracing && lane == 0) { long long* tp_ = a.trace + ((size_t)blockIdx.x * nblocks + (blk)) * 32 + (k); tp_[0] = (long long)gtimer(); tp_[16] = clock64(); } } while (0)
-#define SSTAMP(blk, k) do { if (tracing && warp == 0 && lane == 0) { long long* tp_ = a.trace + ((size_t)blockIdx.x * nblocks + (blk)) * 32 + (k); tp_[0] = (long long)gtimer(); tp_[16] = clock64(); } } while (0)
+#define SSTAMPW(blk, k) do { if (tracing && lane == 0) { long long* tp_ = a.trace + ((size_t)blockIdx.x * nblocks + (blk)) * 32 + (k); tp_[0] = (long long)globaltimer_ns(); tp_[16] = clock64(); } } while (0)
+#define SSTAMP(blk, k) do { if (tracing && warp == 0 && lane == 0) { long long* tp_ = a.trace + ((size_t)blockIdx.x * nblocks + (blk)) * 32 + (k); tp_[0] = (long long)globaltimer_ns(); tp_[16] = clock64(); } } while (0)
 
   if (warp < kSolveWarps) {
     if (use_inv && warp >= kInvWarp0) {
@@ -685,7 +625,7 @@ __global__ void __launch_bounds__(kT, 1) sweep_pipe_kernel(PipeArgs a) {
           for (int i = 0; i < 32; i++) mt[4 * i] = x[i];
         }
         mbar_arrive(&S.in_ready[slot]);
-        if (tracing && warp == kInvWarp0 && lane == 0) { long long* tp_ = a.trace + ((size_t)blockIdx.x * nblocks + nb) * 32 + 3; tp_[0] = (long long)gtimer(); tp_[16] = clock64(); }
+        if (tracing && warp == kInvWarp0 && lane == 0) { long long* tp_ = a.trace + ((size_t)blockIdx.x * nblocks + nb) * 32 + 3; tp_[0] = (long long)globaltimer_ns(); tp_[16] = clock64(); }
       }
     }
     if (CL && warp >= kCommWarp0) {
@@ -732,7 +672,7 @@ __global__ void __launch_bounds__(kT, 1) sweep_pipe_kernel(PipeArgs a) {
           *reinterpret_cast<volatile unsigned int*>(a.started) = a.started_val;
           __threadfence_system();
         }
-        if (tracing && ct == 0) { long long* tp_ = a.trace + ((size_t)blockIdx.x * nblocks + b) * 32 + 4; tp_[0] = (long long)gtimer(); tp_[16] = clock64(); }
+        if (tracing && ct == 0) { long long* tp_ = a.trace + ((size_t)blockIdx.x * nblocks + b) * 32 + 4; tp_[0] = (long long)globaltimer_ns(); tp_[16] = clock64(); }
         // until the partials of the next block arrive these warps are idle: three of them take one tile each of the lower-
         // triangular product dE = T r of the block they just delivered ((2,2), (3,2), (3,3)); the solve warps add the tile sums in
         // the same order as when they compute all tiles themselves, so the result is bit-identical to the flat topology
@@ -1274,7 +1214,7 @@ __global__ void __launch_bounds__(kT, 1) sweep_pipe_kernel(PipeArgs a) {
     // thread ht = marker ht of the block.  Marker ids are fetched two blocks ahead and the per-marker scalars one block
     // ahead into registers, so the HBM round trips of these tiny gathers never sit on the per-block path.
     const int ht = (warp - kPreWarp0) * 32 + lane;  // 0..127
-#define PSTAMP(k) do { if (tracing && ht == 0) { long long* tp_ = a.trace + ((size_t)blockIdx.x * nblocks + nb) * 32 + (k); tp_[0] = (long long)gtimer(); tp_[16] = clock64(); } } while (0)
+#define PSTAMP(k) do { if (tracing && ht == 0) { long long* tp_ = a.trace + ((size_t)blockIdx.x * nblocks + nb) * 32 + (k); tp_[0] = (long long)globaltimer_ns(); tp_[16] = clock64(); } } while (0)
     constexpr int kPipeSys = 2;  // systems whose scalars are register-pipelined (more systems: loaded in place)
     auto perm_at = [&](int blk) { const int pos = blk * 128 + ht; return (blk < nblocks && pos < p) ? a.perm[pos] : -1; };
     int j_cur = perm_at(0), j_nxt = perm_at(1);
@@ -1302,9 +1242,9 @@ __global__ void __launch_bounds__(kT, 1) sweep_pipe_kernel(PipeArgs a) {
           const int tile = it >> 1, rr = rr0 + 16 * (it & 1);
           const int hi = kHi[tile], lo = kLo[tile];
           const int grow_ = kLinear ? 32 * hi + rr : 32 * lo + rr, gcol = kLinear ? 32 * lo + 4 * c4 : 32 * hi + 4 * c4;
-          cp_async16(smem_u32(Gb + (size_t)tile * kTileF + rr * kTS + 4 * c4), src + (size_t)grow_ * tstride + gcol, 16u);
+          cp_async16_zfill(smem_u32(Gb + (size_t)tile * kTileF + rr * kTS + 4 * c4), src + (size_t)grow_ * tstride + gcol, 16u);
         }
-        asm volatile("cp.async.commit_group;" ::: "memory");
+        cp_async_commit();
       }
       PSTAMP(1);
       // issue the gathers of the following blocks now; they are consumed in the next iteration
@@ -1374,7 +1314,7 @@ __global__ void __launch_bounds__(kT, 1) sweep_pipe_kernel(PipeArgs a) {
         }
       }
       PSTAMP(2);
-      asm volatile("cp.async.wait_group 0;" ::: "memory");
+      cp_async_wait<0>();
       if (use_inv) mbar_arrive(&S.raw_ready[slot]);
       else mbar_arrive(&S.in_ready[slot]);
       PSTAMP(7);
