@@ -11,9 +11,9 @@ LIB_PATH = os.environ.get("BWGR_LIB") or os.path.join(_HERE, "lib", "libbwgr_b20
 # every symbol include/bwgr_b200.h declares (tests check the shared object exports all of them)
 SYMBOLS = [
     "bwgr_create", "bwgr_destroy", "bwgr_last_error", "bwgr_version", "bwgr_set_stream", "bwgr_set_tuning",
-    "bwgr_fitted", "bwgr_geno_load_f64", "bwgr_geno_load_f64_centred", "bwgr_geno_load_bed", "bwgr_geno_load_i8", "bwgr_geno_load_i8_device", "bwgr_geno_unpack_i8", "bwgr_geno_raw",
+    "bwgr_fitted", "bwgr_fitted_sys", "bwgr_geno_load_f64", "bwgr_geno_load_f64_centred", "bwgr_geno_load_bed", "bwgr_geno_load_i8", "bwgr_geno_load_i8_device", "bwgr_geno_unpack_i8", "bwgr_geno_raw",
     "bwgr_geno_info", "bwgr_geno_stats", "bwgr_em_fit", "bwgr_em_begin", "bwgr_em_sweeps", "bwgr_em_end",
-    "bwgr_gibbs_fit", "bwgr_kmup_sweep", "bwgr_kmup2_sweep", "bwgr_wgr_fit_bag", "bwgr_gs_fit", "bwgr_wgr_fit", "bwgr_mrr3_fit", "bwgr_dist_unique_id", "bwgr_dist_init", "bwgr_dist_connect", "bwgr_launch_count", "bwgr_debug_gram", "bwgr_debug_gram_band", "bwgr_debug_narrow", "bwgr_trim", "bwgr_profile", "bwgr_profile_read",
+    "bwgr_gibbs_fit", "bwgr_gibbs_fit_sys", "bwgr_kmup_sweep", "bwgr_kmup2_sweep", "bwgr_wgr_fit_bag", "bwgr_gs_fit", "bwgr_wgr_fit", "bwgr_mrr3_fit", "bwgr_dist_unique_id", "bwgr_dist_init", "bwgr_dist_connect", "bwgr_launch_count", "bwgr_debug_gram", "bwgr_debug_gram_band", "bwgr_debug_narrow", "bwgr_trim", "bwgr_profile", "bwgr_profile_read",
 ]
 
 
@@ -36,6 +36,10 @@ class EmOut(C.Structure):
 class GibbsParams(C.Structure):
     _fields_ = [("model", C.c_int), ("nchains", C.c_int), ("it", C.c_int), ("bi", C.c_int), ("pi", C.c_double),
                 ("df", C.c_double), ("R2", C.c_double), ("seed", C.c_uint64)]
+
+
+class GibbsSysParams(C.Structure):
+    _fields_ = [("base", GibbsParams), ("nsys", C.c_int), ("row_mask", C.c_void_p), ("chain0", C.c_int)]
 
 
 class GibbsOut(C.Structure):
@@ -75,7 +79,9 @@ def load():
         lib.bwgr_em_sweeps.argtypes = [C.c_void_p, C.c_int]
         lib.bwgr_em_end.argtypes = [C.c_void_p, C.POINTER(EmOut)]
         lib.bwgr_gibbs_fit.argtypes = [C.c_void_p, C.POINTER(GibbsParams), C.c_void_p, C.POINTER(GibbsOut)]
+        lib.bwgr_gibbs_fit_sys.argtypes = [C.c_void_p, C.POINTER(GibbsSysParams), C.c_void_p, C.POINTER(GibbsOut)]
         lib.bwgr_fitted.argtypes = [C.c_void_p, C.c_void_p, C.c_double, C.c_void_p]
+        lib.bwgr_fitted_sys.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]
         lib.bwgr_kmup_sweep.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                         C.c_double, C.c_double, C.c_uint64]
         lib.bwgr_kmup2_sweep.argtypes = [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,

@@ -10,7 +10,7 @@ import ctypes as C
 import numpy as np
 
 from . import _lib
-from ._lib import EmOut, EmParams, GibbsOut, GibbsParams, check
+from ._lib import EmOut, EmParams, GibbsOut, GibbsParams, GibbsSysParams, check
 
 STORE_I8, STORE_2BIT, STORE_F32 = 0, 1, 2
 PATH_AUTO, PATH_SMALL_N, PATH_BLOCKED, PATH_GRID = 0, 1, 2, 3
@@ -136,11 +136,21 @@ class Genotypes:
         return xx, sx
 
     def fitted(self, b, mu=0.0):
-        """mu + X b on the store (bwgr_fitted)."""
-        b = np.ascontiguousarray(b, dtype=np.float64)
-        _need(b.size == self.p, "b must have p = %d values" % self.p)
-        hat = np.empty(self.n)
-        check(self.lib.bwgr_fitted(self.h, _ptr(b), float(mu), _ptr(hat)))
+        """mu + X b on the store: b is p (bwgr_fitted) or p x k with mu a scalar or k values (bwgr_fitted_sys: k systems, one pass
+        over the store, hat n x k)."""
+        b = np.asarray(b, dtype=np.float64)
+        if b.ndim == 1:
+            b = np.ascontiguousarray(b)
+            _need(b.size == self.p, "b must have p = %d values" % self.p)
+            hat = np.empty(self.n)
+            check(self.lib.bwgr_fitted(self.h, _ptr(b), float(mu), _ptr(hat)))
+            return hat
+        _need(b.ndim == 2 and b.shape[0] == self.p and b.shape[1] >= 1, "b must be p x k with p = %d" % self.p)
+        B = np.asfortranarray(b)
+        k = B.shape[1]
+        m = np.ascontiguousarray(np.broadcast_to(np.asarray(mu, dtype=np.float64), (k,)))
+        hat = np.empty((self.n, k), order="F")
+        check(self.lib.bwgr_fitted_sys(self.h, k, _ptr(B), _ptr(m), _ptr(hat)))
         return hat
 
     def gram_blocks(self, perm, block=128):
@@ -339,22 +349,32 @@ def lasso(y, gen, **kw):
     return em_fit("lasso", y, gen, **kw)
 
 
-def gibbs_fit(model, y, X, it=1500, bi=500, pi=0.95, df=5.0, R2=0.5, seed=1, nchains=1, **store_kw):
+def gibbs_fit(model, y, X, it=1500, bi=500, pi=0.95, df=5.0, R2=0.5, seed=1, nchains=1, row_mask=None, chain0=0, **store_kw):
+    """Generic entry of the seven samplers.  y is n (one trait) or n x k (k traits / CV folds sharing X, one call); row_mask (n x k, like
+    em_fit's) fits column t on the rows it keeps.  Column t runs `nchains` chains: system s = t * nchains + c draws from Philox chain
+    chain0 + s.  A 1-D y without a mask returns what the single-trait call returns (a trailing chain axis when nchains > 1); an n x k y
+    returns arrays with a trailing system axis of k * nchains, and hat covers every row, the ones a mask leaves out included."""
     g, own = _store(X, **store_kw)
     try:
-        y = np.ascontiguousarray(y, dtype=np.float64)
-        _need(y.size == g.n, "y has %d values, the genotype store %d rows" % (y.size, g.n))
-        nc = int(nchains)
-        mu = np.zeros(nc)
-        b = np.zeros((g.p, nc), order="F")
-        d = np.zeros((g.p, nc), order="F")
-        hat = np.zeros((g.n, nc), order="F")
-        vb = np.zeros((g.p, nc), order="F")
-        scal = np.zeros((NSCAL, nc), order="F")
-        par = GibbsParams(_GIBBS[model], nc, int(it), int(bi), pi, df, R2, seed)
+        y = np.asarray(y, dtype=np.float64)
+        _need(y.ndim in (1, 2) and y.shape[0] == g.n and y.size % g.n == 0, "y has %d rows, the genotype store %d" % (y.shape[0], g.n))
+        Y = np.asfortranarray(y.reshape(g.n, -1, order="F"))
+        k = Y.shape[1]
+        nc = max(1, int(nchains))
+        ns = k * nc
+        mask = None
+        if row_mask is not None:
+            mask = np.asfortranarray(np.asarray(row_mask).reshape(g.n, k, order="F") != 0, dtype=np.uint8)
+        mu = np.zeros(ns)
+        b = np.zeros((g.p, ns), order="F")
+        d = np.zeros((g.p, ns), order="F")
+        hat = np.zeros((g.n, ns), order="F")
+        vb = np.zeros((g.p, ns), order="F")
+        scal = np.zeros((NSCAL, ns), order="F")
+        par = GibbsSysParams(GibbsParams(_GIBBS[model], nc, int(it), int(bi), pi, df, R2, seed), k, _ptr(mask), int(chain0))
         out = GibbsOut(_ptr(mu), _ptr(b), _ptr(d), _ptr(hat), _ptr(vb), _ptr(scal))
-        check(g.lib.bwgr_gibbs_fit(g.h, C.byref(par), _ptr(y), C.byref(out)))
-        sq = nc == 1
+        check(g.lib.bwgr_gibbs_fit_sys(g.h, C.byref(par), _ptr(Y), C.byref(out)))
+        sq = ns == 1 and y.ndim == 1
 
         def v(a):
             return a[:, 0].copy() if sq else a

@@ -164,6 +164,7 @@ struct Fit {
   int rows_per_cta = 0, grid = 0, nblocks = 0;
   bool gram_cached = false;
   uint64_t seed = 0;
+  int chain0 = 0;                       // Philox chain index of system 0
   std::vector<SysScalars> sc0;
   std::vector<float> vy, MSx, cxx;      // per system constants needed for outputs
   std::vector<int> order;               // host marker order (cumulative shuffles)
@@ -865,6 +866,7 @@ struct FitSpec {
   float df, R2, Pi, alpha, pi;
   int it, bi;
   uint64_t seed;
+  int chain0 = 0;  // Philox chain index of system 0 (Gibbs): system t draws from chain chain0 + t
 };
 
 // Geometry of the pipelined sweep: W streaming CTAs (row slabs of R rows, R <= 512) + one solver CTA, look-ahead D,
@@ -1047,7 +1049,7 @@ int fit_begin(bwgr_handle* h, const FitSpec& s, const double* y) {
   const int64_t n = h->n, p = h->p, ld = h->ld;
   const int ns = s.nsys;
   f.model = s.model; f.nsys = ns; f.shuffled = s.shuffled; f.blocked = blocked; f.gridfam = family == 2; f.masked = s.row_mask != nullptr; f.weighted = false;
-  f.sweeps_issued = 0; f.seed = s.seed; f.gram_cached = false; f.skip_epilogue = false; f.wgr_mode = false; f.gram_p = nullptr;
+  f.sweeps_issued = 0; f.seed = s.seed; f.chain0 = s.chain0; f.gram_cached = false; f.skip_epilogue = false; f.wgr_mode = false; f.gram_p = nullptr;
   f.overlap = false; f.gram_ahead = -1;
   if (h->side) CU(cudaStreamSynchronize(h->side));  // a band computed ahead for a sweep the previous fit never ran
   f.xx_over.release(); f.wst.release(); f.sx_dev.release(); f.cshift.release(); f.wts.release();
@@ -1402,7 +1404,7 @@ int fit_sweeps(bwgr_handle* h, int nsweeps) {
       a.g = g; a.model = rule_model(f.model); a.nsys = f.nsys; a.perm = d_perm; a.nblocks = f.nblocks; a.gram = f.gram_p; a.nband = f.nband; a.tinv = f.full_inv ? f.tinv.p : nullptr;
       a.e = f.e.p; a.b = f.b.p; a.d = f.d.p; a.vbv = f.vbv.p; a.xx = f.xx_over.p ? f.xx_over.p : h->xx_f.p; a.sx = f.sx_dev.p; a.cshift = f.cshift.p; a.sc = f.sc.p;
       a.part = f.part.p; a.hred = f.part.p + (size_t)8 * f.nsys * 128 * 160; a.dew = f.dew.p; a.tag = ++f.tag;
-      a.seed_lo = (uint32_t)f.seed; a.seed_hi = (uint32_t)(f.seed >> 32); a.chain0 = 0;
+      a.seed_lo = (uint32_t)f.seed; a.seed_hi = (uint32_t)(f.seed >> 32); a.chain0 = f.chain0;
       a.rows_per_cta = f.rows_per_cta; a.nworkers = f.nworkers; a.D = f.lookahead; a.nbuf = f.nbuf; a.sring = f.sring; a.err = h->err.p;
       a.world = h->world; a.rank = h->rank; a.gen0 = h->dist_gen;
       a.cl = f.cl; a.nclusters = f.nclusters; a.cx = f.cx.p;
@@ -1456,7 +1458,7 @@ int fit_sweeps(bwgr_handle* h, int nsweeps) {
         a.gram_quantum = h->storage == BWGR_STORE_F32 ? (float)std::ldexp(1.0, ex - 50) : (float)std::ldexp(1.0, std::max(0, ex - 50));
       }
       a.sc = f.sc.p; a.acc = f.gridacc.p; a.g_quantum = quantum; a.seed_lo = (uint32_t)f.seed; a.seed_hi = (uint32_t)(f.seed >> 32);
-      a.chain0 = 0; a.rows_per_cta = f.rows_per_cta; a.err = h->err.p;
+      a.chain0 = f.chain0; a.rows_per_cta = f.rows_per_cta; a.err = h->err.p;
       CU(cudaMemsetAsync(f.gridacc.p, 0, sizeof(unsigned long long) * f.gridacc.n, h->stream));
       cudaEvent_t pe = h->prof_begin(1);
       const cudaError_t le = launch_grid_sweep(a, f.grid, h->stream);
@@ -1469,7 +1471,7 @@ int fit_sweeps(bwgr_handle* h, int nsweeps) {
       a.g = g; a.model = rule_model(f.model); a.nsys = f.nsys; a.perms = d_perm; a.y = f.y.p; a.e = f.e.p; a.b = f.b.p; a.d = f.d.p;
       a.vbv = f.vbv.p; a.xx = f.masked ? f.xx_sys.p : (f.xx_over.p ? f.xx_over.p : h->xx_f.p); a.xx_per_sys = f.masked ? 1 : 0; a.mask = f.mask.p;
       a.xx2 = f.xx_over.p; a.row_w = f.weighted ? f.row_w.p : nullptr;
-      a.sc = f.sc.p; a.seed_lo = (uint32_t)f.seed; a.seed_hi = (uint32_t)(f.seed >> 32); a.chain0 = 0; a.err = h->err.p;
+      a.sc = f.sc.p; a.seed_lo = (uint32_t)f.seed; a.seed_hi = (uint32_t)(f.seed >> 32); a.chain0 = f.chain0; a.err = h->err.p;
       cudaEvent_t pe = h->prof_begin(1);
       launch_small_n(a, h->smem_optin, h->stream);
       h->prof_end(pe);
@@ -1492,7 +1494,7 @@ int fit_sweeps(bwgr_handle* h, int nsweeps) {
       ea.d = f.d.p; ea.vbv = f.vbv.p; ea.b_prev = f.b_prev.p; ea.mask = f.mask.p; ea.sc = f.sc.p; ea.B = f.B.p; ea.D = f.D.p;
       ea.xx = f.masked ? f.xx_sys.p : (f.xx_over.p ? f.xx_over.p : h->xx_f.p); ea.xx_per_sys = f.masked ? 1 : 0;
       ea.wts = f.wts.p;
-      ea.VBv = f.VBv.p; ea.seed_lo = (uint32_t)f.seed; ea.seed_hi = (uint32_t)(f.seed >> 32); ea.chain0 = 0;
+      ea.VBv = f.VBv.p; ea.seed_lo = (uint32_t)f.seed; ea.seed_hi = (uint32_t)(f.seed >> 32); ea.chain0 = f.chain0;
       cudaEvent_t pe2 = h->prof_begin(2);
       if (h->world > 1) {  // sums over individuals: per rank, then all-reduced; everything else is replicated
         launch_epilogue_partial(ea, f.esum.p, f.emaxv.p, h->stream);
@@ -1512,32 +1514,38 @@ int fit_sweeps(bwgr_handle* h, int nsweeps) {
   return 0;
 }
 
-// hat = mu + X b for system t, into a device buffer
-int fit_hat(bwgr_handle* h, const float* b_dev, const float* mu_dev, float* hat_dev) {
+constexpr int kHatSplits = 64;           // column splits of the fitted values (they fix each row's summation order)
+constexpr size_t kHatWorkBytes = 512u << 20;  // bound of the partial sums [k][splits][ld] of one launch of the fitted values
+
+// hat[t] = mu[t] + X b_t for the k systems of b [k][p] into hat [k][ld] (device buffers): one launch per group of systems whose partial
+// sums fit kHatWorkBytes (all k at once up to n ~ 10^5 for k = 16)
+int fit_hat(bwgr_handle* h, int k, const float* b_dev, const float* mu_dev, float* hat_dev) {
   Fit& f = h->fit;
-  const int splits = 64;
-  if (f.work.n < (size_t)splits * h->ld && f.work.alloc((size_t)splits * h->ld) != cudaSuccess) return fail(BWGR_ERR_CUDA, "cudaMalloc failed");
-  launch_gemv_hat(h->view(), b_dev, mu_dev, hat_dev, f.work.p, splits, h->stream);
-  h->launches += 2;
+  const size_t per_sys = (size_t)kHatSplits * h->ld;
+  int per = (int)std::max<size_t>(1, std::min<size_t>((size_t)k, kHatWorkBytes / (per_sys * sizeof(float))));
+  if (per < k && per >= kHatChunk) per -= per % kHatChunk;
+  if (f.work.n < (size_t)per * per_sys && f.work.alloc((size_t)per * per_sys) != cudaSuccess) return fail(BWGR_ERR_CUDA, "cudaMalloc failed");
+  for (int t0 = 0; t0 < k; t0 += per) {
+    const int kc = std::min(per, k - t0);
+    launch_gemv_hat(h->view(), b_dev + (size_t)t0 * h->p, kc, mu_dev + t0, hat_dev + (size_t)t0 * h->ld, f.work.p, kHatSplits, h->stream);
+    h->launches += 2;
+  }
   return 0;
 }
 
 // Fitted values of nsys systems read back to the host: hat[t * n + i] = mu[t] + x_i'b_t.  b: nsys x p floats, on the device or, with
 // b_on_host, on the host.
 int fitted_values(bwgr_handle* h, int nsys, const float* b, bool b_on_host, const float* mu, std::vector<float>& hat) {
-  const int64_t n = h->n, p = h->p;
+  const int64_t n = h->n, p = h->p, ld = h->ld;
   DevBuf<float> bdev, mudev, hatd;
-  if ((b_on_host && bdev.alloc((size_t)nsys * p) != cudaSuccess) || mudev.alloc(nsys) != cudaSuccess || hatd.alloc(h->ld) != cudaSuccess)
+  if ((b_on_host && bdev.alloc((size_t)nsys * p) != cudaSuccess) || mudev.alloc(nsys) != cudaSuccess || hatd.alloc((size_t)nsys * ld) != cudaSuccess)
     return fail(BWGR_ERR_CUDA, "cudaMalloc failed");
   if (b_on_host) CU(cudaMemcpyAsync(bdev.p, b, sizeof(float) * nsys * p, cudaMemcpyHostToDevice, h->stream));
   CU(cudaMemcpyAsync(mudev.p, mu, sizeof(float) * nsys, cudaMemcpyHostToDevice, h->stream));
-  const float* bd = b_on_host ? bdev.p : b;
+  const int rc = fit_hat(h, nsys, b_on_host ? bdev.p : b, mudev.p, hatd.p);
+  if (rc) return rc;
   hat.resize((size_t)nsys * n);
-  for (int t = 0; t < nsys; t++) {
-    const int rc = fit_hat(h, bd + (size_t)t * p, mudev.p + t, hatd.p);
-    if (rc) return rc;
-    CU(cudaMemcpyAsync(hat.data() + (size_t)t * n, hatd.p, sizeof(float) * n, cudaMemcpyDeviceToHost, h->stream));
-  }
+  CU(cudaMemcpy2DAsync(hat.data(), sizeof(float) * n, hatd.p, sizeof(float) * ld, sizeof(float) * n, nsys, cudaMemcpyDeviceToHost, h->stream));
   CU(cudaStreamSynchronize(h->stream));
   return 0;
 }
@@ -1771,21 +1779,33 @@ int bwgr_gs_fit(bwgr_handle* h, int which, const double* y, double* e, double* b
 }
 
 // ---- Gibbs -------------------------------------------------------------------------------------------
-int bwgr_gibbs_fit(bwgr_handle* h, const bwgr_gibbs_params* par, const double* y, bwgr_gibbs_out* out) {
-  if (!h || !par || !out || !y) return fail(BWGR_ERR_ARG, "null argument");
+// nsys phenotype columns x nchains chains = S systems; system s = t * nchains + c fits column t (on the rows of its mask) and draws
+// from Philox chain chain0 + s.  bwgr_gibbs_fit is the case nsys = 1, no mask, chain0 = 0.
+int bwgr_gibbs_fit_sys(bwgr_handle* h, const bwgr_gibbs_sys_params* sp, const double* Y, bwgr_gibbs_out* out) {
+  if (!h || !sp || !out || !Y) return fail(BWGR_ERR_ARG, "null argument");
   if (!h->p) return fail(BWGR_ERR_STATE, "no genotypes loaded");
+  const bwgr_gibbs_params* par = &sp->base;
   if (par->model < 0 || par->model > BWGR_GIBBS_DPI) return fail(BWGR_ERR_ARG, "bad Gibbs model %d", par->model);
   static const int kGibbsModel[] = {M_BRR, M_BA, M_BB, M_BC, M_BL, M_BCPI, M_BDPI};
   const bool has_pi = par->model == BWGR_GIBBS_CPI || par->model == BWGR_GIBBS_DPI;  // these two start at pi = 0.5 (:870, :934), not an argument
   if (par->it < 1 || par->bi < 0 || par->bi >= par->it) return fail(BWGR_ERR_ARG, "need 0 <= bi < it");
+  if (sp->nsys < 1) return fail(BWGR_ERR_ARG, "bad nsys %d", sp->nsys);
+  if (sp->chain0 < 0) return fail(BWGR_ERR_ARG, "bad chain0 %d", sp->chain0);
   const int nc = par->nchains < 1 ? 1 : par->nchains;
+  if ((int64_t)sp->nsys * nc > 4096) return fail(BWGR_ERR_ARG, "nsys x nchains = %lld systems (at most 4096)", (long long)sp->nsys * nc);
+  const int ns = sp->nsys * nc;
   const int64_t n = h->n, p = h->p;
-  std::vector<double> yy((size_t)nc * n);
-  for (int c = 0; c < nc; c++) memcpy(yy.data() + (size_t)c * n, y, sizeof(double) * n);
+  std::vector<double> yy((size_t)ns * n);
+  std::vector<uint8_t> mm(sp->row_mask ? (size_t)ns * n : 0);
+  for (int s = 0; s < ns; s++) {
+    const size_t t = (size_t)(s / nc);
+    memcpy(yy.data() + (size_t)s * n, Y + t * n, sizeof(double) * n);
+    if (sp->row_mask) memcpy(mm.data() + (size_t)s * n, sp->row_mask + t * n, (size_t)n);
+  }
   FitSpec s;
-  s.model = kGibbsModel[par->model]; s.nsys = nc; s.shuffled = false; s.row_mask = nullptr;
+  s.model = kGibbsModel[par->model]; s.nsys = ns; s.shuffled = false; s.row_mask = sp->row_mask ? mm.data() : nullptr;
   s.df = (float)par->df; s.R2 = (float)par->R2; s.Pi = 0; s.alpha = 0; s.pi = has_pi ? 0.5f : (float)par->pi;
-  s.it = par->it; s.bi = par->bi; s.seed = par->seed;
+  s.it = par->it; s.bi = par->bi; s.seed = par->seed; s.chain0 = sp->chain0;
   FitGuard guard{h};
   int rc = fit_begin(h, s, yy.data());
   if (rc) return rc;
@@ -1794,19 +1814,19 @@ int bwgr_gibbs_fit(bwgr_handle* h, const bwgr_gibbs_params* par, const double* y
   if (rc) return rc;
   rc = check_err_flag(h, "gibbs sweep");
   if (rc) return rc;
-  std::vector<SysScalars> sc(nc);
-  CU(cudaMemcpyAsync(sc.data(), f.sc.p, sizeof(SysScalars) * nc, cudaMemcpyDeviceToHost, h->stream));
-  std::vector<float> B((size_t)nc * p), D, V;
+  std::vector<SysScalars> sc(ns);
+  CU(cudaMemcpyAsync(sc.data(), f.sc.p, sizeof(SysScalars) * ns, cudaMemcpyDeviceToHost, h->stream));
+  std::vector<float> B((size_t)ns * p), D, V;
   CU(cudaMemcpyAsync(B.data(), f.B.p, sizeof(float) * B.size(), cudaMemcpyDeviceToHost, h->stream));
-  if (f.D.p) { D.resize((size_t)nc * p); CU(cudaMemcpyAsync(D.data(), f.D.p, sizeof(float) * D.size(), cudaMemcpyDeviceToHost, h->stream)); }
-  if (f.VBv.p) { V.resize((size_t)nc * p); CU(cudaMemcpyAsync(V.data(), f.VBv.p, sizeof(float) * V.size(), cudaMemcpyDeviceToHost, h->stream)); }
+  if (f.D.p) { D.resize((size_t)ns * p); CU(cudaMemcpyAsync(D.data(), f.D.p, sizeof(float) * D.size(), cudaMemcpyDeviceToHost, h->stream)); }
+  if (f.VBv.p) { V.resize((size_t)ns * p); CU(cudaMemcpyAsync(V.data(), f.VBv.p, sizeof(float) * V.size(), cudaMemcpyDeviceToHost, h->stream)); }
   CU(cudaStreamSynchronize(h->stream));
   const float MCMC = (float)par->it - (float)par->bi;  // sic (:626): divisor it-bi although i>bi keeps it-bi-1 draws
-  std::vector<float> Bm(B.size()), MU(nc), hh;
+  std::vector<float> Bm(B.size()), MU(ns), hh;
   for (size_t i = 0; i < B.size(); i++) Bm[i] = B[i] / MCMC;
-  for (int c = 0; c < nc; c++) MU[c] = (float)(sc[c].MU / MCMC);
-  if ((rc = fitted_values(h, nc, Bm.data(), true, MU.data(), hh))) return rc;
-  for (int c = 0; c < nc; c++) {
+  for (int c = 0; c < ns; c++) MU[c] = (float)(sc[c].MU / MCMC);
+  if ((rc = fitted_values(h, ns, Bm.data(), true, MU.data(), hh))) return rc;  // every row, the ones a mask leaves out included
+  for (int c = 0; c < ns; c++) {
     const float VE = (float)(sc[c].VE / MCMC), VBs = (float)(sc[c].VB / MCMC);
     float vg;
     if (f.VBv.p) { double sv = 0; for (int64_t j = 0; j < p; j++) sv += V[(size_t)c * p + j] / MCMC; vg = (float)sv; }
@@ -1827,6 +1847,13 @@ int bwgr_gibbs_fit(bwgr_handle* h, const bwgr_gibbs_params* par, const double* y
   if (out->d && !D.empty()) for (size_t i = 0; i < D.size(); i++) out->d[i] = D[i] / MCMC;
   if (out->hat) for (size_t i = 0; i < hh.size(); i++) out->hat[i] = hh[i];
   return 0;
+}
+
+int bwgr_gibbs_fit(bwgr_handle* h, const bwgr_gibbs_params* par, const double* y, bwgr_gibbs_out* out) {
+  if (!par) return fail(BWGR_ERR_ARG, "null argument");
+  bwgr_gibbs_sys_params sp;
+  sp.base = *par; sp.nsys = 1; sp.row_mask = nullptr; sp.chain0 = 0;
+  return bwgr_gibbs_fit_sys(h, &sp, y, out);
 }
 
 // Common start of KMUP / wgr: a one-system M_KMUP fit whose state (b, d, e, per-marker L, Ve, pi) is set by the caller.
@@ -1925,21 +1952,24 @@ int bwgr_kmup_sweep(bwgr_handle* h, double* b, double* d, const double* xx, doub
 
 // Fitted values of the handle's store: hat = mu + X b.  What the reference's drivers form as X * b (emML2's u1 = X1 * b1,
 // Rcpp20260726ai.cpp:1275-1276; the fit of the two-design samplers :1063, :1151, :1212; wgr's gen0 %*% B, R/wgr.R:147).
-int bwgr_fitted(bwgr_handle* h, const double* b, double mu, double* hat) {
+int bwgr_fitted_sys(bwgr_handle* h, int k, const double* B, const double* mu, double* hat) {
   if (!h || !h->p) return fail(BWGR_ERR_STATE, "no genotypes loaded");
-  if (!b || !hat) return fail(BWGR_ERR_ARG, "null argument");
+  if (!B || !mu || !hat) return fail(BWGR_ERR_ARG, "null argument");
+  if (k < 1) return fail(BWGR_ERR_ARG, "bad k %d", k);
   if (h->world > 1) return fail(BWGR_ERR_UNSUPPORTED, "bwgr_fitted on a row-sharded store");
   if (h->col_offset.size()) return fail(BWGR_ERR_UNSUPPORTED, "this store holds integer codes + a constant per column: use the solvers that centre the columns themselves");
   CU(cudaSetDevice(h->device));
   const int64_t n = h->n, p = h->p;
-  std::vector<float> bf(p), hh;
-  for (int64_t j = 0; j < p; j++) bf[j] = (float)b[j];
-  const float m0 = (float)mu;
-  const int rc = fitted_values(h, 1, bf.data(), true, &m0, hh);
+  std::vector<float> bf((size_t)k * p), m0(k), hh;
+  for (size_t j = 0; j < bf.size(); j++) bf[j] = (float)B[j];
+  for (int t = 0; t < k; t++) m0[t] = (float)mu[t];
+  const int rc = fitted_values(h, k, bf.data(), true, m0.data(), hh);
   if (rc) return rc;
-  for (int64_t i = 0; i < n; i++) hat[i] = hh[i];
+  for (size_t i = 0; i < (size_t)k * n; i++) hat[i] = hh[i];
   return 0;
 }
+
+int bwgr_fitted(bwgr_handle* h, const double* b, double mu, double* hat) { return bwgr_fitted_sys(h, 1, b, &mu, hat); }
 
 // wgr(y, X, it, bi, th, bag, rp, iv, de, pi, df, R2, eigK = NULL) (R/wgr.R:2-169) with the MCMC loop on the device.
 // bag = 1: `it` KMUP sweeps, each followed by the driver's step on the device (wgr_mode).
@@ -2039,7 +2069,7 @@ static int wgr_fit(bwgr_handle* h, const double* y, int it, int bi, int th, doub
       }
       if ((rc = fit_sweeps(h, 1))) return rc;                                    // KMUP2 over the rows in use
       launch_wgr_bag_phase(w, 1, h->num_sms, h->stream);                          // Vb (with the old Ve), Va, Ve from the rows in use
-      if ((rc = fit_hat(h, f.b.p, reinterpret_cast<const float*>(f.sc.p), hatd.p))) return rc;  // mu + X b  (SysScalars starts with mu)
+      if ((rc = fit_hat(h, 1, f.b.p, reinterpret_cast<const float*>(f.sc.p), hatd.p))) return rc;  // mu + X b  (SysScalars starts with mu)
       launch_wgr_bag_phase(w, 2, h->num_sms, h->stream);                          // e = y - hat, intercept draw, L, posterior sums
       h->launches += 3;
     }

@@ -266,64 +266,142 @@ __global__ void __launch_bounds__(256) d_to_float_kernel(const double* __restric
 }
 void launch_d_to_float(const double* src, float* dst, int n, cudaStream_t st) { d_to_float_kernel<<<(n + 255) / 256, 256, 0, st>>>(src, dst, n); }
 
-// hat = mu + X b.  CTA (x = row tile of 256*16 rows, y = column split): partial[y][row] = sum over its
-// columns; then a second kernel adds the splits in a fixed order (deterministic).
-__global__ void __launch_bounds__(256) gemv_partial_kernel(GenoView g, const float* __restrict__ b, float* __restrict__ work,
-                                                           int splits) {
-  const int row0 = (blockIdx.x * 256 + threadIdx.x) * 16;
-  if (row0 >= g.ld) return;
-  float acc[16];
+// hat[t] = mu[t] + X b_t for k systems with one stream of X.
+// Split `y` of a column split takes the columns j = y, y + splits, ...; every row's partial sum of a system runs over them in increasing j
+// as one FMA chain, and a second kernel adds the splits in a fixed order (deterministic; k = 1 is the single-system fitted values).
+// A row's chain does not depend on which thread holds the row or on the other systems, so a thread takes R rows x KC systems:
+// each genotype is converted once and used KC times, each b_tj (staged in shared memory, kHatCols columns of the split at a time) R times.
+// CTAs of the same (row tile, split) and consecutive system chunks are adjacent in launch order (blockIdx.x = chunk): they read the
+// same X tile at about the same time, so HBM serves it once and L2 the rest.
+// A zero b_tj is not skipped: acc starts at +0 and an FMA never turns it into -0, so fmaf(x, 0, acc) == acc for every finite x.
+constexpr int kHatCols = 128;
+constexpr int kHatThreads = 256;
+
+template <int R>
+__device__ __forceinline__ void hat_rows(const GenoView& g, int64_t j, int64_t row0, float (&x)[R]) {
+  static_assert(R == 4 || R == 16, "rows per thread");
+  if (g.storage == 2) {  // float32 store
+    const float4* v = reinterpret_cast<const float4*>(g.xf + j * g.ld + row0);
 #pragma unroll
-  for (int q = 0; q < 16; q++) acc[q] = 0.0f;
-  for (int j = blockIdx.y; j < g.p; j += splits) {
-    const float bj = __ldg(b + j);
-    if (bj == 0.0f) continue;
-    if (g.storage == 2) {  // float32 store
-      const float4* v = reinterpret_cast<const float4*>(g.xf + (int64_t)j * g.ld + row0);
-#pragma unroll
-      for (int q = 0; q < 4; q++) {
-        const float4 x = __ldg(v + q);
-        acc[4 * q + 0] = fmaf(x.x, bj, acc[4 * q + 0]); acc[4 * q + 1] = fmaf(x.y, bj, acc[4 * q + 1]);
-        acc[4 * q + 2] = fmaf(x.z, bj, acc[4 * q + 2]); acc[4 * q + 3] = fmaf(x.w, bj, acc[4 * q + 3]);
-      }
-      continue;
+    for (int q = 0; q < R / 4; q++) {
+      const float4 f = __ldg(v + q);
+      x[4 * q + 0] = f.x; x[4 * q + 1] = f.y; x[4 * q + 2] = f.z; x[4 * q + 3] = f.w;
     }
-    uint32_t w[4];
-    if (g.storage == 0) {
-      const uint4 v = __ldg(reinterpret_cast<const uint4*>(g.x8 + (int64_t)j * g.ld + row0));
+    return;
+  }
+  uint32_t w[R / 4];
+  if (g.storage == 0) {
+    if constexpr (R == 16) {
+      const uint4 v = __ldg(reinterpret_cast<const uint4*>(g.x8 + j * g.ld + row0));
       w[0] = v.x; w[1] = v.y; w[2] = v.z; w[3] = v.w;
     } else {
-      const uint32_t pk = __ldg(reinterpret_cast<const uint32_t*>(g.x2 + (int64_t)j * g.ldb + (row0 >> 2)));
-#pragma unroll
-      for (int q = 0; q < 4; q++) {
-        const uint32_t byte = (pk >> (8 * q)) & 0xFFu;
-        w[q] = (byte & 3u) | (((byte >> 2) & 3u) << 8) | (((byte >> 4) & 3u) << 16) | (((byte >> 6) & 3u) << 24);
-      }
+      w[0] = __ldg(reinterpret_cast<const uint32_t*>(g.x8 + j * g.ld + row0));
     }
+  } else {  // 2-bit store: R / 4 packed bytes
+    uint32_t pk;
+    if constexpr (R == 16) pk = __ldg(reinterpret_cast<const uint32_t*>(g.x2 + j * g.ldb + (row0 >> 2)));
+    else pk = __ldg(g.x2 + j * g.ldb + (row0 >> 2));
 #pragma unroll
-    for (int q = 0; q < 4; q++) {
-      const uint32_t x = w[q] ^ 0x80808080u;
-#pragma unroll
-      for (int t = 0; t < 4; t++) acc[4 * q + t] = fmaf(byte_to_float(x, t), bj, acc[4 * q + t]);
+    for (int q = 0; q < R / 4; q++) {
+      const uint32_t byte = (pk >> (8 * q)) & 0xFFu;
+      w[q] = (byte & 3u) | (((byte >> 2) & 3u) << 8) | (((byte >> 4) & 3u) << 16) | (((byte >> 6) & 3u) << 24);
     }
   }
-  float* out = work + (int64_t)blockIdx.y * g.ld + row0;
 #pragma unroll
-  for (int q = 0; q < 16; q += 4) *reinterpret_cast<float4*>(out + q) = make_float4(acc[q], acc[q + 1], acc[q + 2], acc[q + 3]);
+  for (int q = 0; q < R / 4; q++) {
+    const uint32_t xw = w[q] ^ 0x80808080u;
+#pragma unroll
+    for (int t = 0; t < 4; t++) x[4 * q + t] = byte_to_float(xw, t);
+  }
 }
-__global__ void gemv_reduce_kernel(const float* __restrict__ work, int64_t ld, int n, int splits, const float* mu,
-                                   float* __restrict__ hat) {
-  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+
+// work[t][y][row] = sum over the columns of split y of x_row,j b_tj, for the KC systems of chunk blockIdx.x
+template <int R, int KC>
+__global__ void __launch_bounds__(kHatThreads) gemv_hat_partial_kernel(GenoView g, const float* __restrict__ b, int k,
+                                                                      float* __restrict__ work, int splits) {
+  static_assert(KC == 1 || KC % 4 == 0, "systems per thread");
+  __shared__ __align__(16) float bs[KC == 1 ? 1 : kHatCols][KC];
+  const int t0 = blockIdx.x * KC, split = blockIdx.z;
+  const int64_t row0 = ((int64_t)blockIdx.y * kHatThreads + threadIdx.x) * R;
+  const bool live = row0 < g.ld;  // KC > 1: no early return, the thread takes part in staging b
+  float acc[R][KC];
+#pragma unroll
+  for (int r = 0; r < R; r++)
+#pragma unroll
+    for (int t = 0; t < KC; t++) acc[r][t] = 0.0f;
+  if constexpr (KC == 1) {  // one system: b_j read in place, zero effects cost no load
+    if (!live) return;
+    for (int64_t j = split; j < g.p; j += splits) {
+      const float bj = __ldg(b + j);
+      if (bj == 0.0f) continue;
+      float x[R];
+      hat_rows<R>(g, j, row0, x);
+#pragma unroll
+      for (int r = 0; r < R; r++) acc[r][0] = fmaf(x[r], bj, acc[r][0]);
+    }
+    float* out = work + (int64_t)split * g.ld + row0;
+#pragma unroll
+    for (int q = 0; q < R; q += 4) *reinterpret_cast<float4*>(out + q) = make_float4(acc[q][0], acc[q + 1][0], acc[q + 2][0], acc[q + 3][0]);
+  } else {
+    const int ncol = (g.p - split + splits - 1) / splits;
+    for (int m0 = 0; m0 < ncol; m0 += kHatCols) {
+      const int mc = min(kHatCols, ncol - m0);
+      __syncthreads();  // the previous columns' b are consumed
+      for (int q = threadIdx.x; q < kHatCols * KC; q += kHatThreads) {
+        const int t = q / kHatCols, m = q - t * kHatCols;
+        bs[m][t] = (m < mc && t0 + t < k) ? __ldg(b + (int64_t)(t0 + t) * g.p + split + (int64_t)splits * (m0 + m)) : 0.0f;
+      }
+      __syncthreads();
+      if (!live) continue;
+#pragma unroll 2
+      for (int m = 0; m < mc; m++) {
+        float x[R];
+        hat_rows<R>(g, split + (int64_t)splits * (m0 + m), row0, x);
+#pragma unroll
+        for (int t4 = 0; t4 < KC; t4 += 4) {
+          const float4 bt = *reinterpret_cast<const float4*>(&bs[m][t4]);
+#pragma unroll
+          for (int r = 0; r < R; r++) {
+            acc[r][t4 + 0] = fmaf(x[r], bt.x, acc[r][t4 + 0]); acc[r][t4 + 1] = fmaf(x[r], bt.y, acc[r][t4 + 1]);
+            acc[r][t4 + 2] = fmaf(x[r], bt.z, acc[r][t4 + 2]); acc[r][t4 + 3] = fmaf(x[r], bt.w, acc[r][t4 + 3]);
+          }
+        }
+      }
+    }
+    if (!live) return;
+#pragma unroll
+    for (int t = 0; t < KC; t++) {
+      if (t0 + t >= k) break;
+      float* out = work + ((int64_t)(t0 + t) * splits + split) * g.ld + row0;
+#pragma unroll
+      for (int q = 0; q < R; q += 4) *reinterpret_cast<float4*>(out + q) = make_float4(acc[q][t], acc[q + 1][t], acc[q + 2][t], acc[q + 3][t]);
+    }
+  }
+}
+
+
+__global__ void __launch_bounds__(256) gemv_hat_reduce_kernel(const float* __restrict__ work, int64_t ld, int n, int splits,
+                                                              const float* __restrict__ mu, float* __restrict__ hat) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x, t = blockIdx.y;
   if (i >= n) return;
+  const float* w = work + (int64_t)t * splits * ld + i;
   float s = 0.0f;
-  for (int k = 0; k < splits; k++) s += work[(int64_t)k * ld + i];
-  hat[i] = s + mu[0];
+  for (int y = 0; y < splits; y++) s += w[(int64_t)y * ld];
+  hat[(int64_t)t * ld + i] = s + mu[t];
 }
-void launch_gemv_hat(const GenoView& g, const float* b, const float* mu_dev, float* hat, float* work, int splits,
-                     cudaStream_t st) {
-  dim3 grid((unsigned)((g.ld + 4095) / 4096), splits);
-  gemv_partial_kernel<<<grid, 256, 0, st>>>(g, b, work, splits);
-  gemv_reduce_kernel<<<(g.n + 255) / 256, 256, 0, st>>>(work, g.ld, g.n, splits, mu_dev, hat);
+
+template <int R, int KC>
+static void launch_hat_partial(const GenoView& g, const float* b, int k, float* work, int splits, cudaStream_t st) {
+  const int rows = kHatThreads * R;
+  dim3 grid((unsigned)((k + KC - 1) / KC), (unsigned)((g.ld + rows - 1) / rows), (unsigned)splits);
+  gemv_hat_partial_kernel<R, KC><<<grid, kHatThreads, 0, st>>>(g, b, k, work, splits);
+}
+
+void launch_gemv_hat(const GenoView& g, const float* b, int k, const float* mu, float* hat, float* work, int splits, cudaStream_t st) {
+  if (k == 1) launch_hat_partial<16, 1>(g, b, k, work, splits, st);
+  else if (k <= 4) launch_hat_partial<16, 4>(g, b, k, work, splits, st);
+  else launch_hat_partial<4, kHatChunk>(g, b, k, work, splits, st);
+  gemv_hat_reduce_kernel<<<dim3((unsigned)((g.n + 255) / 256), (unsigned)k), 256, 0, st>>>(work, g.ld, g.n, splits, mu, hat);
 }
 
 }  // namespace bwgr

@@ -41,9 +41,10 @@ void launch_col_stats_f32(const GenoView& g, const uint8_t* mask, double* xx, do
 // row multiplicities cnt[i] (uint8) instead of a 0/1 mask; any store
 void launch_col_stats_cnt(const GenoView& g, const uint8_t* cnt, double* xx, double* sx, cudaStream_t st);
 void launch_d_to_float(const double* src, float* dst, int n, cudaStream_t st);
-// hat = mu + X b (deterministic two-stage reduction). work: [splits][ld] floats.
-void launch_gemv_hat(const GenoView& g, const float* b, const float* mu_dev, float* hat, float* work, int splits,
-                     cudaStream_t st);
+// hat[t] = mu[t] + X b_t for k systems, one stream of X (deterministic two-stage reduction; each system's sum does not depend on k).
+// b: [k][p], mu: [k], hat: [k][ld], work: [k][splits][ld] floats (all device).
+constexpr int kHatChunk = 16;  // systems per thread when k > 4
+void launch_gemv_hat(const GenoView& g, const float* b, int k, const float* mu, float* hat, float* work, int splits, cudaStream_t st);
 
 // ---- small-n path: one persistent CTA per system -------------------------------------------------
 struct SmallNArgs {

@@ -30,11 +30,12 @@ def _merge(parts, axis_keys):
     return out
 
 
-def fit_sharded(fit_fn, Y, row_mask=None, group=None, **kw):
+def fit_sharded(fit_fn, Y, row_mask=None, group=None, offset_kw=None, **kw):
     """Run `fit_fn(Y_cols, row_mask=mask_cols, **kw)` (e.g. functools.partial(bw.em_fit, "emBC", gen=store)) on this
     rank's share of the columns of Y (n x nsys) and gather every rank's result dict on all ranks.  Works on any
     torch.distributed backend (nccl on the GPU box, gloo in the CPU tests); without an initialised process group it
-    degenerates to one rank."""
+    degenerates to one rank.  offset_kw: name of a keyword that receives the index of the rank's first column, e.g. "chain0"
+    with bw.gibbs_fit (one chain per column), so that the sharded systems draw the streams of the one-GPU fit."""
     import torch.distributed as dist
     Y = np.asarray(Y)
     nsys = Y.shape[1]
@@ -46,7 +47,8 @@ def fit_sharded(fit_fn, Y, row_mask=None, group=None, **kw):
     mine = None
     if e > s:
         m = None if row_mask is None else np.asarray(row_mask)[:, s:e]
-        res = fit_fn(Y[:, s:e], row_mask=m, **kw) if row_mask is not None else fit_fn(Y[:, s:e], **kw)
+        fkw = dict(kw) if offset_kw is None else dict(kw, **{offset_kw: s})
+        res = fit_fn(Y[:, s:e], row_mask=m, **fkw) if row_mask is not None else fit_fn(Y[:, s:e], **fkw)
         mine = {k: np.asarray(v) for k, v in res.items()}
     if world == 1:
         return _merge([mine], None)

@@ -158,7 +158,7 @@ typedef struct {
 } bwgr_gibbs_params;
 
 typedef struct {
-  double* mu;   /* [nchains] */
+  double* mu;   /* [nchains] (bwgr_gibbs_fit_sys: [S] here and below) */
   double* b;    /* [p x nchains] posterior means */
   double* d;    /* [p x nchains] (BayesB/C/Cpi/Dpi; the reference's PVAL is -log(1 - d)) or NULL */
   double* hat;  /* [n x nchains] */
@@ -167,6 +167,23 @@ typedef struct {
 } bwgr_gibbs_out;
 
 BWGR_API int bwgr_gibbs_fit(bwgr_handle* h, const bwgr_gibbs_params* par, const double* y, bwgr_gibbs_out* out);
+
+/* Several traits / CV folds in one call (not in the reference: its samplers take one y).  Column t of Y runs base.nchains chains, so
+ * there are S = nsys * nchains systems; system s = t * nchains + c draws from Philox chain index chain0 + s (disjoint streams; a caller
+ * that splits the columns over GPUs passes its first system as chain0 and gets the draws of the one-GPU fit).  A masked system fits
+ * its column on the rows its mask keeps: the draws are addressed by (sweep, marker, chain), so it is the fit of those rows alone under
+ * the same chain index, with MSx and the variance draws from those rows.  Every output of bwgr_gibbs_out has S columns; hat covers
+ * all n rows, the held-out ones included (their prediction).  bwgr_gibbs_fit = nsys 1, no mask, chain0 0.
+ * BWGR_ERR_ARG: nsys < 1, NaN in Y, a mask column that keeps fewer than 2 rows.  BWGR_ERR_UNSUPPORTED: a mask on a row-sharded
+ * store, or a shape no kernel family takes (more than 32 masked systems whose residual does not fit one SM). */
+typedef struct {
+  bwgr_gibbs_params base;   /* model, nchains, it, bi, pi, df, R2, seed: as for bwgr_gibbs_fit */
+  int nsys;                 /* phenotype columns of Y (traits / folds) */
+  const uint8_t* row_mask;  /* optional n x nsys, 1 = row used by that column's systems; NULL = all */
+  int chain0;               /* Philox chain index of the first system */
+} bwgr_gibbs_sys_params;
+BWGR_API int bwgr_gibbs_fit_sys(bwgr_handle* h, const bwgr_gibbs_sys_params* par, const double* Y /* n x nsys */,
+                                bwgr_gibbs_out* out);
 
 /* One Kuo-Mallick sweep, drop-in for KMUP(X,b,d,xx,e,L,Ve,pi) (:12-38); b,d,e updated in place.
  * The inclusion probability uses BayesB's ratio form (:673-674), algebraically identical to
@@ -177,6 +194,9 @@ BWGR_API int bwgr_kmup_sweep(bwgr_handle* h, double* b, double* d, const double*
 /* hat[n] = mu + X b on the handle's store: the X * b the reference's drivers form around the marker loop (emML2's u1 = X1 * b1,
  * Rcpp20260726ai.cpp:1275-1276; the fitted values of the two-design samplers :1063, :1151, :1212; wgr's gen0 %*% B, R/wgr.R:147). */
 BWGR_API int bwgr_fitted(bwgr_handle* h, const double* b, double mu, double* hat);
+/* The same for k systems with one pass over the store: hat[:, t] = mu[t] + X B[:, t].  B: p x k, mu: [k], hat: n x k (column-major).
+ * Every column is bit-identical to bwgr_fitted of that column alone (the summation order of a row does not depend on k). */
+BWGR_API int bwgr_fitted_sys(bwgr_handle* h, int k, const double* B, const double* mu, double* hat);
 
 /* KMUP2(X,Use,b,d,xx,E,L,Ve,pi) (:41-77), the bagged sweep of wgr(bag != 1): only the rows Use (0-based, as R passes them) enter.
  * b, d updated in place; e_out [nuse] = the residuals of the rows in use, in the order of Use (the reference's third list element).
