@@ -1814,6 +1814,7 @@ int bwgr_gibbs_fit_sys(bwgr_handle* h, const bwgr_gibbs_sys_params* sp, const do
   if (rc) return rc;
   rc = check_err_flag(h, "gibbs sweep");
   if (rc) return rc;
+  dump_trace(h);
   std::vector<SysScalars> sc(ns);
   CU(cudaMemcpyAsync(sc.data(), f.sc.p, sizeof(SysScalars) * ns, cudaMemcpyDeviceToHost, h->stream));
   std::vector<float> B((size_t)ns * p), D, V;

@@ -730,9 +730,9 @@ def test_full_size_properties():
 
 
 # ======================================================================================================================
-# Parity at the geometry the bench runs (VERDICT r1, next-round item 1): n = 50,000 rows -> 143 workers x 352 rows, 3 row atoms,
-# the same sweep kernel configuration as bench.py; p is cut to 2,048 markers so that the CPU oracle finishes in seconds
-# (its cost per marker does not depend on p).
+# Parity at the geometry the bench runs (VERDICT r1, next-round item 1): n = 50,000 rows -> the clustered plan with 4 row atoms per
+# worker (on a B200), the same sweep kernel configuration as bench.py; p is cut to 2,048 markers so that the CPU oracle finishes in
+# seconds (its cost per marker does not depend on p).  The plan is read from the sweep's trace header.
 # ======================================================================================================================
 @pytest.fixture(scope="module")
 def bench_slice():
@@ -741,13 +741,21 @@ def bench_slice():
 
 
 @pytest.mark.parametrize("model", ["emRR", "emBA", "emBC"])
-def test_blocked_path_at_bench_geometry(bench_slice, model):
+def test_blocked_path_at_bench_geometry(bench_slice, model, monkeypatch, tmp_path):
     X, y = bench_slice
     it = 8
     ref = O.em(model, y, X.astype(np.float32), it=it)
     ref64 = O.em(model, y, X.astype(np.float32), it=it, use_double=True)
+    trace = tmp_path / "trace.bin"
+    monkeypatch.setenv("BWGR_TRACE", str(trace))
     with bw.Genotypes(X, path=2) as g:
         out = bw.em_fit(model, y, g, it=it)
+    ctas, blocks, _, D = (int(v) for v in np.fromfile(trace, dtype=np.int64, count=4))
+    ld = (X.shape[0] + 127) // 128 * 128
+    W = 7 * ctas // 8                      # clustered: 7 workers per cluster of 8 CTAs
+    R = -(-(-(-ld // W)) // 16) * 16
+    print("bench geometry plan: %d CTAs, %d workers x %d rows, %d row atoms, look-ahead %d" % (ctas, W, R, -(-R // 128), D))
+    assert ctas % 8 == 0 and blocks == 16 and D == 1 and -(-R // 128) == 4 and R <= 512, (ctas, blocks, D, R)
     _close_em(out, ref, model, ref64)
 
 
