@@ -262,6 +262,7 @@ struct bwgr_handle {
   DevBuf<long long> xx_i, sx_i;
   DevBuf<float> xx_f;
   std::vector<double> h_xx, h_sx;
+  double xx_max = 0;  // max_j h_xx[j]: bounds every Gram entry and every |x_j'x_k| (Cauchy-Schwarz)
   std::vector<double> col_offset;  // bwgr_geno_load_f64_centred: x = code + col_offset[j]
   bool has_offset = false;
   DevBuf<int> err;
@@ -386,6 +387,8 @@ int finish_store(bwgr_handle* h, int storage) {
   CU(cudaStreamSynchronize(h->stream));
   h->h_xx.assign(xx.begin(), xx.end());
   h->h_sx.assign(sx.begin(), sx.end());
+  h->xx_max = 0;
+  for (double v : h->h_xx) h->xx_max = std::max(h->xx_max, v);
   std::vector<float> xf(h->p);
   for (int64_t j = 0; j < h->p; j++) xf[j] = (float)xx[j];
   CU(cudaMemcpyAsync(h->xx_f.p, xf.data(), sizeof(float) * h->p, cudaMemcpyHostToDevice, h->stream));
@@ -393,9 +396,7 @@ int finish_store(bwgr_handle* h, int storage) {
   int flag = 0, rc = 0;
   {  // codes 0..7 everywhere?  (one more streaming pass at load time)
     h->fp8_codes = 0;
-    double xxmax = 0;  // every Gram entry and every partial sum of non-negative codes is bounded by max_j xx_j (Cauchy-Schwarz)
-    for (double v : h->h_xx) xxmax = std::max(xxmax, v);
-    if (xxmax < 16777216.0) {
+    if (h->xx_max < 16777216.0) {  // every Gram entry and every partial sum of non-negative codes is bounded by max_j xx_j
       launch_check_range_i8(h->x8, h->ld, (int)h->n, (int)h->p, 0, 7, h->err.p, h->stream);
       h->launches++;
       if ((rc = take_err_flag(h, &flag))) return rc;
@@ -646,6 +647,8 @@ static int load_f64_real(bwgr_handle* h, const double* X, int64_t n, int64_t p, 
   CU(cudaMemcpyAsync(h->h_xx.data(), dxx.p, sizeof(double) * p, cudaMemcpyDeviceToHost, h->stream));
   CU(cudaMemcpyAsync(h->h_sx.data(), dsx.p, sizeof(double) * p, cudaMemcpyDeviceToHost, h->stream));
   CU(cudaStreamSynchronize(h->stream));
+  h->xx_max = 0;
+  for (double v : h->h_xx) h->xx_max = std::max(h->xx_max, v);
   h->n_global = h->n;
   h->storage = BWGR_STORE_F32;
   h->fp8_codes = 0;
@@ -1275,13 +1278,10 @@ int fit_begin(bwgr_handle* h, const FitSpec& s, const double* y) {
     PipePlan pl;
     if (!plan_pipe(h, s.model, ns, &pl)) return fail(BWGR_ERR_UNSUPPORTED, "the shape does not fit the pipelined blocked sweep");
     if (dist) {
-      {  // the per-rank Gram bands are summed in float by ncclAllReduce: exact (= independent of the sharding) only below 2^24.
-         // |G_jk| <= max_j xx_j (Cauchy-Schwarz) over ALL individuals; h_xx holds the all-reduced column statistics.
-        double xxmax = 0;
-        for (double v : h->h_xx) xxmax = std::max(xxmax, v);
-        if (!(xxmax < 16777216.0))
-          return fail(BWGR_ERR_UNSUPPORTED, "row-sharded fit: max_j sum_i x_ij^2 = %.0f >= 2^24, the float sum of the per-GPU Gram bands would depend on the sharding", xxmax);
-      }
+      // the per-rank Gram bands are summed in float by ncclAllReduce: exact (= independent of the sharding) only below 2^24.
+      // |G_jk| <= max_j xx_j (Cauchy-Schwarz) over ALL individuals; h_xx holds the all-reduced column statistics.
+      if (!(h->xx_max < 16777216.0))
+        return fail(BWGR_ERR_UNSUPPORTED, "row-sharded fit: max_j sum_i x_ij^2 = %.0f >= 2^24, the float sum of the per-GPU Gram bands would depend on the sharding", h->xx_max);
       // stale words of a previous fit (another nsys = another ring layout) must not be mistaken for this fit's: zero my ring,
       // then a collective as the barrier that no peer writes into it before it is clean
       CU(cudaMemsetAsync(h->hx_own.p, 0, sizeof(unsigned long long) * h->hx_own.n, h->stream));
@@ -1335,8 +1335,7 @@ int fit_begin(bwgr_handle* h, const FitSpec& s, const double* y) {
 
 // Fixed-point quantum of g = x'e: a power of two such that 64 x the Cauchy-Schwarz bound stays below 2^50.
 void g_fixed_point(bwgr_handle* h, const Fit& f, float* quantum, float* limit) {
-  double xxmax = 1;
-  for (double v : h->h_xx) xxmax = std::max(xxmax, v);
+  const double xxmax = std::max(1.0, h->xx_max);
   double yy = 0;
   for (size_t t = 0; t < f.vy.size(); t++) yy = std::max(yy, (double)f.vy[t] * (double)(h->n - 1));
   const double bound = 64.0 * (f.weighted ? 256.0 : 1.0) * std::sqrt(xxmax * std::max(yy, 1e-30));  // row multiplicities <= 255
@@ -1346,12 +1345,28 @@ void g_fixed_point(bwgr_handle* h, const Fit& f, float* quantum, float* limit) {
   *limit = (float)std::ldexp(1.0, ex);
 }
 
+// The fit's state as the sweep kernels and the epilogue take it.  The rule divides by the per-system xx of masked systems, else by
+// the caller's (KMUP) or the centred (MRR3) xx when the fit has one, else by the store's; the blocked family never has masked
+// systems.  Only the KMUP2 rule reads xx2.
+SweepState sweep_state(const bwgr_handle* h) {
+  const Fit& f = h->fit;
+  SweepState s;
+  s.g = h->view(); s.nsys = f.nsys;
+  s.e = f.e.p; s.b = f.b.p; s.d = f.d.p; s.vbv = f.vbv.p;
+  s.xx = f.masked ? f.xx_sys.p : (f.xx_over.p ? f.xx_over.p : h->xx_f.p); s.xx_per_sys = f.masked ? 1 : 0;
+  s.xx2 = f.model == M_KMUP2 ? f.xx_over.p : nullptr;
+  s.mask = f.mask.p; s.sc = f.sc.p;
+  s.seed_lo = (uint32_t)f.seed; s.seed_hi = (uint32_t)(f.seed >> 32); s.chain0 = f.chain0;
+  s.err = h->err.p;
+  return s;
+}
+
 int fit_sweeps(bwgr_handle* h, int nsweeps) {
   Fit& f = h->fit;
   if (!h || !f.active) return fail(BWGR_ERR_STATE, "no fit in progress");
   CU(cudaSetDevice(h->device));
-  const int64_t p = h->p, ld = h->ld;
-  const GenoView g = h->view();
+  const int64_t p = h->p;
+  const SweepState state = sweep_state(h);
   float quantum = 1, limit = 1;
   if (f.gridfam) g_fixed_point(h, f, &quantum, &limit);
   for (int k = 0; k < nsweeps; k++) {
@@ -1392,8 +1407,7 @@ int fit_sweeps(bwgr_handle* h, int nsweeps) {
       }
       if (f.full_inv) {  // the step coefficients change every sweep (lambda), the inverses with them
         cudaEvent_t pi = h->prof_begin(3);
-        launch_block_inverse(f.model, d_perm, (int)p, f.nblocks, f.gram_p, f.nband, f.xx_over.p ? f.xx_over.p : h->xx_f.p, f.vbv.p, f.sc.p,
-                             f.tinv.p, h->stream);
+        launch_block_inverse(f.model, d_perm, (int)p, f.nblocks, f.gram_p, f.nband, state.xx, state.vbv, state.sc, f.tinv.p, h->stream);
         h->prof_end(pi);
         h->launches++;
       }
@@ -1401,11 +1415,10 @@ int fit_sweeps(bwgr_handle* h, int nsweeps) {
       else CU(cudaMemsetAsync(f.part.p, 0, sizeof(unsigned long long) * f.part.n, h->stream));
       PipeArgs a;
       memset(&a, 0, sizeof a);
-      a.g = g; a.model = rule_model(f.model); a.nsys = f.nsys; a.perm = d_perm; a.nblocks = f.nblocks; a.gram = f.gram_p; a.nband = f.nband; a.tinv = f.full_inv ? f.tinv.p : nullptr;
-      a.e = f.e.p; a.b = f.b.p; a.d = f.d.p; a.vbv = f.vbv.p; a.xx = f.xx_over.p ? f.xx_over.p : h->xx_f.p; a.sx = f.sx_dev.p; a.cshift = f.cshift.p; a.sc = f.sc.p;
+      a.s = state; a.model = rule_model(f.model); a.perm = d_perm; a.nblocks = f.nblocks; a.gram = f.gram_p; a.nband = f.nband; a.tinv = f.full_inv ? f.tinv.p : nullptr;
+      a.sx = f.sx_dev.p; a.cshift = f.cshift.p;
       a.part = f.part.p; a.hred = f.part.p + (size_t)8 * f.nsys * 128 * 160; a.dew = f.dew.p; a.tag = ++f.tag;
-      a.seed_lo = (uint32_t)f.seed; a.seed_hi = (uint32_t)(f.seed >> 32); a.chain0 = f.chain0;
-      a.rows_per_cta = f.rows_per_cta; a.nworkers = f.nworkers; a.D = f.lookahead; a.nbuf = f.nbuf; a.sring = f.sring; a.err = h->err.p;
+      a.rows_per_cta = f.rows_per_cta; a.nworkers = f.nworkers; a.D = f.lookahead; a.nbuf = f.nbuf; a.sring = f.sring;
       a.world = h->world; a.rank = h->rank; a.gen0 = h->dist_gen;
       a.cl = f.cl; a.nclusters = f.nclusters; a.cx = f.cx.p;
       for (int r = 0; r < 8; r++) a.hx[r] = h->hx[r];
@@ -1445,20 +1458,15 @@ int fit_sweeps(bwgr_handle* h, int nsweeps) {
     } else if (f.gridfam) {
       GridArgs a;
       memset(&a, 0, sizeof a);
-      a.g = g; a.model = f.model; a.nsys = f.nsys; a.perm = d_perm; a.e = f.e.p; a.b = f.b.p; a.d = f.d.p; a.vbv = f.vbv.p;
-      a.xx = f.masked ? f.xx_sys.p : (f.xx_over.p ? f.xx_over.p : h->xx_f.p); a.xx_per_sys = f.masked ? 1 : 0;
-      a.mask = f.weighted ? f.cnt.p : f.mask.p;  // row multiplicities ride in the mask bytes (they weigh the dot products only)
-      a.xx2 = f.model == M_KMUP2 ? f.xx_over.p : nullptr;
+      a.s = state; a.model = f.model; a.perm = d_perm;
+      a.s.mask = f.weighted ? f.cnt.p : f.mask.p;  // row multiplicities ride in the mask bytes (they weigh the dot products only)
       a.blocked = f.grid_blocked ? 1 : 0;
       {  // cross products are bounded by max_j x_j'x_j (Cauchy-Schwarz): one unit = 1 (exact integers) unless that exceeds 2^50
-        double xxmax = 1;
-        for (double v : h->h_xx) xxmax = std::max(xxmax, v);
         int ex = 0;
-        std::frexp(xxmax, &ex);
+        std::frexp(std::max(1.0, h->xx_max), &ex);
         a.gram_quantum = h->storage == BWGR_STORE_F32 ? (float)std::ldexp(1.0, ex - 50) : (float)std::ldexp(1.0, std::max(0, ex - 50));
       }
-      a.sc = f.sc.p; a.acc = f.gridacc.p; a.g_quantum = quantum; a.seed_lo = (uint32_t)f.seed; a.seed_hi = (uint32_t)(f.seed >> 32);
-      a.chain0 = f.chain0; a.rows_per_cta = f.rows_per_cta; a.err = h->err.p;
+      a.acc = f.gridacc.p; a.g_quantum = quantum; a.rows_per_cta = f.rows_per_cta;
       CU(cudaMemsetAsync(f.gridacc.p, 0, sizeof(unsigned long long) * f.gridacc.n, h->stream));
       cudaEvent_t pe = h->prof_begin(1);
       const cudaError_t le = launch_grid_sweep(a, f.grid, h->stream);
@@ -1468,13 +1476,11 @@ int fit_sweeps(bwgr_handle* h, int nsweeps) {
     } else {
       SmallNArgs a;
       memset(&a, 0, sizeof a);
-      a.g = g; a.model = rule_model(f.model); a.nsys = f.nsys; a.perms = d_perm; a.y = f.y.p; a.e = f.e.p; a.b = f.b.p; a.d = f.d.p;
-      a.vbv = f.vbv.p; a.xx = f.masked ? f.xx_sys.p : (f.xx_over.p ? f.xx_over.p : h->xx_f.p); a.xx_per_sys = f.masked ? 1 : 0; a.mask = f.mask.p;
-      a.xx2 = f.xx_over.p; a.row_w = f.weighted ? f.row_w.p : nullptr;
-      a.sc = f.sc.p; a.seed_lo = (uint32_t)f.seed; a.seed_hi = (uint32_t)(f.seed >> 32); a.chain0 = f.chain0; a.err = h->err.p;
+      a.s = state; a.model = rule_model(f.model); a.perms = d_perm; a.row_w = f.weighted ? f.row_w.p : nullptr;
       cudaEvent_t pe = h->prof_begin(1);
-      launch_small_n(a, h->smem_optin, h->stream);
+      const cudaError_t le = launch_small_n(a, h->smem_optin, h->stream);
       h->prof_end(pe);
+      if (le != cudaSuccess) return fail(BWGR_ERR_CUDA, "small-n sweep launch failed: %s", cudaGetErrorString(le));
       h->launches++;
     }
     if (f.shuffled) { CU(cudaEventRecord(f.perm_free[slot], h->stream)); f.perm_ev_valid[slot] = true; }
@@ -1490,11 +1496,8 @@ int fit_sweeps(bwgr_handle* h, int nsweeps) {
         if (f.esum.n < (size_t)4 * f.nsys && (f.esum.alloc((size_t)4 * f.nsys) != cudaSuccess || f.emaxv.alloc(f.nsys) != cudaSuccess))
           return fail(BWGR_ERR_CUDA, "cudaMalloc failed");
       }
-      ea.model = f.model; ea.nsys = f.nsys; ea.n = (int)h->n; ea.p = (int)p; ea.ld = ld; ea.e = f.e.p; ea.y = f.y.p; ea.b = f.b.p;
-      ea.d = f.d.p; ea.vbv = f.vbv.p; ea.b_prev = f.b_prev.p; ea.mask = f.mask.p; ea.sc = f.sc.p; ea.B = f.B.p; ea.D = f.D.p;
-      ea.xx = f.masked ? f.xx_sys.p : (f.xx_over.p ? f.xx_over.p : h->xx_f.p); ea.xx_per_sys = f.masked ? 1 : 0;
-      ea.wts = f.wts.p;
-      ea.VBv = f.VBv.p; ea.seed_lo = (uint32_t)f.seed; ea.seed_hi = (uint32_t)(f.seed >> 32); ea.chain0 = f.chain0;
+      ea.s = state; ea.model = f.model; ea.y = f.y.p; ea.b_prev = f.b_prev.p; ea.wts = f.wts.p;
+      ea.B = f.B.p; ea.D = f.D.p; ea.VBv = f.VBv.p;
       cudaEvent_t pe2 = h->prof_begin(2);
       if (h->world > 1) {  // sums over individuals: per rank, then all-reduced; everything else is replicated
         launch_epilogue_partial(ea, f.esum.p, f.emaxv.p, h->stream);
@@ -2461,8 +2464,6 @@ int mrr3_general(bwgr_handle* h, int f32_variant, const double* Y, int k, const 
     CU(cudaStreamSynchronize(st));
   }
   std::vector<double> TrXSX(k), see(k);
-  double xxmax = 0;
-  for (int64_t j = 0; j < p; j++) xxmax = std::max(xxmax, h->h_xx[j]);
   for (int t = 0; t < k; t++) see[t] = vy[t] * (nn[t] - 1.0);  // e = y at the start
   if (F.TH) xsx.resize((size_t)p * k);
   for (int64_t j = 0; j < p; j++) {
@@ -2518,7 +2519,7 @@ int mrr3_general(bwgr_handle* h, int f32_variant, const double* Y, int k, const 
       std::vector<double> scl(64, 0.0);
       for (int t = 0; t < k; t++) {
         int ex = 0;
-        std::frexp(16.0 * std::sqrt(xxmax * see[t]) + 1e-300, &ex);
+        std::frexp(16.0 * std::sqrt(h->xx_max * see[t]) + 1e-300, &ex);
         scl[t] = std::ldexp(1.0, 52 - ex); scl[32 + t] = std::ldexp(1.0, ex - 52);
       }
       CU(cudaMemcpyAsync(d_scale, scl.data(), sizeof(double) * 64, cudaMemcpyHostToDevice, st));

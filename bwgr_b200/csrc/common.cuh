@@ -3,6 +3,8 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include <type_traits>
+
 namespace bwgr {
 
 // Unified model ids used on the device (EM = bwgr_em_model, Gibbs = 10 + bwgr_gibbs_model).
@@ -22,6 +24,31 @@ enum Model : int {
 __host__ __device__ constexpr int rule_model(int m) {
   // emML with weights steps like emDE too: the per-marker slot carries Lmb / d_j, refreshed by the epilogue after every sweep
   return m == M_EMML ? M_EMRR : m == M_EMBCPI ? M_EMBC : m == M_BCPI ? M_BC : (m == M_GSRR || m == M_GSFLM || m == M_EMMLD) ? M_EMDE : m;
+}
+// The one list of rules the sweep kernels are instantiated for: calls f(std::integral_constant<int, rule_model(m)>()), or nothing
+// when m is not a model id.  A kernel family leaves out, with if constexpr on the constant, the rules it is never launched with.
+template <class F>
+void with_rule(int m, F&& f) {
+  switch (rule_model(m)) {
+    case M_EMRR: f(std::integral_constant<int, M_EMRR>()); break;
+    case M_EMBA: f(std::integral_constant<int, M_EMBA>()); break;
+    case M_EMBB: f(std::integral_constant<int, M_EMBB>()); break;
+    case M_EMBC: f(std::integral_constant<int, M_EMBC>()); break;
+    case M_EMBL: f(std::integral_constant<int, M_EMBL>()); break;
+    case M_EMEN: f(std::integral_constant<int, M_EMEN>()); break;
+    case M_EMDE: f(std::integral_constant<int, M_EMDE>()); break;
+    case M_LASSO: f(std::integral_constant<int, M_LASSO>()); break;
+    case M_BRR: f(std::integral_constant<int, M_BRR>()); break;
+    case M_BA: f(std::integral_constant<int, M_BA>()); break;
+    case M_BB: f(std::integral_constant<int, M_BB>()); break;
+    case M_BC: f(std::integral_constant<int, M_BC>()); break;
+    case M_KMUP: f(std::integral_constant<int, M_KMUP>()); break;
+    case M_MRR: f(std::integral_constant<int, M_MRR>()); break;
+    case M_BL: f(std::integral_constant<int, M_BL>()); break;
+    case M_BDPI: f(std::integral_constant<int, M_BDPI>()); break;
+    case M_KMUP2: f(std::integral_constant<int, M_KMUP2>()); break;
+    default: break;
+  }
 }
 
 // Per-system scalar state, device resident, updated by the sweep epilogue.
@@ -278,6 +305,17 @@ __device__ __forceinline__ float byte_to_float(uint32_t word_xored, int byte_idx
   const uint32_t sel = 0x7440u | (uint32_t)byte_idx;  // result bytes {u_i, 0x00, 0x00, 0x4B} from (word, 0x4B000000)
   asm("prmt.b32 %0, %1, %2, %3;" : "=r"(r) : "r"(word_xored), "r"(0x4B000000u), "r"(sel));
   return __uint_as_float(r) - 8388736.0f;
+}
+
+// 2-bit store: expand 4 packed bytes (16 rows, row r in bits 2*(r%4) of byte r/4) into 16 int8 bytes.
+__device__ __forceinline__ uint4 expand_2bit(uint32_t pk) {
+  uint32_t w[4];
+#pragma unroll
+  for (int q = 0; q < 4; q++) {
+    const uint32_t byte = (pk >> (8 * q)) & 0xFFu;
+    w[q] = (byte & 3u) | (((byte >> 2) & 3u) << 8) | (((byte >> 4) & 3u) << 16) | (((byte >> 6) & 3u) << 24);
+  }
+  return make_uint4(w[0], w[1], w[2], w[3]);
 }
 
 __device__ __forceinline__ float warp_sum(float v) {

@@ -42,25 +42,25 @@ __global__ void __cluster_dims__(kEpiCl, 1, 1) __launch_bounds__(1024) epilogue_
   __shared__ int s_acc;
   const int cr = (int)cluster.block_rank();
   const int sys = blockIdx.x / kEpiCl, tid = threadIdx.x, T = blockDim.x * kEpiCl, gt = cr * (int)blockDim.x + tid;
-  SysScalars* scp = a.sc + sys;
+  SysScalars* scp = a.s.sc + sys;
   if (scp->done) return;
-  float* e = a.e + (size_t)sys * a.ld;
-  const float* y = a.y + (size_t)sys * a.ld;
-  float* b = a.b + (size_t)sys * a.p;
-  const float* d = a.d ? a.d + (size_t)sys * a.p : nullptr;
-  float* vbv = a.vbv ? a.vbv + (size_t)sys * a.p : nullptr;
-  const uint8_t* mask = a.mask ? a.mask + (size_t)sys * a.ld : nullptr;
+  float* e = a.s.e + (size_t)sys * a.s.g.ld;
+  const float* y = a.y + (size_t)sys * a.s.g.ld;
+  float* b = a.s.b + (size_t)sys * a.s.g.p;
+  const float* d = a.s.d ? a.s.d + (size_t)sys * a.s.g.p : nullptr;
+  float* vbv = a.s.vbv ? a.s.vbv + (size_t)sys * a.s.g.p : nullptr;
+  const uint8_t* mask = a.s.mask ? a.s.mask + (size_t)sys * a.s.g.ld : nullptr;
   const int model = a.model;
 
   double se = 0, see = 0, sey = 0, sy = 0;
   float emax = 0.0f;
   if (!a.esum)  // row-sharded fit: the sums over individuals were taken per rank and all-reduced (a.esum)
-    for (int i0 = gt; i0 < a.n; i0 += 8 * T) {  // one CTA walks the vector: eight loads in flight per thread, or latency is all there is
+    for (int i0 = gt; i0 < a.s.g.n; i0 += 8 * T) {  // one CTA walks the vector: eight loads in flight per thread, or latency is all there is
       float ev[8], yv[8];
 #pragma unroll
       for (int u = 0; u < 8; u++) {
         const int i = i0 + u * T;
-        const bool ok = i < a.n && (!mask || mask[i]);
+        const bool ok = i < a.s.g.n && (!mask || mask[i]);
         ev[u] = ok ? e[i] : 0.0f;
         yv[u] = ok ? y[i] : 0.0f;
       }
@@ -79,15 +79,15 @@ __global__ void __cluster_dims__(kEpiCl, 1, 1) __launch_bounds__(1024) epilogue_
   emax = 0.0f;
   for (int w = 0; w < (int)(blockDim.x >> 5); w++) emax = fmaxf(emax, sh_max[w]);
   double sbb = 0, sd = 0, scnv = 0;
-  for (int j0 = gt; j0 < a.p; j0 += 8 * T) {
+  for (int j0 = gt; j0 < a.s.g.p; j0 += 8 * T) {
     float bv[8], dv[8], pv[8];
 #pragma unroll
     for (int u = 0; u < 8; u++) {
       const int j = j0 + u * T;
-      const bool ok = j < a.p;
+      const bool ok = j < a.s.g.p;
       bv[u] = ok ? b[j] : 0.0f;
       dv[u] = (ok && d) ? d[j] : 0.0f;
-      pv[u] = (ok && a.b_prev) ? a.b_prev[(size_t)sys * a.p + j] : bv[u];
+      pv[u] = (ok && a.b_prev) ? a.b_prev[(size_t)sys * a.s.g.p + j] : bv[u];
     }
 #pragma unroll
     for (int u = 0; u < 8; u++) {
@@ -118,7 +118,7 @@ __global__ void __cluster_dims__(kEpiCl, 1, 1) __launch_bounds__(1024) epilogue_
 
   if (cr == 0 && tid == 0) {
     SysScalars s = *scp;
-    const float n = s.n_eff, p = (float)a.p;
+    const float n = s.n_eff, p = (float)a.s.g.p;
     const float ee = (float)see, bb = (float)sbb;
     float eM = (float)(se / (double)n);
     int accumulate = 0;
@@ -135,7 +135,7 @@ __global__ void __cluster_dims__(kEpiCl, 1, 1) __launch_bounds__(1024) epilogue_
           break;
         case M_EMBC:
           s.ve = (ee + s.Se) / (n + s.df);
-          s.vb = (bb + s.Sa) / (p + s.df) / ((float)(sd / (double)a.p) - s.Pi);
+          s.vb = (bb + s.Sa) / (p + s.df) / ((float)(sd / (double)a.s.g.p) - s.Pi);
           s.lmb = s.ve / s.vb;
           break;
         case M_EMEN: {
@@ -171,7 +171,7 @@ __global__ void __cluster_dims__(kEpiCl, 1, 1) __launch_bounds__(1024) epilogue_
           break;
         }
         case M_EMBCPI: {  // :1529-1536 ; pi_mix = the prior Pi, cxx = sum of the marker variances
-          const float dm = (float)(sd / (double)a.p);
+          const float dm = (float)(sd / (double)a.s.g.p);
           s.Pi = ((1.0f - dm) * p + s.pi_mix * s.df) / (p + s.df);
           s.Pi0 = (1.0f - s.Pi) / s.Pi;
           s.MSx = s.cxx * s.Pi * (1.0f - s.Pi);
@@ -204,26 +204,26 @@ __global__ void __cluster_dims__(kEpiCl, 1, 1) __launch_bounds__(1024) epilogue_
       s.its += 1;
     } else {
       // Gibbs: intercept draw, then variances (counter = (0xFFFFFFFF, sweep, chain, purpose))
-      const uint32_t chain = (uint32_t)(a.chain0 + sys), sw = (uint32_t)s.sweep;
+      const uint32_t chain = (uint32_t)(a.s.chain0 + sys), sw = (uint32_t)s.sweep;
       uint32_t c[4] = {0xFFFFFFFFu, sw, chain, 0u};
-      philox4x32_10(c, a.seed_lo, a.seed_hi);
+      philox4x32_10(c, a.s.seed_lo, a.s.seed_hi);
       float z, z2;
       box_muller(c[0], c[1], z, z2);
       eM = eM + sqrtf(s.ve / n) * z;
       const float ee2 = (float)(see - 2.0 * (double)eM * se + (double)n * (double)eM * (double)eM);
-      const float chi_e = rchisq_philox(n + s.df, 0xFFFFFFFFu, sw, chain, 1u, a.seed_lo, a.seed_hi);
+      const float chi_e = rchisq_philox(n + s.df, 0xFFFFFFFFu, sw, chain, 1u, a.s.seed_lo, a.s.seed_hi);
       if (model == M_BRR || model == M_BC || model == M_BCPI) {
-        const float chi_b = rchisq_philox(p + s.df, 0xFFFFFFFFu, sw, chain, 2u, a.seed_lo, a.seed_hi);
+        const float chi_b = rchisq_philox(p + s.df, 0xFFFFFFFFu, sw, chain, 2u, a.s.seed_lo, a.s.seed_hi);
         s.ve = (ee2 + s.Se) / chi_e;
         s.vb = (bb + s.Sb) / chi_b;
         s.lmb = s.ve / s.vb;
         if (model == M_BCPI) {  // :906-907 ; the mixing odds Pi0 stay as they were
-          s.Pi = (float)(sd / (double)a.p);
+          s.Pi = (float)(sd / (double)a.s.g.p);
           s.Sb = s.df * s.R2 * s.vy / s.MSx / (1.0f - s.Pi);
         }
       } else {
         s.ve = (ee2 + s.Se) / chi_e;
-        if (model == M_BDPI) s.Pi = (float)(sd / (double)a.p);  // :969
+        if (model == M_BDPI) s.Pi = (float)(sd / (double)a.s.g.p);  // :969
       }
       s.C = -0.5f / sqrtf(s.ve);
       if (s.sweep > s.burn) {  // sic: i > bi, divided later by it-bi (:624-627)
@@ -248,9 +248,9 @@ __global__ void __cluster_dims__(kEpiCl, 1, 1) __launch_bounds__(1024) epilogue_
   cluster.sync();  // CTA 0 stays until its shared memory has been read
   const float eM = s_eM;
   if (model == M_EMDE && vbv) {  // :293-296 ; Vb_j = b_j^2 + Ve/(xx_j + Lmb_j + 1e-4), Lmb_j = sqrt(cxx Ve / Vb_j)
-    const float* xx = a.xx + (a.xx_per_sys ? (size_t)sys * a.p : 0);
+    const float* xx = a.s.xx + (a.s.xx_per_sys ? (size_t)sys * a.s.g.p : 0);
     const float Ve = s_ve, cxx = s_cxx;
-    for (int j = gt; j < a.p; j += T) {
+    for (int j = gt; j < a.s.g.p; j += T) {
       float xxj = xx[j];
       if (xxj == 0.0f) xxj = 0.1f;  // :261
       const float Vb = b[j] * b[j] + Ve / (xxj + vbv[j] + 0.0001f);
@@ -258,12 +258,12 @@ __global__ void __cluster_dims__(kEpiCl, 1, 1) __launch_bounds__(1024) epilogue_
     }
   }
   if (model == M_EMMLD && vbv && a.wts) {  // :495 ; the penalty of marker j is Lmb / d_j
-    for (int j = gt; j < a.p; j += T) vbv[j] = s_lmb / a.wts[j];
+    for (int j = gt; j < a.s.g.p; j += T) vbv[j] = s_lmb / a.wts[j];
   }
   if ((model == M_GSRR || model == M_GSFLM) && vbv) {  // the per-marker slot carries Lmb_j + 0.01 (the rule's denominator)
-    const float* xx = a.xx + (a.xx_per_sys ? (size_t)sys * a.p : 0);
+    const float* xx = a.s.xx + (a.s.xx_per_sys ? (size_t)sys * a.s.g.p : 0);
     const float vna = s_ve, phi = s_cxx;
-    for (int j = gt; j < a.p; j += T) {
+    for (int j = gt; j < a.s.g.p; j += T) {
       if (model == M_GSRR) vbv[j] = s_lmb + 0.01f;  // :1621-1623
       else {                                        // :1588-1589 ; Vb_j = b_j^2 + vna/(xx_j + Lmb_j), Lmb_j = sqrt(phi vna / Vb_j)
         const float Vb = b[j] * b[j] + vna / (xx[j] + (vbv[j] - 0.01f));
@@ -272,18 +272,18 @@ __global__ void __cluster_dims__(kEpiCl, 1, 1) __launch_bounds__(1024) epilogue_
     }
   }
   if (eM != 0.0f)
-    for (int i0 = gt; i0 < a.n; i0 += 8 * T) {
+    for (int i0 = gt; i0 < a.s.g.n; i0 += 8 * T) {
       float ev[8];
 #pragma unroll
-      for (int u = 0; u < 8; u++) { const int i = i0 + u * T; ev[u] = i < a.n ? e[i] : 0.0f; }
+      for (int u = 0; u < 8; u++) { const int i = i0 + u * T; ev[u] = i < a.s.g.n ? e[i] : 0.0f; }
 #pragma unroll
-      for (int u = 0; u < 8; u++) { const int i = i0 + u * T; if (i < a.n && (!mask || mask[i])) e[i] = ev[u] - eM; }
+      for (int u = 0; u < 8; u++) { const int i = i0 + u * T; if (i < a.s.g.n && (!mask || mask[i])) e[i] = ev[u] - eM; }
     }
   if (s_acc && a.B) {
-    float* B = a.B + (size_t)sys * a.p;
-    for (int j = gt; j < a.p; j += T) B[j] += b[j];
-    if (a.D && d) { float* D = a.D + (size_t)sys * a.p; for (int j = gt; j < a.p; j += T) D[j] += d[j]; }
-    if (a.VBv && vbv) { float* V = a.VBv + (size_t)sys * a.p; for (int j = gt; j < a.p; j += T) V[j] += vbv[j]; }
+    float* B = a.B + (size_t)sys * a.s.g.p;
+    for (int j = gt; j < a.s.g.p; j += T) B[j] += b[j];
+    if (a.D && d) { float* D = a.D + (size_t)sys * a.s.g.p; for (int j = gt; j < a.s.g.p; j += T) D[j] += d[j]; }
+    if (a.VBv && vbv) { float* V = a.VBv + (size_t)sys * a.s.g.p; for (int j = gt; j < a.s.g.p; j += T) V[j] += vbv[j]; }
   }
 }
 
@@ -384,11 +384,11 @@ __global__ void __launch_bounds__(1024) epilogue_partial_kernel(EpilogueArgs a, 
   __shared__ double sh[32];
   __shared__ float sh_max[32];
   const int sys = blockIdx.x, tid = threadIdx.x, T = blockDim.x;
-  const float* e = a.e + (size_t)sys * a.ld;
-  const float* y = a.y + (size_t)sys * a.ld;
+  const float* e = a.s.e + (size_t)sys * a.s.g.ld;
+  const float* y = a.y + (size_t)sys * a.s.g.ld;
   double se = 0, see = 0, sey = 0, sy = 0;
   float emax = 0.0f;
-  for (int i = tid; i < a.n; i += T) {
+  for (int i = tid; i < a.s.g.n; i += T) {
     const double ev = e[i], yv = y[i];
     se += ev; see += ev * ev; sey += ev * yv; sy += yv;
     emax = fmaxf(emax, fabsf(e[i]));
@@ -408,7 +408,7 @@ __global__ void __launch_bounds__(1024) epilogue_partial_kernel(EpilogueArgs a, 
 }  // namespace
 
 void launch_epilogue_partial(const EpilogueArgs& a, double* out, float* emax_out, cudaStream_t st) {
-  epilogue_partial_kernel<<<a.nsys, 1024, 0, st>>>(a, out, emax_out);
+  epilogue_partial_kernel<<<a.s.nsys, 1024, 0, st>>>(a, out, emax_out);
 }
 
 // bagged wgr: phase 1 (variances) before the fitted values are rebuilt, phase 2 (intercept, posterior sums, per-marker part) after
@@ -428,6 +428,6 @@ void launch_wgr_step(const WgrArgs& a, int num_sms, cudaStream_t st) {
   wgr_markers_kernel<<<num_sms, 256, 0, st>>>(a);
 }
 
-void launch_epilogue(const EpilogueArgs& a, cudaStream_t st) { epilogue_kernel<<<a.nsys * kEpiCl, 1024, 0, st>>>(a); }
+void launch_epilogue(const EpilogueArgs& a, cudaStream_t st) { epilogue_kernel<<<a.s.nsys * kEpiCl, 1024, 0, st>>>(a); }
 
 }  // namespace bwgr

@@ -301,11 +301,9 @@ __device__ __forceinline__ void hat_rows(const GenoView& g, int64_t j, int64_t r
     uint32_t pk;
     if constexpr (R == 16) pk = __ldg(reinterpret_cast<const uint32_t*>(g.x2 + j * g.ldb + (row0 >> 2)));
     else pk = __ldg(g.x2 + j * g.ldb + (row0 >> 2));
-#pragma unroll
-    for (int q = 0; q < R / 4; q++) {
-      const uint32_t byte = (pk >> (8 * q)) & 0xFFu;
-      w[q] = (byte & 3u) | (((byte >> 2) & 3u) << 8) | (((byte >> 4) & 3u) << 16) | (((byte >> 6) & 3u) << 24);
-    }
+    const uint4 v = expand_2bit(pk);
+    w[0] = v.x;
+    if constexpr (R == 16) { w[1] = v.y; w[2] = v.z; w[3] = v.w; }
   }
 #pragma unroll
   for (int q = 0; q < R / 4; q++) {

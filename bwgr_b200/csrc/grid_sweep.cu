@@ -56,37 +56,37 @@ __global__ void __launch_bounds__(kT, 1) grid_sweep_kernel(GridArgs a) {
   __shared__ float s_de[32];
   __shared__ float s_wred[8][33];
   GridSmem s;
-  const int ns = a.nsys, rp = a.rows_per_cta, p = a.g.p;
-  const bool masked = a.mask != nullptr;
+  const int ns = a.s.nsys, rp = a.rows_per_cta, p = a.s.g.p;
+  const bool masked = a.s.mask != nullptr;
   grid_carve(smem_raw, ns, rp, masked, (int)sizeof(XT), &s);
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, G = (int)gridDim.x, cta = blockIdx.x;
-  const int64_t ld = a.g.ld, r0 = (int64_t)cta * rp;
+  const int64_t ld = a.s.g.ld, r0 = (int64_t)cta * rp;
   for (int q = tid; q < ns * rp; q += kT) {
     const int t = q / rp, i = q - t * rp;
     const bool in = r0 + i < ld;
-    s.E[q] = in ? a.e[(size_t)t * ld + r0 + i] : 0.0f;
-    if (masked) s.M[q] = in ? a.mask[(size_t)t * ld + r0 + i] : (uint8_t)0;
+    s.E[q] = in ? a.s.e[(size_t)t * ld + r0 + i] : 0.0f;
+    if (masked) s.M[q] = in ? a.s.mask[(size_t)t * ld + r0 + i] : (uint8_t)0;
   }
   for (int q = tid; q < kD * rp * (int)sizeof(XT); q += kT) s.xs[0][q] = 0;  // the ring slots are contiguous (rp is a multiple of 16)
-  if (tid < ns) s.sc[tid] = a.sc[tid];
+  if (tid < ns) s.sc[tid] = a.s.sc[tid];
   if (tid == 0) s_abort = 0;
   const int nch = rp * (int)sizeof(XT) / 16;  // 16-byte chunks of a slab
   constexpr int kRowsPerChunk = 16 / (int)sizeof(XT);
-  const float* xxbase = a.xx;
+  const float* xxbase = a.s.xx;
   int Jnext = a.perm ? a.perm[0] : 0;
   auto prefetch = [&](int m) {
     if (m < p) {
       const int J = Jnext, slot = m % kD;
       if (m + 1 < p) Jnext = a.perm ? a.perm[m + 1] : m + 1;
-      const unsigned char* col = sizeof(XT) == 1 ? reinterpret_cast<const unsigned char*>(a.g.x8 + (int64_t)J * ld + r0)
-                                                 : reinterpret_cast<const unsigned char*>(a.g.xf + (int64_t)J * ld + r0);
+      const unsigned char* col = sizeof(XT) == 1 ? reinterpret_cast<const unsigned char*>(a.s.g.x8 + (int64_t)J * ld + r0)
+                                                 : reinterpret_cast<const unsigned char*>(a.s.g.xf + (int64_t)J * ld + r0);
       for (int c = tid; c < nch; c += kT)
         if (r0 + (int64_t)kRowsPerChunk * c < ld) cp_async16(s.xs[slot] + 16 * c, col + 16 * c);
       float* v = s.vin[slot];
-      if (tid < 32) { if (tid < ns) cp_async4(v + tid, a.b + (size_t)tid * p + J); }
-      else if (tid < 64) { const int t = tid - 32; if (t < ns && a.vbv) cp_async4(v + 32 + t, a.vbv + (size_t)t * p + J); }
-      else if (tid < 96) { const int t = tid - 64; if (t < ns) cp_async4(v + 64 + t, xxbase + (a.xx_per_sys ? (size_t)t * p : 0) + J); }
-      else if (tid == 96 && a.xx2) cp_async4(v + 96, a.xx2 + J);
+      if (tid < 32) { if (tid < ns) cp_async4(v + tid, a.s.b + (size_t)tid * p + J); }
+      else if (tid < 64) { const int t = tid - 32; if (t < ns && a.s.vbv) cp_async4(v + 32 + t, a.s.vbv + (size_t)t * p + J); }
+      else if (tid < 96) { const int t = tid - 64; if (t < ns) cp_async4(v + 64 + t, xxbase + (a.s.xx_per_sys ? (size_t)t * p : 0) + J); }
+      else if (tid == 96 && a.s.xx2) cp_async4(v + 96, a.s.xx2 + J);
       if (tid == 0) s.Js[slot] = J;
     }
     cp_async_commit();
@@ -95,7 +95,7 @@ __global__ void __launch_bounds__(kT, 1) grid_sweep_kernel(GridArgs a) {
   for (int m = 0; m < kD - 1; m++) prefetch(m);
   __syncthreads();
   if (model_is_gibbs(MODEL) && warp == 1 && lane < ns)  // draws of marker 0
-    s.dr[lane] = marker_draws(MODEL, (uint32_t)s.Js[0], (uint32_t)s.sc[lane].sweep, (uint32_t)(a.chain0 + lane), s.sc[lane].df, a.seed_lo, a.seed_hi);
+    s.dr[lane] = marker_draws(MODEL, (uint32_t)s.Js[0], (uint32_t)s.sc[lane].sweep, (uint32_t)(a.s.chain0 + lane), s.sc[lane].df, a.s.seed_lo, a.s.seed_hi);
   const unsigned long long t_start = globaltimer_ns();
   const double inv_q = (double)a.g_quantum;  // value of one fixed-point unit
   const double qinv = 1.0 / (double)a.g_quantum;
@@ -140,9 +140,9 @@ __global__ void __launch_bounds__(kT, 1) grid_sweep_kernel(GridArgs a) {
         double v = 0.0;
 #pragma unroll
         for (int w = 0; w < 8; w++) v += (double)s_wred[w][lane];
-        grid_add(a.acc + ((size_t)m * kGridCopies + (cta & (kGridCopies - 1))) * 32 + lane, v * qinv, a.err);
+        grid_add(a.acc + ((size_t)m * kGridCopies + (cta & (kGridCopies - 1))) * 32 + lane, v * qinv, a.s.err);
       }
-      const long long tot = grid_wait_total(a.acc + (size_t)m * kGridCopies * 32 + (on ? lane : 0), on, G, a.err, t_start, &s_abort);
+      const long long tot = grid_wait_total(a.acc + (size_t)m * kGridCopies * 32 + (on ? lane : 0), on, G, a.s.err, t_start, &s_abort);
       if (on) {
         const float g = (float)((double)tot * inv_q);
         const SysScalars& sc = s.sc[lane];
@@ -151,21 +151,21 @@ __global__ void __launch_bounds__(kT, 1) grid_sweep_kernel(GridArgs a) {
           MarkerDraws dr;
           if (model_is_gibbs(MODEL)) dr = s.dr[(m & 1) * 32 + lane];
           else { dr.z1 = dr.z2 = dr.u = 0.0f; dr.chi = 1.0f; }
-          const float vbj = a.vbv ? vin[32 + lane] : 0.0f;
-          const RuleOut r = marker_rule<MODEL>(g, vin[64 + lane], vin[lane], vbj, sc, dr, a.xx2 ? vin[96] : 0.0f);
+          const float vbj = a.s.vbv ? vin[32 + lane] : 0.0f;
+          const RuleOut r = marker_rule<MODEL>(g, vin[64 + lane], vin[lane], vbj, sc, dr, a.s.xx2 ? vin[96] : 0.0f);
           de = r.de;
           if (cta == 0) {
             const size_t q = (size_t)lane * p + s.Js[slot];
-            a.b[q] = r.b;
-            if (model_has_d(MODEL) && a.d) a.d[q] = r.d;
-            if (model_rule_writes_vbj(MODEL) && a.vbv) a.vbv[q] = r.vbj;
+            a.s.b[q] = r.b;
+            if (model_has_d(MODEL) && a.s.d) a.s.d[q] = r.d;
+            if (model_rule_writes_vbj(MODEL) && a.s.vbv) a.s.vbv[q] = r.vbj;
           }
         }
         s_de[lane] = de;
       }
     } else if (model_is_gibbs(MODEL) && warp == 1 && lane < ns && m + 1 < p) {  // the next marker's draws, off the chain
-      s.dr[((m + 1) & 1) * 32 + lane] = marker_draws(MODEL, (uint32_t)s.Js[(m + 1) % kD], (uint32_t)s.sc[lane].sweep, (uint32_t)(a.chain0 + lane),
-                                                     s.sc[lane].df, a.seed_lo, a.seed_hi);
+      s.dr[((m + 1) & 1) * 32 + lane] = marker_draws(MODEL, (uint32_t)s.Js[(m + 1) % kD], (uint32_t)s.sc[lane].sweep, (uint32_t)(a.s.chain0 + lane),
+                                                     s.sc[lane].df, a.s.seed_lo, a.s.seed_hi);
     }
     __syncthreads();
     if (s_abort) return;  // the host reports the error flag; the residuals of this launch are not written back
@@ -186,7 +186,7 @@ __global__ void __launch_bounds__(kT, 1) grid_sweep_kernel(GridArgs a) {
   __syncthreads();
   for (int q = tid; q < ns * rp; q += kT) {
     const int t = q / rp, i = q - t * rp;
-    if (r0 + i < ld) a.e[(size_t)t * ld + r0 + i] = s.E[q];
+    if (r0 + i < ld) a.s.e[(size_t)t * ld + r0 + i] = s.E[q];
   }
 }
 
@@ -247,18 +247,18 @@ __global__ void __launch_bounds__(kTB, 1) grid_block_kernel(GridArgs a) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   __shared__ int s_abort;
   GridBlockSmem s;
-  const int ns = a.nsys, rp = a.rows_per_cta, p = a.g.p;
+  const int ns = a.s.nsys, rp = a.rows_per_cta, p = a.s.g.p;
   grid_block_carve(smem_raw, ns, rp, (int)sizeof(XT), model_is_gibbs(MODEL), &s);
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, G = (int)gridDim.x, cta = blockIdx.x;
-  const int64_t ld = a.g.ld, r0 = (int64_t)cta * rp;
+  const int64_t ld = a.s.g.ld, r0 = (int64_t)cta * rp;
   const int nblk = (p + kGB - 1) / kGB, W = grid_block_words(ns), ndot = kGB * ns;
   for (int q = tid; q < ns * rp; q += kTB) {
     const int t = q / rp, i = q - t * rp;
-    s.E[q] = (r0 + i < ld) ? a.e[(size_t)t * ld + r0 + i] : 0.0f;
+    s.E[q] = (r0 + i < ld) ? a.s.e[(size_t)t * ld + r0 + i] : 0.0f;
   }
   for (int q = tid; q < kGR * kGB * rp * (int)sizeof(XT); q += kTB) s.xs[0][q] = 0;  // slots are contiguous
   for (int q = tid; q < kGR * kGB * 100; q += kTB) s.vin[0][q] = 0.0f;
-  if (tid < ns) s.sc[tid] = a.sc[tid];
+  if (tid < ns) s.sc[tid] = a.s.sc[tid];
   if (tid == 0) s_abort = 0;
   for (int j = 1 + warp; j < kGB; j += kTB / 32)
     for (int i = lane; i < j; i += 32) s.pj[j * (j - 1) / 2 + i] = (unsigned char)j;
@@ -283,7 +283,7 @@ __global__ void __launch_bounds__(kTB, 1) grid_block_kernel(GridArgs a) {
         const int j = q / nch, c = q - j * nch;
         if (r0 + (int64_t)kRowsPerChunk * c < ld) {
           const int64_t off = (int64_t)Jv[j] * ld + r0;
-          const unsigned char* col = sizeof(XT) == 1 ? reinterpret_cast<const unsigned char*>(a.g.x8 + off) : reinterpret_cast<const unsigned char*>(a.g.xf + off);
+          const unsigned char* col = sizeof(XT) == 1 ? reinterpret_cast<const unsigned char*>(a.s.g.x8 + off) : reinterpret_cast<const unsigned char*>(a.s.g.xf + off);
           cp_async16(s.xs[slot] + (size_t)j * rp * sizeof(XT) + 16 * c, col + 16 * c);
         }
       }
@@ -293,9 +293,9 @@ __global__ void __launch_bounds__(kTB, 1) grid_block_kernel(GridArgs a) {
         if (t < ns) {
           const int J = Jv[j];
           float* v = s.vin[slot] + j * 100 + 32 * w + t;
-          if (w == 0) cp_async4(v, a.b + (size_t)t * p + J);
-          else if (w == 1) { if (a.vbv) cp_async4(v, a.vbv + (size_t)t * p + J); }
-          else cp_async4(v, a.xx + (a.xx_per_sys ? (size_t)t * p : 0) + J);
+          if (w == 0) cp_async4(v, a.s.b + (size_t)t * p + J);
+          else if (w == 1) { if (a.s.vbv) cp_async4(v, a.s.vbv + (size_t)t * p + J); }
+          else cp_async4(v, a.s.xx + (a.s.xx_per_sys ? (size_t)t * p : 0) + J);
         }
       }
     }
@@ -307,8 +307,8 @@ __global__ void __launch_bounds__(kTB, 1) grid_block_kernel(GridArgs a) {
     for (int q = tid - 32; q < nb * ns; q += kTB - 32) {
       if (q < 0) break;
       const int j = q / ns, t = q - j * ns;
-      s.dr[((blk & 1) * kGB + j) * 32 + t] = marker_draws(MODEL, (uint32_t)s.Js[blk % kJR][j], (uint32_t)s.sc[t].sweep, (uint32_t)(a.chain0 + t),
-                                                          s.sc[t].df, a.seed_lo, a.seed_hi);
+      s.dr[((blk & 1) * kGB + j) * 32 + t] = marker_draws(MODEL, (uint32_t)s.Js[blk % kJR][j], (uint32_t)s.sc[t].sweep, (uint32_t)(a.s.chain0 + t),
+                                                          s.sc[t].df, a.s.seed_lo, a.s.seed_hi);
     }
   };
   const unsigned long long t_start = globaltimer_ns();
@@ -366,7 +366,7 @@ __global__ void __launch_bounds__(kTB, 1) grid_block_kernel(GridArgs a) {
         float acc = 0.0f;
         for (int i = lane; i < rp; i += 32) acc = fmaf((float)xj[i], s.E[i], acc);
         const double v = (double)warp_sum(acc) * qinv;
-        if (lane == 0) grid_add(accw + j, v, a.err);
+        if (lane == 0) grid_add(accw + j, v, a.s.err);
       } else {
         for (int t0 = 0; t0 < ns; t0 += 4) {
           const int nt = min(4, ns - t0);
@@ -381,7 +381,7 @@ __global__ void __launch_bounds__(kTB, 1) grid_block_kernel(GridArgs a) {
           for (int q = 0; q < 4; q++) {
             if (q < nt) {
               const double v = (double)warp_sum(acc[q]) * qinv;
-              if (lane == 0) grid_add(accw + j * ns + t0 + q, v, a.err);
+              if (lane == 0) grid_add(accw + j * ns + t0 + q, v, a.s.err);
             }
           }
         }
@@ -405,8 +405,8 @@ __global__ void __launch_bounds__(kTB, 1) grid_block_kernel(GridArgs a) {
         }
         if (done) { s.tot[tid] = (float)((double)tot * (tid < ndot ? inv_q : inv_qG)); break; }
         if ((++spins & 0x3ffu) == 0) {
-          if (*reinterpret_cast<volatile int*>(a.err) != 0) { s_abort = 1; break; }
-          if (globaltimer_ns() - t_start > kGridTimeoutNs) { atomicExch(a.err, 3); s_abort = 1; break; }
+          if (*reinterpret_cast<volatile int*>(a.s.err) != 0) { s_abort = 1; break; }
+          if (globaltimer_ns() - t_start > kGridTimeoutNs) { atomicExch(a.s.err, 3); s_abort = 1; break; }
         }
       }
     }
@@ -429,13 +429,13 @@ __global__ void __launch_bounds__(kTB, 1) grid_block_kernel(GridArgs a) {
             if (model_is_gibbs(MODEL)) dr = s.dr[((blk & 1) * kGB + j) * 32 + lane];
             else { dr.z1 = dr.z2 = dr.u = 0.0f; dr.chi = 1.0f; }
             const float* v = vin + j * 100;
-            const RuleOut r = marker_rule<MODEL>(g, v[64 + lane], v[lane], a.vbv ? v[32 + lane] : 0.0f, sc, dr, 0.0f);
+            const RuleOut r = marker_rule<MODEL>(g, v[64 + lane], v[lane], a.s.vbv ? v[32 + lane] : 0.0f, sc, dr, 0.0f);
             de[j] = r.de;
             if (cta == 0) {
               const size_t q = (size_t)lane * p + Jcur[j];
-              a.b[q] = r.b;
-              if (model_has_d(MODEL) && a.d) a.d[q] = r.d;
-              if (model_rule_writes_vbj(MODEL) && a.vbv) a.vbv[q] = r.vbj;
+              a.s.b[q] = r.b;
+              if (model_has_d(MODEL) && a.s.d) a.s.d[q] = r.d;
+              if (model_rule_writes_vbj(MODEL) && a.s.vbv) a.s.vbv[q] = r.vbj;
             }
           }
           s.de[j * 32 + lane] = de[j];
@@ -462,19 +462,19 @@ __global__ void __launch_bounds__(kTB, 1) grid_block_kernel(GridArgs a) {
   __syncthreads();
   for (int q = tid; q < ns * rp; q += kTB) {
     const int t = q / rp, i = q - t * rp;
-    if (r0 + i < ld) a.e[(size_t)t * ld + r0 + i] = s.E[q];
+    if (r0 + i < ld) a.s.e[(size_t)t * ld + r0 + i] = s.E[q];
   }
 }
 
 template <int MODEL>
 cudaError_t launch_grid_model(const GridArgs& a, int grid, cudaStream_t st) {
-  const bool real = a.g.storage == 2;
-  size_t smem = grid_sweep_smem(a.nsys, a.rows_per_cta, a.mask != nullptr, real);
+  const bool real = a.s.g.storage == 2;
+  size_t smem = grid_sweep_smem(a.s.nsys, a.rows_per_cta, a.s.mask != nullptr, real);
   int threads = kT;
   const void* fn = real ? reinterpret_cast<const void*>(grid_sweep_kernel<MODEL, float>) : reinterpret_cast<const void*>(grid_sweep_kernel<MODEL, int8_t>);
   if (a.blocked) {
     if constexpr (MODEL != M_KMUP2) {
-      smem = grid_block_smem(a.nsys, a.rows_per_cta, real, model_is_gibbs(MODEL));
+      smem = grid_block_smem(a.s.nsys, a.rows_per_cta, real, model_is_gibbs(MODEL));
       fn = real ? reinterpret_cast<const void*>(grid_block_kernel<MODEL, float>) : reinterpret_cast<const void*>(grid_block_kernel<MODEL, int8_t>);
       threads = kTB;
     }
@@ -497,26 +497,14 @@ size_t grid_sweep_smem(int nsys, int rows_per_cta, bool masked, bool real_store)
   return grid_carve(nullptr, nsys, rows_per_cta, masked, real_store ? 4 : 1, nullptr) + 16;
 }
 
+// Every rule but MRR3's rotated systems, which run on the pipelined blocked sweep only.
 cudaError_t launch_grid_sweep(const GridArgs& a, int grid, cudaStream_t st) {
-  switch (rule_model(a.model)) {
-    case M_EMRR: return launch_grid_model<M_EMRR>(a, grid, st);
-    case M_EMBA: return launch_grid_model<M_EMBA>(a, grid, st);
-    case M_EMBB: return launch_grid_model<M_EMBB>(a, grid, st);
-    case M_EMBC: return launch_grid_model<M_EMBC>(a, grid, st);
-    case M_EMBL: return launch_grid_model<M_EMBL>(a, grid, st);
-    case M_EMEN: return launch_grid_model<M_EMEN>(a, grid, st);
-    case M_EMDE: return launch_grid_model<M_EMDE>(a, grid, st);
-    case M_LASSO: return launch_grid_model<M_LASSO>(a, grid, st);
-    case M_BL: return launch_grid_model<M_BL>(a, grid, st);
-    case M_BDPI: return launch_grid_model<M_BDPI>(a, grid, st);
-    case M_BRR: return launch_grid_model<M_BRR>(a, grid, st);
-    case M_BA: return launch_grid_model<M_BA>(a, grid, st);
-    case M_BB: return launch_grid_model<M_BB>(a, grid, st);
-    case M_BC: return launch_grid_model<M_BC>(a, grid, st);
-    case M_KMUP: return launch_grid_model<M_KMUP>(a, grid, st);
-    case M_KMUP2: return launch_grid_model<M_KMUP2>(a, grid, st);
-    default: return cudaErrorInvalidValue;
-  }
+  cudaError_t e = cudaErrorInvalidValue;
+  with_rule(a.model, [&](auto rule) {
+    constexpr int M = decltype(rule)::value;
+    if constexpr (M != M_MRR) e = launch_grid_model<M>(a, grid, st);
+  });
+  return e;
 }
 
 }  // namespace bwgr

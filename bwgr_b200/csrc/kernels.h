@@ -46,33 +46,34 @@ void launch_d_to_float(const double* src, float* dst, int n, cudaStream_t st);
 constexpr int kHatChunk = 16;  // systems per thread when k > 4
 void launch_gemv_hat(const GenoView& g, const float* b, int k, const float* mu, float* hat, float* work, int splits, cudaStream_t st);
 
-// ---- small-n path: one persistent CTA per system -------------------------------------------------
-struct SmallNArgs {
+// ---- the state of a fit's systems, as every sweep kernel and the epilogue read it ----------------
+// The order puts fields that are read together (b and d, vbv and xx, the seed words and chain0) in one 16-byte word of the
+// parameter bank, where one instruction loads them; the sweep kernels keep the registers they had with their own copies.
+struct SweepState {
   GenoView g;
-  int model;
   int nsys;
-  int sweep0, nsweeps;     // absolute sweep range of this launch
-  const int* perms;        // [nsweeps_total][p] marker order per sweep, or nullptr for natural order
-  int perm_stride_sweeps;  // perms row used = (sweep - perm_base)
-  int perm_base;
-  const float* y;          // [nsys][ld]  (centred later; raw y)
+  const uint8_t* mask;     // [nsys][ld] or nullptr
   float* e;                // [nsys][ld]  residuals (state, persists across launches)
   float* b;                // [nsys][p]
   float* d;                // [nsys][p] or nullptr
   float* vbv;              // [nsys][p] per-marker variance (or KMUP lambda) or nullptr
   const float* xx;         // [nxx][p]  (nxx = 1 shared or nsys when masked)
-  const float* xx2;        // KMUP2: the caller's xx(j) * bg [p] (the rule's denominator; xx carries H'H of the rows in use)
-  int xx_per_sys;
-  const uint8_t* mask;     // [nsys][ld] or nullptr
-  const float* row_w;      // KMUP2 on rows sampled with replacement: [ld] row multiplicities as floats (nsys = 1), or nullptr
+  const float* xx2;        // KMUP2: the caller's xx(j) * bg [p] (the rule's denominator; xx carries H'H of the rows in use), else nullptr
   SysScalars* sc;          // [nsys]
-  // Gibbs posterior sums
-  float* B; float* D; float* VBv;  // [nsys][p] or nullptr
+  int xx_per_sys;
   uint32_t seed_lo, seed_hi;
   int chain0;              // chain id offset for the RNG counter
   int* err;                // device error flag
 };
-void launch_small_n(const SmallNArgs& a, size_t smem_limit, cudaStream_t st);
+
+// ---- small-n path: one persistent CTA per system -------------------------------------------------
+struct SmallNArgs {
+  SweepState s;
+  int model;               // the rule (rule_model)
+  const int* perms;        // [p] marker order of this sweep, or nullptr for natural order
+  const float* row_w;      // KMUP2 on rows sampled with replacement: [ld] row multiplicities as floats (nsys = 1), or nullptr
+};
+cudaError_t launch_small_n(const SmallNArgs& a, size_t smem_limit, cudaStream_t st);
 bool small_n_fits(const GenoView& g, bool masked, size_t smem_limit, bool weighted = false);
 
 // ---- blocked path ---------------------------------------------------------------------------------
@@ -99,22 +100,17 @@ double column_min(const double* src, int64_t n);
 
 // Pipelined blocked sweep (sweep_pipe.cu): nworkers streaming CTAs + one solver CTA, look-ahead D (0 or 1).
 struct PipeArgs {
-  GenoView g;
-  int model;
-  int nsys;
+  SweepState s;          // unmasked systems: xx is one [p] for all
+  int model;             // the rule (rule_model)
   const int* perm;       // this sweep's marker order [p] (device)
   int nblocks;
   const float* gram;     // [nblocks][128][nband*128] Gram band as float (exact below 2^24)
   int nband;
   const float* tinv;     // [nblocks][128][128] (I + A L)^-1 of every block (block_inv.cu), given exactly when the sweep
                          // has one linear system on uncentred columns; else nullptr
-  float* e;              // [nsys][ld]
-  float* b; float* d; float* vbv;  // [nsys][p]
-  const float* xx;       // [p]
   const float* sx;       // [p] column sums, or nullptr.  Non-null = the columns are centred (MRR3): the Gram band is the
                          // centred one and g gets the running mean-shift term c * sx_j (the workers stay uncentred)
   float* cshift;         // [nsys] out: the mean shift c accumulated over the sweep (e_true = e_stored + c)
-  SysScalars* sc;        // [nsys]
   unsigned long long* part;  // [8][nsys][128][160] per-worker integer partials of h: (value << 12) | block tag; zeroed before launch
   unsigned long long* hred;  // [8][nsys][128] reduced h, same word format; zeroed before launch
   // row-sharded fit over `world` GPUs of a node: hx[r] = rank r's exchange ring [8][world][nsys][128] mapped into this
@@ -123,20 +119,17 @@ struct PipeArgs {
   unsigned long long* hx[8];
   unsigned long long gen0;
   unsigned long long* dew;  // [nblocks][nsys][136] published steps: (int32 q << 32) | tag, word 128 = (float scale << 32) | tag
-  uint32_t tag;          // unique per launch, never 0
-  uint32_t seed_lo, seed_hi;
-  int chain0;
   int rows_per_cta;      // multiple of 16, <= 512
   int nworkers;
   int D;                 // look-ahead depth
   int nbuf;              // X tiles in the ring of a worker (>= D + 1)
   int sring;             // blocks of solve inputs in flight in the solver CTA (2 or 3)
-  int* err;
-  long long* trace;      // optional [nblocks][16] clock64 stamps (BWGR_TRACE), else nullptr
+  uint32_t tag;          // unique per launch, never 0
   // clustered topology: nclusters thread-block clusters of 8 CTAs = one solver + seven workers each (nworkers = 7 * nclusters);
   // cx = [8][nclusters][nsys][128] per-cluster sums of h, same word format as hred; zeroed before launch
-  int cl, nclusters;
   unsigned long long* cx;
+  long long* trace;      // optional [nblocks][16] clock64 stamps (BWGR_TRACE), else nullptr
+  int cl, nclusters;
   // optional: cluster 0 stores started_val here once the first grid sum has gone round, i.e. when every CTA of the launch is
   // resident -- a side stream waits on it (cuStreamWaitValue32) before it fills the SMs this launch leaves idle
   unsigned int* started;
@@ -153,16 +146,11 @@ void launch_block_inverse(int model, const int* perm, int p, int nblocks, const 
 // Sweep epilogue (both paths use the same arithmetic): reductions + hyper-parameter update +
 // e -= mean(e). One CTA per system.
 struct EpilogueArgs {
-  int model, nsys, n, p;
-  int64_t ld;
-  float* e; const float* y; float* b; const float* d; float* vbv; const float* b_prev;  // b_prev: convergence (model_has_cnv)
-  const float* xx; int xx_per_sys;  // emDE: the per-marker penalty update needs xx_j
+  SweepState s;                     // xx: emDE's per-marker penalty update needs xx_j
+  int model;                        // the full model
+  const float* y; const float* b_prev;  // b_prev: convergence (model_has_cnv)
   const float* wts;                 // emML with marker weights: d_j (one system)
-  const uint8_t* mask;
-  SysScalars* sc;
   float* B; float* D; float* VBv;
-  uint32_t seed_lo, seed_hi;
-  int chain0;
   // row-sharded fit: all-reduced sums over individuals [nsys][4] {sum e, sum e^2, sum e.y, sum y} and max|e| [nsys]; else nullptr
   const double* esum; const float* emaxv;
 };
@@ -206,25 +194,14 @@ void launch_pair_reduce(const float* A, const float* B, int64_t lda, int64_t ldb
 // (4, 8 and 16 measured alike with grid_block_kernel)
 constexpr int kGridCopies = 8;
 struct GridArgs {
-  GenoView g;
-  int model;
-  int nsys;               // <= 32
-  const int* perm;        // marker order of this sweep [p], or nullptr = natural order
-  float* e;               // [nsys][ld]
-  float* b; float* d; float* vbv;  // [nsys][p]
-  const float* xx;        // [nxx][p]
-  int xx_per_sys;
-  const float* xx2;       // KMUP2 only
-  const uint8_t* mask;    // [nsys][ld] or nullptr
-  SysScalars* sc;         // [nsys]
+  SweepState s;           // nsys <= 32; a mask byte may be a row multiplicity (KMUP2 on rows drawn with replacement)
+  int model;              // the full model
   unsigned long long* acc;  // [p][kGridCopies][32]: (fixed-point sum << 8) + arrivals; zeroed before launch
   float g_quantum;        // value of one fixed-point unit of g
   float gram_quantum;     // blocked variant: value of one fixed-point unit of a cross product x_j'x_i (<= 1 for the int8 store: exact)
+  const int* perm;        // marker order of this sweep [p], or nullptr = natural order
   int blocked;            // blocked variant (unmasked systems): acc is [nblocks][kGridCopies][grid_block_words(nsys)]
-  uint32_t seed_lo, seed_hi;
-  int chain0;
   int rows_per_cta;       // multiple of 16; grid * rows_per_cta >= ld
-  int* err;
 };
 size_t grid_block_smem(int nsys, int rows_per_cta, bool real_store, bool gibbs);
 size_t grid_block_acc_words(int nsys, int p);

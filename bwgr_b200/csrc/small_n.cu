@@ -13,27 +13,15 @@ namespace bwgr {
 
 namespace {
 
-
-// Expand 4 packed 2-bit bytes (16 rows) into 16 int8 bytes.
-__device__ __forceinline__ uint4 expand_2bit(uint32_t pk) {
-  uint32_t w[4];
-#pragma unroll
-  for (int q = 0; q < 4; q++) {
-    const uint32_t byte = (pk >> (8 * q)) & 0xFFu;
-    w[q] = (byte & 3u) | (((byte >> 2) & 3u) << 8) | (((byte >> 4) & 3u) << 16) | (((byte >> 6) & 3u) << 24);
-  }
-  return make_uint4(w[0], w[1], w[2], w[3]);
-}
-
 // kRing = genotype columns in flight per CTA (8, 4 or 2 depending on how much shared memory e leaves).
 template <int MODEL, int kRing>
 __global__ void __launch_bounds__(1024, 1) small_n_sweep_kernel(SmallNArgs a) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   const int sys = blockIdx.x;
   const int tid = threadIdx.x, T = blockDim.x, lane = tid & 31, warp = tid >> 5, nwarps = T >> 5;
-  const int ld = (int)a.g.ld, p = a.g.p;
+  const int ld = (int)a.s.g.ld, p = a.s.g.p;
   const int nchunks = ld >> 4;
-  const bool two_bit = a.g.storage != 0;
+  const bool two_bit = a.s.g.storage != 0;
   const int col_bytes = two_bit ? (ld >> 2) : ld;  // bytes of one column slot in the ring
 
   // e in shared memory, quarter-chunk major: rows 16c + 4q .. 16c + 4q + 3 of chunk c sit at float4 index q * nchunks + c, so that the
@@ -44,7 +32,7 @@ __global__ void __launch_bounds__(1024, 1) small_n_sweep_kernel(SmallNArgs a) {
   auto e_idx = [&](int i) { return ((((i >> 2) & 3) * nchunks + (i >> 4)) << 2) + (i & 3); };
   unsigned char* ring = smem_raw + (size_t)ld * 4;                          // [kRing][col_bytes]
   unsigned char* mask_s = ring + (size_t)kRing * col_bytes;                 // [ld] (only if mask)
-  float* red = reinterpret_cast<float*>(mask_s + (a.mask ? ld : 0));        // [2][32]
+  float* red = reinterpret_cast<float*>(mask_s + (a.s.mask ? ld : 0));        // [2][32]
   MarkerDraws* draws = reinterpret_cast<MarkerDraws*>(red + 64);            // [2][T] (Gibbs)
   int* ord_s = reinterpret_cast<int*>(draws + (model_is_gibbs(MODEL) ? 2 * T : 0));  // [2][T]: the marker order, two chunks of T positions
   // KMUP2 on rows drawn with replacement (R/wgr.R:68, rp = TRUE): H'e0 counts a row as often as it was drawn (:57-60), the residual
@@ -54,24 +42,24 @@ __global__ void __launch_bounds__(1024, 1) small_n_sweep_kernel(SmallNArgs a) {
     if (a.row_w) w_s = reinterpret_cast<const float*>((reinterpret_cast<uintptr_t>(ord_s + 2 * T) + 15) & ~(uintptr_t)15);
   __shared__ SysScalars sc;
 
-  if (tid == 0) sc = a.sc[sys];
+  if (tid == 0) sc = a.s.sc[sys];
   __syncthreads();
   if (sc.done) return;
 
-  float* e_g = a.e + (size_t)sys * ld;
+  float* e_g = a.s.e + (size_t)sys * ld;
   for (int i = tid; i < ld; i += T) e_s[e_idx(i)] = e_g[i];
-  if (a.mask)
-    for (int i = tid; i < ld; i += T) mask_s[i] = a.mask[(size_t)sys * ld + i];
+  if (a.s.mask)
+    for (int i = tid; i < ld; i += T) mask_s[i] = a.s.mask[(size_t)sys * ld + i];
   if (w_s)
     for (int i = tid; i < ld; i += T) const_cast<float*>(w_s)[e_idx(i)] = a.row_w[i];
 
-  float* b = a.b + (size_t)sys * p;
-  float* dvec = a.d ? a.d + (size_t)sys * p : nullptr;
-  float* vbv = a.vbv ? a.vbv + (size_t)sys * p : nullptr;
-  const float* xx = a.xx + (a.xx_per_sys ? (size_t)sys * p : 0);
+  float* b = a.s.b + (size_t)sys * p;
+  float* dvec = a.s.d ? a.s.d + (size_t)sys * p : nullptr;
+  float* vbv = a.s.vbv ? a.s.vbv + (size_t)sys * p : nullptr;
+  const float* xx = a.s.xx + (a.s.xx_per_sys ? (size_t)sys * p : 0);
   const int* order = a.perms;  // nullptr = natural order
   const int sweep = sc.sweep;
-  const uint32_t chain = (uint32_t)(a.chain0 + sys);
+  const uint32_t chain = (uint32_t)(a.s.chain0 + sys);
 
   // the order is read through shared memory: straight from global memory the index load sat in front of every column address and
   // every per-marker input (a dependent L2 round trip per marker in every thread)
@@ -91,10 +79,10 @@ __global__ void __launch_bounds__(1024, 1) small_n_sweep_kernel(SmallNArgs a) {
     if (pos < p) {
       unsigned char* slot = ring + (size_t)(pos % kRing) * col_bytes;
       if (!two_bit) {
-        const int8_t* src = a.g.x8 + (int64_t)j * a.g.ld;
+        const int8_t* src = a.s.g.x8 + (int64_t)j * a.s.g.ld;
         for (int c = tid; c < nchunks; c += T) cp_async16(slot + 16 * c, src + 16 * c);
       } else {
-        const uint8_t* src = a.g.x2 + (int64_t)j * a.g.ldb;
+        const uint8_t* src = a.s.g.x2 + (int64_t)j * a.s.g.ldb;
         for (int c = tid; c < nchunks; c += T) cp_async4(slot + 4 * c, src + 4 * c);
       }
     }
@@ -110,7 +98,7 @@ __global__ void __launch_bounds__(1024, 1) small_n_sweep_kernel(SmallNArgs a) {
   float bA = b[jA], xA = xx[jA], vA = vbv ? vbv[jA] : 0.0f;
   float bB = b[jB], xB = xx[jB], vB = vbv ? vbv[jB] : 0.0f;
   float hA = 0.0f, hB = 0.0f;  // KMUP2: the second per-marker scale
-  if constexpr (MODEL == M_KMUP2) { hA = a.xx2[jA]; hB = a.xx2[jB]; }
+  if constexpr (MODEL == M_KMUP2) { hA = a.s.xx2[jA]; hB = a.s.xx2[jB]; }
 
 #pragma unroll 1
   for (int pos = 0; pos < p; pos++) {
@@ -124,12 +112,12 @@ __global__ void __launch_bounds__(1024, 1) small_n_sweep_kernel(SmallNArgs a) {
     if (pos + 2 < p) {
       jB = marker_ahead(pos, 2);
       bB = b[jB]; xB = xx[jB]; vB = vbv ? vbv[jB] : 0.0f;
-      if constexpr (MODEL == M_KMUP2) hB = a.xx2[jB];
+      if constexpr (MODEL == M_KMUP2) hB = a.s.xx2[jB];
     }
     if (model_is_gibbs(MODEL) && pm == 0) {  // draws of the next T markers, one per thread
       const int q = pos + tid;
       if (q < p)
-        draws[pb * T + tid] = marker_draws(MODEL, (uint32_t)marker_ahead(pos, tid), (uint32_t)sweep, chain, sc.df, a.seed_lo, a.seed_hi);
+        draws[pb * T + tid] = marker_draws(MODEL, (uint32_t)marker_ahead(pos, tid), (uint32_t)sweep, chain, sc.df, a.s.seed_lo, a.s.seed_hi);
     }
     issue_col(pos + kRing - 1, pos + kRing - 1 < p ? marker_ahead(pos, kRing - 1) : 0);
     cp_async_wait<kRing - 1>();
@@ -145,7 +133,7 @@ __global__ void __launch_bounds__(1024, 1) small_n_sweep_kernel(SmallNArgs a) {
         const int c = tid;
         uint4 w = two_bit ? expand_2bit(*reinterpret_cast<const uint32_t*>(slot + 4 * c))
                           : *reinterpret_cast<const uint4*>(slot + 16 * c);
-        if (a.mask) {
+        if (a.s.mask) {
           const uint4 m = *reinterpret_cast<const uint4*>(mask_s + 16 * c);
           w.x &= m.x * 0xFFu; w.y &= m.y * 0xFFu; w.z &= m.z * 0xFFu; w.w &= m.w * 0xFFu;
         }
@@ -167,7 +155,7 @@ __global__ void __launch_bounds__(1024, 1) small_n_sweep_kernel(SmallNArgs a) {
     for (int c = tid; c < nchunks; c += T) {
       uint4 w = two_bit ? expand_2bit(*reinterpret_cast<const uint32_t*>(slot + 4 * c))
                         : *reinterpret_cast<const uint4*>(slot + 16 * c);
-      if (a.mask) {
+      if (a.s.mask) {
         const uint4 m = *reinterpret_cast<const uint4*>(mask_s + 16 * c);
         w.x &= m.x * 0xFFu; w.y &= m.y * 0xFFu; w.z &= m.z * 0xFFu; w.w &= m.w * 0xFFu;
       }
@@ -217,7 +205,7 @@ __global__ void __launch_bounds__(1024, 1) small_n_sweep_kernel(SmallNArgs a) {
       for (int c = tid; c < nchunks; c += T) {
         uint4 w = two_bit ? expand_2bit(*reinterpret_cast<const uint32_t*>(slot + 4 * c))
                           : *reinterpret_cast<const uint4*>(slot + 16 * c);
-        if (a.mask) {
+        if (a.s.mask) {
           const uint4 m = *reinterpret_cast<const uint4*>(mask_s + 16 * c);
           w.x &= m.x * 0xFFu; w.y &= m.y * 0xFFu; w.z &= m.z * 0xFFu; w.w &= m.w * 0xFFu;
         }
@@ -244,23 +232,23 @@ __global__ void __launch_bounds__(1024, 1) small_n_sweep_kernel(SmallNArgs a) {
 }  // namespace
 
 static size_t small_n_smem(const SmallNArgs& a, int ring, int T) {
-  const size_t ld = (size_t)a.g.ld;
-  const size_t col_bytes = a.g.storage ? (ld >> 2) : ld;
-  return ld * 4 + (size_t)ring * col_bytes + (a.mask ? ld : 0) + 64 * 4 +
+  const size_t ld = (size_t)a.s.g.ld;
+  const size_t col_bytes = a.s.g.storage ? (ld >> 2) : ld;
+  return ld * 4 + (size_t)ring * col_bytes + (a.s.mask ? ld : 0) + 64 * 4 +
          (model_is_gibbs(a.model) ? 2 * (size_t)T * sizeof(MarkerDraws) : 0) + 2 * (size_t)T * sizeof(int) + 16 + (a.row_w ? ld * 4 + 16 : 0);
 }
 
 // Largest n this path takes: e (4 B/row) + two ring slots must fit the 227 KB of one SM.
 bool small_n_fits(const GenoView& g, bool masked, size_t smem_limit, bool weighted) {
   SmallNArgs a;
-  a.g = g; a.mask = masked ? reinterpret_cast<const uint8_t*>(1) : nullptr; a.model = M_BB;
+  a.s.g = g; a.s.mask = masked ? reinterpret_cast<const uint8_t*>(1) : nullptr; a.model = M_BB;
   a.row_w = weighted ? reinterpret_cast<const float*>(1) : nullptr;
   return small_n_smem(a, 2, 1024) <= smem_limit;
 }
 
 template <int MODEL>
-static void launch_small_model(const SmallNArgs& a, size_t smem_limit, cudaStream_t st) {
-  const int nchunks = (int)(a.g.ld >> 4);
+static cudaError_t launch_small_model(const SmallNArgs& a, size_t smem_limit, cudaStream_t st) {
+  const int nchunks = (int)(a.s.g.ld >> 4);
   int T = ((nchunks + 31) / 32) * 32;
   if (T > 1024) T = 1024;
   if (T < 32) T = 32;
@@ -268,38 +256,28 @@ static void launch_small_model(const SmallNArgs& a, size_t smem_limit, cudaStrea
   {                                                                                                               \
     const size_t smem = small_n_smem(a, RING, T);                                                                 \
     if (smem <= smem_limit) {                                                                                     \
-      cudaFuncSetAttribute(small_n_sweep_kernel<MODEL, RING>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem); \
-      small_n_sweep_kernel<MODEL, RING><<<a.nsys, T, smem, st>>>(a);                                              \
-      return;                                                                                                     \
+      const cudaError_t e =                                                                                       \
+          cudaFuncSetAttribute(small_n_sweep_kernel<MODEL, RING>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem); \
+      if (e != cudaSuccess) return e;                                                                             \
+      small_n_sweep_kernel<MODEL, RING><<<a.s.nsys, T, smem, st>>>(a);                                            \
+      return cudaSuccess;                                                                                         \
     }                                                                                                             \
   }
   BWGR_TRY_RING(8)
   BWGR_TRY_RING(4)
   BWGR_TRY_RING(2)
 #undef BWGR_TRY_RING
+  return cudaErrorInvalidValue;
 }
 
-void launch_small_n(const SmallNArgs& a, size_t smem_limit, cudaStream_t st) {
-  switch (rule_model(a.model)) {
-    case M_EMRR: launch_small_model<M_EMRR>(a, smem_limit, st); break;
-    case M_EMBA: launch_small_model<M_EMBA>(a, smem_limit, st); break;
-    case M_EMBB: launch_small_model<M_EMBB>(a, smem_limit, st); break;
-    case M_EMBC: launch_small_model<M_EMBC>(a, smem_limit, st); break;
-    case M_EMBL: launch_small_model<M_EMBL>(a, smem_limit, st); break;
-    case M_EMEN: launch_small_model<M_EMEN>(a, smem_limit, st); break;
-    case M_EMDE: launch_small_model<M_EMDE>(a, smem_limit, st); break;
-    case M_LASSO: launch_small_model<M_LASSO>(a, smem_limit, st); break;
-    case M_BL: launch_small_model<M_BL>(a, smem_limit, st); break;
-    case M_BDPI: launch_small_model<M_BDPI>(a, smem_limit, st); break;
-    case M_BRR: launch_small_model<M_BRR>(a, smem_limit, st); break;
-    case M_BA: launch_small_model<M_BA>(a, smem_limit, st); break;
-    case M_BB: launch_small_model<M_BB>(a, smem_limit, st); break;
-    case M_BC: launch_small_model<M_BC>(a, smem_limit, st); break;
-    case M_KMUP: launch_small_model<M_KMUP>(a, smem_limit, st); break;
-    case M_KMUP2: launch_small_model<M_KMUP2>(a, smem_limit, st); break;
-    case M_MRR: launch_small_model<M_MRR>(a, smem_limit, st); break;
-    default: break;
-  }
+// Every rule but MRR3's rotated systems, which run on the pipelined blocked sweep only.
+cudaError_t launch_small_n(const SmallNArgs& a, size_t smem_limit, cudaStream_t st) {
+  cudaError_t e = cudaErrorInvalidValue;
+  with_rule(a.model, [&](auto rule) {
+    constexpr int M = decltype(rule)::value;
+    if constexpr (M != M_MRR) e = launch_small_model<M>(a, smem_limit, st);
+  });
+  return e;
 }
 
 }  // namespace bwgr

@@ -200,7 +200,7 @@ __global__ void __launch_bounds__(kT, 1) sweep_pipe_kernel(PipeArgs a) {
   __shared__ Sync S;
   __shared__ SysScalars sc[32];
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  const int ns = a.nsys, p = a.g.p, W = a.nworkers, D = a.D, nblocks = a.nblocks;
+  const int ns = a.s.nsys, p = a.s.g.p, W = a.nworkers, D = a.D, nblocks = a.nblocks;
   unsigned char* base = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
   // clustered topology (CL): rank 0 of every cluster is a solver (all solvers run the identical solve on the identical integer
   // sums, like the ranks of a row-sharded fit), ranks 1..7 are its workers; worker index = cluster * 7 + rank - 1
@@ -210,7 +210,7 @@ __global__ void __launch_bounds__(kT, 1) sweep_pipe_kernel(PipeArgs a) {
   const bool writer = !CL || cluster == 0;  // the solver that writes b / d / vb back to HBM
   bool dead = false;
 
-  if (tid < ns) sc[tid] = a.sc[tid];
+  if (tid < ns) sc[tid] = a.s.sc[tid];
   if (tid == 0) {
     for (int i = 0; i < 8; i++) { mbar_init(&S.tile_full[i], 128); mbar_init(&S.tile_empty[i], 1); }
     for (int i = 0; i < 4; i++) { mbar_init(&S.u_done_at[i], 1); mbar_init(&S.el_full_at[i], 128); }
@@ -258,7 +258,7 @@ __global__ void __launch_bounds__(kT, 1) sweep_pipe_kernel(PipeArgs a) {
     for (int s = 0; s < ns; s++)
       for (int i = tid; i < RS; i += kT) {
         const int r = row0 + i;
-        const float e = (i < R && r < a.g.ld) ? a.e[(size_t)s * a.g.ld + r] : 0.0f;
+        const float e = (i < R && r < a.s.g.ld) ? a.s.e[(size_t)s * a.s.g.ld + r] : 0.0f;
         Es[s * RS + i] = e;
         if (i < R) {
           const float sv = e * sc[s].e_qinv;
@@ -292,10 +292,10 @@ __global__ void __launch_bounds__(kT, 1) sweep_pipe_kernel(PipeArgs a) {
       // number of those barriers, < 0 = the limbs written at start-up).  The two tensor-core passes and the epilogue overlap by halves.
       auto issue_g = [&](int c, int use) {
         const unsigned char* Xt = Xs + (size_t)(c % nbuf) * NA * kAtomBytes;
-        mbar_wait(&S.tile_full[c % nbuf], (uint32_t)(c / nbuf) & 1u, dead, a.err);
-        if (c > 0) mbar_wait(&S.g_empty, (uint32_t)(c - 1) & 1u, dead, a.err);
+        mbar_wait(&S.tile_full[c % nbuf], (uint32_t)(c / nbuf) & 1u, dead, a.s.err);
+        if (c > 0) mbar_wait(&S.g_empty, (uint32_t)(c - 1) & 1u, dead, a.s.err);
         for (int g = 0; g * kAtomsPerGroup < NA; g++) {
-          if (use >= 0) mbar_wait(&S.el_full_at[g], (uint32_t)use & 1u, dead, a.err);
+          if (use >= 0) mbar_wait(&S.el_full_at[g], (uint32_t)use & 1u, dead, a.s.err);
           tc_fence_after();
           if (elect_one()) {
             for (int at = g * kAtomsPerGroup; at < NA && at < (g + 1) * kAtomsPerGroup; at++) {
@@ -313,7 +313,7 @@ __global__ void __launch_bounds__(kT, 1) sweep_pipe_kernel(PipeArgs a) {
       for (int c = 0; c <= npro; c++) issue_g(c, -1);
       for (int b = 0; b < nblocks; b++) {
         const unsigned char* Xt = Xs + (size_t)(b % nbuf) * NA * kAtomBytes;
-        mbar_wait(&S.dl_full[b & 1], (uint32_t)(b >> 1) & 1u, dead, a.err);
+        mbar_wait(&S.dl_full[b & 1], (uint32_t)(b >> 1) & 1u, dead, a.s.err);
         tc_fence_after();
         if (tracing && lane == 0) WSTAMP(b, 8);
         if (elect_one()) {
@@ -342,7 +342,7 @@ __global__ void __launch_bounds__(kT, 1) sweep_pipe_kernel(PipeArgs a) {
       const uint32_t tlane = (uint32_t)(quarter * 32) << 16;
       const bool t0 = tracing && q == 0;
       auto g_epilogue = [&](int c) {
-        mbar_wait(&S.g_done, (uint32_t)c & 1u, dead, a.err);
+        mbar_wait(&S.g_done, (uint32_t)c & 1u, dead, a.s.err);
         if (t0) WSTAMP(c, 6);
         tc_fence_after();
         // partial of marker q, system s -> part[c % ring][s][this worker][q] (full 32-byte sectors): (value << 12) | block tag
@@ -372,7 +372,7 @@ __global__ void __launch_bounds__(kT, 1) sweep_pipe_kernel(PipeArgs a) {
           unsigned char* dl = DL + (size_t)(b & 1) * (N / 8) * 1024;
           // epilogue warp e receives the systems s = e, e+4, ...: lane l polls step words l, l+32, l+64, l+96 and lane 0 the
           // scale word as well (one L2 round trip when the step is already there), then writes the limbs of those markers
-          if (CL) mbar_wait(&S.de_in[b & 1], (uint32_t)(b >> 1) & 1u, dead, a.err);
+          if (CL) mbar_wait(&S.de_in[b & 1], (uint32_t)(b >> 1) & 1u, dead, a.s.err);
           for (int s = quarter; s < ns; s += 4) {
             const unsigned long long* ws = wv + (size_t)s * kDewStride;
             unsigned long long v[4] = {0, 0, 0, 0}, vq = 0;
@@ -389,7 +389,7 @@ __global__ void __launch_bounds__(kT, 1) sweep_pipe_kernel(PipeArgs a) {
               for (int t = 0; t < 4; t++) { v[t] = ld_relaxed_u64(ws + 32 * t + lane); ok = ok && ((uint32_t)v[t] == a.tag); }
               if (lane == 0) { vq = ld_relaxed_u64(ws + 128); ok = ok && ((uint32_t)vq == a.tag); }
               if (__all_sync(0xffffffffu, ok)) break;
-              if (++spin > kSpin || ((spin & 255u) == 255u && *reinterpret_cast<volatile int*>(a.err) != 0)) { dead = true; atomicCAS(a.err, 0, 3); }
+              if (++spin > kSpin || ((spin & 255u) == 255u && *reinterpret_cast<volatile int*>(a.s.err) != 0)) { dead = true; atomicCAS(a.s.err, 0, 3); }
             }
             if (lane == 0) dqs[(b & 1) * 32 + s] = __uint_as_float((uint32_t)(vq >> 32));
 #pragma unroll
@@ -412,7 +412,7 @@ __global__ void __launch_bounds__(kT, 1) sweep_pipe_kernel(PipeArgs a) {
         // ---- E_slab -= X_b dE_b, then the limbs of the new residual (B operand of the next G pass)
         // group by group (two row atoms each), as the issuer commits them
         for (int g = 0; g * kAtomsPerGroup < NA; g++) {
-          mbar_wait(&S.u_done_at[g], (uint32_t)b & 1u, dead, a.err);
+          mbar_wait(&S.u_done_at[g], (uint32_t)b & 1u, dead, a.s.err);
           if (t0 && g == 0) WSTAMP(b, 3);
           tc_fence_after();
           const int at0 = g * kAtomsPerGroup;
@@ -455,7 +455,7 @@ __global__ void __launch_bounds__(kT, 1) sweep_pipe_kernel(PipeArgs a) {
       for (int s = 0; s < ns; s++)
         for (int i = q; i < R; i += 128) {
           const int r = row0 + i;
-          if (r < a.g.ld) a.e[(size_t)s * a.g.ld + r] = Es[s * RS + i];
+          if (r < a.s.g.ld) a.s.e[(size_t)s * a.s.g.ld + r] = Es[s * RS + i];
         }
     } else if ((warp >= 5 && warp <= 8) || (warp >= 10 && warp <= 13)) {
       // ------------------------------------------------------------------ X tile gather
@@ -466,15 +466,15 @@ __global__ void __launch_bounds__(kT, 1) sweep_pipe_kernel(PipeArgs a) {
       const int grp = warp >= 10 ? 1 : 0, ngrp = nbuf >= 2 ? 2 : 1;
       const int lw = warp - (grp ? 10 : 5);
       const int nchunk = R >> 4;
-      const bool act = lane < nchunk && row0 + 16 * lane < a.g.ld;
+      const bool act = lane < nchunk && row0 + 16 * lane < a.s.g.ld;
       const uint32_t choff = (uint32_t)((lane >> 3) * kAtomBytes + ((lane & 7) << 4));
-      const int8_t* xrow = a.g.x8 + row0 + 16 * lane;
+      const int8_t* xrow = a.s.g.x8 + row0 + 16 * lane;
       const uint64_t pol = policy_evict_first();
       for (int t = grp; t < nblocks && grp < ngrp; t += ngrp) {
         const int buf = t % nbuf;
         const int pos = t * 128 + lw + 4 * lane;
         const int myid = pos < p ? a.perm[pos] : -1;
-        if (t >= nbuf) mbar_wait(&S.tile_empty[buf], (uint32_t)(t / nbuf - 1) & 1u, dead, a.err);
+        if (t >= nbuf) mbar_wait(&S.tile_empty[buf], (uint32_t)(t / nbuf - 1) & 1u, dead, a.s.err);
         const uint32_t dst = smem_u32(Xs + (size_t)buf * NA * kAtomBytes);
 #pragma unroll 8
         for (int i = 0; i < 32; i++) {
@@ -483,7 +483,7 @@ __global__ void __launch_bounds__(kT, 1) sweep_pipe_kernel(PipeArgs a) {
           if (lane < nchunk) {
             const uint32_t dm = dst + (uint32_t)(m * 128) + (choff ^ (uint32_t)((m & 7) << 4));
             const bool ok = act && j >= 0;
-            cp_async16_stream(dm, ok ? xrow + (int64_t)j * a.g.ld : a.g.x8, ok ? 16u : 0u, pol);
+            cp_async16_stream(dm, ok ? xrow + (int64_t)j * a.s.g.ld : a.s.g.x8, ok ? 16u : 0u, pol);
           }
         }
         cp_async_commit();
@@ -520,7 +520,7 @@ __global__ void __launch_bounds__(kT, 1) sweep_pipe_kernel(PipeArgs a) {
               }
             }
             if (__all_sync(0xffffffffu, ok)) break;
-            if (++spin > kSpin || ((spin & 255u) == 255u && *reinterpret_cast<volatile int*>(a.err) != 0)) { dead = true; atomicCAS(a.err, 0, 3); sum = 0; }
+            if (++spin > kSpin || ((spin & 255u) == 255u && *reinterpret_cast<volatile int*>(a.s.err) != 0)) { dead = true; atomicCAS(a.s.err, 0, 3); sum = 0; }
           }
           if (tracing && lane == 0 && task == (int)blockIdx.x) WSTAMP(c, 14);
 #pragma unroll
@@ -536,7 +536,7 @@ __global__ void __launch_bounds__(kT, 1) sweep_pipe_kernel(PipeArgs a) {
         }
       }
     }
-    if (bad) atomicExch(a.err, 4);
+    if (bad) atomicExch(a.s.err, 4);
     tc_fence_before();
     __syncthreads();
     if (warp == 0) tmem_dealloc(tmem_base, tmem_cols);
@@ -580,7 +580,7 @@ __global__ void __launch_bounds__(kT, 1) sweep_pipe_kernel(PipeArgs a) {
   // a worker's step inbox sits at the same shared-window offset in every CTA of this launch
   const uint32_t dein_u32 = smem_u32(base) + (uint32_t)worker_layout(a.rows_per_cta, ns, a.nbuf, CL).di;
   const bool centred = a.sx != nullptr;
-  const float inv_n = 1.0f / (float)a.g.n;
+  const float inv_n = 1.0f / (float)a.s.g.n;
   if (tid < 64) cs[tid] = 0.0f;
   const int gstride = a.nband * 128;  // floats per Gram row in HBM
   const int nsw = ns < kSolveWarps ? ns : kSolveWarps;
@@ -595,7 +595,7 @@ __global__ void __launch_bounds__(kT, 1) sweep_pipe_kernel(PipeArgs a) {
       // invert the four 32x32 diagonal blocks of I + A L (E-independent), one block of markers ahead of the solve
       for (int nb = 0; nb < nblocks; nb++) {
         const int slot = nb % sring;
-        mbar_wait(&S.raw_ready[slot], (uint32_t)(nb / sring) & 1u, dead, a.err);
+        mbar_wait(&S.raw_ready[slot], (uint32_t)(nb / sring) & 1u, dead, a.s.err);
         const float* Gb = Gs + (size_t)slot * 10 * kTileF;
         for (int task = warp - kInvWarp0; task < ns * 4; task += 4) {
           const int s = task >> 2, d = task & 3;
@@ -638,7 +638,7 @@ __global__ void __launch_bounds__(kT, 1) sweep_pipe_kernel(PipeArgs a) {
       const int C = a.nclusters;
       for (int b = 0; b < nblocks; b++) {
         const int slot = b & 1;
-        mbar_wait(&S.h_in[slot], (uint32_t)(b >> 1) & 1u, dead, a.err);
+        mbar_wait(&S.h_in[slot], (uint32_t)(b >> 1) & 1u, dead, a.s.err);
         const unsigned long long tagb = tag_of((unsigned long long)(b / kRing));
         unsigned long long* ring = a.cx + (size_t)(b % kRing) * C * ns * 128;
         for (int pair = ct; pair < ns * 128; pair += 128) {
@@ -660,7 +660,7 @@ __global__ void __launch_bounds__(kT, 1) sweep_pipe_kernel(PipeArgs a) {
               ok = ok && word_ok(wv[cl], tagb);
             }
             if (__all_sync(0xffffffffu, ok)) break;
-            if (++spins > kSpin || ((spins & 255u) == 255u && *reinterpret_cast<volatile int*>(a.err) != 0)) { dead = true; atomicCAS(a.err, 0, 3); }
+            if (++spins > kSpin || ((spins & 255u) == 255u && *reinterpret_cast<volatile int*>(a.s.err) != 0)) { dead = true; atomicCAS(a.s.err, 0, 3); }
           }
           long long tot = 0;
 #pragma unroll
@@ -708,7 +708,7 @@ __global__ void __launch_bounds__(kT, 1) sweep_pipe_kernel(PipeArgs a) {
         const int slot = b % sring;
         const float* Gb = Gs + (size_t)slot * 10 * kTileF;
         const MarkerCol* mc = mcol + slot * 128;
-        mbar_wait(&S.in_ready[slot], (uint32_t)(b / sring) & 1u, dead, a.err);
+        mbar_wait(&S.in_ready[slot], (uint32_t)(b / sring) & 1u, dead, a.s.err);
         const SysScalars Sy = sc[0];
         const MarkerSys* mk = msys + (size_t)slot * 128;
         const MarkerDraws* drb = drw + (size_t)slot * 128;
@@ -718,7 +718,7 @@ __global__ void __launch_bounds__(kT, 1) sweep_pipe_kernel(PipeArgs a) {
           long long qq = 0;
           uint32_t spins = 0;
           if (CL) {
-            mbar_wait(&S.h_ready[b & 1], (uint32_t)(b >> 1) & 1u, dead, a.err);
+            mbar_wait(&S.h_ready[b & 1], (uint32_t)(b >> 1) & 1u, dead, a.s.err);
             qq = dead ? 0 : hsum[(size_t)(b & 1) * 128 + jj];
           } else if (a.world > 1) {
             const unsigned long long gen = a.gen0 + (unsigned long long)b;
@@ -734,7 +734,7 @@ __global__ void __launch_bounds__(kT, 1) sweep_pipe_kernel(PipeArgs a) {
                 ok = ok && word_ok(wv[src], tagx);
               }
               if (__all_sync(0xffffffffu, ok)) break;
-              if (++spins > kSpin || ((spins & 255u) == 255u && *reinterpret_cast<volatile int*>(a.err) != 0)) { dead = true; atomicCAS(a.err, 0, 3); }
+              if (++spins > kSpin || ((spins & 255u) == 255u && *reinterpret_cast<volatile int*>(a.s.err) != 0)) { dead = true; atomicCAS(a.s.err, 0, 3); }
             }
 #pragma unroll
             for (int src = 0; src < 8; src++) qq += dead ? 0 : word_val(wv[src]);  // tag-only filler words carry value 0
@@ -745,7 +745,7 @@ __global__ void __launch_bounds__(kT, 1) sweep_pipe_kernel(PipeArgs a) {
             while (!dead) {
               wv = ld_relaxed_u64(gq);
               if (__all_sync(0xffffffffu, word_ok(wv, tagb))) break;
-              if (++spins > kSpin || ((spins & 255u) == 255u && *reinterpret_cast<volatile int*>(a.err) != 0)) { dead = true; atomicCAS(a.err, 0, 3); }
+              if (++spins > kSpin || ((spins & 255u) == 255u && *reinterpret_cast<volatile int*>(a.s.err) != 0)) { dead = true; atomicCAS(a.s.err, 0, 3); }
             }
             qq = dead ? 0 : word_val(wv);
           }
@@ -757,7 +757,7 @@ __global__ void __launch_bounds__(kT, 1) sweep_pipe_kernel(PipeArgs a) {
           g = (float)((double)qq * (double)Sy.e_q);
         }
         if (D > 0 && b > 0) {
-          mbar_wait(&S.corr_ready[0], (uint32_t)(b - 1) & 1u, dead, a.err);
+          mbar_wait(&S.corr_ready[0], (uint32_t)(b - 1) & 1u, dead, a.s.err);
           g -= tcor[(b & 1) * ns * 128 + jj];
         }
         if (w == 0) SSTAMPW(b, 9);
@@ -811,7 +811,7 @@ __global__ void __launch_bounds__(kT, 1) sweep_pipe_kernel(PipeArgs a) {
         if (mx > 0.0f && mx < 3.0e38f) ex = (int)((__float_as_uint(mx) >> 23) & 0xFFu) - 126;
         if (ex < -90) ex = -90;
         const float dq = __uint_as_float((uint32_t)(ex - 30 + 127) << 23), dqinv = __uint_as_float((uint32_t)(30 - ex + 127) << 23);
-        if (!(mx < 3.0e38f)) atomicExch(a.err, 4);
+        if (!(mx < 3.0e38f)) atomicExch(a.s.err, 4);
         unsigned long long* wv = a.dew + (size_t)b * kDewStride;
         const bool valid = jj < nvalid && !Sy.done;
         const int qv = valid ? __float2int_rn(de * dqinv) : 0;
@@ -837,8 +837,8 @@ __global__ void __launch_bounds__(kT, 1) sweep_pipe_kernel(PipeArgs a) {
           if (MODEL == M_EMBA) vnew = (Sy.Sb + bnew * bnew) / (Sy.df + 1.0f);
           if (MODEL == M_BA || MODEL == M_BL) vnew = (Sy.Sb + bnew * bnew) / drb[jj].chi;
           const int j = mc[jj].j;
-          a.b[j] = bnew;
-          if (model_rule_writes_vbj(MODEL) && a.vbv) a.vbv[j] = vnew;
+          a.s.b[j] = bnew;
+          if (model_rule_writes_vbj(MODEL) && a.s.vbv) a.s.vbv[j] = vnew;
         }
         __syncwarp();
         if (lane == 0) mbar_arrive(&S.solve_done[slot]);
@@ -851,7 +851,7 @@ __global__ void __launch_bounds__(kT, 1) sweep_pipe_kernel(PipeArgs a) {
         const int slot = b % sring;
         const float* Gb = Gs + (size_t)slot * 10 * kTileF;
         const MarkerCol* mc = mcol + slot * 128;
-        mbar_wait(&S.in_ready[slot], (uint32_t)(b / sring) & 1u, dead, a.err);
+        mbar_wait(&S.in_ready[slot], (uint32_t)(b / sring) & 1u, dead, a.s.err);
         for (int s = warp; s < ns; s += kSolveWarps) {
           const SysScalars Sy = sc[s];
           const MarkerSys* mk = msys + ((size_t)slot * ns + s) * 128;
@@ -861,7 +861,7 @@ __global__ void __launch_bounds__(kT, 1) sweep_pipe_kernel(PipeArgs a) {
             long long qq[4] = {0, 0, 0, 0};
             uint32_t spins = 0;
             if (CL) {
-              mbar_wait(&S.h_ready[b & 1], (uint32_t)(b >> 1) & 1u, dead, a.err);
+              mbar_wait(&S.h_ready[b & 1], (uint32_t)(b >> 1) & 1u, dead, a.s.err);
 #pragma unroll
               for (int t = 0; t < 4; t++) qq[t] = dead ? 0 : hsum[(size_t)((b & 1) * ns + s) * 128 + 32 * t + lane];
             } else if (a.world > 1) {
@@ -880,7 +880,7 @@ __global__ void __launch_bounds__(kT, 1) sweep_pipe_kernel(PipeArgs a) {
                     w4[t] = word_val(w);
                   }
                   if (__all_sync(0xffffffffu, ok)) break;
-                  if (++spins > kSpin || ((spins & 255u) == 255u && *reinterpret_cast<volatile int*>(a.err) != 0)) { dead = true; atomicCAS(a.err, 0, 3); }
+                  if (++spins > kSpin || ((spins & 255u) == 255u && *reinterpret_cast<volatile int*>(a.s.err) != 0)) { dead = true; atomicCAS(a.s.err, 0, 3); }
                 }
 #pragma unroll
                 for (int t = 0; t < 4; t++) qq[t] += w4[t];
@@ -897,7 +897,7 @@ __global__ void __launch_bounds__(kT, 1) sweep_pipe_kernel(PipeArgs a) {
                   qq[t] = word_val(w);
                 }
                 if (__all_sync(0xffffffffu, ok)) break;
-                if (++spins > kSpin || ((spins & 255u) == 255u && *reinterpret_cast<volatile int*>(a.err) != 0)) { dead = true; atomicCAS(a.err, 0, 3); }
+                if (++spins > kSpin || ((spins & 255u) == 255u && *reinterpret_cast<volatile int*>(a.s.err) != 0)) { dead = true; atomicCAS(a.s.err, 0, 3); }
               }
             }
             if (s == 0) SSTAMP(b, 8);
@@ -912,7 +912,7 @@ __global__ void __launch_bounds__(kT, 1) sweep_pipe_kernel(PipeArgs a) {
             }
           }
           if (D > 0 && b > 0) {
-            mbar_wait(&S.corr_ready[s], (uint32_t)(b - 1) & 1u, dead, a.err);
+            mbar_wait(&S.corr_ready[s], (uint32_t)(b - 1) & 1u, dead, a.s.err);
 #pragma unroll
             for (int t = 0; t < 4; t++) g[t] -= tcor[((b & 1) * ns + s) * 128 + 32 * t + lane];
           }
@@ -1110,7 +1110,7 @@ __global__ void __launch_bounds__(kT, 1) sweep_pipe_kernel(PipeArgs a) {
           if (mx > 0.0f && mx < 3.0e38f) frexpf(mx, &ex);
           if (ex < -90) ex = -90;
           const float dq = ldexpf(1.0f, ex - 30), dqinv = ldexpf(1.0f, 30 - ex);
-          if (!(mx < 3.0e38f)) atomicExch(a.err, 4);
+          if (!(mx < 3.0e38f)) atomicExch(a.s.err, 4);
           unsigned long long* wv = a.dew + ((size_t)b * ns + s) * kDewStride;
           int qv[4];
 #pragma unroll
@@ -1149,9 +1149,9 @@ __global__ void __launch_bounds__(kT, 1) sweep_pipe_kernel(PipeArgs a) {
                 bnew = nb[t];
               }
               const int j = mc[jj].j;
-              a.b[(size_t)s * p + j] = bnew;
-              if (model_has_d(MODEL) && a.d) a.d[(size_t)s * p + j] = dnew;
-              if (model_rule_writes_vbj(MODEL) && a.vbv) a.vbv[(size_t)s * p + j] = vnew;
+              a.s.b[(size_t)s * p + j] = bnew;
+              if (model_has_d(MODEL) && a.s.d) a.s.d[(size_t)s * p + j] = dnew;
+              if (model_rule_writes_vbj(MODEL) && a.s.vbv) a.s.vbv[(size_t)s * p + j] = vnew;
             }
           }
         }
@@ -1184,7 +1184,7 @@ __global__ void __launch_bounds__(kT, 1) sweep_pipe_kernel(PipeArgs a) {
         }
         auto chunk = [&](const float (&cv)[32], int d) {
           for (int s = 0; s < ns; s++) {
-            mbar_wait(&S.de_ready[s][d], (uint32_t)b & 1u, dead, a.err);
+            mbar_wait(&S.de_ready[s][d], (uint32_t)b & 1u, dead, a.s.err);
             const float4* dv = reinterpret_cast<const float4*>(dehist + s * 128 + 32 * d);
             float fa[4] = {0.f, 0.f, 0.f, 0.f};
 #pragma unroll
@@ -1218,16 +1218,16 @@ __global__ void __launch_bounds__(kT, 1) sweep_pipe_kernel(PipeArgs a) {
     constexpr int kPipeSys = 2;  // systems whose scalars are register-pipelined (more systems: loaded in place)
     auto perm_at = [&](int blk) { const int pos = blk * 128 + ht; return (blk < nblocks && pos < p) ? a.perm[pos] : -1; };
     int j_cur = perm_at(0), j_nxt = perm_at(1);
-    float xx_cur = j_cur >= 0 ? a.xx[j_cur] : 1.0f, sx_cur = (j_cur >= 0 && a.sx) ? a.sx[j_cur] : 0.0f, b_cur[kPipeSys], v_cur[kPipeSys];
+    float xx_cur = j_cur >= 0 ? a.s.xx[j_cur] : 1.0f, sx_cur = (j_cur >= 0 && a.sx) ? a.sx[j_cur] : 0.0f, b_cur[kPipeSys], v_cur[kPipeSys];
 #pragma unroll
     for (int s = 0; s < kPipeSys; s++) {
-      b_cur[s] = (s < ns && j_cur >= 0) ? a.b[(size_t)s * p + j_cur] : 0.0f;
-      v_cur[s] = (s < ns && j_cur >= 0 && model_has_vbj(MODEL) && a.vbv) ? a.vbv[(size_t)s * p + j_cur] : 1.0f;
+      b_cur[s] = (s < ns && j_cur >= 0) ? a.s.b[(size_t)s * p + j_cur] : 0.0f;
+      v_cur[s] = (s < ns && j_cur >= 0 && model_has_vbj(MODEL) && a.s.vbv) ? a.s.vbv[(size_t)s * p + j_cur] : 1.0f;
     }
     const int rr0 = ht >> 3, c4 = ht & 7;
     for (int nb = 0; nb < nblocks; nb++) {
       const int slot = nb % sring;
-      if (nb >= sring) mbar_wait(&S.solve_done[slot], (uint32_t)(nb / sring - 1) & 1u, dead, a.err);
+      if (nb >= sring) mbar_wait(&S.solve_done[slot], (uint32_t)(nb / sring - 1) & 1u, dead, a.s.err);
       PSTAMP(0);
       // Gram triangle of block nb: linear rules read tile (hi, lo) = G[32 hi + r][32 lo + c];
       // the scalar chain reads the transposed triangle, stored in the same slots
@@ -1250,11 +1250,11 @@ __global__ void __launch_bounds__(kT, 1) sweep_pipe_kernel(PipeArgs a) {
       // issue the gathers of the following blocks now; they are consumed in the next iteration
       const int j_nn = perm_at(nb + 2);
       float xx_nxt = 1.0f, sx_nxt = 0.0f, b_nxt[kPipeSys], v_nxt[kPipeSys];
-      if (j_nxt >= 0) { xx_nxt = a.xx[j_nxt]; if (a.sx) sx_nxt = a.sx[j_nxt]; }
+      if (j_nxt >= 0) { xx_nxt = a.s.xx[j_nxt]; if (a.sx) sx_nxt = a.sx[j_nxt]; }
 #pragma unroll
       for (int s = 0; s < kPipeSys; s++) {
-        b_nxt[s] = (s < ns && j_nxt >= 0) ? a.b[(size_t)s * p + j_nxt] : 0.0f;
-        v_nxt[s] = (s < ns && j_nxt >= 0 && model_has_vbj(MODEL) && a.vbv) ? a.vbv[(size_t)s * p + j_nxt] : 1.0f;
+        b_nxt[s] = (s < ns && j_nxt >= 0) ? a.s.b[(size_t)s * p + j_nxt] : 0.0f;
+        v_nxt[s] = (s < ns && j_nxt >= 0 && model_has_vbj(MODEL) && a.s.vbv) ? a.s.vbv[(size_t)s * p + j_nxt] : 1.0f;
       }
       {
         const int j = j_cur;
@@ -1266,13 +1266,13 @@ __global__ void __launch_bounds__(kT, 1) sweep_pipe_kernel(PipeArgs a) {
           if (j >= 0 && !sc[s].done) {
             if (s < kPipeSys) { in.b0 = b_cur[s < kPipeSys ? s : 0]; in.vbj = v_cur[s < kPipeSys ? s : 0]; }
             else {
-              in.b0 = a.b[(size_t)s * p + j];
-              in.vbj = (model_has_vbj(MODEL) && a.vbv) ? a.vbv[(size_t)s * p + j] : 1.0f;
+              in.b0 = a.s.b[(size_t)s * p + j];
+              in.vbj = (model_has_vbj(MODEL) && a.s.vbv) ? a.s.vbv[(size_t)s * p + j] : 1.0f;
             }
             MarkerDraws dr;
             dr.z1 = dr.z2 = dr.u = 0.0f; dr.chi = 1.0f;
             if (kGibbs) {
-              dr = marker_draws(MODEL, (uint32_t)j, (uint32_t)sc[s].sweep, (uint32_t)(a.chain0 + s), sc[s].df, a.seed_lo, a.seed_hi);
+              dr = marker_draws(MODEL, (uint32_t)j, (uint32_t)sc[s].sweep, (uint32_t)(a.s.chain0 + s), sc[s].df, a.s.seed_lo, a.s.seed_hi);
               drw[((size_t)slot * ns + s) * 128 + ht] = dr;
             }
             if (kLinear) {
@@ -1378,45 +1378,28 @@ size_t sweep_pipe_smem(int rows_per_cta, int nsys, int model, int nbuf, int srin
   return (w > s ? w : s) + 1024;
 }
 
-#define BWGR_MODEL_SWITCH(CALL)                 \
-  switch (rule_model(model)) {                  \
-    case M_EMRR: return CALL(M_EMRR);           \
-    case M_EMBA: return CALL(M_EMBA);           \
-    case M_EMBB: return CALL(M_EMBB);           \
-    case M_EMBC: return CALL(M_EMBC);           \
-    case M_EMBL: return CALL(M_EMBL);           \
-    case M_EMEN: return CALL(M_EMEN);           \
-    case M_BRR: return CALL(M_BRR);             \
-    case M_BA: return CALL(M_BA);               \
-    case M_BB: return CALL(M_BB);               \
-    case M_BC: return CALL(M_BC);               \
-    case M_KMUP: return CALL(M_KMUP);           \
-    case M_MRR: return CALL(M_MRR);             \
-    case M_EMDE: return CALL(M_EMDE);           \
-    case M_LASSO: return CALL(M_LASSO);         \
-    case M_BL: return CALL(M_BL);               \
-    case M_BDPI: return CALL(M_BDPI);           \
-    default: break;                             \
-  }
-
 // The clustered topology needs the solver's warps 4-7 free (comm warps): at most four systems and no in-kernel 32 x 32 inverses.
 bool sweep_pipe_cluster_ok(int model, int nsys, int full_inv) {
   return nsys <= 4 && !(!full_inv && pipe_use_inv(model, nsys));
 }
+// Every rule but KMUP2's, which always comes with a row mask (the pipelined sweep takes unmasked systems only).
 int sweep_pipe_max_clusters(int model, size_t smem) {
-#define BWGR_CALL(M) max_clusters_model<M>(smem)
-  BWGR_MODEL_SWITCH(BWGR_CALL)
-#undef BWGR_CALL
-  return 0;
+  int n = 0;
+  with_rule(model, [&](auto rule) {
+    constexpr int M = decltype(rule)::value;
+    if constexpr (M != M_KMUP2) n = max_clusters_model<M>(smem);
+  });
+  return n;
 }
 
 cudaError_t launch_sweep_pipe(const PipeArgs& a, cudaStream_t st) {
-  const size_t smem = sweep_pipe_smem(a.rows_per_cta, a.nsys, a.model, a.nbuf, a.sring, a.tinv != nullptr, a.cl);
-  const int model = a.model;
-#define BWGR_CALL(M) launch_model<M>(a, smem, st)
-  BWGR_MODEL_SWITCH(BWGR_CALL)
-#undef BWGR_CALL
-  return cudaErrorInvalidValue;
+  const size_t smem = sweep_pipe_smem(a.rows_per_cta, a.s.nsys, a.model, a.nbuf, a.sring, a.tinv != nullptr, a.cl);
+  cudaError_t e = cudaErrorInvalidValue;
+  with_rule(a.model, [&](auto rule) {
+    constexpr int M = decltype(rule)::value;
+    if constexpr (M != M_KMUP2) e = launch_model<M>(a, smem, st);
+  });
+  return e;
 }
 
 }  // namespace bwgr
