@@ -179,7 +179,7 @@ struct Fit {
   int lookahead = 0, nbuf = 0, sring = 2, nworkers = 0, nc = 1, nband = 1, full_inv = 0, cl = 0, nclusters = 0;
   DevBuf<float> tinv;                   // (I + A L)^-1 of every block of the current sweep (block_inv.cu)
   uint32_t tag = 0;
-  DevBuf<unsigned long long> dew, part, cx;
+  DevBuf<unsigned long long> dew, part, hsum;
   DevBuf<float> wts;  // emML: marker weights d_j
   float* gram_p = nullptr;              // Gram band in use: f.gram (per fit) or the handle's natural-order cache
   // Gram band of sweep s + 1 computed on the handle's side stream while sweep s runs (the clustered sweep leaves SMs idle)
@@ -896,9 +896,9 @@ bool plan_pipe(const bwgr_handle* h, int model, int ns, PipePlan* pl) {
   // (MRR3's centred systems keep the stepwise solve.)
   const int full_inv = model_is_linear(model) && ns == 1 && model != M_MRR;
   pl->cl = 0; pl->nclusters = 0;
-  // Clustered topology (sweep_pipe.cu): thread-block clusters of one solver + seven workers; partial sums and steps travel
-  // through distributed shared memory, one L2 hop per block is left (the exchange of the cluster sums between the solvers).
-  // Single GPU at the default grid, at most four systems; otherwise the flat topology (one solver CTA, two-hop L2 tree).  Row-sharded
+  // Clustered topology (sweep_pipe.cu): thread-block clusters of one solver + seven workers; steps travel through distributed shared
+  // memory, and every worker adds its partial sums to L2 grid-sum words: one L2 hop per block.
+  // Single GPU at the default grid, at most three systems; otherwise the flat topology (one solver CTA, two-hop L2 tree).  Row-sharded
   // fits use the flat one: a clustered variant with a third (NVLink) hop after the cluster exchange measured 1.79 ms against 1.43 ms per sweep.
   if (h->world <= 1 && h->grid <= 1 && sweep_pipe_cluster_ok(model, ns, full_inv)) {
     {
@@ -1317,8 +1317,13 @@ int fit_begin(bwgr_handle* h, const FitSpec& s, const double* y) {
     if (!f.full_inv) f.tinv.release();
     if (f.part.alloc((size_t)8 * ns * 128 * 161) != cudaSuccess || f.dew.alloc((size_t)f.nblocks * ns * 136) != cudaSuccess)
       return fail(BWGR_ERR_CUDA, "cudaMalloc(blocked workspace) failed");
-    if (f.cl && f.cx.alloc((size_t)8 * f.nclusters * ns * 128) != cudaSuccess) return fail(BWGR_ERR_CUDA, "cudaMalloc(cluster ring) failed");
-    if (!f.cl) f.cx.release();
+    // clustered topology: two sets of the grid-sum words of h, used by alternate sweeps; each sweep zeroes the other set
+    if (f.cl) {
+      if (f.hsum.alloc((size_t)2 * f.nblocks * ns * 128 * kGridCopies) != cudaSuccess) return fail(BWGR_ERR_CUDA, "cudaMalloc(grid sums of h) failed");
+      CU(cudaMemsetAsync(f.hsum.p, 0, sizeof(unsigned long long) * f.hsum.n, h->stream));
+    } else {
+      f.hsum.release();
+    }
     CU(cudaMemsetAsync(f.dew.p, 0, sizeof(unsigned long long) * f.dew.n, h->stream));
   }
   if (f.gridfam) {
@@ -1411,8 +1416,7 @@ int fit_sweeps(bwgr_handle* h, int nsweeps) {
         h->prof_end(pi);
         h->launches++;
       }
-      if (f.cl) CU(cudaMemsetAsync(f.cx.p, 0, sizeof(unsigned long long) * f.cx.n, h->stream));
-      else CU(cudaMemsetAsync(f.part.p, 0, sizeof(unsigned long long) * f.part.n, h->stream));
+      if (!f.cl) CU(cudaMemsetAsync(f.part.p, 0, sizeof(unsigned long long) * f.part.n, h->stream));
       PipeArgs a;
       memset(&a, 0, sizeof a);
       a.s = state; a.model = rule_model(f.model); a.perm = d_perm; a.nblocks = f.nblocks; a.gram = f.gram_p; a.nband = f.nband; a.tinv = f.full_inv ? f.tinv.p : nullptr;
@@ -1420,7 +1424,11 @@ int fit_sweeps(bwgr_handle* h, int nsweeps) {
       a.part = f.part.p; a.hred = f.part.p + (size_t)8 * f.nsys * 128 * 160; a.dew = f.dew.p; a.tag = ++f.tag;
       a.rows_per_cta = f.rows_per_cta; a.nworkers = f.nworkers; a.D = f.lookahead; a.nbuf = f.nbuf; a.sring = f.sring;
       a.world = h->world; a.rank = h->rank; a.gen0 = h->dist_gen;
-      a.cl = f.cl; a.nclusters = f.nclusters; a.cx = f.cx.p;
+      a.cl = f.cl; a.nclusters = f.nclusters;
+      if (f.cl) {
+        const size_t set = f.hsum.n / 2;
+        a.hsum = f.hsum.p + (sweep & 1) * set; a.hsum_next = f.hsum.p + ((sweep + 1) & 1) * set;
+      }
       for (int r = 0; r < 8; r++) a.hx[r] = h->hx[r];
       if (h->world > 1) h->dist_gen += (unsigned long long)f.nblocks;
       if (getenv("BWGR_TRACE")) {

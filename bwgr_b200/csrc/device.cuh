@@ -126,7 +126,7 @@ __device__ __forceinline__ void tmem_ld_x32(uint32_t taddr, uint32_t (&v)[32]) {
 }
 __device__ __forceinline__ void tmem_ld_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
 
-// ---- the L2 grid sum (grid family, general MRR3) -----------------------------------------------------------------------------
+// ---- the L2 grid sum (grid family, general MRR3, clustered sweep) ------------------------------------------------------------
 // A sum over the CTAs of a grid lives in 64-bit words of global memory, zeroed before the launch: (fixed-point sum << 8) + arrivals.
 // Every CTA adds its fixed-point partial, plus one, with a single atomic, so the low byte counts the CTAs that have added and the
 // data is its own flag (one L2 hop, no fence, no barrier).  Integer sums are order-free: every CTA reads bit-identical totals.
@@ -143,11 +143,17 @@ __device__ __forceinline__ void grid_add(unsigned long long* w, double v, int* e
   if (!(fabs(v) < 4503599627370496.0)) atomicExch(err, 4);
   atomicAdd(w, grid_word(v));
 }
+// the same with an integer partial (the sweep's exact fixed-point sums)
+__device__ __forceinline__ void grid_add(unsigned long long* w, long long v, int* err) {
+  if (!(v < 4503599627370496ll && v > -4503599627370496ll)) atomicExch(err, 4);
+  atomicAdd(w, ((unsigned long long)v << 8) + 1ull);
+}
 // Warp-collective wait for the words of one marker, copy c at w + 32 c: returns the lane's total once the words of every lane with
 // `on` set are complete.  Every 4096 spins lane 0 looks at the error flag and, two minutes after t_start, raises err = 3; either ends
-// the wait for the whole warp with *abort = 1 (the total is then meaningless).
+// the wait for the whole warp with *abort = 1 (the total is then meaningless).  backoff_ns > 0: the warp sleeps that long between
+// polls (it issues nothing meanwhile: a poller that shares its SM with a latency-bound chain leaves the chain the issue slots).
 __device__ __forceinline__ long long grid_wait_total(const unsigned long long* w, bool on, int G, int* err, unsigned long long t_start,
-                                                     int* abort) {
+                                                     int* abort, unsigned int backoff_ns = 0) {
   unsigned long long v[kGridCopies];
   unsigned int spins = 0;
   for (;;) {
@@ -157,6 +163,7 @@ __device__ __forceinline__ long long grid_wait_total(const unsigned long long* w
 #pragma unroll
     for (int c = 0; c < kGridCopies; c++) pending |= grid_word_count(v[c]) != grid_copy_count(G, c);
     if (!__any_sync(0xffffffffu, on && pending)) break;
+    if (backoff_ns) __nanosleep(backoff_ns);
     if ((++spins & 0xfffu) == 0) {
       int ab = 0;
       if ((threadIdx.x & 31) == 0) {

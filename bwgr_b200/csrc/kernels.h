@@ -126,11 +126,13 @@ struct PipeArgs {
   int sring;             // blocks of solve inputs in flight in the solver CTA (2 or 3)
   uint32_t tag;          // unique per launch, never 0
   // clustered topology: nclusters thread-block clusters of 8 CTAs = one solver + seven workers each (nworkers = 7 * nclusters);
-  // cx = [8][nclusters][nsys][128] per-cluster sums of h, same word format as hred; zeroed before launch
-  unsigned long long* cx;
+  // hsum = [nblocks][nsys][4][kGridCopies][32] L2 grid-sum words of h (device.cuh), word (block, system, marker m) at
+  // [block][system][m / 32][copy][m % 32]; zero at launch.  hsum_next = the set of the next launch: this launch zeroes it
+  unsigned long long* hsum;
+  unsigned long long* hsum_next;
   long long* trace;      // optional [nblocks][16] clock64 stamps (BWGR_TRACE), else nullptr
   int cl, nclusters;
-  // optional: cluster 0 stores started_val here once the first grid sum has gone round, i.e. when every CTA of the launch is
+  // optional: cluster 0 stores started_val here once the first grid sum is complete, i.e. when every CTA of the launch is
   // resident -- a side stream waits on it (cuStreamWaitValue32) before it fills the SMs this launch leaves idle
   unsigned int* started;
   unsigned int started_val;

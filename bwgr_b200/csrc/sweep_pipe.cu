@@ -111,9 +111,6 @@ __device__ __forceinline__ uint32_t mapa_u32(uint32_t addr, uint32_t rank) {
   return r;
 }
 // remote shared-memory store that counts its bytes on the destination CTA's mbarrier (no flag, no polling)
-__device__ __forceinline__ void st_async_u64(uint32_t raddr, unsigned long long v, uint32_t rbar) {
-  asm volatile("st.async.weak.shared::cluster.mbarrier::complete_tx::bytes.b64 [%0], %1, [%2];" ::"r"(raddr), "l"(v), "r"(rbar) : "memory");
-}
 __device__ __forceinline__ void st_async_u32(uint32_t raddr, uint32_t v, uint32_t rbar) {
   asm volatile("st.async.weak.shared::cluster.mbarrier::complete_tx::bytes.b32 [%0], %1, [%2];" ::"r"(raddr), "r"(v), "r"(rbar) : "memory");
 }
@@ -125,10 +122,12 @@ __device__ __forceinline__ void cluster_sync_all() {
 }
 constexpr int kClSize = 8;             // CTAs per cluster: one solver + seven workers
 constexpr int kClWorkers = kClSize - 1;
-constexpr int kMaxCl = 18;             // clusters whose sums a solver gathers (B200: 15 co-resident clusters of 8 at ~200 KB per CTA)
 constexpr int kDeStride = 132;         // 32-bit words per (parity, system) of a worker's step inbox: 128 steps + the scale (+ pad)
 constexpr int kAtomsPerGroup = 2;      // row atoms whose U epilogue / G issue are handled together (see the worker)
-constexpr int kCommWarp0 = 4;          // clustered solver: warps 4-7 gather the partial sums (they are idle whenever CL is eligible)
+constexpr int kCommWarp0 = 4;          // clustered solver: warps 4-7 wait for the grid sums of h (they are idle whenever CL is eligible)
+constexpr unsigned int kPollBackoffNs = 128;  // their sleep between polls (they share the SM with the solve chain)
+// word of (block b, system s, marker m) among the grid-sum words of h (PipeArgs::hsum); copy c at + 32 c
+__host__ __device__ inline size_t hsum_word(int b, int ns, int s, int m) { return (((size_t)b * ns + s) * 4 + (m >> 5)) * kGridCopies * 32 + (m & 31); }
 
 // Self-validating 64-bit words of the grid reduction: (signed value << 12) | tag, tag = 1 + (use index of the ring slot) mod 4095
 // (never 0 = freshly zeroed memory; consecutive uses of a slot always differ).  |value| < 2^51: a rank's sum of 143 worker
@@ -151,8 +150,8 @@ struct Sync {
   uint64_t tile_full[8], tile_empty[8], dl_full[2], u_done, el_full, g_done, g_empty;
   // solver
   uint64_t raw_ready[3], in_ready[3], solve_done[3], corr_ready[32], de_ready[32][4];
-  // clustered topology: step inbox of a worker, partial inbox of a solver, gathered sums ready for the solve warps
-  uint64_t de_in[2], h_in[2], h_ready[2];
+  // clustered topology: step inbox of a worker, grid sums of h ready for the solve warps
+  uint64_t de_in[2], h_ready[2];
   // per 128-row atom: U accumulator complete (tcgen05.commit) / new residual limbs of the atom written (128 epilogue threads)
   uint64_t u_done_at[4], el_full_at[4];
   uint32_t tmem_base;
@@ -172,7 +171,7 @@ __host__ __device__ inline WLayout worker_layout(int R, int ns, int nbuf, bool c
   L.total = o;
   return L;
 }
-struct SLayout { size_t gs, mt, ms, mc, drw, tc, dh, rb, cs, hi, hs, total; };
+struct SLayout { size_t gs, mt, ms, mc, drw, tc, dh, rb, cs, hs, total; };
 // sring = blocks of solve inputs in flight in the solver CTA (2 or 3)
 __host__ __device__ inline SLayout solver_layout(int ns, bool gibbs, bool use_inv, int sring, bool cl = false) {
   SLayout L;
@@ -187,8 +186,7 @@ __host__ __device__ inline SLayout solver_layout(int ns, bool gibbs, bool use_in
   L.rb = o; o += (size_t)kSolveWarps * 32 * 4;
   L.cs = o; o += (size_t)32 * 2 * 4 + 2 * 4 * 4;  // running mean shift per system (centred columns): {current, before the last block}
   o = (o + 15) & ~(size_t)15;
-  L.hi = o; o += cl ? (size_t)2 * kClWorkers * ns * 128 * 8 : 0;  // partial inbox [parity][worker][system][marker], written by the workers
-  L.hs = o; o += cl ? (size_t)2 * ns * 128 * 8 : 0;               // h summed over the whole grid [parity][system][marker]
+  L.hs = o; o += cl ? (size_t)2 * ns * 128 * 8 : 0;  // h summed over the whole grid [parity][system][marker]
   L.total = o;
   return L;
 }
@@ -222,14 +220,10 @@ __global__ void __launch_bounds__(kT, 1) sweep_pipe_kernel(PipeArgs a) {
       mbar_init(&S.corr_ready[s], 128);
       for (int d = 0; d < 4; d++) mbar_init(&S.de_ready[s][d], 1);
     }
-    for (int i = 0; i < 2; i++) { mbar_init(&S.de_in[i], 1); mbar_init(&S.h_in[i], 1); mbar_init(&S.h_ready[i], 128); }
+    for (int i = 0; i < 2; i++) { mbar_init(&S.de_in[i], 1); mbar_init(&S.h_ready[i], 128); }
     fence_mbar_init();
-    if (CL) {  // expected bytes of the first two blocks (every later phase is armed by the consumer of the phase before)
-      for (int i = 0; i < 2 && i < nblocks; i++) {
-        if (is_solver) mbar_expect_tx(&S.h_in[i], (uint32_t)(kClWorkers * ns * 128 * 8));
-        else mbar_expect_tx(&S.de_in[i], (uint32_t)(ns * 129 * 4));
-      }
-    }
+    if (CL && !is_solver)  // expected bytes of the first two steps (every later phase is armed by the consumer of the phase before)
+      for (int i = 0; i < 2 && i < nblocks; i++) mbar_expect_tx(&S.de_in[i], (uint32_t)(ns * 129 * 4));
   }
   if (CL) cluster_sync_all();  // every CTA's barriers exist before the first remote store
 
@@ -241,8 +235,6 @@ __global__ void __launch_bounds__(kT, 1) sweep_pipe_kernel(PipeArgs a) {
     const int R = a.rows_per_cta, NA = L.NA, N = L.N, RS = NA * 128, nbuf = L.nbuf;
     const int row0 = widx * R;
     const uint32_t* dein = reinterpret_cast<const uint32_t*>(base + L.di);
-    // the solver's partial inbox sits at the same shared-window offset in every CTA of this launch
-    const uint32_t hin_u32 = smem_u32(base) + (uint32_t)solver_layout(ns, model_is_gibbs(MODEL), false, a.sring, CL).hi;
     unsigned char* Xs = base + L.xs;
     unsigned char* EL = base + L.el;
     unsigned char* DL = base + L.dl;
@@ -348,15 +340,13 @@ __global__ void __launch_bounds__(kT, 1) sweep_pipe_kernel(PipeArgs a) {
         // partial of marker q, system s -> part[c % ring][s][this worker][q] (full 32-byte sectors): (value << 12) | block tag
         unsigned long long* hb = a.part + (((size_t)(c % kRing) * ns) * kWPad + (CL ? 0 : blockIdx.x)) * 128 + q;
         const unsigned long long tagc = tag_of((unsigned long long)(c / kRing));
-        // CL: the partial goes into the cluster solver's shared memory and counts itself on that solver's barrier
-        const uint32_t rdst = CL ? mapa_u32(hin_u32 + (uint32_t)((((c & 1) * kClWorkers + (crank - 1)) * ns) * 128 + q) * 8u, 0u) : 0u;
-        const uint32_t rbar = CL ? mapa_u32(smem_u32(&S.h_in[c & 1]), 0u) : 0u;
         for (int s = 0; s < ns; s++) {
           int s0, s1, s2, s3;
           tmem_ld4(tmem_g + tlane + (uint32_t)(4 * s), s0, s1, s2, s3);
           tmem_ld_wait();
           const long long gq = combine_limbs(s0, s1, s2, s3);
-          if (CL) st_async_u64(rdst + (uint32_t)s * 1024u, (unsigned long long)gq, rbar);
+          // CL: straight into copy (worker % kGridCopies) of the grid-sum word of (block c, system s, marker q)
+          if (CL) grid_add(a.hsum + hsum_word(c, ns, s, q) + (widx % kGridCopies) * 32, gq, a.s.err);
           else st_relaxed_u64(hb + (size_t)s * kWPad * 128, pack_word(gq, tagc));
         }
         tc_fence_before();
@@ -493,7 +483,13 @@ __global__ void __launch_bounds__(kT, 1) sweep_pipe_kernel(PipeArgs a) {
         mbar_arrive(&S.tile_full[buf]);
         if (tracing && lw == 0 && lane == 0) WSTAMP(t, 13);
       }
-    } else if (warp == kRedWarp && !CL) {
+    } else if (warp == kRedWarp && CL) {
+      // ------------------------------------------------------------------ zero the grid-sum words of the next launch
+      // (this warp is idle in the clustered topology; the words are in use again only after this launch has ended)
+      const size_t n16 = (size_t)nblocks * ns * 128 * kGridCopies / 2;
+      uint4* z = reinterpret_cast<uint4*>(a.hsum_next);
+      for (size_t i = (size_t)widx * 32 + lane; i < n16; i += (size_t)W * 32) z[i] = make_uint4(0, 0, 0, 0);
+    } else if (warp == kRedWarp) {
       // ------------------------------------------------------------------ second hop of the grid reduction
       // row (block c, system s, marker m) of the partials is summed by worker (s*128 + m) % W; plain loads and one store,
       // no atomics (143 x 128 L2 atomics per block cost ~7 us; this tree costs two L2 round trips)
@@ -575,7 +571,6 @@ __global__ void __launch_bounds__(kT, 1) sweep_pipe_kernel(PipeArgs a) {
   float* dehist = reinterpret_cast<float*>(base + L.dh);
   float* rb = reinterpret_cast<float*>(base + L.rb);
   float* cs = reinterpret_cast<float*>(base + L.cs);
-  const long long* hin = reinterpret_cast<const long long*>(base + L.hi);
   long long* hsum = reinterpret_cast<long long*>(base + L.hs);
   // a worker's step inbox sits at the same shared-window offset in every CTA of this launch
   const uint32_t dein_u32 = smem_u32(base) + (uint32_t)worker_layout(a.rows_per_cta, ns, a.nbuf, CL).di;
@@ -630,45 +625,28 @@ __global__ void __launch_bounds__(kT, 1) sweep_pipe_kernel(PipeArgs a) {
     }
     if (CL && warp >= kCommWarp0) {
       // ------------------------------------------------------------------ clustered topology: gather h_b
-      // 1. the seven workers of this cluster have stored their partials into this CTA (st.async; the barrier counts the bytes);
-      // 2. their sum goes to the L2 ring as one self-validating word per (system, marker) -- the only L2 hop of a block --
-      //    and the sums of all clusters are polled back, all words of a thread in flight at once;
-      // 3. the grid total (an integer: the same on every solver) is handed to the solve warps through shared memory.
+      // every worker has added its partial to the grid-sum words of h_b (one atomic per (system, marker): the only L2 hop of a
+      // block); these warps wait for the words, all copies of a word in flight at once, and hand the total (an integer: the same
+      // on every solver) to the solve warps through shared memory -- the solve warps never wait on L2 themselves.
       const int ct = tid - kCommWarp0 * 32;  // 0..127
-      const int C = a.nclusters;
+      const unsigned long long t_start = globaltimer_ns();
       for (int b = 0; b < nblocks; b++) {
         const int slot = b & 1;
-        mbar_wait(&S.h_in[slot], (uint32_t)(b >> 1) & 1u, dead, a.s.err);
-        const unsigned long long tagb = tag_of((unsigned long long)(b / kRing));
-        unsigned long long* ring = a.cx + (size_t)(b % kRing) * C * ns * 128;
+        // h_b cannot be complete before the step of block b - 2 is published (the workers' G(b) follows U(b - 2)): sleep on that
+        // barrier, not on the words, so that a long solve chain is not slowed by these warps' polls.  The hsum slot is next used by
+        // block b + 2 for the same reason.
+        if (b >= 2) mbar_wait(&S.solve_done[(b - 2) % sring], (uint32_t)((b - 2) / sring) & 1u, dead, a.s.err);
         for (int pair = ct; pair < ns * 128; pair += 128) {
-          long long own = 0;
-#pragma unroll
-          for (int wr = 0; wr < kClWorkers; wr++) own += hin[(size_t)((slot * kClWorkers + wr) * ns) * 128 + pair];
-          st_relaxed_u64(ring + (size_t)cluster * ns * 128 + pair, pack_word(dead ? 0 : own, tagb));
-        }
-        // the slot is next used by block b + 2, whose partials cannot be sent before this block's step is published
-        if (ct == 0 && b + 2 < nblocks) mbar_expect_tx(&S.h_in[slot], (uint32_t)(kClWorkers * ns * 128 * 8));
-        for (int pair = ct; pair < ns * 128; pair += 128) {
-          unsigned long long wv[kMaxCl];
-          uint32_t spins = 0;
-          while (!dead) {
-            bool ok = true;
-#pragma unroll
-            for (int cl = 0; cl < kMaxCl; cl++) {
-              wv[cl] = cl < C ? ld_relaxed_u64(ring + (size_t)cl * ns * 128 + pair) : tagb;
-              ok = ok && word_ok(wv[cl], tagb);
-            }
-            if (__all_sync(0xffffffffu, ok)) break;
-            if (++spins > kSpin || ((spins & 255u) == 255u && *reinterpret_cast<volatile int*>(a.s.err) != 0)) { dead = true; atomicCAS(a.s.err, 0, 3); }
-          }
           long long tot = 0;
-#pragma unroll
-          for (int cl = 0; cl < kMaxCl; cl++) tot += dead ? 0 : word_val(wv[cl]);  // tag-only filler words carry value 0
+          if (!dead) {
+            int ab = 0;
+            tot = grid_wait_total(a.hsum + hsum_word(b, ns, pair >> 7, pair & 127), true, W, a.s.err, t_start, &ab, kPollBackoffNs);
+            if (__shfl_sync(0xffffffffu, ab, 0)) { dead = true; tot = 0; }
+          }
           hsum[(size_t)slot * ns * 128 + pair] = tot;
         }
         mbar_arrive(&S.h_ready[slot]);
-        if (b == 0 && ct == 0 && cluster == 0 && a.started) {  // every cluster has delivered a sum: the whole grid is resident
+        if (b == 0 && ct == 0 && cluster == 0 && a.started) {  // every worker has added its partial: the whole grid is resident
           *reinterpret_cast<volatile unsigned int*>(a.started) = a.started_val;
           __threadfence_system();
         }
@@ -1378,9 +1356,11 @@ size_t sweep_pipe_smem(int rows_per_cta, int nsys, int model, int nbuf, int srin
   return (w > s ? w : s) + 1024;
 }
 
-// The clustered topology needs the solver's warps 4-7 free (comm warps): at most four systems and no in-kernel 32 x 32 inverses.
+// The clustered topology needs the solver's warps 4-7 free (comm warps) and no in-kernel 32 x 32 inverses.  At most three systems:
+// four never fitted next to the partial inboxes the solver once had, and without them are not measured (the comm warps would
+// wait for four words per thread one after the other).
 bool sweep_pipe_cluster_ok(int model, int nsys, int full_inv) {
-  return nsys <= 4 && !(!full_inv && pipe_use_inv(model, nsys));
+  return nsys <= 3 && !(!full_inv && pipe_use_inv(model, nsys));
 }
 // Every rule but KMUP2's, which always comes with a row mask (the pipelined sweep takes unmasked systems only).
 int sweep_pipe_max_clusters(int model, size_t smem) {

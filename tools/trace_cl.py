@@ -1,7 +1,11 @@
 #!/usr/bin/env python
 """Summarise a BWGR_TRACE file of the CLUSTERED pipelined sweep: [cta][block][32] = 16 globaltimer (ns) + 16 clock64 stamps.
 CTA 8c = solver of cluster c (8 h received, 9 corrected, 10 solved, 11 published; 4 = comm warps: grid sum ready),
-CTA 8c + r = its workers (0 step received, 1 DL written, 2 U issued, 3 u_done, 4 U-epilogue done, 5 G issued, 6 g_done, 7 partial sent)."""
+CTA 8c + r = its workers (0 step received, 1 DL written, 2 U issued, 3 u_done, 4 U-epilogue done, 5 G issued, 6 g_done, 7 partial sent
+= added to the grid-sum words of h).
+Traces of the kernel before the grid-sum words (partials summed per cluster, the cluster sums exchanged through an L2 ring) also
+carry, on the solver, 5 = the seven partials of the cluster arrived, 6 = the cluster's sum stored, 12 = the last cluster's word
+seen; the leg "last partial sent -> grid sum ready" is then split at those stamps."""
 import sys
 import numpy as np
 raw = np.fromfile(sys.argv[1], dtype=np.int64)
@@ -35,3 +39,14 @@ first_recv = allw[:, b, 0].min(0); last_recv = allw[:, b, 0].max(0)
 print("step received: first worker - solver0 published %.0f ns, last worker %.0f ns" % (np.median(first_recv - S[b, 11]), np.median(last_recv - S[b, 11])))
 sent = allw[:, c, 7]
 print("partial sent (block c=b+1+D) relative to step received (block b): med %.0f ns, slowest worker med %.0f ns" % (np.median(sent - allw[:, b, 0]), np.median((sent - allw[:, b, 0]).max(0))))
+# the leg "last partial sent -> grid sum ready", split (older kernel only).  Cycles on solver 0's SM; ns (globaltimer) across SMs
+if bool((S[b, 5] != 0).all()):
+    has12 = bool((S[b, 12] != 0).all())
+    print("solver 0 cycles: partials in -> cluster sum stored %d | stored -> %s %d" % (
+        np.median(S[c, ck + 6] - S[c, ck + 5]),
+        "last cluster word seen %d | seen -> grid sum ready" % np.median(S[c, ck + 12] - S[c, ck + 6]) if has12 else "grid sum ready",
+        np.median(S[c, ck + 4] - S[c, ck + (12 if has12 else 6)])))
+    last_stored = sol[:, c, 6].max(0)
+    print("last partial sent by ANY worker -> last cluster's partials in (any solver): med %.0f ns ; -> last cluster sum stored (any solver): med %.0f ns ; "
+          "last cluster sum stored -> grid sum ready at solver 0: med %.0f ns" % (
+              np.median(sol[:, c, 5].max(0) - last_sent), np.median(last_stored - last_sent), np.median(S[c, 4] - last_stored)))
