@@ -773,7 +773,10 @@ _MRR3_DEFAULTS = dict(
 
 def MRR3(Y, X, f32_variant=False, verbose=False, **kw):
     """MRR3(Y, X, ...) of R/RcppExports.R:180 (same argument names and defaults, same returned list).
-    The marker loop runs as k rotated ridge systems in the blocked sweep kernel (csrc/mrr.cu)."""
+    The marker loop runs as k rotated ridge systems in the blocked sweep kernel (csrc/mrr.cu).
+    X may be a row-sharded store (Genotypes.enable_row_sharding): every rank passes its rows of Y and gets the common
+    b / mu / h2 / GC / vb / ve / MSx / Its and hat for its rows.  Only the fast path runs sharded (complete Y, no InnerGS, TH,
+    NLfactor or MRR3F NoInv); otherwise every rank raises BwgrError(BWGR_ERR_UNSUPPORTED)."""
     par = dict(_MRR3_DEFAULTS)
     for key, v in kw.items():
         if key not in par:

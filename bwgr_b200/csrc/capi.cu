@@ -394,32 +394,44 @@ int finish_store(bwgr_handle* h, int storage) {
   CU(cudaMemcpyAsync(h->xx_f.p, xf.data(), sizeof(float) * h->p, cudaMemcpyHostToDevice, h->stream));
   CU(cudaStreamSynchronize(h->stream));
   int flag = 0, rc = 0;
+  // row shards: which Gram kernel runs, and so the band's layout, the sweep's geometry and the collectives of a fit, must be the
+  // same on every rank -- a code any rank holds counts for all
+  auto agree = [h](int* f) -> int {
+    double v = *f;
+    const int r = dist_allreduce_host(h, &v, 1, true);
+    *f = v != 0.0 ? 1 : 0;
+    return r;
+  };
   {  // codes 0..7 everywhere?  (one more streaming pass at load time)
     h->fp8_codes = 0;
     if (h->xx_max < 16777216.0) {  // every Gram entry and every partial sum of non-negative codes is bounded by max_j xx_j
       launch_check_range_i8(h->x8, h->ld, (int)h->n, (int)h->p, 0, 7, h->err.p, h->stream);
       h->launches++;
-      if ((rc = take_err_flag(h, &flag))) return rc;
+      if ((rc = take_err_flag(h, &flag)) || (rc = agree(&flag))) return rc;
       h->fp8_codes = flag ? 0 : 1;
     }
   }
   h->x2f.release();
   if (h->fp8_codes && storage == BWGR_STORE_I8) {  // FP4 Gram shadow copy (gram_fp4.cu): only when every code is 0, 1 or 2
+    flag = 1;
     if (h->x2f.alloc((size_t)(h->ld / 4) * h->p) == cudaSuccess) {
       launch_pack_2bit_fp4(h->x8, h->ld, (int)h->p, h->x2f.p, h->err.p, h->stream);
       h->launches++;
       if ((rc = take_err_flag(h, &flag))) return rc;
-      if (flag) h->x2f.release();  // a code 3..7: the E4M3 path
     }
+    if ((rc = agree(&flag))) return rc;
+    if (flag) h->x2f.release();  // a code 3..7 (or no room for the copy): the E4M3 path
   }
   h->x2g.release();
   if (h->fp8_codes && storage == BWGR_STORE_I8 && !h->x2f.p) {  // E4M3 Gram shadow copy (codes 0..3)
+    flag = 1;
     if (h->x2g.alloc((size_t)(h->ld / 4) * h->p) == cudaSuccess) {
       launch_pack_2bit_gram(h->x8, h->ld, (int)h->p, h->x2g.p, h->err.p, h->stream);
       h->launches++;
       if ((rc = take_err_flag(h, &flag))) return rc;
-      if (flag) h->x2g.release();  // a code 3..7: keep the int8 gather
     }
+    if ((rc = agree(&flag))) return rc;
+    if (flag) h->x2g.release();  // a code 3..7 (or no room for the copy): keep the int8 gather
   }
   CU(cudaGetLastError());  // a store kernel that failed to launch must not go unnoticed
   h->storage = BWGR_STORE_I8;
@@ -562,8 +574,10 @@ int64_t bwgr_launch_count(bwgr_handle* h) { return h ? h->launches : 0; }
 // pinned staging buffers, each chunk of columns copied to the device while the next ones are narrowed.
 // offsets != nullptr (the centred loader): a column may be "integer codes + one constant" (CNT(gen), or any integer-valued
 // column): the constant -- the fractional part of the first value plus the column minimum, so that the stored codes start at 0 --
-// goes to offsets[j]; the codes must still be integers to 1e-4, the resolution of a float32 column mean.
-static int narrow_columns(const double* X, int64_t ld_src, int64_t n, int64_t ld_dst, int64_t j0, int64_t j1, int8_t* dst, int lo, int hi, double* offsets) {
+// goes to offsets[j]; the codes must still be integers to 1e-4, the resolution of a float32 column mean.  mins (row-sharded store):
+// the column minima over all ranks, so that every rank shifts a column by the same integer.
+static int narrow_columns(const double* X, int64_t ld_src, int64_t n, int64_t ld_dst, int64_t j0, int64_t j1, int8_t* dst, int lo, int hi, double* offsets,
+                          const double* mins) {
   int flag = 0;
   for (int64_t j = j0; j < j1; j++) {
     const double* src = X + j * ld_src;
@@ -573,7 +587,7 @@ static int narrow_columns(const double* X, int64_t ld_src, int64_t n, int64_t ld
       double frac = v0 - std::floor(v0);
       if (!(frac == frac) || frac < 1e-4 || frac > 1.0 - 1e-4) frac = 0.0;
       // also for an integer-valued column: the solver centres anyway, and codes starting at 0 keep the store on the FP4 / E4M3 Gram paths
-      const double base = std::nearbyint(bwgr::column_min(src, n) - frac);
+      const double base = std::nearbyint((mins ? mins[j] : bwgr::column_min(src, n)) - frac);
       flag |= bwgr::narrow_column_shifted(src, n, out, frac + base, lo, hi);
       offsets[j] = frac + base;
     } else {
@@ -665,6 +679,19 @@ static int load_f64_common(bwgr_handle* h, const double* X, int64_t n, int64_t p
   if (allow_offset) h->col_offset.assign((size_t)p, 0.0);
   double* offs = allow_offset ? h->col_offset.data() : nullptr;
   const int lo = storage == BWGR_STORE_2BIT ? 0 : -128, hi = storage == BWGR_STORE_2BIT ? 2 : 127;
+  std::vector<double> mins;  // row-sharded centred store: column minima over all ranks (min = -max of the negated values)
+  if (allow_offset && h->world > 1) {
+    mins.resize((size_t)p);
+    std::vector<std::thread> pool;
+    const int nthr = (int)std::min<int64_t>(loader_threads(), p);
+    for (int t = 0; t < nthr; t++)
+      pool.emplace_back([&, t]() { for (int64_t j = t; j < p; j += nthr) mins[(size_t)j] = -bwgr::column_min(X + j * ld, n); });
+    for (auto& th : pool) th.join();
+    rc = dist_allreduce_host(h, mins.data(), (int)p, true);
+    if (rc) return rc;
+    for (double& v : mins) v = -v;
+  }
+  const double* gmins = mins.empty() ? nullptr : mins.data();
   const int64_t ldd = h->ld;
   constexpr int kStage = 4;
   const int64_t chunk_cols = std::max<int64_t>(1, std::min<int64_t>(p, ((int64_t)32 << 20) / ldd));
@@ -707,7 +734,7 @@ static int load_f64_common(bwgr_handle* h, const double* X, int64_t n, int64_t p
       const int sl = (int)(t % nslice);
       const int64_t j0 = c * chunk_cols, pc = std::min(chunk_cols, p - j0);
       const int64_t a = pc * sl / nslice, b = pc * (sl + 1) / nslice;
-      if (b > a && narrow_columns(X, ld, n, ldd, j0 + a, j0 + b, s_stage[c % kStage] + a * ldd, lo, hi, offs)) bad.store(1);
+      if (b > a && narrow_columns(X, ld, n, ldd, j0 + a, j0 + b, s_stage[c % kStage] + a * ldd, lo, hi, offs, gmins)) bad.store(1);
       left[(size_t)c].fetch_sub(1, std::memory_order_release);
     }
   };
@@ -1043,7 +1070,7 @@ int fit_begin(bwgr_handle* h, const FitSpec& s, const double* y) {
   if (dist) {
     if (!h->hx_connected) return fail(BWGR_ERR_STATE, "row-sharded handle: call bwgr_dist_connect before fitting");
     if (s.row_mask) return fail(BWGR_ERR_UNSUPPORTED, "row-sharded fits take unmasked systems");
-    if (s.model == M_MRR || s.model == M_KMUP || s.model == M_KMUP2) return fail(BWGR_ERR_UNSUPPORTED, "row sharding covers the univariate EM and Gibbs solvers");
+    if (s.model == M_KMUP || s.model == M_KMUP2) return fail(BWGR_ERR_UNSUPPORTED, "row sharding covers the EM and Gibbs solvers and MRR3's fast path");
   }
   // row-sharded fits and MRR3's rotated systems run on the pipelined blocked sweep only
   int rc = choose_path(h, s, dist || s.model == M_MRR ? BWGR_PATH_BLOCKED : h->path, &family);
@@ -1366,6 +1393,18 @@ SweepState sweep_state(const bwgr_handle* h) {
   return s;
 }
 
+// Row-sharded fit: the uncentred Gram band of this rank's rows -> the band over all individuals (exact: integers below 2^24 in
+// fp32), centred afterwards when the fit's columns are (MRR3), with the same arithmetic as one GPU's Gram kernel.
+int sum_gram_band(bwgr_handle* h, float* gram, const int* perm, ncclComm_t comm, cudaStream_t st) {
+  const Fit& f = h->fit;
+  NC(nccl().AllReduce(gram, gram, (size_t)f.nblocks * kBlk * kBlk * f.nband, ncclFloat, ncclSum, comm, st));
+  if (f.sx_dev.p) {
+    launch_gram_centre(gram, perm, (int)h->p, f.nblocks, f.nband, f.sx_dev.p, 1.0f / (float)h->n_global, st);
+    h->launches++;
+  }
+  return 0;
+}
+
 int fit_sweeps(bwgr_handle* h, int nsweeps) {
   Fit& f = h->fit;
   if (!h || !f.active) return fail(BWGR_ERR_STATE, "no fit in progress");
@@ -1399,16 +1438,21 @@ int fit_sweeps(bwgr_handle* h, int nsweeps) {
         CU(cudaStreamWaitEvent(h->stream, h->side_done[sweep & 1], 0));
       } else if (f.shuffled || !f.gram_cached) {
         cudaEvent_t pe = h->prof_begin(0);
+        // row shards: each rank's band is uncentred (integers below 2^24 in fp32, so the float all-reduce is exact) and is
+        // centred once the sum is complete
+        const float* sx_in_kernel = h->world > 1 ? nullptr : f.sx_dev.p;
         if (h->x2f.p && f.nband == 2) {
-          const cudaError_t ge = launch_gram_fp4(h->x2f.p, h->ld, (int)h->p, (int)h->n_global, d_perm, f.nblocks, f.gram_p, h->err.p, h->num_sms, f.sx_dev.p, h->stream);
+          const cudaError_t ge = launch_gram_fp4(h->x2f.p, h->ld, (int)h->p, (int)h->n_global, d_perm, f.nblocks, f.gram_p, h->err.p, h->num_sms, sx_in_kernel, h->stream);
           if (ge != cudaSuccess) return fail(BWGR_ERR_CUDA, "FP4 Gram launch failed: %s", cudaGetErrorString(ge));
-        } else launch_gram_tc(gram_view(h), d_perm, f.nblocks, f.gram_p, 1, f.nband, h->fp8_codes, h->err.p, h->num_sms, f.sx_dev.p, h->stream);
+        } else launch_gram_tc(gram_view(h), d_perm, f.nblocks, f.gram_p, 1, f.nband, h->fp8_codes, h->err.p, h->num_sms, sx_in_kernel, h->stream);
         h->prof_end(pe);
         h->launches++;
         f.gram_cached = true;
         if (!f.shuffled && f.gram_p == h->gram_nat.p) h->gram_nat_band = f.nband;
-        if (h->world > 1)  // row shards: the Gram band is a sum over individuals (exact: integers below 2^24 in fp32)
-          NC(nccl().AllReduce(f.gram_p, f.gram_p, (size_t)f.nblocks * kBlk * kBlk * f.nband, ncclFloat, ncclSum, h->comm, h->stream));
+        if (h->world > 1) {
+          int rc = sum_gram_band(h, f.gram_p, d_perm, h->comm, h->stream);
+          if (rc) return rc;
+        }
       }
       if (f.full_inv) {  // the step coefficients change every sweep (lambda), the inverses with them
         cudaEvent_t pi = h->prof_begin(3);
@@ -1420,7 +1464,7 @@ int fit_sweeps(bwgr_handle* h, int nsweeps) {
       PipeArgs a;
       memset(&a, 0, sizeof a);
       a.s = state; a.model = rule_model(f.model); a.perm = d_perm; a.nblocks = f.nblocks; a.gram = f.gram_p; a.nband = f.nband; a.tinv = f.full_inv ? f.tinv.p : nullptr;
-      a.sx = f.sx_dev.p; a.cshift = f.cshift.p;
+      a.sx = f.sx_dev.p; a.cshift = f.cshift.p; a.n_total = (int)h->n_global;
       a.part = f.part.p; a.hred = f.part.p + (size_t)8 * f.nsys * 128 * 160; a.dew = f.dew.p; a.tag = ++f.tag;
       a.rows_per_cta = f.rows_per_cta; a.nworkers = f.nworkers; a.D = f.lookahead; a.nbuf = f.nbuf; a.sring = f.sring;
       a.world = h->world; a.rank = h->rank; a.gen0 = h->dist_gen;
@@ -1451,12 +1495,13 @@ int fit_sweeps(bwgr_handle* h, int nsweeps) {
           if (h->wait32(h->side, flag, a.started_val, CU_STREAM_WAIT_VALUE_GEQ) != CUDA_SUCCESS) return fail(BWGR_ERR_CUDA, "cuStreamWaitValue32 failed");
           CU(upload_order(sweep + 1, h->side));
           const int* np_ = f.perm.p + (size_t)((sweep + 1) % kPermRing) * p;
-          const cudaError_t ge = launch_gram_fp4(h->x2f.p, h->ld, (int)h->p, (int)h->n_global, np_, f.nblocks, ((sweep + 1) & 1) ? f.gram2.p : f.gram.p,
-                                                 h->err.p, h->num_sms, f.sx_dev.p, h->side, true);
+          float* gn = ((sweep + 1) & 1) ? f.gram2.p : f.gram.p;
+          const cudaError_t ge = launch_gram_fp4(h->x2f.p, h->ld, (int)h->p, (int)h->n_global, np_, f.nblocks, gn, h->err.p, h->num_sms,
+                                                 h->world > 1 ? nullptr : f.sx_dev.p, h->side, true);
           if (ge != cudaSuccess) return fail(BWGR_ERR_CUDA, "FP4 Gram launch failed: %s", cudaGetErrorString(ge));
-          if (h->world > 1) {  // row shards: the band is a sum over individuals; its own communicator, so it never queues behind (or ahead of) the main stream's
-            float* gn = ((sweep + 1) & 1) ? f.gram2.p : f.gram.p;
-            NC(nccl().AllReduce(gn, gn, (size_t)f.nblocks * kBlk * kBlk * f.nband, ncclFloat, ncclSum, h->comm_side, h->side));
+          if (h->world > 1) {  // row shards: its own communicator, so it never queues behind (or ahead of) the main stream's
+            int rc = sum_gram_band(h, gn, np_, h->comm_side, h->side);
+            if (rc) return rc;
           }
           CU(cudaEventRecord(h->side_done[(sweep + 1) & 1], h->side));
           f.gram_ahead = sweep + 1;
@@ -2624,35 +2669,54 @@ int bwgr_mrr3_fit(bwgr_handle* h, int f32_variant, const double* Y, int k, const
   const MrrOut out{mu_out, b_out, hat_out, h2_out, GC_out, vb_out, ve_out, MSx_out, cnv_out, W_out, its_out};
   const int maxit = F.maxit;
   if (maxit < 1) return fail(BWGR_ERR_ARG, "maxit < 1");
-  const int64_t n = h->n, p = h->p, ld = h->ld;
+  // n: this rank's rows (all of them on one GPU); ng: the individuals every sum over individuals runs over
+  const int64_t n = h->n, p = h->p, ld = h->ld, ng = h->n_global;
+  const bool dist = h->world > 1;
   bool missing = false;
   for (int64_t i = 0; i < n * k && !missing; i++) missing = !(Y[i] == Y[i]);
   // Everything the rotation cannot express -- missing phenotypes (per-trait XX), the inner Gauss-Seidel solve, marker weights,
   // MRR3F's NoInv system, the tilde-hat estimator -- runs on the general device path (mrr_gen.cu); BWGR_MRR=general forces it.
   const char* force = getenv("BWGR_MRR");
-  if (missing || F.TH || F.NLfactor != 0 || F.InnerGS || (f32_variant && F.NoInv) || (force && !strcmp(force, "general")))
+  const bool options = F.TH || F.NLfactor != 0 || F.InnerGS || (f32_variant && F.NoInv);
+  const bool forced = force && !strcmp(force, "general");
+  if (dist) {
+    // A row-sharded store has the fast path only, and every rank must take the same road: the reasons any rank has to refuse are
+    // all-reduced before any other collective, and then every rank refuses or none does.
+    PipePlan pl;
+    const bool no_fit = !h->hx_connected || h->storage != BWGR_STORE_I8 || !(h->xx_max < 16777216.0) || !plan_pipe(h, M_MRR, k, &pl);
+    double why[4] = {missing ? 1.0 : 0.0, options ? 1.0 : 0.0, forced ? 1.0 : 0.0, no_fit ? 1.0 : 0.0};
+    int rc = dist_allreduce_host(h, why, 4, true);
+    if (rc) return rc;
+    if (why[0] || why[1] || why[2] || why[3])
+      return fail(BWGR_ERR_UNSUPPORTED, "the general MRR3 path does not run on a row-sharded store (%s)",
+                  why[0] ? "missing phenotypes on some rank" : why[1] ? "TH, NLfactor, InnerGS or MRR3F's NoInv" :
+                  why[2] ? "BWGR_MRR=general on some rank" : "the shard does not fit the pipelined blocked sweep on some rank");
+  } else if (missing || options || forced) {
     return mrr3_general(h, f32_variant, Y, k, F, out);
+  }
   auto M = [k](int r, int c) { return (size_t)r + (size_t)c * k; };
   // ---- setup (:359-432), double on the host
   MrrVar V;
-  V.mu.resize(k); V.vy.resize(k); V.nn.assign(k, (double)n);
+  V.mu.assign(k, 0.0); V.vy.assign(k, 0.0); V.nn.assign(k, (double)ng);
+  for (int t = 0; t < k; t++)
+    for (int64_t i = 0; i < n; i++) V.mu[t] += Y[(size_t)t * n + i];
+  int rc = dist_allreduce_host(h, V.mu.data(), k, false);
+  if (rc) return rc;
   for (int t = 0; t < k; t++) {
-    double s = 0;
-    for (int64_t i = 0; i < n; i++) s += Y[(size_t)t * n + i];
-    V.mu[t] = s / (double)n;
-    double ss = 0;
-    for (int64_t i = 0; i < n; i++) { const double v = Y[(size_t)t * n + i] - V.mu[t]; ss += v * v; }
-    V.vy[t] = ss / ((double)n - 1.0);
+    V.mu[t] /= (double)ng;
+    for (int64_t i = 0; i < n; i++) { const double v = Y[(size_t)t * n + i] - V.mu[t]; V.vy[t] += v * v; }
   }
+  if ((rc = dist_allreduce_host(h, V.vy.data(), k, false))) return rc;
+  for (int t = 0; t < k; t++) V.vy[t] /= ((double)ng - 1.0);
   std::vector<float> xxc(p), sxf(p);
   double msx = 0;
   for (int64_t j = 0; j < p; j++) {
-    const double c = h->h_xx[j] - h->h_sx[j] * h->h_sx[j] / (double)n;  // XX(J,t) = sum (x - mean)^2, same for every trait (:382-385)
+    const double c = h->h_xx[j] - h->h_sx[j] * h->h_sx[j] / (double)ng;  // XX(J,t) = sum (x - mean)^2, same for every trait (:382-385)
     xxc[j] = (float)c; sxf[j] = (float)h->h_sx[j];
-    msx += c / (double)n;                                              // XSX (:386-388): the centred column sums to zero
+    msx += c / (double)ng;                                              // XSX (:386-388): the centred column sums to zero
   }
   if (!(msx > 0)) return fail(BWGR_ERR_ARG, "genotypes have no variance");
-  const double TrXSX = (double)n * msx;
+  const double TrXSX = (double)ng * msx;
   V.MSx.assign(k, msx);
   mrr_start(F, k, V);
   // ---- device state through the common fit machinery: k systems of the rotated ridge rule
@@ -2660,8 +2724,8 @@ int bwgr_mrr3_fit(bwgr_handle* h, int f32_variant, const double* Y, int k, const
   s.model = M_MRR; s.nsys = k; s.shuffled = true; s.row_mask = nullptr;
   s.df = 0; s.R2 = (float)F.R2; s.Pi = 0; s.alpha = 0; s.pi = 0; s.it = maxit; s.bi = 0; s.seed = 0;
   FitGuard guard{h};
-  int rc = fit_begin(h, s, Y);
-  if (rc == BWGR_ERR_UNSUPPORTED)  // the shape does not fit the pipelined blocked sweep (row slabs above 512 rows): general path
+  rc = fit_begin(h, s, Y);
+  if (rc == BWGR_ERR_UNSUPPORTED && !dist)  // the shape does not fit the pipelined blocked sweep (row slabs above 512 rows): general path
     return mrr3_general(h, f32_variant, Y, k, F, out);
   if (rc) return rc;
   Fit& f = h->fit;
@@ -2680,6 +2744,7 @@ int bwgr_mrr3_fit(bwgr_handle* h, int f32_variant, const double* Y, int k, const
   CU(cudaMemcpyAsync(f.y.p, f.e.p, sizeof(float) * k * ld, cudaMemcpyDeviceToDevice, h->stream));
   launch_xty(h->view(), f.y.p, k, tilde.p, h->stream);  // tilde = X'y (:420)
   h->launches++;
+  if (dist) NC(nccl().AllReduce(tilde.p, tilde.p, (size_t)k * p, ncclFloat, ncclSum, h->comm, h->stream));
   std::vector<double> hred((size_t)k * k + 3 * k);
   std::vector<float> Tf(32 * 32), Tif(32 * 32), hmax(32);
   std::vector<SysScalars> sc(f.sc0);
@@ -2703,6 +2768,8 @@ int bwgr_mrr3_fit(bwgr_handle* h, int f32_variant, const double* Y, int k, const
     launch_rotate(f.b.p, b_alt.p, p, (int)p, k, Tdev.p, nullptr, nullptr, h->num_sms, h->stream);
     h->launches += 2;
     f.e.swap(e_alt); f.b.swap(b_alt);
+    // the fixed-point words of X_B'E the ranks exchange are summable only at one scale: max|e| over all individuals
+    if (dist) NC(nccl().AllReduce(amax.p, amax.p, 32, ncclFloat, ncclMax, h->comm, h->stream));
     CU(cudaMemcpyAsync(hmax.data(), amax.p, sizeof(float) * 32, cudaMemcpyDeviceToHost, h->stream));
     CU(cudaStreamSynchronize(h->stream));
     for (int t = 0; t < k; t++) {
@@ -2725,6 +2792,10 @@ int bwgr_mrr3_fit(bwgr_handle* h, int f32_variant, const double* Y, int k, const
     launch_pair_reduce(b_old.p, f.b.p, p, p, (int)p, k, 1, red.p + (size_t)k * k, h->stream);
     launch_pair_reduce(f.e.p, nullptr, ld, ld, (int)n, k, 2, red.p + (size_t)k * k + k, h->stream);
     h->launches += 6;
+    if (dist) {  // e.y and the column sums of e run over individuals; b'tilde and |beta0 - b|^2 are the same on every rank
+      NC(nccl().AllReduce(red2.p, red2.p, (size_t)k * k, ncclDouble, ncclSum, h->comm, h->stream));
+      NC(nccl().AllReduce(red.p + (size_t)k * k + k, red.p + (size_t)k * k + k, (size_t)k, ncclDouble, ncclSum, h->comm, h->stream));
+    }
     std::vector<double> ey((size_t)k * k), small(2 * k);
     CU(cudaMemcpyAsync(hred.data(), red.p, sizeof(double) * ((size_t)k * k + 2 * k), cudaMemcpyDeviceToHost, h->stream));
     CU(cudaMemcpyAsync(ey.data(), red2.p, sizeof(double) * k * k, cudaMemcpyDeviceToHost, h->stream));
@@ -2738,7 +2809,7 @@ int bwgr_mrr3_fit(bwgr_handle* h, int f32_variant, const double* Y, int k, const
     { const std::vector<double> Tr((size_t)k, TrXSX); mrr_varcomp(F, k, TildeHat, Tr, V.h2, V); }
     if (F.updateMu) {  // :651-655 (complete Y: Z = 1)
       std::vector<float> sh(k);
-      for (int t = 0; t < k; t++) { const double m = small[k + t] / ((double)n - 1.0); V.mu[t] += m; sh[t] = (float)(-m); }
+      for (int t = 0; t < k; t++) { const double m = small[k + t] / ((double)ng - 1.0); V.mu[t] += m; sh[t] = (float)(-m); }
       // e -= m: a rotation by the identity with a shift
       std::vector<float> I((size_t)k * k, 0.0f);
       for (int t = 0; t < k; t++) I[(size_t)t * k + t] = 1.0f;
@@ -2756,7 +2827,7 @@ int bwgr_mrr3_fit(bwgr_handle* h, int f32_variant, const double* Y, int k, const
   CU(cudaStreamSynchronize(h->stream));
   for (int t = 0; t < k; t++) {
     double shift = 0;
-    for (int64_t j = 0; j < p; j++) shift += (h->h_sx[j] / (double)n) * (double)hb[(size_t)t * p + j];
+    for (int64_t j = 0; j < p; j++) shift += (h->h_sx[j] / (double)ng) * (double)hb[(size_t)t * p + j];
     m0[t] = (float)(V.mu[t] - shift);
   }
   rc = fitted_values(h, k, f.b.p, false, m0.data(), hh);

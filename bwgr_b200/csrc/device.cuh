@@ -180,4 +180,9 @@ __device__ __forceinline__ long long grid_wait_total(const unsigned long long* w
   return tot;
 }
 
+// ---- centred Gram band (MRR3 centres every column, RcppEigen20230423.cpp:378-379) ----------------------------------------------
+// x_ci'x_ck = x_i'x_k - sx_i sx_k / n, rounded as one FMA on the exact integer entry g.  The Gram kernels apply it in their epilogue
+// and gram_centre_kernel to a band that was summed over the ranks of a row-sharded fit: the same operands, so the same bits.
+__device__ __forceinline__ float gram_centre(float g, float sx_i, float sx_k, float inv_n) { return fmaf(-(sx_i * inv_n), sx_k, g); }
+
 }  // namespace bwgr

@@ -178,9 +178,9 @@ __global__ void __launch_bounds__(kThreads, 1) gram_fp4_kernel(const uint8_t* __
       float* out_d = gram + ((size_t)blk * 128 + row) * 256;              // diagonal block of b
       float* out_c = gram + ((size_t)(blk + 1) * 128 + row) * 256 + 128;  // cross block of b + 1 (its row r = marker r of block b)
       float sxr = 0.0f;
-      if (sx) {  // centred Gram (MRR3 centres every column): x_ci'x_ck = x_i'x_k - sx_i sx_k / n
+      if (sx) {  // centred Gram (gram_centre)
         const int pos = blk * 128 + row;
-        sxr = pos < p ? sx[perm[pos]] * inv_n : 0.0f;
+        sxr = pos < p ? sx[perm[pos]] : 0.0f;
         named_bar(1, 128);
         for (int q = row; q < 256; q += 128) { const int pq = blk * 128 + q; S->sxc[q] = pq < p ? sx[perm[pq]] : 0.0f; }
         named_bar(1, 128);
@@ -193,7 +193,7 @@ __global__ void __launch_bounds__(kThreads, 1) gram_fp4_kernel(const uint8_t* __
         tmem_ld_wait();
         if (sx) {
 #pragma unroll
-          for (int q = 0; q < 32; q++) v[q] = __float_as_uint(fmaf(-sxr, S->sxc[c * 32 + q], __uint_as_float(v[q])));
+          for (int q = 0; q < 32; q++) v[q] = __float_as_uint(gram_centre(__uint_as_float(v[q]), sxr, S->sxc[c * 32 + q], inv_n));
         }
         if (c < 4) {
 #pragma unroll

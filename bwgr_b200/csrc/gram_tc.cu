@@ -254,7 +254,7 @@ __global__ void __launch_bounds__(416, 1) gram_tc_kernel(GenoView g, const int* 
       ok = mbar_wait(&S->tmem_full[as], aphase, err);
       tc_fence_after();
       int32_t* out = gram + ((size_t)blk * 128 + row) * (NBAND * 128);
-      // centred Gram (MRR3 centres every column, RcppEigen20230423.cpp:378-379): x_ci'x_ck = x_i'x_k - sx_i sx_k / n
+      // centred Gram (gram_centre)
       float sxr0 = 0.0f, sxr1 = 0.0f;
       if (sx) {
         const int pos0 = blk * 128 + row, pos1 = (blk - 1) * 128 + row;
@@ -281,9 +281,9 @@ __global__ void __launch_bounds__(416, 1) gram_tc_kernel(GenoView g, const int* 
           for (int q = 0; q < 32; q++) v[q] = __float_as_uint(__int2float_rn((int)v[q]));
         }
         if (sx && out_f32) {
-          const float sr = (c < 4 ? sxr0 : sxr1) * inv_n;
+          const float sr = c < 4 ? sxr0 : sxr1;
 #pragma unroll
-          for (int q = 0; q < 32; q++) v[q] = __float_as_uint(fmaf(-sr, S->sxc[(c & 3) * 32 + q], __uint_as_float(v[q])));
+          for (int q = 0; q < 32; q++) v[q] = __float_as_uint(gram_centre(__uint_as_float(v[q]), sr, S->sxc[(c & 3) * 32 + q], inv_n));
         }
         if (ok) {
 #pragma unroll
@@ -302,7 +302,26 @@ __global__ void __launch_bounds__(416, 1) gram_tc_kernel(GenoView g, const int* 
   if (warp == 4) tmem_dealloc(tmem_base, 2u * kAccCols);
 }
 
+// Centres a band the kernel above (or gram_fp4.cu) wrote uncentred: row r of block b, column c of band d is x_{b-d,r}'x_{b,c}.
+// One CTA per band row; block 0's cross half (no predecessor) is left as it is, as the Gram kernels leave it.
+__global__ void __launch_bounds__(128) gram_centre_kernel(float* __restrict__ gram, const int* __restrict__ perm, int p, int nband,
+                                                          const float* __restrict__ sx, float inv_n) {
+  const int blk = blockIdx.x >> 7, r = blockIdx.x & 127, c = threadIdx.x;
+  const int pc = blk * 128 + c;
+  const float sxc = pc < p ? sx[perm[pc]] : 0.0f;
+  float* row = gram + (size_t)blockIdx.x * nband * 128;
+  for (int d = 0; d < nband && d <= blk; d++) {
+    const int pr = (blk - d) * 128 + r;
+    const float sxr = pr < p ? sx[perm[pr]] : 0.0f;
+    row[d * 128 + c] = gram_centre(row[d * 128 + c], sxr, sxc, inv_n);
+  }
+}
+
 }  // namespace
+
+void launch_gram_centre(float* gram, const int* perm, int p, int nblocks, int nband, const float* sx, float inv_n, cudaStream_t st) {
+  gram_centre_kernel<<<nblocks * 128, 128, 0, st>>>(gram, perm, p, nband, sx, inv_n);
+}
 
 template <int NBAND, bool FP8>
 static void launch_gram_band(const GenoView& g, const int* perm, int nblocks, void* gram, int out_f32, int* err, int num_sms,

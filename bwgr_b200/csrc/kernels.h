@@ -93,6 +93,9 @@ void launch_gram_tc(const GenoView& g, const int* perm, int nblocks, void* gram,
 void launch_pack_2bit_fp4(const int8_t* src, int64_t ld, int p, uint8_t* dst, int* bad, cudaStream_t st);
 cudaError_t launch_gram_fp4(const uint8_t* x2f, int64_t ld, int p, int n, const int* perm, int nblocks, float* gram, int* err,
                             int num_sms, const float* sx, cudaStream_t st, bool block_per_cta = false);
+// Centres an uncentred float band in place (gram_tc.cu): what sx != nullptr does inside the Gram kernels, bit for bit, for a band
+// summed over the ranks of a row-sharded fit first (sx = column sums and inv_n = 1 / n over all individuals).
+void launch_gram_centre(float* gram, const int* perm, int p, int nblocks, int nband, const float* sx, float inv_n, cudaStream_t st);
 // host_narrow.cpp: one column of R's double matrix -> int8 codes, exactly (nonzero = not an integer code in [lo, hi])
 int narrow_column(const double* src, int64_t n, int8_t* out, int lo, int hi);
 int narrow_column_shifted(const double* src, int64_t n, int8_t* out, double shift, int lo, int hi);
@@ -111,6 +114,7 @@ struct PipeArgs {
   const float* sx;       // [p] column sums, or nullptr.  Non-null = the columns are centred (MRR3): the Gram band is the
                          // centred one and g gets the running mean-shift term c * sx_j (the workers stay uncentred)
   float* cshift;         // [nsys] out: the mean shift c accumulated over the sweep (e_true = e_stored + c)
+  int n_total;           // individuals over all ranks: the mean shift is sum_j sx_j dE_j / n_total
   unsigned long long* part;  // [8][nsys][128][160] per-worker integer partials of h: (value << 12) | block tag; zeroed before launch
   unsigned long long* hred;  // [8][nsys][128] reduced h, same word format; zeroed before launch
   // row-sharded fit over `world` GPUs of a node: hx[r] = rank r's exchange ring [8][world][nsys][128] mapped into this

@@ -575,7 +575,7 @@ __global__ void __launch_bounds__(kT, 1) sweep_pipe_kernel(PipeArgs a) {
   // a worker's step inbox sits at the same shared-window offset in every CTA of this launch
   const uint32_t dein_u32 = smem_u32(base) + (uint32_t)worker_layout(a.rows_per_cta, ns, a.nbuf, CL).di;
   const bool centred = a.sx != nullptr;
-  const float inv_n = 1.0f / (float)a.s.g.n;
+  const float inv_n = 1.0f / (float)a.n_total;
   if (tid < 64) cs[tid] = 0.0f;
   const int gstride = a.nband * 128;  // floats per Gram row in HBM
   const int nsw = ns < kSolveWarps ? ns : kSolveWarps;

@@ -4,7 +4,8 @@ One process per GPU (torchrun / torch.distributed).  Systems are partitioned ove
 genotypes (they are shared by all fits) and runs its share through the ordinary single-GPU entry points; there is NO
 data-path collective -- only the host-side gather of the small result vectors at the end, which is what the reference's
 caller does with `lapply` results (R/cv.R:80).  The single large fit (config 5) shards rows instead and needs a per-block
-exchange inside the sweep kernel; see DESIGN.md section 6.
+exchange inside the sweep kernel; see DESIGN.md section 6.  A row-sharded store (Genotypes.enable_row_sharding) takes the EM
+and Gibbs fits and MRR3 / MRR3F (bw.MRR3(Y[rows], g)) on their fast path.
 """
 import numpy as np
 

@@ -233,7 +233,11 @@ BWGR_API int bwgr_wgr_fit_bag(bwgr_handle* h, const double* y, int it, int bi, i
  *  - everything else -- NaN in Y (missing phenotypes, :359-365), InnerGS = TRUE (:510-514), TH = TRUE (:423, :549-571), NLfactor != 0
  *    (:524-533), MRR3F with NoInv = TRUE (:878-882): one k x k system per marker with per-trait observation masks, float64 device
  *    state (csrc/mrr_gen.cu); needs the int8 store.
- * BWGR_ERR_UNSUPPORTED: k > 32, row-sharded stores, a trait with fewer than two observations is BWGR_ERR_ARG. */
+ * On a row-sharded store (bwgr_dist_*) only the first path runs: each rank passes its rows of Y and gets the common b, mu, h2, GC,
+ * vb, ve, MSx, cnv and Its, and hat for its rows.  Whether the fit can run is decided by all ranks together: if any rank meets
+ * something only the general path handles (NaN in its rows of Y, InnerGS, TH, NLfactor, MRR3F's NoInv, BWGR_MRR=general) or a
+ * shard the pipelined sweep cannot take, every rank returns BWGR_ERR_UNSUPPORTED.
+ * BWGR_ERR_UNSUPPORTED: k > 32; a trait with fewer than two observations is BWGR_ERR_ARG. */
 BWGR_API int bwgr_mrr3_fit(bwgr_handle* h, int f32_variant, const double* Y, int k, const double* par, double* mu, double* b,
                   double* hat, double* h2, double* GC, double* vb, double* ve, double* MSx, double* cnv, double* W,
                   int* its);
@@ -244,7 +248,9 @@ BWGR_API int bwgr_mrr3_fit(bwgr_handle* h, int f32_variant, const double* Y, int
  * Per 128-marker block the reduced partial X_B'E of a rank is stored straight into every peer's exchange ring inside the
  * sweep kernel (peer memory over NVLink, no host involvement); NCCL all-reduces the per-sweep Gram band and scalars.
  * Call order on every rank: bwgr_create -> bwgr_dist_init -> (exchange the 64-byte handles) -> bwgr_dist_connect ->
- * bwgr_geno_load_* -> fits.  Supports the blocked family (unmasked systems, int8 store). */
+ * bwgr_geno_load_* -> fits.  Supports the blocked family (unmasked systems, int8 store): the EM and Gibbs solvers and MRR3 /
+ * MRR3F's rotated fast path (bwgr_mrr3_fit; a refusal there is taken by all ranks together, so no rank waits in a collective the
+ * others never reach).  bwgr_geno_load_f64_centred agrees each column's constant over the ranks. */
 BWGR_API int bwgr_dist_unique_id(void* id128);  /* rank 0 creates it, the host framework broadcasts the 128 bytes */
 BWGR_API int bwgr_dist_init(bwgr_handle* h, int rank, int world, const void* id128, void* ipc_handle_out64);
 BWGR_API int bwgr_dist_connect(bwgr_handle* h, const void* ipc_handles_all /* world x 64 bytes, rank order */);
