@@ -12,7 +12,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OBJ = os.path.join(HERE, "lib", "obj")
 LIB = os.path.join(HERE, "lib", "libbwgr_b200.so")
-SOURCES = ["capi.cu", "geno.cu", "small_n.cu", "grid_sweep.cu", "epilogue.cu", "gram_tc.cu", "gram_fp4.cu", "sweep_pipe.cu", "mrr.cu", "mrr_gen.cu", "block_inv.cu", "host_narrow.cpp"]
+SOURCES = ["handle.cu", "store.cu", "fit.cu", "solvers.cu", "mrr_host.cu", "geno.cu", "small_n.cu", "grid_sweep.cu", "epilogue.cu", "gram_tc.cu", "gram_fp4.cu", "sweep_pipe.cu", "mrr.cu", "mrr_gen.cu", "block_inv.cu", "host_narrow.cpp"]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17", "-Xcompiler", "-fPIC",
          "--expt-relaxed-constexpr"]

@@ -1,5 +1,5 @@
 // device.cuh -- the inline-PTX wrappers that more than one kernel file uses, and the L2 grid-sum word.  Device code only: the
-// kernel .cu files include it, the host layer (capi.cu, kernels.h) does not.
+// kernel .cu files include it, the host layer (host.h, kernels.h) does not.
 #pragma once
 #include "kernels.h"
 

@@ -1,4 +1,4 @@
-// kernels.h -- internal launch interface between the C-ABI host layer (capi.cu) and the kernels.
+// kernels.h -- internal launch interface between the C-ABI host layer (host.h and its .cu files) and the kernels.
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>

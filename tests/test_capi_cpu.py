@@ -69,7 +69,7 @@ def test_cv_host_logic():
 
 @pytest.mark.parametrize("level", [0, 1, 2, -1])
 def test_float64_loader_narrowing_paths(level):
-    """The loader of R's double matrix (capi.cu load_f64_common -> csrc/host_narrow.cpp): every code path (plain, AVX2, AVX-512)
+    """The loader of R's double matrix (store.cu load_f64_common -> csrc/host_narrow.cpp): every code path (plain, AVX2, AVX-512)
     narrows exact integer codes bit for bit and flags anything else -- fractions, NaN, infinities, out-of-range codes -- wherever in
     the column it sits (vector body or scalar tail)."""
     import ctypes as C

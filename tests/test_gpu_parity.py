@@ -363,7 +363,7 @@ def test_blocked_sweep_is_deterministic(tpod):
 
 
 def test_gram_band_computed_ahead_changes_nothing():
-    """The next sweep's Gram band is computed on a side stream while the clustered sweep runs (capi.cu fit_sweeps): the fit is
+    """The next sweep's Gram band is computed on a side stream while the clustered sweep runs (fit.cu fit_sweeps): the fit is
     bit-identical to the one-stream schedule (what a profiled handle runs), for straight fits, stepped fits and back-to-back fits
     on one store."""
     X, y = synth(20000, 4000, seed=33)

@@ -86,7 +86,7 @@ def _assert_small_n(n, geo, ring, case, **kw):
 # ---- general MRR3 path (csrc/mrr_gen.cu) ----------------------------------------------------------------------------------------
 
 def _mrr_gen_plan(n, sms):
-    """(NJ, rows_per_cta, CTAs): grid_geometry (capi.cu) and launch_mrr_gen_sweep restated.  rows_per_cta = max(64, ceil(ld / SMs)
+    """(NJ, rows_per_cta, CTAs): grid_geometry (fit.cu) and launch_mrr_gen_sweep restated.  rows_per_cta = max(64, ceil(ld / SMs)
     rounded up to 16); a thread keeps ceil(rows_per_cta / 32) rows per trait in registers, the kernel instance with NJ = 2, 4, 8, 12 or
     16 such rows, or NJ = 0 (slab in shared memory) above 512 rows per CTA."""
     ld = _ld(n)
@@ -109,7 +109,7 @@ def _mrr_n(geo, nj):
 # ---- blocked family (csrc/sweep_pipe.cu): the plan from the trace header ---------------------------------------------------------
 
 def _clusters(sms):
-    return min(18, max(2, (sms - 36) // 8))  # plan_pipe's first choice (capi.cu): leave 36 SMs to the next sweep's Gram band
+    return min(18, max(2, (sms - 36) // 8))  # plan_pipe's first choice (fit.cu): leave 36 SMs to the next sweep's Gram band
 
 
 def _n_clustered(geo, rows):
